@@ -6,6 +6,7 @@ m=4M,n=256; GA evals/sec; 1/2/4/8 B200").
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W              # our arm, row-sharded over N GPUs (strong scaling)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's own CPU code on the host cores
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # + what the last timed step computed, as DIR/*.npy
 
 Workload (config.workload = "cfg5"): Levenberg-Marquardt on the tree-summed Lorentzian curve fit of SURVEY.md 8(d),
 m = 4 000 000 residuals x n = 256 parameters, FP64. One STEP = one LM iteration of
@@ -35,6 +36,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True     # the tree may be read-only; the modules imported below must not leave caches in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -295,6 +297,47 @@ class LMDevice:
         self.rejected += rej
 
 
+DUMP_SEED = 20240607               # fixed: the sampled rows are the same in every run and every build
+DUMP_BUDGET = {"residual": 32 << 20, "jacobian": 16 << 20, "jtj": 8 << 20}     # bytes per array: 56 MiB + the n-vectors in all
+
+
+def _sample_rows(rows, row_bytes, budget, rng):
+    """None if all `rows` rows fit the budget, else a sorted seeded sample of as many rows as fit with their 8-byte indices"""
+    if rows * row_bytes <= budget:
+        return None
+    return np.sort(rng.choice(rows, size=max(1, budget // (row_bytes + 8)), replace=False))
+
+
+def dump_outputs(out_dir, ctx, prob, lo):
+    """Writes what the last timed LM iteration left to its caller, as float64 .npy files: the iterate `x`, `lambda`, `chisq`, and
+    the device buffers the caller passed to pnol_lm_iterate: `residual` F at x, `jacobian` J of the last step and `jtj` / `rhs`
+    (J^T J and -J^T F). An array over its byte budget is a fixed seeded sample of its rows, with the (global) row indices
+    beside it as `<name>_rows`. With the rows sharded over several GPUs, this rank's rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    m, n = prob.m, prob.n
+    rng = np.random.default_rng(DUMP_SEED)
+    out = {"x": prob.X, "lambda": np.array([prob.lam]), "chisq": np.array([prob.chi])}
+    F = ctx.to_host(prob.F, m)
+    rows = _sample_rows(m, 8, DUMP_BUDGET["residual"], rng)
+    out["residual"] = F if rows is None else F[rows]
+    if rows is not None:
+        out["residual_rows"] = (lo + rows).astype(np.float64)
+    rows = _sample_rows(m, 8 * n, DUMP_BUDGET["jacobian"], rng)
+    rows = np.arange(m) if rows is None else rows
+    J = np.empty((rows.size, n))
+    for j, i in enumerate(rows):
+        ctx.memcpy(J[j], prob.J + int(i) * n * 8, n * 8)
+    out["jacobian"], out["jacobian_rows"] = J, (lo + rows).astype(np.float64)
+    W = ctx.to_host(prob.JTJ, n * n + n)
+    rows = _sample_rows(n, 8 * n, DUMP_BUDGET["jtj"], rng)
+    out["jtj"] = W[:n * n].reshape(n, n) if rows is None else W[:n * n].reshape(n, n)[rows]
+    if rows is not None:
+        out["jtj_rows"] = rows.astype(np.float64)
+    out["rhs"] = W[n * n:]
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     from parallelnonlinearoptimizationlibrary_b200 import capi, hostapi, launch, problems
@@ -365,6 +408,8 @@ def run_ours(args):
         if cnt:
             timers[name] = {"ms_avg": ms / cnt, "count": cnt}
     accepted, rejected = prob.accepted, prob.rejected
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, prob, lo)
     # the small scopes: the same steps once more, untimed, with every scope on
     ctx.timer_enable(1)
     ctx.timer_reset()
@@ -748,7 +793,10 @@ def main():
     ap.add_argument("--no-ga", action="store_true")
     ap.add_argument("--no-dense", action="store_true", help="skip the cfg3 dense-kernel lines (matvec, rank-2 / literal update, solve)")
     ap.add_argument("--no-scaled-shapes", action="store_true", help="cpu baseline: skip the measured m=4M,n=16 / m=200k,n=64 reference runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -1,16 +1,95 @@
-"""Pins the oracle (oracle/pnol_oracle.cpp, a restatement) against the VERBATIM reference compiled from
-/root/reference/Source against oracle/shim (oracle/_ref/pnol_ref_cli). Runs wherever oracle/_ref has been built (this
-container builds it in __graft_entry__.build(); the binary travels to the GPU box). Bit-exact everywhere: both sides are
-plain sequential C++ built without FMA contraction."""
+"""Pins the oracle (oracle/pnol_oracle.cpp, a restatement) against the VERBATIM reference compiled from the reference's Source/
+against oracle/shim (oracle/_ref/pnol_ref_cli). Bit-exact everywhere: both sides are plain sequential C++ built without FMA
+contraction.
+
+The reference's side of every comparison is stored in tests/golden/oracle_vs_ref_golden.json (tests/golden/make_oracle_vs_ref_golden.py),
+keyed by the call: shape and SHA-256 of every array (-0.0 read as 0.0, as np.array_equal does), and the values of the small ones. So
+the module runs without the reference's sources; where oracle/_ref is built, every call is also run fresh and must give the same bits."""
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
 import oracle_lib as O
 
-pytestmark = pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref/pnol_ref_cli not built (needs /root/reference)")
+HERE = os.path.dirname(os.path.abspath(__file__))
+RECORDED = os.path.join(HERE, "golden", "oracle_vs_ref_golden.json")
+RECORD_ENV = "PNOL_RECORD_ORACLE_VS_REF"          # set by make_oracle_vs_ref_golden.py: collect the recording instead of checking it
+RECORD = {} if os.environ.get(RECORD_ENV) else None
+REC = None if RECORD is not None else json.load(open(RECORDED))
+SMALL = 64                                         # arrays up to this size are recorded with their values
 
 ROSEN, POWER, BOOTH, GOLD, RAST, EXPS = 1, 2, 3, 4, 5, 6
 EXPC, CUBIC, LOR = 101, 102, 103
+
+
+def call_key(cmd, arrays, kw):
+    h = hashlib.sha1(cmd.encode())
+    for k in sorted(kw):
+        h.update(("%s=%r;" % (k, kw[k])).encode())
+    for k in sorted(arrays):
+        h.update(k.encode() + np.ascontiguousarray(arrays[k], dtype=np.float64).tobytes())
+    return h.hexdigest()[:20]
+
+
+def record_of(v):
+    v = np.ascontiguousarray(v, dtype=np.float64) + 0.0
+    assert not np.isnan(v).any()
+    rec = {"shape": list(v.shape), "sha256": hashlib.sha256(v.tobytes()).hexdigest()}
+    if v.size <= SMALL:
+        rec["values"] = v.ravel().tolist()
+    return rec
+
+
+def matches(got, rec):
+    return record_of(np.asarray(got).reshape(rec["shape"])) == rec
+
+
+def ref(cmd, arrays, golden=None, **kw):
+    """The reference's outputs of one pnol_ref_cli call (as arrays; recorded with their values): the recording, and a fresh run that
+    must equal it where oracle/_ref is built. `golden` names the case of tests/golden/ref_golden.npz that holds the reference's
+    output of this very call: the recording takes it from there (used where the oracle does not reproduce the reference's bits)."""
+    key = call_key(cmd, arrays, kw)
+    if RECORD is not None:
+        G = np.load(os.path.join(HERE, "golden", "ref_golden.npz"))
+        RECORD[key] = {k.split("/", 1)[1]: record_of(G[k]) for k in G.files if k.startswith(golden + "/")}
+        rec = RECORD[key]
+    else:
+        rec = REC.get(key)
+        assert rec, "no recorded reference output for %s %r" % (cmd, kw)
+        if O.have_ref():
+            r = O.ref_cli(cmd, arrays=arrays, **kw)
+            for k, v in rec.items():
+                assert matches(r[k], v), (cmd, k)
+    return {k: np.array(v["values"]).reshape(v["shape"]) for k, v in rec.items() if "values" in v}
+
+
+def same(cmd, arrays, want, **kw):
+    """the reference, given `arrays` and `kw`, returns `want` (the oracle's outputs, by name) bit for bit"""
+    want = {k: np.reshape(v, -1) if np.ndim(v) == 0 else np.asarray(v) for k, v in want.items()}
+    key = call_key(cmd, arrays, kw)
+    if RECORD is not None:
+        RECORD.setdefault(key, {}).update({k: record_of(v) for k, v in want.items()})
+        return
+    rec = REC.get(key)
+    assert rec, "no recorded reference output for %s %r" % (cmd, kw)
+    for k, v in want.items():
+        assert k in rec and record_of(v) == rec[k], (cmd, k)
+    if O.have_ref():
+        r = O.ref_cli(cmd, arrays=arrays, **kw)
+        for k, v in want.items():
+            assert np.array_equal(np.asarray(r[k]).reshape(v.shape), v), (cmd, k)
+
+
+@pytest.fixture(scope="module", autouse=True)
+def _write_recording():
+    yield
+    if RECORD is not None:
+        with open(os.environ[RECORD_ENV], "w") as f:
+            json.dump(RECORD, f, indent=0, sort_keys=True)
+            f.write("\n")
 
 
 def expcurve_cols():
@@ -29,12 +108,10 @@ def test_fd_gradient_and_hessian(spec, kind, ints, n, nprocs):
     dx = np.full(n, 1e-6)
     f = O.OFunctor(kind, (), ints)
     g, f0 = O.fd_gradient(f, x, dx)
-    r = O.ref_cli("fdgrad", arrays=dict(x=x, dx=dx), obj=spec, nprocs=nprocs)
-    assert np.array_equal(r["g"], g) and np.array_equal(r["g_mpi"], g) and r["f"][0] == f0
+    same("fdgrad", dict(x=x, dx=dx), dict(g=g, g_mpi=g, f=f0), obj=spec, nprocs=nprocs)
     if nprocs == 1 and n <= 12:
         B = O.fd_hessian(f, x, np.full(n, 1e-3))
-        rh = O.ref_cli("hessian", arrays=dict(x=x, dx=np.full(n, 1e-3)), obj=spec)
-        assert np.array_equal(rh["B"].reshape(n, n), B)
+        same("hessian", dict(x=x, dx=np.full(n, 1e-3)), dict(B=B), obj=spec)
 
 
 def test_reference_pow_objects_match_the_product_form():
@@ -42,7 +119,7 @@ def test_reference_pow_objects_match_the_product_form():
     # above through obj=rosenbrock, which instantiates the reference class); PowerObject's run-time pow(x,3) does not
     # fold and may differ from x*x*x in the last ulp: the FD gradient then agrees to FD-noise level only (SURVEY 7.1)
     x = np.full(5, 3.0)
-    r = O.ref_cli("fdgrad", arrays=dict(x=x, dx=np.full(5, 1e-6)), obj="power:3")
+    r = ref("fdgrad", dict(x=x, dx=np.full(5, 1e-6)), golden="testGradientEvaluation", obj="power:3")
     g, _ = O.fd_gradient(O.OFunctor(POWER, (), (3,)), x, np.full(5, 1e-6))
     assert np.allclose(r["g"], g, rtol=1e-7)
     assert r["g"][0] == 27.000008998356861          # SURVEY.md Appendix C known answer
@@ -58,8 +135,7 @@ def test_recur_gradient():
     f = O.OFunctor(ROSEN)
     g, f0 = O.fd_gradient_recur(f, xr, dxr, xfull, ind)
     for P in (1, 4):
-        r = O.ref_cli("recur", arrays=dict(x=xr, dx=dxr, constx=xfull, ind=ind), obj="rosenbrock", nprocs=P)
-        assert np.array_equal(r["g"], g) and np.array_equal(r["g_mpi"], g) and r["f"][0] == f0
+        same("recur", dict(x=xr, dx=dxr, constx=xfull, ind=ind), dict(g=g, g_mpi=g, f=f0), obj="rosenbrock", nprocs=P)
     # SURVEY.md Appendix C: testGradientApproxMultMPIRecur known values (full gradient minus the 4th entry)
     want = np.array([-2.0000190090740944, 10.600067000154922, 15.600064998011476, 6.4000969928201812, -2.9998690038723907,
                      -12.399822999498156, 68.000100000631392])
@@ -77,22 +153,19 @@ def test_fd_jacobian_lorentz(K, m, P):
     f = O.OFunctor(LOR, (pr["w"],), (), (pr["t"], pr["y"]), m)
     dx = np.full(pr["n"], 1e-7)
     J, F = O.fd_jacobian(f, pr["x0"], dx)
-    r = O.ref_cli("fdjac", arrays=dict(x=pr["x0"], dx=dx, t=pr["t"], y=pr["y"]), obj="lorentz", w=pr["w"], nprocs=P)
-    assert np.array_equal(r["J"].reshape(m, -1), J) and np.array_equal(r["J_mpi"].reshape(m, -1), J) and np.array_equal(r["F"], F)
+    same("fdjac", dict(x=pr["x0"], dx=dx, t=pr["t"], y=pr["y"]), dict(J=J, J_mpi=J, F=F), obj="lorentz", w=pr["w"], nprocs=P)
 
 
 def test_fd_jacobian_cubic_reference_class():
     # CubicObjective is the reference's own class (data built by its constructor with libm pow)
     x = np.full(4, 0.1)
-    r = O.ref_cli("fdjac", arrays=dict(x=x, dx=np.full(4, 1e-6)), obj="cubic")
     xs = np.linspace(-5, 5, 100)
     # columns as the reference builds them: linspace by the shim, pow(x,3) by libm -- take x^3 via Python's pow (libm)
     x3 = np.array([pow(float(v), 3) for v in xs])
     y = np.array([0.3 * pow(float(v), 3) + 1.1 * pow(float(v), 2) - 4.3 * float(v) + 7.3 for v in xs])
     f = O.OFunctor(CUBIC, (), (), (x3, xs, y), 100)
     J, F = O.fd_jacobian(f, x, np.full(4, 1e-6))
-    assert np.array_equal(r["F"], F)
-    assert np.array_equal(r["J"].reshape(100, 4), J)
+    same("fdjac", dict(x=x, dx=np.full(4, 1e-6)), dict(F=F, J=J), obj="cubic")
 
 
 @pytest.mark.parametrize("K,m,iters,P", [(8, 2000, 12, 1), (8, 2000, 5, 4), (16, 600, 6, 2)])
@@ -100,20 +173,19 @@ def test_lm_loop(K, m, iters, P):
     pr = _lorentz(m, K)
     f = O.OFunctor(LOR, (pr["w"],), (), (pr["t"], pr["y"]), m)
     w = O.lm(f, pr["x0"], 0.001, 10.0, 1e-7, iters, 0.0)
-    r = O.ref_cli("lm", arrays=dict(x=pr["x0"], t=pr["t"], y=pr["y"]), obj="lorentz", w=pr["w"], lambda0=0.001, factor=10.0,
-                  dxgrad=1e-7, maxiter=iters, xmindiff=0.0, nprocs=P)
-    assert np.array_equal(r["X"], w["X"]) and np.array_equal(r["F"], w["F"]) and np.array_equal(r["F0"], w["F0"])
-    rs = O.ref_cli("lm", arrays=dict(x=pr["x0"], t=pr["t"], y=pr["y"]), obj="lorentz", w=pr["w"], lambda0=0.001, factor=10.0,
-                   dxgrad=1e-7, maxiter=iters, xmindiff=0.0, serial=1)
-    assert np.array_equal(rs["X"], w["X"])
+    same("lm", dict(x=pr["x0"], t=pr["t"], y=pr["y"]), dict(X=w["X"], F=w["F"], F0=w["F0"]), obj="lorentz", w=pr["w"], lambda0=0.001,
+         factor=10.0, dxgrad=1e-7, maxiter=iters, xmindiff=0.0, nprocs=P)
+    same("lm", dict(x=pr["x0"], t=pr["t"], y=pr["y"]), dict(X=w["X"]), obj="lorentz", w=pr["w"], lambda0=0.001, factor=10.0,
+         dxgrad=1e-7, maxiter=iters, xmindiff=0.0, serial=1)
 
 
 def test_lm_reference_known_answers():
     # testLMExpMPI / testLMCubicLinearCoef (Source/Examples.cpp:128-160, 415-450), values of SURVEY.md Appendix C
-    r = O.ref_cli("lm", arrays=dict(x=np.array([9.0, 0.5, 0.3])), obj="expcurve_ref", lambda0=0.001, factor=10.0, dxgrad=1e-6,
-                  maxiter=100, xmindiff=1e-6)
+    r = ref("lm", dict(x=np.array([9.0, 0.5, 0.3])), golden="testLMExpMPI", obj="expcurve_ref", lambda0=0.001, factor=10.0,
+            dxgrad=1e-6, maxiter=100, xmindiff=1e-6)
     assert np.allclose(r["X"], [10.2, 0.4, 0.1], rtol=1e-8)
-    r = O.ref_cli("lm", arrays=dict(x=np.full(4, 0.1)), obj="cubic", lambda0=0.001, factor=10.0, dxgrad=1e-6, maxiter=100, xmindiff=1e-6)
+    r = ref("lm", dict(x=np.full(4, 0.1)), golden="testLMCubicLinearCoef", obj="cubic", lambda0=0.001, factor=10.0, dxgrad=1e-6,
+            maxiter=100, xmindiff=1e-6)
     assert np.allclose(r["X"], [0.3, 1.1, -4.3, 7.3], rtol=1e-10)
 
 
@@ -124,8 +196,7 @@ def test_update_hinv(n):
     D = M @ M.T / n + np.eye(n)
     g = rng.normal(size=n)
     s = 0.1 * g + 0.05 * rng.normal(size=n)
-    r = O.ref_cli("updhinv", arrays=dict(D=D, g=g, s=s))
-    assert np.array_equal(r["D"].reshape(n, n), O.update_hinv(D, g, s))
+    same("updhinv", dict(D=D, g=g, s=s), dict(D=O.update_hinv(D, g, s)))
 
 
 @pytest.mark.parametrize("P", [1, 3])
@@ -136,22 +207,22 @@ def test_alpha_pool_against_the_reference_class(P):
     n = 9
     x, p = rng.uniform(-1.5, 1.5, n), rng.normal(size=n)
     alpha = np.array([0.0, 1e-3, 0.1, 0.37, 1.0, 2.5])
-    r = O.ref_cli("alphapool", arrays=dict(x=x, p=p, alpha=alpha), obj="rosenbrock", dalpha=1e-6, nprocs=P)
     phi, dphi, bad = O.alpha_pool(O.OFunctor(ROSEN), x, p, alpha, 1e-6)
-    assert bad == 0 and np.array_equal(r["phi"], phi) and np.array_equal(r["dphi"], dphi)
+    assert bad == 0
+    same("alphapool", dict(x=x, p=p, alpha=alpha), dict(phi=phi, dphi=dphi), obj="rosenbrock", dalpha=1e-6, nprocs=P)
     nf = 12
     ind = np.zeros(nf)
     ind[[2, 5, 9]] = 1
     constx = rng.uniform(-1, 1, nf)
     xr = rng.uniform(-1, 1, n)
-    r = O.ref_cli("alphapool", arrays=dict(x=xr, p=p, alpha=alpha, constx=constx, ind=ind), obj="rastrigin", dalpha=1e-6, nprocs=P)
     phi, dphi, bad = O.alpha_pool(O.OFunctor(RAST), xr, p, alpha, 1e-6, const_x=constx, const_ind=ind)
-    assert bad == 0 and np.array_equal(r["phi"], phi) and np.array_equal(r["dphi"], dphi)
+    assert bad == 0
+    same("alphapool", dict(x=xr, p=p, alpha=alpha, constx=constx, ind=ind), dict(phi=phi, dphi=dphi), obj="rastrigin", dalpha=1e-6, nprocs=P)
     xb = x.copy()
     xb[0] = 1e200                                      # f overflows: every entry comes back as the sentinel
-    r = O.ref_cli("alphapool", arrays=dict(x=xb, p=p, alpha=alpha), obj="rosenbrock", dalpha=1e-6, nprocs=P)
     phi, dphi, bad = O.alpha_pool(O.OFunctor(ROSEN), xb, p, alpha, 1e-6)
-    assert bad == alpha.size and np.all(phi == 1e10) and np.array_equal(r["phi"], phi)
+    assert bad == alpha.size and np.all(phi == 1e10)
+    same("alphapool", dict(x=xb, p=p, alpha=alpha), dict(phi=phi), obj="rosenbrock", dalpha=1e-6, nprocs=P)
 
 
 def test_box_helpers():
@@ -162,11 +233,10 @@ def test_box_helpers():
     p = rng.normal(size=n)
     p[7] = 0.0
     xin = np.clip(x, lb, ub)
-    r = O.ref_cli("box", arrays=dict(x=xin, xlb=lb, xub=ub, p=p))
-    assert r["alphabnd"][0] == O.compute_alpha_bnd(xin, lb, ub, p)
-    r = O.ref_cli("box", arrays=dict(x=x, xlb=lb, xub=ub))
+    same("box", dict(x=xin, xlb=lb, xub=ub, p=p), dict(alphabnd=O.compute_alpha_bnd(xin, lb, ub, p)))
     xw, cnt = O.check_box_bounds(x, lb, ub)
-    assert cnt > 0 and np.array_equal(r["X"], xw)
+    assert cnt > 0
+    same("box", dict(x=x, xlb=lb, xub=ub), dict(X=xw))
 
 
 @pytest.mark.parametrize("spec,kind,ints,n,npop,gens,box", [("powerprod:2", POWER, (2,), 4, 150, 6, 10.0), ("rastrigin", RAST, (), 6, 200, 5, 5.12),
@@ -177,9 +247,8 @@ def test_ga(spec, kind, ints, n, npop, gens, box):
     scale = 1.0 - 1.0 / npop
     w = O.ga(O.OFunctor(kind, (), ints), x0, lb, ub, npop, gens, dict(seed=777, scale=scale))
     for kw in (dict(nprocs=1), dict(nprocs=4), dict(serial=1)):
-        r = O.ref_cli("ga", arrays=dict(x=x0, xlb=lb, xub=ub), obj=spec, npop=npop, maxgen=gens, seed=777, scale=scale, **kw)
-        assert np.array_equal(r["X"], w["X"]) and r["fOpt"][0] == w["fOpt"] and r["f0"][0] == w["f0"]
-        assert int(r["stream_pos"][0]) == w["stream_pos"]
+        same("ga", dict(x=x0, xlb=lb, xub=ub), dict(X=w["X"], fOpt=w["fOpt"], f0=w["f0"], stream_pos=w["stream_pos"]), obj=spec, npop=npop,
+             maxgen=gens, seed=777, scale=scale, **kw)
 
 
 def test_ga_stages():
@@ -189,12 +258,10 @@ def test_ga_stages():
     X = rng.uniform(-1.4, 1.4, size=(npop, n))
     X[7] = X[100]
     F = np.round(rng.uniform(0.1, 9, npop), 1)
-    r = O.ref_cli("popsort", arrays=dict(xpop=X, F=F), n=n)
     Xw, Fw = O.ga_pop_sort(X, F)
-    assert np.array_equal(r["F"], Fw) and np.array_equal(r["xpop"].reshape(npop, n), Xw)
-    r = O.ref_cli("checkbounds", arrays=dict(xpop=X, xlb=lb, xub=ub), n=n, seed=5, scale=1.0)
+    same("popsort", dict(xpop=X, F=F), dict(F=Fw, xpop=Xw), n=n)
     Xw, iw, pw = O.ga_check_bounds(X, lb, ub, dict(seed=5, scale=1.0))
-    assert int(r["stream_pos"][0]) == pw and np.array_equal(r["xpop"].reshape(npop, n), Xw) and np.array_equal(r["ind"], iw)
-    r = O.ref_cli("checkidentical", arrays=dict(xpop=X, xlb=lb, xub=ub), n=n, seed=5, scale=1.0)
+    same("checkbounds", dict(xpop=X, xlb=lb, xub=ub), dict(stream_pos=pw, xpop=Xw, ind=iw), n=n, seed=5, scale=1.0)
     Xw, iw, pw = O.ga_check_identical(X, lb, ub, dict(seed=5, scale=1.0))
-    assert int(r["stream_pos"][0]) == pw == n and np.array_equal(r["xpop"].reshape(npop, n), Xw) and np.array_equal(r["ind"], iw)
+    assert pw == n
+    same("checkidentical", dict(xpop=X, xlb=lb, xub=ub), dict(stream_pos=pw, xpop=Xw, ind=iw), n=n, seed=5, scale=1.0)
