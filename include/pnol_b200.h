@@ -266,7 +266,8 @@ int pnol_lm_damp(pnol_ctx * ctx, const double * JTJ, int n, double lambda, doubl
  *   JTJ         device, n*n + n doubles: receives J^T J followed by -J^T F. reuse_jtj != 0: J^T J / rhs are taken from it instead of
  *               being recomputed (x unchanged after a rejected step), only the damping is redone with the new lambda
  *   sigma_out, x_trial_out (host, n), sumsq_trial_out, spd_info_out (host): the step, the trial point, sum Ftrial^2 over all
- *               ranks and the Cholesky status (k > 0: pivot k not positive; the step is then NaN, which the caller's chi^2 test rejects) */
+ *               ranks and the Cholesky status (k > 0: pivot k rejected, see pnol_spd_solve; the step is then NaN, which the caller's
+ *               chi^2 test rejects). n <= 704 (the solve's range) */
 int pnol_lm_step(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * dx, int n, double * J, const double * F,
                  double * Ftrial, double lambda, int jac_mode, int reuse_jtj, double * JTJ, double * sigma_out, double * x_trial_out,
                  double * sumsq_trial_out, int * spd_info_out);
@@ -304,8 +305,12 @@ int pnol_lm_last_run(pnol_ctx * ctx, int * stopped_out, double * xdiff_out);
 int pnol_lm_normal_eq_fused(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * dx, int n,
                             double lambda, double * JTJ, double * A, double * rhs, double * F);
 
-/* a9: damped solve  A sigma = rhs  by Cholesky (A symmetric positive definite, only the lower triangle is
- * read). *info = 0 ok, k > 0: pivot k not positive. Replaces luSolve (Source/LevenbergMarquardtMPI.cpp:88). */
+/* a9: damped solve  A sigma = rhs  by Cholesky, 1 <= n <= 704 (PNOL_ERR_INVALID otherwise). A is symmetric positive definite;
+ * only its lower triangle (diagonal included) is read, the strict upper triangle may hold anything, NaN included. Every pivot
+ * (the Schur complement's diagonal entry d_k when column k is eliminated) must lie in [2^-1022, 2^1000): zero, negative, subnormal,
+ * too large or NaN pivots are rejected. On success *info = 0 and x = sigma. On a rejected pivot the call returns PNOL_ERR_NOT_SPD
+ * with *info = k > 0, the 1-based index of the first rejected pivot (named in pnol_last_error), and every entry of x is NaN.
+ * Replaces luSolve (Source/LevenbergMarquardtMPI.cpp:88). */
 int pnol_spd_solve(pnol_ctx * ctx, const double * A, const double * rhs, int n, double * x, int * info);
 
 /* General inverse Ainv = A^-1 by LU with partial pivoting (first largest |entry| on ties) and one pair of substitutions per unit

@@ -1079,7 +1079,7 @@ extern "C" int pnol_spd_solve(pnol_ctx * ctx, const double * A, const double * r
 	PNOL_CUDA(ctx, cudaMemcpyAsync(&inf, info_dev, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
 	PNOL_CHECK(finish(ctx));
 	if (info) *info = inf;
-	if (inf != 0) { PNOL_SET_ERR(ctx, "spd_solve: pivot %d is not positive", inf); return PNOL_ERR_NOT_SPD; }
+	if (inf != 0) { PNOL_SET_ERR(ctx, "spd_solve: pivot %d is outside [2^-1022, 2^1000)", inf); return PNOL_ERR_NOT_SPD; }
 	return PNOL_OK;
 }
 
