@@ -54,7 +54,9 @@ class Runtime {
 	// BFGS inverse-Hessian update form (PNOL_HINV_RANK2 default, PNOL_HINV_LITERAL = the reference's two products)
 	int hessianUpdateMode() const { return hinvMode_; }
 	void setHessianUpdateMode(int m) { hinvMode_ = m; }
-	// Jacobian mode for LM (PNOL_JAC_AUTO / PNOL_JAC_BLACKBOX)
+	// Jacobian mode of LevMarq[MPI]::findMin and MultiObjective::gradientApproximation: PNOL_JAC_AUTO (default) / PNOL_JAC_BLACKBOX /
+	// PNOL_JAC_STRUCTURED forward differences, or PNOL_JAC_ANALYTIC: the model's own derivative (R::jacobian, include/pnol/functors.hpp;
+	// a model without one makes the call fail with PNOL_ERR_NO_FUNCTOR)
 	int jacobianMode() const { return jacMode_; }
 	void setJacobianMode(int m) { jacMode_ = m; }
 	// LM: keep J^T J across a rejected step (X restored, so J is unchanged). The reference recomputes the identical J

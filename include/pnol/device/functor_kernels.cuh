@@ -7,7 +7,8 @@
  * implementing objEval (Source/PNOL_Objective.hpp:29, :57). Here the device side of that plug-in point is:
  *
  *   1. write the functor once, __host__ __device__, to the concept of include/pnol/functors.hpp (scalar: eval(P, X, n);
- *      residual model: residual(P, X, n, i); optionally kSeparable / sep_init / sep_term for the fast population sweep);
+ *      residual model: residual(P, X, n, i), optionally jacobian(P, X, n, i, Ji) for PNOL_JAC_ANALYTIC; optionally kSeparable /
+ *      sep_init / sep_term for the fast population sweep);
  *   2. in ONE .cu file of your own, compiled with
  *        nvcc -gencode arch=compute_100a,code=sm_100a -fmad=false -Xcompiler -ffp-contract=off -I<repo>/include ...
  *      write   PNOL_REGISTER_SCALAR_FUNCTOR(kind, MyFunctor, n_columns)   or   PNOL_REGISTER_RESIDUAL_FUNCTOR(kind, MyModel, n_columns)
@@ -581,6 +582,72 @@ int fd_jacobian(const pnol_launch_env * env, const FunctorParams & P, const doub
 	return PNOL_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------
+// analytic Jacobian (PNOL_JAC_ANALYTIC) of a residual functor that defines R::jacobian (functors.hpp: has_jacobian)
+//   J[i][j] = d r_i / d x_j
+// One row per thread: R::jacobian writes the thread's row into a shared-memory tile (odd pitch: the threads' rows fall in different
+// banks), the block then writes its rows out with coalesced stores -- the rows of a block are one contiguous range of J. Rows too
+// wide for a tile of kJacRowsMin rows are written by R::jacobian straight to global memory. F (optional) from R::residual.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kJacRows = 128;        // rows per block when the tile fits
+constexpr int kJacRowsMin = 32;      // smallest tile
+
+template <class R>
+__global__ void __launch_bounds__(kJacRows)
+jacobian_kernel(FunctorParams P, const double * __restrict__ x, int n, double * __restrict__ J, double * __restrict__ F, int tiled)
+{
+	extern __shared__ double sm[];
+	double * xs = sm;                       // n
+	double * tile = sm + n;                 // blockDim.x x (n | 1), when tiled
+	const int pitch = n | 1;
+	for (int j = threadIdx.x; j < n; j += blockDim.x) xs[j] = x[j];
+	__syncthreads();
+	const PtrAcc acc{xs};
+	for (long long row0 = (long long) blockIdx.x * blockDim.x; row0 < P.m; row0 += (long long) gridDim.x * blockDim.x) {
+		const long long i = row0 + threadIdx.x;
+		const bool live = i < P.m;
+		if (live && F) F[i] = R::residual(P, acc, n, i);
+		if (!tiled) {
+			if (live) R::jacobian(P, acc, n, i, J + i * n);
+			continue;
+		}
+		if (live) R::jacobian(P, acc, n, i, tile + threadIdx.x * pitch);
+		__syncthreads();
+		const int rows = (int) min((long long) blockDim.x, P.m - row0);
+		double * dst = J + row0 * n;
+		for (int e = threadIdx.x; e < rows * n; e += blockDim.x) {
+			const int r = e / n;
+			dst[e] = tile[r * pitch + (e - r * n)];
+		}
+		__syncthreads();
+	}
+}
+
+template <class R>
+int jacobian(const pnol_launch_env * env, const FunctorParams & P, const double * x, int n, double * J, double * F)
+{
+	const long long m = P.m;
+	if (m <= 0) return PNOL_OK;
+	const size_t xbytes = (size_t) n * sizeof(double);
+	const size_t row_bytes = (size_t) (n | 1) * sizeof(double);
+	PNOL_DEV_REQUIRE(env, xbytes <= env->smem_optin, "analytic jacobian: n = %d does not fit in shared memory", n);
+	int threads = kJacRows;
+	while (threads > kJacRowsMin && xbytes + threads * row_bytes > env->smem_optin) threads /= 2;
+	const int tiled = xbytes + threads * row_bytes <= env->smem_optin;
+	if (!tiled) threads = kJacRows;
+	const size_t smem = xbytes + (tiled ? threads * row_bytes : 0);
+	auto kern = jacobian_kernel<R>;
+	PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+	int per_sm = 1;
+	PNOL_DEV_CUDA(env, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
+	if (per_sm < 1) per_sm = 1;
+	const long long blocks = (m + threads - 1) / threads;
+	const long long cap = (long long) env->sm_count * per_sm;
+	const long long grid = blocks < cap ? blocks : cap;
+	PNOL_DEV_LAUNCH(env, kern, (unsigned) grid, threads, smem, P, x, n, J, F, tiled);
+	return PNOL_OK;
+}
+
 /* ---- launch tables (pnol_functor_vtable) of a functor type ---- */
 template <class F> struct ScalarTable {
 	static int eval_batch_(const pnol_launch_env * env, const pnol_functor_params * P, const double * pts, long long B, int n, long long ld,
@@ -609,6 +676,8 @@ template <class R> struct ResidualTable {
 	static int residual_(const pnol_launch_env * env, const pnol_functor_params * P, const double * x, int n, double * F) { return residual<R>(env, *P, x, n, F); }
 	static int fd_jacobian_(const pnol_launch_env * env, const pnol_functor_params * P, const double * x, const double * dx, int n, double * J,
 	                        double * F) { return fd_jacobian<R>(env, *P, x, dx, n, J, F); }
+	static int jacobian_(const pnol_launch_env * env, const pnol_functor_params * P, const double * x, int n, double * J, double * F)
+	{ return jacobian<R>(env, *P, x, n, J, F); }
 	static pnol_functor_vtable make(int n_columns)
 	{
 		pnol_functor_vtable vt = {};
@@ -616,6 +685,7 @@ template <class R> struct ResidualTable {
 		vt.n_columns = n_columns;
 		vt.residual = residual_;
 		vt.fd_jacobian = fd_jacobian_;
+		if constexpr (has_jacobian<R>::value) vt.jacobian = jacobian_;      // NULL otherwise: PNOL_JAC_ANALYTIC is refused
 		return vt;
 	}
 };

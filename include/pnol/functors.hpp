@@ -15,6 +15,10 @@
  * Residual functor concept (row i of the residual vector, data columns in FunctorParams::col):
  *     struct R { static constexpr int kKind;  template<class Acc> static double residual(const FunctorParams&, const Acc& X, int n, long long i); };
  * Acc needs only `double operator[](int) const`.
+ * A residual functor MAY also define its analytic Jacobian row (PNOL_JAC_ANALYTIC; detected by has_jacobian below):
+ *     template<class Acc> static void jacobian(const FunctorParams&, const Acc& X, int n, long long i, double * Ji);
+ * which writes all n entries Ji[j] = d r_i / d x_j. That one definition is the specification: the kernels (the generic template of
+ * device/functor_kernels.cuh and any specialised kernel of a built-in model) return its bits, host and device alike.
  */
 #ifndef PNOL_FUNCTORS_HPP_
 #define PNOL_FUNCTORS_HPP_
@@ -155,6 +159,15 @@ struct ExpCurveFunctor {
 		double func = X[0] * exp_hd(X[1] * P.col[0][i]) + X[2];
 		return P.col[1][i] - func;
 	}
+	/* r = y - (x0 e + x2), e = exp(x1 t):  dr/dx0 = -e, dr/dx1 = -((x0 e) t), dr/dx2 = -1 */
+	template <class Acc> PNOL_HD static void jacobian(const FunctorParams & P, const Acc & X, int, long long i, double * Ji)
+	{
+		const double t = P.col[0][i];
+		const double e = exp_hd(X[1] * t);
+		Ji[0] = -e;
+		Ji[1] = -((X[0] * e) * t);
+		Ji[2] = -1.0;
+	}
 };
 
 /* Source/ExampleObjectives.hpp:170-179; columns {x^3 computed by the host's pow(x,3), x, y}; pow(x,2) -> x*x */
@@ -165,6 +178,15 @@ struct CubicFunctor {
 		double x3 = P.col[0][i], x = P.col[1][i];
 		double func = X[0] * x3 + X[1] * (x * x) + X[2] * x + X[3];
 		return P.col[2][i] - func;
+	}
+	/* dr/dx = -(x^3, x*x, x, 1) */
+	template <class Acc> PNOL_HD static void jacobian(const FunctorParams & P, const Acc &, int, long long i, double * Ji)
+	{
+		const double x3 = P.col[0][i], x = P.col[1][i];
+		Ji[0] = -x3;
+		Ji[1] = -(x * x);
+		Ji[2] = -x;
+		Ji[3] = -1.0;
 	}
 };
 
@@ -180,6 +202,19 @@ PNOL_HD double lorentz_term(double a, double c, double w, double t)
 	double e = w * q;
 	double den = 1.0 + e;
 	return a / den;
+}
+
+/* Derivatives of one term of the residual r = y - S: ja = dr/da = -1/den, jc = dr/dc = -2 a w (t - c) / den^2, in this operation
+ * order (the first four operations are lorentz_term's). Every kernel and test of the analytic Jacobian follows it. */
+PNOL_HD void lorentz_term_grad(double a, double c, double w, double t, double & ja, double & jc)
+{
+	double d = t - c;
+	double q = d * d;
+	double e = w * q;
+	double den = 1.0 + e;
+	double u = 1.0 / den;
+	ja = -u;
+	jc = -((a * u) * u * ((w + w) * d));
 }
 
 struct LorentzSumFunctor {
@@ -203,6 +238,21 @@ struct LorentzSumFunctor {
 		while ((1 << top) < K) top++;
 		return P.col[1][i] - stack[top];
 	}
+	/* the terms are independent: Ji = (ja_0, jc_0, ja_1, jc_1, ...), no tree */
+	template <class Acc> PNOL_HD static void jacobian(const FunctorParams & P, const Acc & X, int n, long long i, double * Ji)
+	{
+		const double w = P.scalars[0];
+		const double t = P.col[0][i];
+		for (int k = 0; k < n / 2; k++) lorentz_term_grad(X[2 * k], X[2 * k + 1], w, t, Ji[2 * k], Ji[2 * k + 1]);
+	}
+};
+
+/* has_jacobian<R>::value: R defines the analytic Jacobian row of the concept above */
+template <class R> struct has_jacobian {
+	template <class T>
+	static constexpr bool test(decltype(&T::template jacobian<PtrAcc>)) { return true; }
+	template <class T> static constexpr bool test(...) { return false; }
+	static constexpr bool value = test<R>(nullptr);
 };
 
 } // namespace pnol

@@ -138,13 +138,14 @@ typedef struct {
  * A user objective brings its own instantiations of the library's kernel templates (include/pnol/device/functor_kernels.cuh, compiled
  * out of tree by the user's nvcc) and registers their launchers under a kind of its choice:
  *     kinds [PNOL_F_USER_SCALAR_BASE, +1000)   scalar objectives  (eval_batch, fd_points, fd_hessian, alpha_pool)
- *     kinds [PNOL_F_USER_RESIDUAL_BASE, +1000) residual models    (residual, fd_jacobian)
+ *     kinds [PNOL_F_USER_RESIDUAL_BASE, +1000) residual models    (residual, fd_jacobian; optionally jacobian: PNOL_JAC_ANALYTIC)
  * pnol_functor_create and every entry point that takes a functor then work for that kind as for the built-ins; libpnol_b200.so is not
  * rebuilt. PNOL_REGISTER_SCALAR_FUNCTOR / PNOL_REGISTER_RESIDUAL_FUNCTOR in that header fill the table and call pnol_register_functor
  * at load time. INTEGRATION.md section A shows the whole recipe; tests/test_gpu_user_functor.py does it end to end. */
 #define PNOL_F_USER_SCALAR_BASE 1000
 #define PNOL_F_USER_RESIDUAL_BASE 2000
-#define PNOL_FUNCTOR_ABI 1
+/* 2: pnol_functor_vtable ends in `jacobian`; version-1 tables (without it) are still accepted */
+#define PNOL_FUNCTOR_ABI 2
 
 /* parameters of a functor as the kernels see them (POD, passed by value as a kernel argument; pnol::FunctorParams) */
 typedef struct pnol_functor_params {
@@ -166,7 +167,7 @@ typedef struct pnol_launch_env {
 
 /* launch table of one functor kind; every pointer argument is a DEVICE pointer, every call only enqueues on env->stream */
 typedef struct pnol_functor_vtable {
-	int abi_version;                             /* PNOL_FUNCTOR_ABI */
+	int abi_version;                             /* PNOL_FUNCTOR_ABI (2), or 1 for a table that ends at fd_jacobian */
 	int n_columns;                               /* data columns the functor expects in pnol_functor_desc */
 	int (*eval_batch)(const pnol_launch_env *, const pnol_functor_params *, const double * pts, long long B, int n, long long ld,
 	                  const unsigned char * indicator, double * f_out);
@@ -180,10 +181,14 @@ typedef struct pnol_functor_vtable {
 	int (*residual)(const pnol_launch_env *, const pnol_functor_params *, const double * x, int n, double * F);
 	int (*fd_jacobian)(const pnol_launch_env *, const pnol_functor_params *, const double * x, const double * dx, int n, double * J,
 	                   double * F /* may be NULL */);
+	/* ABI 2, residual models only, may be NULL: analytic Jacobian J[i][j] = dr_i/dx_j (PNOL_JAC_ANALYTIC), F (may be NULL) = r(x) */
+	int (*jacobian)(const pnol_launch_env *, const pnol_functor_params *, const double * x, int n, double * J, double * F);
 } pnol_functor_vtable;
 
-/* registers (or replaces) the launch table of a user kind; the table must outlive its use. Thread-safe; callable before any context
- * exists (static initialisers). Returns PNOL_OK, or PNOL_ERR_INVALID for a kind outside the user ranges, a missing launcher or another ABI. */
+/* registers (or replaces) the launch table of a user kind. The library keeps its own copy of the table: of a version-1 table only the
+ * version-1 prefix is read (its `jacobian` is taken as NULL). Thread-safe; callable before any context exists (static initialisers).
+ * Returns PNOL_OK, or PNOL_ERR_INVALID for a kind outside the user ranges, a missing launcher, an abi_version other than 1 or 2, or a
+ * scalar kind whose table sets `jacobian`. */
 int pnol_register_functor(int kind, const pnol_functor_vtable * vt);
 int pnol_functor_registered(int kind);                     /* 1 for built-in and registered kinds */
 
@@ -242,8 +247,14 @@ int pnol_residual_eval(pnol_ctx * ctx, const pnol_functor * f, const double * x,
 /* a7 / a8: forward-difference Jacobian J[i][j] = (F_i(x + dx[j] e_j) - F_i(x)) / dx[j], J is m x n row-major,
  * F (optional) receives F(x). Replaces MultiObjective::gradientApproximation[MPI]
  * (Source/PNOL_Objective.cpp:165-197, 202-299). mode: PNOL_JAC_AUTO picks the structured kernel when the
- * functor has one; PNOL_JAC_BLACKBOX forces n+1 full model evaluations per row. Results are bit-identical. */
-enum { PNOL_JAC_AUTO = 0, PNOL_JAC_BLACKBOX = 1, PNOL_JAC_STRUCTURED = 2 };
+ * functor has one; PNOL_JAC_BLACKBOX forces n+1 full model evaluations per row. Results are bit-identical.
+ * These three forward-difference modes are unchanged by the fourth:
+ *   PNOL_JAC_ANALYTIC  J[i][j] = dF_i/dx_j from the functor's own derivative (R::jacobian, include/pnol/functors.hpp; for a user kind
+ *                      the `jacobian` launcher of its table); dx is ignored and may be NULL. Built-in models: all three have one. A functor
+ *                      without one is refused with PNOL_ERR_NO_FUNCTOR (never a silent forward difference). F, when requested, has
+ *                      the bits of pnol_residual_eval. Accepted by pnol_fd_jacobian, pnol_lm_step and pnol_lm_iterate (J stored or NULL).
+ * Other values of mode are taken as PNOL_JAC_AUTO. */
+enum { PNOL_JAC_AUTO = 0, PNOL_JAC_BLACKBOX = 1, PNOL_JAC_STRUCTURED = 2, PNOL_JAC_ANALYTIC = 3 };
 int pnol_fd_jacobian(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * dx, int n,
                      double * J, double * F, int mode);
 
@@ -260,7 +271,7 @@ int pnol_lm_damp(pnol_ctx * ctx, const double * JTJ, int n, double lambda, doubl
 /* One LM iteration's device work behind one call and ONE host synchronisation (Source/LevenbergMarquardtMPI.cpp:60-108):
  * FD Jacobian at x -> J^T J | J^T F (+ all-reduce over the ranks) -> Marquardt damping -> Cholesky solve -> x_trial = x + sigma ->
  * Ftrial = F(x_trial) and its sum of squares (+ all-reduce). The accept / reject decision stays with the caller as in the reference.
- *   x, dx       host or device, n
+ *   x, dx       host or device, n (dx may be NULL with jac_mode = PNOL_JAC_ANALYTIC)
  *   J           device, m x n work space (m = rows of the functor), or NULL: the normal equations are then summed over row blocks
  *               and J is never stored (see pnol_lm_normal_eq_fused); F device: residuals at x; Ftrial device: receives F(x_trial)
  *   JTJ         device, n*n + n doubles: receives J^T J followed by -J^T F. reuse_jtj != 0: J^T J / rhs are taken from it instead of

@@ -23,7 +23,7 @@ ERR_NAMES = {1: "INVALID", 2: "CUDA", 3: "NO_FUNCTOR", 4: "NONFINITE", 5: "NOT_S
 # functor kinds (include/pnol_b200.h)
 F_ROSENBROCK, F_POWER, F_BOOTH, F_GOLDSTEIN, F_RASTRIGIN, F_EXPCURVE_SINGLE = 1, 2, 3, 4, 5, 6
 F_EXPCURVE, F_CUBIC, F_LORENTZ_SUM = 101, 102, 103
-JAC_AUTO, JAC_BLACKBOX, JAC_STRUCTURED = 0, 1, 2
+JAC_AUTO, JAC_BLACKBOX, JAC_STRUCTURED, JAC_ANALYTIC = 0, 1, 2, 3      # JAC_ANALYTIC: the model's own derivative, dx may be None
 HINV_LITERAL, HINV_RANK2 = 0, 1
 COMM_ID_BYTES = 128
 
@@ -395,7 +395,8 @@ class Context:
                                                C.byref(ss) if want_sumsq else None))
         return F, ss.value
 
-    def fd_jacobian(self, f, x, dx, J=None, F=None, mode=JAC_AUTO, n=None):
+    def fd_jacobian(self, f, x, dx=None, J=None, F=None, mode=JAC_AUTO, n=None):
+        """J (m x n) and F at x; mode=JAC_ANALYTIC: J from the model's analytic derivative, dx ignored (None allowed)"""
         x, dx = _f64(x), _f64(dx)
         n = _len(x, n)
         host = J is None
@@ -426,7 +427,8 @@ class Context:
         return JTJ, A, rhs, F
 
     def lm_step(self, f, x, dx, n, J, F, Ftrial, lam, JTJ, jac_mode=JAC_AUTO, reuse_jtj=False):
-        """one LM iteration's device work, one synchronisation: returns (sigma, x_trial, sumsq_trial, spd_info)"""
+        """one LM iteration's device work, one synchronisation: returns (sigma, x_trial, sumsq_trial, spd_info).
+        dx may be None with jac_mode=JAC_ANALYTIC"""
         x, dx = _f64(x), _f64(dx)
         sigma, xt = np.empty(n), np.empty(n)
         ss, info = C.c_double(), C.c_int()
@@ -436,8 +438,8 @@ class Context:
 
     def lm_iterate(self, f, x, dx, n, J, F, Ftrial, JTJ, lam, chisq, factor, iterations, x_min_diff=0.0, jac_mode=JAC_AUTO):
         """`iterations` LM iterations on device-resident state, accept / reject on the host in C++:
-        returns (x, lambda, chisq, accepted, rejected, swapped)"""
-        x = np.array(x, dtype=np.float64)
+        returns (x, lambda, chisq, accepted, rejected, swapped). dx may be None with jac_mode=JAC_ANALYTIC"""
+        x, dx = np.array(x, dtype=np.float64), _f64(dx)
         lam_c, chi_c = C.c_double(lam), C.c_double(chisq)
         acc, rej, sw = C.c_int(), C.c_int(), C.c_int()
         self.check(self.lib.pnol_lm_iterate(self.h, f.handle, _ptr(x), _ptr(dx), int(n), _ptr(J), _ptr(F), _ptr(Ftrial), _ptr(JTJ),

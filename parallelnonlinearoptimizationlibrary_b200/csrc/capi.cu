@@ -3,6 +3,7 @@
 #include "common.cuh"
 #include "peer.cuh"
 
+#include <memory>
 #include <mutex>
 #include <vector>
 #include <thread>
@@ -324,9 +325,11 @@ extern "C" int pnol_timer_reset(pnol_ctx * ctx)
 // ---------------------------------------------------------------------------------------------------
 // ---- open functor table (include/pnol_b200.h: pnol_register_functor) ----
 namespace {
+// The library's own copies of the registered tables. A replaced table is kept (`copies`): a launch may still be using it.
 struct FunctorRegistry {
 	std::mutex mu;
 	std::map<int, const pnol_functor_vtable *> table;
+	std::vector<std::unique_ptr<pnol_functor_vtable> > copies;
 };
 FunctorRegistry & registry()
 {
@@ -346,13 +349,21 @@ const pnol_functor_vtable * pnol::user_vtable(int kind)
 
 extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
 {
-	if (!vt || vt->abi_version != PNOL_FUNCTOR_ABI || !pnol::is_user_kind(kind)) return PNOL_ERR_INVALID;
-	if (vt->n_columns < 0 || vt->n_columns > PNOL_MAX_COLUMNS) return PNOL_ERR_INVALID;
+	if (!vt || !pnol::is_user_kind(kind)) return PNOL_ERR_INVALID;
+	// abi_version leads every version of the table; a version-1 table ends before `jacobian`, so only that prefix may be read
+	const int abi = vt->abi_version;
+	if (abi != 1 && abi != PNOL_FUNCTOR_ABI) return PNOL_ERR_INVALID;
+	std::unique_ptr<pnol_functor_vtable> copy(new pnol_functor_vtable());
+	memcpy(copy.get(), vt, abi == 1 ? offsetof(pnol_functor_vtable, jacobian) : sizeof(pnol_functor_vtable));
+	const pnol_functor_vtable * c = copy.get();
+	if (c->n_columns < 0 || c->n_columns > PNOL_MAX_COLUMNS) return PNOL_ERR_INVALID;
 	const bool residual = pnol::is_residual_kind(kind);
-	if (residual ? !(vt->residual && vt->fd_jacobian) : !(vt->eval_batch && vt->fd_points && vt->fd_hessian && vt->alpha_pool)) return PNOL_ERR_INVALID;
+	if (residual ? !(c->residual && c->fd_jacobian) : !(c->eval_batch && c->fd_points && c->fd_hessian && c->alpha_pool)) return PNOL_ERR_INVALID;
+	if (!residual && c->jacobian) return PNOL_ERR_INVALID;      // an analytic Jacobian belongs to a residual model
 	FunctorRegistry & r = registry();
 	std::lock_guard<std::mutex> lock(r.mu);
-	r.table[kind] = vt;
+	r.table[kind] = c;
+	r.copies.push_back(std::move(copy));
 	return PNOL_OK;
 }
 
@@ -616,7 +627,7 @@ extern "C" int pnol_fd_jacobian(pnol_ctx * ctx, const pnol_functor * f, const do
                                 double * J, double * F, int mode)
 {
 	if (!ctx || !f) return PNOL_ERR_INVALID;
-	PNOL_REQUIRE(ctx, x && dx && J && n >= 1, "fd_jacobian: bad arguments");
+	PNOL_REQUIRE(ctx, x && (dx || mode == PNOL_JAC_ANALYTIC) && J && n >= 1, "fd_jacobian: bad arguments");
 	const long long m = f->params.m;
 	DevIn<double> dx_, ddx; DevOut<double> dJ, dF;
 	PNOL_CHECK(dx_.init(ctx, x, n));
@@ -766,7 +777,7 @@ extern "C" int pnol_lm_step(pnol_ctx * ctx, const pnol_functor * f, const double
                             double * sumsq_trial_out, int * spd_info_out)
 {
 	if (!ctx || !f) return PNOL_ERR_INVALID;
-	PNOL_REQUIRE(ctx, x && dx && F && Ftrial && JTJ && n >= 1, "lm_step: bad arguments");
+	PNOL_REQUIRE(ctx, x && (dx || jac_mode == PNOL_JAC_ANALYTIC) && F && Ftrial && JTJ && n >= 1, "lm_step: bad arguments");
 	PNOL_REQUIRE(ctx, (!J || is_device_ptr(J)) && is_device_ptr(F) && is_device_ptr(Ftrial) && is_device_ptr(JTJ), "lm_step: J, F, Ftrial and JTJ must be device memory");
 	PNOL_REQUIRE(ctx, is_residual_kind(f->kind), "lm_step: the functor is not a residual model");
 	DevIn<double> dx_, ddx;
@@ -885,7 +896,8 @@ extern "C" int pnol_lm_iterate(pnol_ctx * ctx, const pnol_functor * f, double * 
                                int * swapped_out)
 {
 	if (!ctx || !f) return PNOL_ERR_INVALID;
-	PNOL_REQUIRE(ctx, x && dx && lambda_inout && chisq_inout && iterations >= 0 && n >= 1, "lm_iterate: bad arguments");
+	PNOL_REQUIRE(ctx, x && (dx || jac_mode == PNOL_JAC_ANALYTIC) && lambda_inout && chisq_inout && iterations >= 0 && n >= 1,
+	             "lm_iterate: bad arguments");
 	PNOL_REQUIRE(ctx, !is_device_ptr(x), "lm_iterate: x is the host's in/out parameter vector");
 	PNOL_REQUIRE(ctx, F && Ftrial && JTJ && (!J || is_device_ptr(J)) && is_device_ptr(F) && is_device_ptr(Ftrial) && is_device_ptr(JTJ),
 	             "lm_iterate: J, F, Ftrial and JTJ must be device memory");
