@@ -268,33 +268,26 @@ template <class F> struct SeparableLaunch<F, true> {
 		const size_t smem = (size_t) (kSepThreads / 32) * 32 * pitch * sizeof(double);
 		const bool rowwise_ok = n % 4 == 0 && ld % 4 == 0 && (((size_t) pts) & 31) == 0;
 		if (!rowwise_ok && (smem > env->smem_optin / 2 || B < 64 || n < 24)) return PNOL_OK;   // long / very short genomes, tiny batches: the generic kernels
-		// default: the row-wise kernel (0.059 ms at 1M x 32, 68 % of the HBM roofline; the warp-tile kernel below it 0.078 ms).
-		// PNOL_SWEEP_G = 4 / 8 / 16 forces the warp-tile kernel with that prefetch depth (tuning runs).
-		static const int g = [] { const char * e = getenv("PNOL_SWEEP_G"); return e ? atoi(e) : 0; }();
-		if (g == 0 && rowwise_ok) {
-			static const int deep = [] { const char * e = getenv("PNOL_SWEEP_DEEP"); return e ? atoi(e) : 1; }();      // 0: one load ahead (A/B runs)
-			if (deep && n % 16 == 0)
+		// aligned rows: the row-wise kernel (0.059 ms at 1M x 32, 68 % of the HBM roofline; the warp-tile kernel below it 0.078 ms)
+		if (rowwise_ok) {
+			if (n % 16 == 0)
 				PNOL_DEV_LAUNCH(env, eval_batch_rowwise16_kernel<F>, (unsigned) ((B + 127) / 128), 128, 0, P, pts, B, n, ld, indicator, f_out);
 			else
 				PNOL_DEV_LAUNCH(env, eval_batch_rowwise_kernel<F>, (unsigned) ((B + 127) / 128), 128, 0, P, pts, B, n, ld, indicator, f_out);
 			*done = true;
 			return PNOL_OK;
 		}
-		auto go = [&](auto kern) -> int {
-			PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
-			int per_sm = 1;
-			PNOL_DEV_CUDA(env, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kSepThreads, smem));
-			if (per_sm < 1) per_sm = 1;
-			const long long blocks = ((B + 31) / 32 + kSepThreads / 32 - 1) / (kSepThreads / 32);
-			static const int waves = [] { const char * e = getenv("PNOL_SWEEP_WAVES"); return e ? atoi(e) : 1; }();   // tuning override
-			const long long grid = blocks < (long long) env->sm_count * per_sm * waves ? blocks : (long long) env->sm_count * per_sm * waves;
-			PNOL_DEV_LAUNCH(env, kern, (unsigned) grid, kSepThreads, smem, P, pts, B, n, ld, indicator, f_out, pitch);
-			return PNOL_OK;
-		};
+		// unaligned rows: the warp-tile kernel with eight rows loaded ahead, at most one wave of CTAs
+		auto kern = eval_batch_separable_kernel<F, 8>;
+		PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+		int per_sm = 1;
+		PNOL_DEV_CUDA(env, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kSepThreads, smem));
+		if (per_sm < 1) per_sm = 1;
+		const long long blocks = ((B + 31) / 32 + kSepThreads / 32 - 1) / (kSepThreads / 32);
+		const long long grid = blocks < (long long) env->sm_count * per_sm ? blocks : (long long) env->sm_count * per_sm;
+		PNOL_DEV_LAUNCH(env, kern, (unsigned) grid, kSepThreads, smem, P, pts, B, n, ld, indicator, f_out, pitch);
 		*done = true;
-		if (g == 4) return go(eval_batch_separable_kernel<F, 4>);
-		if (g == 16) return go(eval_batch_separable_kernel<F, 16>);
-		return go(eval_batch_separable_kernel<F, 8>);
+		return PNOL_OK;
 	}
 };
 

@@ -17,21 +17,11 @@
  *     attached with pnol_comm_init(). A context must not be used from two host threads at once.
  *   - reference citations are path:line under /root/reference/.
  *
- * Environment switches read by the library (tuning / A-B timing runs; the defaults are the product path). Read once per
- * process unless stated:
- *   PNOL_SYRK_NO_PAIR=1   J^T J with the stream-K TMA kernel instead of the CTA-pair kernel (n = 256, no F)
- *   PNOL_SYRK_LEGACY=1    J^T J with the LDGSTS-ring kernel (one tile role per CTA)
- *   PNOL_SYRK_WDIAG=w     cost of a diagonal tile's chunk in the stream-K work plan
- *   PNOL_SYRK_NOF=1       J^T J without J^T F (timing only: results lack the right-hand side)
- *   PNOL_SWEEP_DEEP=0     fitness sweep with one load ahead instead of four; PNOL_SWEEP_G / PNOL_SWEEP_WAVES: sweep tile shapes
- *   PNOL_COPY_THREADS=k   host threads of the staged pageable <-> device copies (1..8, default 4)
+ * Environment switches read by the library (the defaults are the product path). Read once per process unless stated:
  *   PNOL_FUSED_MB=x       MB of J per row block of pnol_lm_normal_eq_fused / J == NULL steps (read per call, default 512)
- *   PNOL_GA_LEGACY=1      genetic algorithm with the stage-by-stage generation of round 1 instead of the fused pipeline
- *   PNOL_GA_SHARD=rows|sweep|none   overrides pnol_ga_set_sharding
  *   PNOL_GA_NO_IPC=1      several GPUs: population replicas + all-gather instead of peer mappings (A/B runs, boxes without IPC)
  *   PNOL_GA_SORT=radix    GA popSort with the cooperative radix kernel only (default: splitter buckets in front of it; read per pnol_ga_create)
  *   PNOL_LM_PEER=0        several GPUs: the LM step's two sums through NCCL instead of the fused peer-memory kernels (csrc/peer.cu)
- *   PNOL_LORENTZ_ROWWISE=0  trial residuals of the sum-of-Lorentzians model with the row-per-warp kernel (default: one row per thread)
  * and by the host classes (include/pnol/Runtime.hpp): PNOL_DEVICE, PNOL_POOL_WIDTH, PNOL_LM_JACOBIAN_CACHE.
  */
 #ifndef PNOL_B200_H_
@@ -410,7 +400,7 @@ int pnol_ga_status_get(pnol_ga * ga, pnol_ga_status * st);
  * Results are bit-identical in every mode and at every rank count. */
 enum { PNOL_GA_SHARD_AUTO = 0, PNOL_GA_SHARD_ROWS = 1, PNOL_GA_SHARD_SWEEP = 2, PNOL_GA_SHARD_NONE = 3 };
 int pnol_ga_set_sharding(pnol_ctx * ctx, int mode);
-/* what a GA object does: 0 one rank (or the stage-by-stage generation), 1 rows sharded + peer mappings, 2 rows sharded + replicas
+/* what a GA object does: 0 one rank, 1 rows sharded + peer mappings, 2 rows sharded + replicas
  * (peer mappings unavailable, or PNOL_GA_NO_IPC=1), 3 rows replicated + sweep sharded, 4 replicas (no collective) */
 int pnol_ga_peer_mode(pnol_ga * ga);
 /* sorted population (npop x n) and objective values; either may be NULL */

@@ -148,9 +148,7 @@ extern "C" int pnol_free(pnol_ctx * ctx, void * dev_ptr)
 // pinned buffers and their own stream, so the host-side memcpy of one chunk overlaps the DMA of the others.
 // ---------------------------------------------------------------------------------------------------
 constexpr size_t kStageChunk = (size_t) 4 << 20;
-constexpr int kStageMaxThreads = 8;
-// threads actually used: PNOL_COPY_THREADS (1..8), default 4
-static const int kStageThreads = [] { const char * e = getenv("PNOL_COPY_THREADS"); int t = e ? atoi(e) : 4; return t < 1 ? 1 : (t > kStageMaxThreads ? kStageMaxThreads : t); }();
+constexpr int kStageThreads = 4;
 // copies from 1 MB on take this path; below 8 chunks of 4 MB the chunk shrinks so that every thread still gets two chunks to overlap
 // (a rank's data column at 8 GPUs is 4 MB: one chunk would be one thread's plain staged copy again)
 constexpr size_t kStageMinBytes = (size_t) 1 << 20;
@@ -166,9 +164,9 @@ static bool is_pageable_host(const void * p)
 static int stage_init(pnol_ctx * ctx)
 {
 	if (ctx->stage_pinned) return PNOL_OK;
-	PNOL_CUDA(ctx, cudaHostAlloc(&ctx->stage_pinned, kStageChunk * 2 * kStageMaxThreads, cudaHostAllocDefault));
-	for (int t = 0; t < kStageMaxThreads; t++) PNOL_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->stage_streams[t], cudaStreamNonBlocking));
-	for (int e = 0; e < 2 * kStageMaxThreads; e++) PNOL_CUDA(ctx, cudaEventCreateWithFlags(&ctx->stage_events[e], cudaEventDisableTiming));
+	PNOL_CUDA(ctx, cudaHostAlloc(&ctx->stage_pinned, kStageChunk * 2 * kStageThreads, cudaHostAllocDefault));
+	for (int t = 0; t < kStageThreads; t++) PNOL_CUDA(ctx, cudaStreamCreateWithFlags(&ctx->stage_streams[t], cudaStreamNonBlocking));
+	for (int e = 0; e < 2 * kStageThreads; e++) PNOL_CUDA(ctx, cudaEventCreateWithFlags(&ctx->stage_events[e], cudaEventDisableTiming));
 	return PNOL_OK;
 }
 
@@ -176,7 +174,7 @@ static int stage_init(pnol_ctx * ctx)
 static int staged_copy(pnol_ctx * ctx, void * dst, const void * src, size_t bytes, bool h2d)
 {
 	PNOL_CHECK(stage_init(ctx));
-	cudaError_t errs[kStageMaxThreads];
+	cudaError_t errs[kStageThreads];
 	size_t chunk = (bytes + 2 * (size_t) kStageThreads - 1) / (2 * (size_t) kStageThreads);
 	chunk = (chunk + 65535) & ~(size_t) 65535;
 	if (chunk > kStageChunk) chunk = kStageChunk;
@@ -214,7 +212,7 @@ static int staged_copy(pnol_ctx * ctx, void * dst, const void * src, size_t byte
 		if (e == cudaSuccess) e = cudaStreamSynchronize(st);
 		errs[t] = e;
 	};
-	std::thread th[kStageMaxThreads];
+	std::thread th[kStageThreads];
 	for (int t = 1; t < kStageThreads; t++) th[t - 1] = std::thread(worker, t);
 	worker(0);
 	for (int t = 1; t < kStageThreads; t++) th[t - 1].join();

@@ -736,6 +736,17 @@ syrk_finish_kernel(const double * __restrict__ part_tiles, const double * __rest
 	(void) nb;
 }
 
+// how launch_syrk runs the product: LDGSTS ring with one role per CTA, TMA stream-K without / with the J^T F tiles, CTA pair
+enum { kSyrkPlanLdgsts = 0, kSyrkPlanTma = 1, kSyrkPlanTmaF = 2, kSyrkPlanPair = 3 };
+
+// relative cost of one K chunk of a diagonal role; an off-diagonal one costs 64 (DMMA per k-step on the busiest sub-partition).
+// Diagonal tiles of the TMA kernel: 34, or 38 with the J^T F tiles (measured chunk times: 34.6 and 40.6 balance the two kinds of
+// segment); LDGSTS kernel: 36. The CTA pair has no plan.
+static double syrk_diag_cost(int plan_kind)
+{
+	return plan_kind == kSyrkPlanTmaF ? 40.6 : plan_kind == kSyrkPlanTma ? 34.6 : 36.0;
+}
+
 // stream-K plan (host): the K chunks of all tile roles as one stream in cost units (64 per chunk of an off-diagonal role, wdiag
 // per chunk of a diagonal one), an equal share of the stream per CTA. Out: the segments in stream order (slot = index, so a role's
 // slots are contiguous: slot0 / nslots), the first segment of every CTA (cta_seg0[grid + 1]) and the grid. A CTA holds at most
@@ -807,7 +818,7 @@ int syrk_plan_selftest(long long m, int n, int sm_count, int with_f)
 	if (m < 1 || n < 1 || sm_count < 1) return -1;
 	const int nb = (n + kBT - 1) / kBT, nroles = nb * (nb + 1) / 2;
 	const long long nchunks = (m + 31) / 32;
-	const double wdiag = with_f ? 40.6 : 34.6;
+	const double wdiag = syrk_diag_cost(with_f ? kSyrkPlanTmaF : kSyrkPlanTma);
 	std::vector<SyrkWork> work;
 	std::vector<int> cta_seg0, slot0, nslots;
 	int grid = 0;
@@ -849,31 +860,23 @@ int syrk_plan_selftest(long long m, int n, int sm_count, int with_f)
 int launch_syrk(pnol_ctx * ctx, const double * J, const double * F, long long m, int n, double * packed, const double * rhs_src)
 {
 	PNOL_REQUIRE(ctx, n >= 1 && m >= 0, "syrk: bad shape m=%lld n=%d", m, n);
-	static const int no_f = [] { const char * e = getenv("PNOL_SYRK_NOF"); return e ? atoi(e) : 0; }();      // timing runs: J^T J only
-	if (no_f) F = nullptr;
 	const int nb = (n + kBT - 1) / kBT;
 	const int nroles = nb * (nb + 1) / 2;
 	const long long nchunks = (m + kSKC - 1) / kSKC;
 	const int grid_cap = ctx->sm_count;
 
-	// TMA-fed stream-K kernel when the layout allows the 3-D tensor map (n a multiple of 16, 16-byte aligned J); otherwise, or with
-	// PNOL_SYRK_LEGACY=1 (A/B timing runs), the LDGSTS ring with one role per CTA
-	static const int legacy = [] { const char * e = getenv("PNOL_SYRK_LEGACY"); return e ? atoi(e) : 0; }();
+	// TMA-fed stream-K kernel when the layout allows the 3-D tensor map (n a multiple of 16, 16-byte aligned J); otherwise the LDGSTS
+	// ring with one role per CTA
 	const bool vec16 = (n % 2 == 0) && ((((size_t) J) & 15) == 0);
 	const bool haveF = F != nullptr && (((size_t) F) & 15) == 0;
 	static_assert(kSKC == 32, "the TMA kernel's chunk is 32 rows");
-	const bool use_tma = vec16 && !legacy && n % kTBoxCols == 0 && m > 0 && m < (1LL << 31) && (F == nullptr || haveF) &&
+	const bool use_tma = vec16 && n % kTBoxCols == 0 && m > 0 && m < (1LL << 31) && (F == nullptr || haveF) &&
 	                     tensor_map_encoder() != nullptr;
 
-	// relative cost of one K chunk of a role: DMMA per k-step on the busiest sub-partition, 64 in an off-diagonal tile. Diagonal
-	// tiles of the TMA kernel: 34, or 38 with the J^T F tiles (measured chunk times: 34.6 and 40.6 balance the two kinds of segment);
-	// LDGSTS kernel: 36. PNOL_SYRK_WDIAG overrides (tuning runs)
-	static const double wdiag_env = [] { const char * e = getenv("PNOL_SYRK_WDIAG"); return e ? atof(e) : 0.0; }();
-	// two tile rows and no F: the CTA-pair kernel (J read once); PNOL_SYRK_NO_PAIR=1 keeps the stream-K kernel (A/B runs)
-	static const int no_pair = [] { const char * e = getenv("PNOL_SYRK_NO_PAIR"); return e ? atoi(e) : 0; }();
-	const bool use_pair = use_tma && nb == 2 && F == nullptr && !no_pair && ctx->sm_count >= 2;
-	const int plan_kind = use_pair ? 3 : use_tma ? (haveF ? 2 : 1) : 0;
-	const double wdiag = wdiag_env > 0 ? wdiag_env : (plan_kind == 2 ? 40.6 : plan_kind == 1 ? 34.6 : 36.0);
+	// two tile rows and no F: the CTA-pair kernel (J read once)
+	const bool use_pair = use_tma && nb == 2 && F == nullptr && ctx->sm_count >= 2;
+	const int plan_kind = use_pair ? kSyrkPlanPair : use_tma ? (haveF ? kSyrkPlanTmaF : kSyrkPlanTma) : kSyrkPlanLdgsts;
+	const double wdiag = syrk_diag_cost(plan_kind);
 
 	std::vector<SyrkWork> work;
 	std::vector<int> nslots(nroles, 0), slot0(nroles, 0), cta_seg0;

@@ -1,16 +1,10 @@
-// ga.cu -- genetic algorithm on the device (a15 / a16): GeneticAlgorithmMPI::findMinBnd
-// (Source/GeneticAlgorithmMPI.cpp:12-276) with its free functions popSort / checkIndenticalChildAndReplace /
-// checkPopulationBoundsAndReplace (Source/GeneticAlgorithm.cpp:313-412).
+// ga.cu -- genetic algorithm on the device (a15 / a16): the state object of GeneticAlgorithmMPI::findMinBnd
+// (Source/GeneticAlgorithmMPI.cpp:12-276), its initial population (:55-81), and the free functions popSort /
+// checkIndenticalChildAndReplace / checkPopulationBoundsAndReplace (Source/GeneticAlgorithm.cpp:313-412) as stand-alone
+// stages. One generation runs in the fused pipeline of ga_pipeline.cu.
 //
 // The reference draws every random number from ONE sequential stream (timeRand()); which draw feeds which decision
-// depends on the data (rejection sampling). The kernels below reproduce exactly that consumption order in parallel:
-//   * crossover  : trial t uses draws (base + 2t, base + 2t + 1) whatever its outcome, so accept flags are computed for
-//                  all trials at once and the g-th gene takes the g-th accepted trial (block counts -> scan -> ranks);
-//   * mutation   : a child is [rejected trials]* [accepted trial] [n mutation draws]; the parser state at a block
-//                  boundary is just the offset (0..n+1) of the next trial start, so every block tabulates
-//                  offset -> (exit offset, children) for its n+2 possible entries, the tables are composed
-//                  hierarchically (block -> group -> top) and a second sweep emits the child start positions;
-//   * elite mut. : two draws per gene at fixed positions;
+// depends on the data. The stages below reproduce exactly that consumption order in parallel:
 //   * duplicates : rows are hashed, (hash,row) sorted, equal-hash runs compared exactly; replaced rows take n draws
 //                  each in row order (prefix sum);
 //   * bounds     : out-of-box genes take one draw each in row-major order (prefix sum over per-row counts);
@@ -19,22 +13,9 @@
 #include "ga_common.cuh"
 
 #include <math.h>
-#include <algorithm>
 #include <utility>
 
 namespace pnol {
-
-// one selection trial at stream position q: index = round(u(q) * Npop), accepted iff index != 0 (the reference's
-// while(index == 0) loop never keeps 0), index < Npop (the reference reads out of bounds there) and
-// u(q+1) <= fitness[index] / maxFitness   (Source/GeneticAlgorithmMPI.cpp:134-144, 167-179)
-__device__ __forceinline__ int trial_index(const StreamDev & st, unsigned long long q, const double * __restrict__ fitness,
-                                           double maxFitness, int Npop)
-{
-	int randomIndex = (int) round(st.u(q) * Npop);
-	double selectValue = st.u(q + 1);
-	if (randomIndex <= 0 || randomIndex >= Npop) return 0;
-	return (selectValue <= fitness[randomIndex] / maxFitness) ? randomIndex : 0;
-}
 
 // ---------------------------------------------------------------------------------------------------
 // exclusive prefix sum of unsigned ints (three kernels, deterministic)
@@ -373,9 +354,8 @@ dup_fix_kernel(double * __restrict__ X, long long npop, int n, const double * __
 }
 
 // ---------------------------------------------------------------------------------------------------
-// generation operators
-// ---------------------------------------------------------------------------------------------------
 // initial population (Source/GeneticAlgorithmMPI.cpp:58-68)
+// ---------------------------------------------------------------------------------------------------
 __global__ void ga_init_pop_kernel(double * __restrict__ X, long long npop, int n, const double * __restrict__ x0,
                                    const double * __restrict__ lb, const double * __restrict__ ub, StreamDev st, unsigned long long pos)
 {
@@ -385,218 +365,6 @@ __global__ void ga_init_pop_kernel(double * __restrict__ X, long long npop, int 
 	int j = (int) (e - i * n);
 	if (i == 0) X[e] = x0[j];
 	else X[e] = x0[j] + ((ub[j] - lb[j]) * st.u(pos + (unsigned long long) (e - n)) + lb[j]);
-}
-
-// fitness[k] = (F[Npop-1] - F[k])^2, indicator, elite copy (Source/GeneticAlgorithmMPI.cpp:101-124)
-__global__ void ga_fitness_kernel(const double * __restrict__ F, int npop, int nelite, double * __restrict__ fitness,
-                                  unsigned char * __restrict__ indicator, double * __restrict__ Fnew)
-{
-	int k = blockIdx.x * blockDim.x + threadIdx.x;
-	if (k >= npop) return;
-	double d = F[npop - 1] - F[k];
-	fitness[k] = d * d;
-	indicator[k] = k < nelite ? 0 : 1;
-	if (k < nelite) Fnew[k] = F[k];
-}
-
-__global__ void copy_rows_kernel(const double * __restrict__ src, double * __restrict__ dst, long long count)
-{
-	long long e = (long long) blockIdx.x * blockDim.x + threadIdx.x;
-	if (e < count) dst[e] = src[e];
-}
-
-// ---- crossover: accepted-trial ranks ----
-constexpr int kTrialTile = 4096;      // trials per block (256 threads x 16)
-
-__global__ void __launch_bounds__(256)
-cross_count_kernel(StreamDev st, unsigned long long pos, long long trial0, long long ntrials, const double * __restrict__ fitness,
-                   int npop, unsigned * __restrict__ block_counts)
-{
-	__shared__ unsigned red[256];
-	const double maxFitness = fitness[0];
-	long long base = trial0 + (long long) blockIdx.x * kTrialTile;
-	unsigned c = 0;
-	for (int e = 0; e < 16; e++) {
-		long long t = base + threadIdx.x * 16 + e;
-		if (t < trial0 + ntrials && trial_index(st, pos + 2ULL * (unsigned long long) t, fitness, maxFitness, npop) != 0) c++;
-	}
-	red[threadIdx.x] = c;
-	__syncthreads();
-	for (int o = 128; o > 0; o >>= 1) {
-		if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
-		__syncthreads();
-	}
-	if (threadIdx.x == 0) block_counts[blockIdx.x] = red[0];
-}
-
-// sel[rank] = index for accepted trials with rank < need; the trial index of rank need-1 goes to *last_trial
-__global__ void __launch_bounds__(256)
-cross_emit_kernel(StreamDev st, unsigned long long pos, long long trial0, long long ntrials, const double * __restrict__ fitness,
-                  int npop, const unsigned long long * __restrict__ block_offs, long long rank0, long long need,
-                  int * __restrict__ sel, long long * __restrict__ last_trial)
-{
-	__shared__ unsigned tsum[256];
-	const double maxFitness = fitness[0];
-	long long base = trial0 + (long long) blockIdx.x * kTrialTile;
-	int idx[16];
-	unsigned c = 0;
-	for (int e = 0; e < 16; e++) {
-		long long t = base + threadIdx.x * 16 + e;
-		idx[e] = (t < trial0 + ntrials) ? trial_index(st, pos + 2ULL * (unsigned long long) t, fitness, maxFitness, npop) : 0;
-		if (idx[e]) c++;
-	}
-	tsum[threadIdx.x] = c;
-	__syncthreads();
-	for (int o = 1; o < 256; o <<= 1) {
-		unsigned v = threadIdx.x >= o ? tsum[threadIdx.x - o] : 0;
-		__syncthreads();
-		tsum[threadIdx.x] += v;
-		__syncthreads();
-	}
-	long long rank = rank0 + (long long) block_offs[blockIdx.x] + (threadIdx.x ? tsum[threadIdx.x - 1] : 0);
-	for (int e = 0; e < 16; e++) {
-		if (idx[e]) {
-			if (rank < need) {
-				sel[rank] = idx[e];
-				if (rank == need - 1) *last_trial = base + threadIdx.x * 16 + e;
-			}
-			rank++;
-		}
-	}
-}
-
-// XpopNew[row0 + k][i] = Xpop[sel[k*n + i]][i]   (Source/GeneticAlgorithmMPI.cpp:147-150)
-__global__ void cross_gather_kernel(const double * __restrict__ Xpop, const int * __restrict__ sel, long long count, int n,
-                                    double * __restrict__ XnewRows)
-{
-	long long e = (long long) blockIdx.x * blockDim.x + threadIdx.x;
-	if (e >= count) return;
-	int i = (int) (e % n);
-	XnewRows[e] = Xpop[(long long) sel[e] * n + i];
-}
-
-// ---- mutation: block tables ----
-constexpr int kMutBlock = 2048;        // stream positions per block
-constexpr int kMutGroup = 64;          // blocks per group
-
-// table[(block * S + delta)] = (exit delta, children) for delta in [0, S), S = n + 2
-__global__ void __launch_bounds__(128)
-mut_block_table_kernel(StreamDev st, unsigned long long pos, long long npositions, const double * __restrict__ fitness, int npop,
-                       int n, int S, int * __restrict__ exit_delta, int * __restrict__ children)
-{
-	__shared__ unsigned char acc[kMutBlock];
-	const double maxFitness = fitness[0];
-	const long long b0 = (long long) blockIdx.x * kMutBlock;
-	for (int e = threadIdx.x; e < kMutBlock; e += blockDim.x) {
-		long long q = b0 + e;
-		acc[e] = (q < npositions && trial_index(st, pos + (unsigned long long) q, fitness, maxFitness, npop) != 0) ? 1 : 0;
-	}
-	__syncthreads();
-	for (int d = threadIdx.x; d < S; d += blockDim.x) {
-		int p = d, cnt = 0;
-		while (p < kMutBlock) {
-			if (acc[p]) { cnt++; p += n + 2; } else p += 2;
-		}
-		exit_delta[(size_t) blockIdx.x * S + d] = p - kMutBlock;
-		children[(size_t) blockIdx.x * S + d] = cnt;
-	}
-}
-
-// compose kMutGroup block tables: gtable[(group * S + delta)] = (exit delta, children)
-__global__ void mut_group_table_kernel(const int * __restrict__ exit_delta, const int * __restrict__ children, int nblocks, int S,
-                                       int ngroups, int * __restrict__ gexit, long long * __restrict__ gchildren)
-{
-	int t = blockIdx.x * blockDim.x + threadIdx.x;
-	if (t >= ngroups * S) return;
-	int g = t / S, d = t - g * S;
-	long long cnt = 0;
-	int b1 = min(nblocks, (g + 1) * kMutGroup);
-	for (int b = g * kMutGroup; b < b1; b++) {
-		if (d >= kMutBlock) { d -= kMutBlock; continue; }      // a jump longer than a block (n + 2 > 2048)
-		cnt += children[(size_t) b * S + d];
-		d = exit_delta[(size_t) b * S + d];
-	}
-	gexit[t] = d;
-	gchildren[t] = cnt;
-}
-
-// single thread: entry delta and child base of every group; total children reached -> *total
-__global__ void mut_top_kernel(const int * __restrict__ gexit, const long long * __restrict__ gchildren, int ngroups, int S,
-                               int * __restrict__ gentry, long long * __restrict__ gbase, long long * __restrict__ total)
-{
-	if (blockIdx.x != 0 || threadIdx.x != 0) return;
-	int d = 0;
-	long long cnt = 0;
-	for (int g = 0; g < ngroups; g++) {
-		gentry[g] = d; gbase[g] = cnt;
-		if (d >= S) { d -= kMutBlock * kMutGroup; if (d < 0) d = 0; continue; }   // unreachable for S <= block*group
-		cnt += gchildren[(size_t) g * S + d];
-		d = gexit[(size_t) g * S + d];
-	}
-	*total = cnt;
-}
-
-// one thread per group: entry delta and child base of every block of the group
-__global__ void mut_group_walk_kernel(const int * __restrict__ exit_delta, const int * __restrict__ children, int nblocks, int S,
-                                      int ngroups, const int * __restrict__ gentry, const long long * __restrict__ gbase,
-                                      int * __restrict__ bentry, long long * __restrict__ bbase)
-{
-	int g = blockIdx.x * blockDim.x + threadIdx.x;
-	if (g >= ngroups) return;
-	int d = gentry[g];
-	long long cnt = gbase[g];
-	int b1 = min(nblocks, (g + 1) * kMutGroup);
-	for (int b = g * kMutGroup; b < b1; b++) {
-		bentry[b] = d; bbase[b] = cnt;
-		if (d >= kMutBlock) { d -= kMutBlock; continue; }
-		cnt += children[(size_t) b * S + d];
-		d = exit_delta[(size_t) b * S + d];
-	}
-}
-
-// one thread per block: walk from the block's entry and record the accepted-trial position of each child < need
-__global__ void mut_emit_kernel(StreamDev st, unsigned long long pos, long long npositions, const double * __restrict__ fitness,
-                                int npop, int n, int nblocks, const int * __restrict__ bentry, const long long * __restrict__ bbase,
-                                long long need, long long * __restrict__ child_pos /* relative to pos */, int * __restrict__ child_idx)
-{
-	int b = blockIdx.x * blockDim.x + threadIdx.x;
-	if (b >= nblocks) return;
-	const double maxFitness = fitness[0];
-	long long k = bbase[b];
-	if (k >= need) return;
-	long long q = (long long) b * kMutBlock + bentry[b];
-	const long long bend = (long long) (b + 1) * kMutBlock;
-	while (q < bend && q < npositions && k < need) {
-		int idx = trial_index(st, pos + (unsigned long long) q, fitness, maxFitness, npop);
-		if (idx) { child_pos[k] = q; child_idx[k] = idx; k++; q += n + 2; } else q += 2;
-	}
-}
-
-// XpopNew[row0 + k][j] = Xpop[index_k][j] + spreadRatio * (ub[j] - lb[j]) * u(accepted_k + 2 + j)  (:182-186)
-__global__ void mut_apply_kernel(const double * __restrict__ Xpop, const long long * __restrict__ child_pos, const int * __restrict__ child_idx,
-                                 long long nrand, int n, const double * __restrict__ lb, const double * __restrict__ ub,
-                                 double spreadRatio, StreamDev st, unsigned long long pos, double * __restrict__ XnewRows)
-{
-	long long e = (long long) blockIdx.x * blockDim.x + threadIdx.x;
-	if (e >= nrand * n) return;
-	long long k = e / n;
-	int j = (int) (e - k * n);
-	double mutation = spreadRatio * (ub[j] - lb[j]) * st.u(pos + (unsigned long long) child_pos[k] + 2ULL + (unsigned long long) j);
-	XnewRows[e] = Xpop[(long long) child_idx[k] * n + j] + mutation;
-}
-
-// elite mutation (Source/GeneticAlgorithmMPI.cpp:195-207): two draws per gene at fixed positions
-__global__ void elite_mut_kernel(const double * __restrict__ Xpop, long long nelmut, int n, int nelite, const double * __restrict__ lb,
-                                 const double * __restrict__ ub, double eliteMutationSize, StreamDev st, unsigned long long pos,
-                                 double * __restrict__ XnewRows, int * __restrict__ elite_idx)
-{
-	long long e = (long long) blockIdx.x * blockDim.x + threadIdx.x;
-	if (e >= nelmut * n) return;
-	int j = (int) (e % n);
-	int randomEliteIdx = (int) round(st.u(pos + 2ULL * (unsigned long long) e) * nelite);
-	double mutation = eliteMutationSize * (ub[j] - lb[j]) * st.u(pos + 2ULL * (unsigned long long) e + 1ULL);
-	XnewRows[e] = Xpop[(long long) randomEliteIdx * n + j] + mutation;
-	if (elite_idx) elite_idx[e] = randomEliteIdx;
 }
 
 } // namespace pnol
@@ -658,7 +426,6 @@ extern "C" void pnol_ga_destroy(pnol_ga * ga)
 	cudaStreamSynchronize(ga->ctx->stream);
 	ga_pipe_destroy(ga);
 	for (void * p : ga->owned) cudaFree(p);
-	if (ga->mut_mem) cudaFree(ga->mut_mem);
 	delete ga;
 }
 
@@ -680,8 +447,7 @@ extern "C" int pnol_ga_create(pnol_ctx * ctx, const pnol_functor * f, const pnol
 	ga->ctx = ctx; ga->f = f; ga->prm = *prm; ga->n = n;
 	ga->nelite = nelite; ga->nelmut = nelmut; ga->ncross = ncross; ga->nrand = nrand;
 	ga->stream = *stream; ga->pos = 0; ga->generation = 0; ga->n_static = 0; ga->stopped = 0;
-	ga->f_best = ga->f_best_prev = 0; ga->accept_rate = 0.25;
-	ga->mut_mem = nullptr; ga->mut_bytes = 0; ga->stream_values = nullptr;
+	ga->f_best = ga->f_best_prev = 0; ga->stream_values = nullptr;
 	size_t NN = (size_t) Npop * n;
 	int st = PNOL_OK;
 #define GA_TRY(x) do { st = (x); if (st != PNOL_OK) { pnol_ga_destroy(ga); return st; } } while (0)
@@ -701,13 +467,10 @@ extern "C" int pnol_ga_create(pnol_ctx * ctx, const pnol_functor * f, const pnol
 	GA_TRY(ga_alloc(ga, &ga->exhausted, 4));
 	GA_TRY(ga_alloc(ga, &ga->keys, Npop));
 	GA_TRY(ga_alloc(ga, &ga->perm, Npop));
-	size_t ntrial_blocks = ((size_t) 64 * 1024 * 1024) / kTrialTile;       // room for 64 M trials per batch
-	size_t u32n = std::max((size_t) Npop, ntrial_blocks) + 16;
-	GA_TRY(ga_alloc(ga, &ga->u32a, u32n));
-	GA_TRY(ga_alloc(ga, &ga->u64a, u32n));
-	GA_TRY(ga_alloc(ga, &ga->scan_tmp, u32n / kScanTile + 16));
+	GA_TRY(ga_alloc(ga, &ga->u32a, (size_t) Npop + 16));
+	GA_TRY(ga_alloc(ga, &ga->u64a, (size_t) Npop + 16));
+	GA_TRY(ga_alloc(ga, &ga->scan_tmp, (size_t) Npop / kScanTile + 16));
 	GA_TRY(ga_alloc(ga, &ga->total_dev, 4));
-	GA_TRY(ga_alloc(ga, &ga->ll_dev, 4));
 	{
 		void * sm = nullptr;
 		cudaError_t e = cudaMalloc(&sm, SortScratch::bytes(Npop));
@@ -725,11 +488,7 @@ extern "C" int pnol_ga_create(pnol_ctx * ctx, const pnol_functor * f, const pnol
 	cudaMemcpyAsync(ga->ub, xub, n * sizeof(double), cudaMemcpyDefault, ctx->stream);
 	cudaMemsetAsync(ga->exhausted, 0, 16, ctx->stream);
 	GA_TRY(finish(ctx));
-	// the fused generation pipeline (ga_pipeline.cu) unless PNOL_GA_LEGACY=1 asks for the stage-by-stage generation (A/B runs)
-	{
-		const char * e = getenv("PNOL_GA_LEGACY");
-		if (!(e && atoi(e) != 0)) GA_TRY(ga_pipe_create(ga));
-	}
+	GA_TRY(ga_pipe_create(ga));
 #undef GA_TRY
 	*out = ga;
 	return PNOL_OK;
@@ -837,166 +596,15 @@ extern "C" int pnol_ga_init(pnol_ga * ga, const double * x0, double * f0_out)
 	PNOL_CHECK(ga_check_stream(ga));
 	ga->f_best_prev = fb; ga->f_best = fb;
 	if (f0_out) *f0_out = f0;
-	if (ga->pipe) PNOL_CHECK(ga_pipe_reset(ga));
-	return PNOL_OK;
-}
-
-static int ga_mut_reserve(pnol_ga * ga, size_t bytes)
-{
-	if (bytes <= ga->mut_bytes) return PNOL_OK;
-	if (ga->mut_mem) { PNOL_CUDA(ga->ctx, cudaStreamSynchronize(ga->ctx->stream)); cudaFree(ga->mut_mem); ga->mut_mem = nullptr; ga->mut_bytes = 0; }
-	PNOL_CUDA(ga->ctx, cudaMalloc(&ga->mut_mem, bytes + bytes / 4));
-	ga->mut_bytes = bytes + bytes / 4;
-	return PNOL_OK;
+	return ga_pipe_reset(ga);
 }
 
 // Source/GeneticAlgorithmMPI.cpp:87-249 (one pass of the while loop)
 extern "C" int pnol_ga_generation(pnol_ga * ga)
 {
 	if (!ga) return PNOL_ERR_INVALID;
-	pnol_ctx * ctx = ga->ctx;
 	if (ga->stopped || ga->generation >= ga->prm.max_generations) return PNOL_OK;
-	if (ga->pipe) return ga_pipe_generation(ga);
-	const int Npop = ga->prm.npop, n = ga->n;
-	const int Nelite = ga->nelite, Ncross = ga->ncross, Nrand = ga->nrand, NeliteMut = ga->nelmut;
-	StreamDev st = ga_stream_dev(ga);
-	GaScratch sc = ga_scratch(ga);
-	const int iter = ga->generation;
-
-	// 0b / 1. fitness, indicator, elite copy (:101-124)
-	{
-		TimerScope ts(ctx, "ga_fitness");
-		PNOL_LAUNCH(ctx, ga_fitness_kernel, (Npop + 255) / 256, 256, 0, ga->F, Npop, Nelite, ga->fitness, ga->indicator, ga->Fnew);
-		if (Nelite > 0)
-			PNOL_LAUNCH(ctx, copy_rows_kernel, (unsigned) (((long long) Nelite * n + 255) / 256), 256, 0, ga->Xpop, ga->Xnew, (long long) Nelite * n);
-	}
-	double maxFitness = 0;
-	PNOL_CUDA(ctx, cudaMemcpyAsync(&maxFitness, ga->fitness, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-	PNOL_CHECK(finish(ctx));
-	if (!(maxFitness > 0) || isinf(maxFitness)) {
-		// every trial would compare against NaN/inf: the reference spins forever in its while loops (SURVEY App. B)
-		PNOL_SET_ERR(ctx, "ga: degenerate population (best and worst objective coincide or are not finite): selection cannot proceed");
-		return PNOL_ERR_NONFINITE;
-	}
-
-	// 2. crossover (:128-153): ranks of accepted trials, batch after batch
-	if (Ncross > 0) {
-		TimerScope ts(ctx, "ga_crossover");
-		const long long need = (long long) Ncross * n;
-		long long have = 0, trial0 = 0;
-		long long last_trial = -1;
-		PNOL_CUDA(ctx, cudaMemsetAsync(ga->ll_dev, 0xff, sizeof(long long), ctx->stream));
-		while (have < need) {
-			double rate = ga->accept_rate > 1e-4 ? ga->accept_rate : 1e-4;
-			long long batch = (long long) ((need - have) / rate * 1.15) + 4 * kTrialTile;
-			const long long cap = (long long) 64 * 1024 * 1024;
-			if (batch > cap) batch = cap;
-			int nb = (int) ((batch + kTrialTile - 1) / kTrialTile);
-			batch = (long long) nb * kTrialTile;
-			PNOL_LAUNCH(ctx, cross_count_kernel, nb, 256, 0, st, (unsigned long long) ga->pos, trial0, batch, ga->fitness, Npop, ga->u32a);
-			PNOL_CHECK(exclusive_scan_u32(ctx, ga->u32a, nb, ga->u64a, ga->scan_tmp, ga->total_dev));
-			PNOL_LAUNCH(ctx, cross_emit_kernel, nb, 256, 0, st, (unsigned long long) ga->pos, trial0, batch, ga->fitness, Npop, ga->u64a,
-			            have, need, ga->cross_idx, ga->ll_dev);
-			unsigned long long got = 0;
-			PNOL_CUDA(ctx, cudaMemcpyAsync(&got, ga->total_dev, sizeof got, cudaMemcpyDeviceToHost, ctx->stream));
-			PNOL_CUDA(ctx, cudaMemcpyAsync(&last_trial, ga->ll_dev, sizeof last_trial, cudaMemcpyDeviceToHost, ctx->stream));
-			PNOL_CHECK(finish(ctx));
-			PNOL_CHECK(ga_check_stream(ga));
-			if (got > 0) ga->accept_rate = 0.5 * ga->accept_rate + 0.5 * ((double) got / (double) batch);
-			else ga->accept_rate *= 0.25;
-			have += (long long) got;
-			trial0 += batch;
-			if (ga->accept_rate < 1e-9) { PNOL_SET_ERR(ctx, "ga: selection accepts no trial"); return PNOL_ERR_NONFINITE; }
-		}
-		PNOL_LAUNCH(ctx, cross_gather_kernel, (unsigned) ((need + 255) / 256), 256, 0, ga->Xpop, ga->cross_idx, need, n,
-		            ga->Xnew + (size_t) Nelite * n);
-		ga->pos += 2ULL * (unsigned long long) (last_trial + 1);
-	}
-
-	// 3. random mutations (:159-190)
-	{
-		TimerScope ts(ctx, "ga_mutation");
-		const double spreadRatio = ga->prm.mutation_size * (ga->prm.max_generations - iter) / ga->prm.max_generations;   // (:159)
-		const int S = n + 2;
-		double rate = ga->accept_rate > 1e-4 ? ga->accept_rate : 1e-4;
-		long long npos = (long long) ((double) Nrand * (n + 2.0 / rate) * 1.1) + 8 * kMutBlock;
-		for (;;) {
-			int nblocks = (int) ((npos + kMutBlock - 1) / kMutBlock);
-			npos = (long long) nblocks * kMutBlock;
-			int ngroups = (nblocks + kMutGroup - 1) / kMutGroup;
-			size_t b_tab = (size_t) nblocks * S * sizeof(int);
-			size_t g_tab = (size_t) ngroups * S;
-			size_t need_bytes = 2 * b_tab + g_tab * (sizeof(int) + sizeof(long long)) + (size_t) ngroups * (sizeof(int) + sizeof(long long)) +
-			                    (size_t) nblocks * (sizeof(int) + sizeof(long long)) + 4096;
-			PNOL_CHECK(ga_mut_reserve(ga, need_bytes));
-			unsigned char * p = (unsigned char *) ga->mut_mem;
-			auto take = [&](size_t b) { void * r = p; p += (b + 255) & ~(size_t) 255; return r; };
-			int * exit_delta = (int *) take(b_tab);
-			int * children = (int *) take(b_tab);
-			int * gexit = (int *) take(g_tab * sizeof(int));
-			long long * gchildren = (long long *) take(g_tab * sizeof(long long));
-			int * gentry = (int *) take((size_t) ngroups * sizeof(int));
-			long long * gbase = (long long *) take((size_t) ngroups * sizeof(long long));
-			int * bentry = (int *) take((size_t) nblocks * sizeof(int));
-			long long * bbase = (long long *) take((size_t) nblocks * sizeof(long long));
-			PNOL_LAUNCH(ctx, mut_block_table_kernel, nblocks, 128, 0, st, (unsigned long long) ga->pos, npos + kMutBlock, ga->fitness, Npop, n, S,
-			            exit_delta, children);
-			PNOL_LAUNCH(ctx, mut_group_table_kernel, (ngroups * S + 127) / 128, 128, 0, exit_delta, children, nblocks, S, ngroups, gexit, gchildren);
-			PNOL_LAUNCH(ctx, mut_top_kernel, 1, 32, 0, gexit, gchildren, ngroups, S, gentry, gbase, ga->ll_dev + 1);
-			long long total = 0;
-			PNOL_CUDA(ctx, cudaMemcpyAsync(&total, ga->ll_dev + 1, sizeof total, cudaMemcpyDeviceToHost, ctx->stream));
-			PNOL_CHECK(finish(ctx));
-			PNOL_CHECK(ga_check_stream(ga));
-			if (total < Nrand) {                       // the window was too short: widen it and redo (rare)
-				double grow = total > 0 ? (double) Nrand / (double) total * 1.25 : 4.0;
-				npos = (long long) ((double) npos * grow) + 8 * kMutBlock;
-				if (npos > ((long long) 1 << 40)) { PNOL_SET_ERR(ctx, "ga: mutation selection accepts no trial"); return PNOL_ERR_NONFINITE; }
-				continue;
-			}
-			PNOL_LAUNCH(ctx, mut_group_walk_kernel, (ngroups + 63) / 64, 64, 0, exit_delta, children, nblocks, S, ngroups, gentry, gbase, bentry, bbase);
-			PNOL_LAUNCH(ctx, mut_emit_kernel, (nblocks + 63) / 64, 64, 0, st, (unsigned long long) ga->pos, npos + kMutBlock, ga->fitness, Npop, n,
-			            nblocks, bentry, bbase, (long long) Nrand, ga->mut_pos, ga->mut_idx);
-			break;
-		}
-		PNOL_LAUNCH(ctx, mut_apply_kernel, (unsigned) (((long long) Nrand * n + 255) / 256), 256, 0, ga->Xpop, ga->mut_pos, ga->mut_idx,
-		            (long long) Nrand, n, ga->lb, ga->ub, spreadRatio, st, (unsigned long long) ga->pos,
-		            ga->Xnew + (size_t) (Nelite + Ncross) * n);
-		long long lastpos = 0;
-		PNOL_CUDA(ctx, cudaMemcpyAsync(&lastpos, ga->mut_pos + (Nrand - 1), sizeof lastpos, cudaMemcpyDeviceToHost, ctx->stream));
-		PNOL_CHECK(finish(ctx));
-		ga->pos += (unsigned long long) lastpos + 2ULL + (unsigned long long) n;
-	}
-
-	// 4. mutations of the elite children (:195-207)
-	if (NeliteMut > 0) {
-		TimerScope ts(ctx, "ga_elite_mutation");
-		PNOL_LAUNCH(ctx, elite_mut_kernel, (unsigned) (((long long) NeliteMut * n + 255) / 256), 256, 0, ga->Xpop, (long long) NeliteMut, n, Nelite,
-		            ga->lb, ga->ub, ga->prm.elite_mutation_size, st, (unsigned long long) ga->pos,
-		            ga->Xnew + (size_t) (Nelite + Ncross + Nrand) * n, ga->elite_idx);
-		ga->pos += 2ULL * (unsigned long long) NeliteMut * (unsigned long long) n;
-	}
-
-	// 5a / 5b. identical children, domain boundaries (:211-214)
-	PNOL_CHECK(ga_check_identical_dev(ctx, ga->Xnew, Npop, n, ga->lb, ga->ub, ga->indicator, st, &ga->pos, sc));
-	PNOL_CHECK(ga_check_bounds_dev(ctx, ga->Xnew, Npop, n, ga->lb, ga->ub, ga->indicator, st, &ga->pos, sc));
-
-	// 6. evaluate the new population (:217): the fitness sweep
-	PNOL_CHECK(ga_evaluate(ga, ga->Xnew, ga->indicator, ga->Fnew));
-
-	// 7. sort and copy to the old population (:220-230): sorted rows go straight into Xpop / F
-	PNOL_CHECK(ga_pop_sort_dev(ctx, ga->Xnew, ga->Fnew, Npop, n, ga->Xpop, ga->F, sc));
-
-	// static generations (:234-249)
-	double Fbest = 0;
-	PNOL_CUDA(ctx, cudaMemcpyAsync(&Fbest, ga->F, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-	PNOL_CHECK(finish(ctx));
-	PNOL_CHECK(ga_check_stream(ga));
-	ga->f_best = Fbest;
-	if (Fbest == ga->f_best_prev) ga->n_static++; else ga->n_static = 0;
-	if (ga->n_static > ga->prm.n_static_generations) { ga->stopped = 1; return PNOL_OK; }
-	ga->f_best_prev = Fbest;
-	ga->generation++;
-	return PNOL_OK;
+	return ga_pipe_generation(ga);
 }
 
 extern "C" int pnol_ga_status_get(pnol_ga * ga, pnol_ga_status * s)
@@ -1023,22 +631,13 @@ extern "C" int pnol_ga_peer_mode(pnol_ga * ga)
 extern "C" int pnol_ga_get_population(pnol_ga * ga, double * xpop, double * F)
 {
 	if (!ga) return PNOL_ERR_INVALID;
-	if (ga->pipe) return ga_pipe_get_population(ga, xpop, F);
-	pnol_ctx * ctx = ga->ctx;
-	if (xpop) PNOL_CUDA(ctx, cudaMemcpyAsync(xpop, ga->Xpop, (size_t) ga->prm.npop * ga->n * sizeof(double), cudaMemcpyDefault, ctx->stream));
-	if (F) PNOL_CUDA(ctx, cudaMemcpyAsync(F, ga->F, (size_t) ga->prm.npop * sizeof(double), cudaMemcpyDefault, ctx->stream));
-	return finish(ctx);
+	return ga_pipe_get_population(ga, xpop, F);
 }
 
 extern "C" int pnol_ga_get_indices(pnol_ga * ga, int * cross_idx, int * mut_idx, int * elite_idx)
 {
 	if (!ga) return PNOL_ERR_INVALID;
-	if (ga->pipe) return ga_pipe_get_indices(ga, cross_idx, mut_idx, elite_idx);
-	pnol_ctx * ctx = ga->ctx;
-	if (cross_idx) PNOL_CUDA(ctx, cudaMemcpyAsync(cross_idx, ga->cross_idx, (size_t) ga->ncross * ga->n * sizeof(int), cudaMemcpyDefault, ctx->stream));
-	if (mut_idx) PNOL_CUDA(ctx, cudaMemcpyAsync(mut_idx, ga->mut_idx, (size_t) ga->nrand * sizeof(int), cudaMemcpyDefault, ctx->stream));
-	if (elite_idx) PNOL_CUDA(ctx, cudaMemcpyAsync(elite_idx, ga->elite_idx, (size_t) ga->nelmut * ga->n * sizeof(int), cudaMemcpyDefault, ctx->stream));
-	return finish(ctx);
+	return ga_pipe_get_indices(ga, cross_idx, mut_idx, elite_idx);
 }
 
 // ---------------------------------------------------------------------------------------------------

@@ -1,5 +1,5 @@
-// ga_common.cuh -- pieces shared by the genetic-algorithm translation units (ga.cu: state object, stand-alone stages and the
-// stage-by-stage generation of round 1; ga_pipeline.cu: the fused, sync-free generation).
+// ga_common.cuh -- pieces shared by the genetic-algorithm translation units (ga.cu: state object, initial population and
+// stand-alone stages; ga_pipeline.cu: the fused, sync-free generation).
 #pragma once
 
 #include "common.cuh"
@@ -82,7 +82,7 @@ struct RowTable {
 };
 
 constexpr int kScanTile = 2048;      // elements per block of the three-kernel prefix sum (256 threads x 8)
-constexpr int kSortTile = 2048;      // keys per block of the legacy radix sort: 8 warps x 8 rounds x 32 lanes
+constexpr int kSortTile = 2048;      // keys per block of the radix sort of ga.cu's stages: 8 warps x 8 rounds x 32 lanes
 constexpr int kSortWarps = 8;
 
 struct SortScratch {
@@ -141,25 +141,21 @@ struct pnol_ga {
 	void * sort_mem; pnol::SortScratch sort;
 	unsigned long long * keys; unsigned * perm;
 	unsigned * u32a; unsigned long long * u64a; unsigned long long * scan_tmp; unsigned long long * total_dev;
-	long long * ll_dev;
-	// mutation tables (grown on demand)
-	void * mut_mem; size_t mut_bytes;
 	double * gather = nullptr;           // all-gather buffer of the sharded fitness sweep (multi-GPU)
 	// host state
 	pnol_stream_desc stream;
 	uint64_t pos;
 	int generation, n_static, stopped;
 	double f_best_prev, f_best;
-	double accept_rate;
 	std::vector<void *> owned;
-	// the fused generation pipeline (ga_pipeline.cu); nullptr: stage-by-stage generation of round 1 (PNOL_GA_LEGACY=1)
+	// the fused generation pipeline (ga_pipeline.cu); created by pnol_ga_create, nullptr only while it is being built or torn down
 	struct GaPipe * pipe = nullptr;
 };
 
 
 namespace pnol {
 // ga_pipeline.cu
-int ga_pipe_create(pnol_ga * ga);                 // allocates the pipeline state (after the legacy buffers exist)
+int ga_pipe_create(pnol_ga * ga);                 // allocates the pipeline state (after the buffers of pnol_ga_init exist)
 void ga_pipe_destroy(pnol_ga * ga);
 int ga_pipe_reset(pnol_ga * ga);                  // after pnol_ga_init: sorted population -> pipeline representation
 int ga_pipe_generation(pnol_ga * ga);

@@ -1,9 +1,9 @@
 // ga_pipeline.cu -- one generation of GeneticAlgorithmMPI::findMinBnd (Source/GeneticAlgorithmMPI.cpp:87-249) as a fused,
 // sync-free kernel pipeline: every stage reads the stream position it starts from out of a status block in device memory, so the
 // host enqueues the whole generation and synchronises ONCE at its end to read that block (stream position, best objective, error
-// bits). Bit-exact with the stage-by-stage generation of ga.cu and with the oracle (tests/test_gpu_ga.py).
+// bits). Bit-exact with the oracle (tests/test_gpu_ga.py).
 //
-// What changed against the stage-by-stage generation (2.25 ms at 1M x 32, ~105 launches, 8 host round trips):
+// What changed against the stage-by-stage generation of round 1 (2.25 ms at 1M x 32, ~105 launches, 8 host round trips):
 //   * the population is never physically sorted. Rows stay where the generation that made them wrote them ("child order");
 //     `perm` maps sorted position -> row. Parents are fetched through perm (they are random accesses anyway), so popSort's
 //     gather of 256 MB in and 256 MB out per generation is gone; only pnol_ga_get_population materialises the sorted rows;
@@ -1369,7 +1369,7 @@ int ga_pipe_create(pnol_ga * ga)
 	PNOL_REQUIRE(ctx, ctx->nranks <= kGaMaxRanks, "ga: at most %d ranks", kGaMaxRanks);
 	GaPipe * P = new GaPipe();
 	ga->pipe = P;
-	// Several GPUs, two ways to split a generation (pnol_ga_set_sharding; PNOL_GA_SHARD=rows|sweep overrides):
+	// Several GPUs, two ways to split a generation (pnol_ga_set_sharding):
 	//   rows  : rank r owns child rows [r per, (r+1) per): it creates, repairs and evaluates them, parents are read from their
 	//           owners over NVLink. Memory per GPU falls with the GPU count; at 1M x 32 the gene-wise parent reads (8 bytes each,
 	//           millions of them per rank) are latency-bound on the link and the generation is SLOWER than on one GPU
@@ -1384,7 +1384,6 @@ int ga_pipe_create(pnol_ga * ga)
 	// that the other ranks take over costs more than the all-gather (built-in objectives: streaming time of the population at 4.6 TB/s
 	// against 0.02 ms + 18 ns per KB gathered, the measured figures above; user functors: always, their cost is unknown), else none.
 	int mode = ctx->ga_sharding;
-	if (const char * e = getenv("PNOL_GA_SHARD")) { if (!strcmp(e, "rows")) mode = 1; else if (!strcmp(e, "sweep")) mode = 2; else if (!strcmp(e, "none")) mode = 3; }
 	if (mode == 0) {
 		size_t free_b = 0, total_b = 0;
 		cudaMemGetInfo(&free_b, &total_b);
@@ -1785,7 +1784,7 @@ int ga_pipe_generation(pnol_ga * ga)
 
 int ga_pipe_peer_mode(pnol_ga * ga)
 {
-	if (!ga->pipe || ga->ctx->nranks <= 1) return 0;
+	if (ga->ctx->nranks <= 1) return 0;
 	if (ga->pipe->R <= 1) return ga->pipe->shard_sweep ? 3 : 4;
 	return ga->pipe->use_ipc ? 1 : 2;
 }
@@ -1797,7 +1796,7 @@ int ga_pipe_get_population(pnol_ga * ga, double * xpop, double * F)
 	const long long Npop = ga->prm.npop;
 	const int n = ga->n;
 	if (xpop) {
-		// sorted rows into the (otherwise idle) full-size buffer of the stage-by-stage path
+		// sorted rows into the full-size buffer that pnol_ga_init sorts through (idle between generations)
 		PNOL_LAUNCH(ctx, ga_gather_sorted_kernel, blocks_for(Npop * kRowLanes, 256), 256, 0, P->table[P->cur], P->perm[P->cur], 0LL, Npop, n, ga->Xnew);
 		PNOL_CUDA(ctx, cudaMemcpyAsync(xpop, ga->Xnew, (size_t) Npop * n * sizeof(double), cudaMemcpyDefault, ctx->stream));
 	}
