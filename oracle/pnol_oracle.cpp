@@ -473,14 +473,16 @@ uint64_t oracle_ga_check_identical(double * Xpop, long long Npop, int n, const d
 // run: cross_idx (Ncross x n), mut_idx (Nrand), elite_idx (NeliteMut x n); stream_pos_out.
 // Returns the number of generations completed (iter at exit), or -1 if the fractions are invalid (the reference
 // calls exit(0), :40-44). stopAfter >= 0 ends the loop early with maxGenerations (hence the mutation schedule) unchanged.
-int oracle_ga(int kind, const double * scalars, const long long * ints, const double * const * cols, long long m,
-              double * X, const double * Xlb, const double * Xub, int Nparam, int Npop, int maxGenerations, double eliteFrac,
-              double crossFrac, double eliteMutationFrac, double mutationSize, double eliteMutationSize,
-              double NstaticGenerations, int stopAfter, const double * values, uint64_t n_values, uint64_t seed, double scale,
-              double * f0_out, double * fOpt_out, double * Xpop_out, double * F_out, int * cross_idx, int * mut_idx,
-              int * elite_idx, uint64_t * stream_pos_out)
+// fn != NULL: the objective is fn(x, n) (a user objective compiled into the caller) instead of the built-in kind.
+int oracle_ga_fn(int kind, const double * scalars, const long long * ints, const double * const * cols, long long m,
+                 double (*fn)(const double *, int), double * X, const double * Xlb, const double * Xub, int Nparam, int Npop,
+                 int maxGenerations, double eliteFrac, double crossFrac, double eliteMutationFrac, double mutationSize,
+                 double eliteMutationSize, double NstaticGenerations, int stopAfter, const double * values, uint64_t n_values,
+                 uint64_t seed, double scale, double * f0_out, double * fOpt_out, double * Xpop_out, double * F_out, int * cross_idx,
+                 int * mut_idx, int * elite_idx, uint64_t * stream_pos_out)
 {
 	OFunctor fobj = {kind, scalars, ints, cols, m};
+	auto objective = [&](const double * x) { return fn ? fn(x, Nparam) : o_scalar(fobj, x, Nparam); };
 	OStream st = {values, n_values, seed, scale, 0, 0};
 	size_t NN = (size_t) Npop * Nparam;
 	vector<double> Xpop(NN, 0.0), XpopNew(NN, 0.0), F(Npop, 0), Fnew(Npop, 0), fitness(Npop, 0);
@@ -498,7 +500,7 @@ int oracle_ga(int kind, const double * scalars, const long long * ints, const do
 			Xpop[(size_t) i * Nparam + j] = Xpop[j] + ((Xub[j] - Xlb[j]) * st.next() + Xlb[j]);   // :66
 	o_check_identical(XpopNew.data(), Npop, Nparam, Xlb, Xub, ind.data(), st);                    // :71 (sic: XpopNew)
 	o_check_bounds(Xpop.data(), Npop, Nparam, Xlb, Xub, ind.data(), st);                           // :74
-	for (int i = 0; i < Npop; i++) if (ind[i]) F[i] = o_scalar(fobj, &Xpop[(size_t) i * Nparam], Nparam);   // :77
+	for (int i = 0; i < Npop; i++) if (ind[i]) F[i] = objective(&Xpop[(size_t) i * Nparam]);   // :77
 	double f0 = F[0];                                           // :78
 	o_pop_sort(Xpop.data(), F.data(), Npop, Nparam);            // :81
 
@@ -562,7 +564,7 @@ int oracle_ga(int kind, const double * scalars, const long long * ints, const do
 		}
 		o_check_identical(XpopNew.data(), Npop, Nparam, Xlb, Xub, ind.data(), st);   // :211
 		o_check_bounds(XpopNew.data(), Npop, Nparam, Xlb, Xub, ind.data(), st);      // :214
-		for (int i = 0; i < Npop; i++) if (ind[i]) Fnew[i] = o_scalar(fobj, &XpopNew[(size_t) i * Nparam], Nparam);   // :217
+		for (int i = 0; i < Npop; i++) if (ind[i]) Fnew[i] = objective(&XpopNew[(size_t) i * Nparam]);   // :217
 		o_pop_sort(XpopNew.data(), Fnew.data(), Npop, Nparam);                        // :220
 		for (int i = 0; i < Npop; i++) {                        // :223-230
 			F[i] = Fnew[i];
@@ -582,6 +584,18 @@ int oracle_ga(int kind, const double * scalars, const long long * ints, const do
 	if (F_out) memcpy(F_out, F.data(), (size_t) Npop * sizeof(double));
 	if (stream_pos_out) *stream_pos_out = st.pos;
 	return iter;
+}
+
+int oracle_ga(int kind, const double * scalars, const long long * ints, const double * const * cols, long long m,
+              double * X, const double * Xlb, const double * Xub, int Nparam, int Npop, int maxGenerations, double eliteFrac,
+              double crossFrac, double eliteMutationFrac, double mutationSize, double eliteMutationSize,
+              double NstaticGenerations, int stopAfter, const double * values, uint64_t n_values, uint64_t seed, double scale,
+              double * f0_out, double * fOpt_out, double * Xpop_out, double * F_out, int * cross_idx, int * mut_idx,
+              int * elite_idx, uint64_t * stream_pos_out)
+{
+	return oracle_ga_fn(kind, scalars, ints, cols, m, nullptr, X, Xlb, Xub, Nparam, Npop, maxGenerations, eliteFrac, crossFrac,
+	                    eliteMutationFrac, mutationSize, eliteMutationSize, NstaticGenerations, stopAfter, values, n_values, seed, scale,
+	                    f0_out, fOpt_out, Xpop_out, F_out, cross_idx, mut_idx, elite_idx, stream_pos_out);
 }
 
 } // extern "C"

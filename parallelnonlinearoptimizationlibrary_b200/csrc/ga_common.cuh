@@ -36,7 +36,9 @@ struct StreamDev {
 	}
 };
 
-// order-preserving map of a double onto an unsigned 64-bit key (and back)
+// order-preserving map of a double onto an unsigned 64-bit key (and back). -0 and +0 get the same key: the reference's popSort compares
+// with < (Source/GeneticAlgorithm.cpp:370-412), so the two zeros tie and keep their row order. The key of zero does not tell which zero
+// it was: the sort kernels read that value from F[row] (sorted_value)
 __host__ __device__ __forceinline__ unsigned long long double_to_key(double d)
 {
 #if defined(__CUDA_ARCH__)
@@ -44,12 +46,19 @@ __host__ __device__ __forceinline__ unsigned long long double_to_key(double d)
 #else
 	unsigned long long b; memcpy(&b, &d, 8);
 #endif
+	if (b == 0x8000000000000000ULL) b = 0;
 	return (b >> 63) ? ~b : (b | 0x8000000000000000ULL);
 }
+constexpr unsigned long long kZeroKey = 0x8000000000000000ULL;     // double_to_key(+0.0) == double_to_key(-0.0)
 __device__ __forceinline__ double key_to_double(unsigned long long k)
 {
 	unsigned long long b = (k >> 63) ? (k & 0x7FFFFFFFFFFFFFFFULL) : ~k;
 	return __longlong_as_double((long long) b);
+}
+// the objective value of sorted key k, row r: rebuilt from the key, except a zero, whose sign only F[r] holds
+__device__ __forceinline__ double sorted_value(unsigned long long k, unsigned r, const double * F)
+{
+	return k == kZeroKey ? F[r] : key_to_double(k);
 }
 
 // contribution of gene j (value v) to the order-independent 64-bit row hash of the duplicate check; +0 and -0 compare equal in

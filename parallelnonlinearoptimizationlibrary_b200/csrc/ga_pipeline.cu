@@ -157,20 +157,23 @@ __device__ __forceinline__ unsigned group_sum(unsigned v)
 	return v;
 }
 
-// elite rows (:108-118): child row k = sorted row k, for the rows this rank owns; the row hash travels with the row
+// elite rows (:108-118): child row k = sorted row k, for the rows this rank owns. The row hash is computed from the genes copied: the
+// previous generation's hash of a row predates the duplicate replacement and bounds repair of ga_fix_kernel, which rewrite genes
 __global__ void __launch_bounds__(256)
-ga_elite_copy_kernel(RowTable cur, const unsigned * __restrict__ perm, const unsigned long long * __restrict__ hash_cur, long long lo,
-                     long long hi, int n, double * __restrict__ Xloc, unsigned long long * __restrict__ hash_new,
-                     unsigned * __restrict__ bcount)
+ga_elite_copy_kernel(RowTable cur, const unsigned * __restrict__ perm, long long lo, long long hi, int n, double * __restrict__ Xloc,
+                     unsigned long long * __restrict__ hash_new, unsigned * __restrict__ bcount)
 {
 	const long long row = lo + (((long long) blockIdx.x * blockDim.x + threadIdx.x) / kRowLanes);
 	const int g = threadIdx.x % kRowLanes;
-	if (row >= hi) return;
-	const unsigned from = perm[row];
-	const double * s = cur.row(from);
-	double * d = Xloc + (row - lo) * n;
-	for (int j = g; j < n; j += kRowLanes) d[j] = __ldcg(s + j);
-	if (g == 0) { hash_new[row] = hash_cur[from]; bcount[row] = 0; }
+	const bool live = row < hi;
+	unsigned long long h = 0;
+	if (live) {
+		const double * s = cur.row(perm[row]);
+		double * d = Xloc + (row - lo) * n;
+		for (int j = g; j < n; j += kRowLanes) { const double v = __ldcg(s + j); d[j] = v; h += gene_hash(v, j); }
+	}
+	h = group_sum(h);
+	if (live && g == 0) { hash_new[row] = h; bcount[row] = 0; }
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -980,7 +983,7 @@ ga_sort_kernel(const double * __restrict__ F, long long N, long long range, unsi
 		grid.sync();
 	}
 	// sorted objective values and the permutation sorted position -> row
-	for (long long i = lo + tid; i < hi; i += kSortThreads) { Fsorted[i] = key_to_double(kin[i]); perm_out[i] = vin[i]; }
+	for (long long i = lo + tid; i < hi; i += kSortThreads) { const unsigned r = vin[i]; Fsorted[i] = sorted_value(kin[i], r, F); perm_out[i] = r; }
 	if (cta == 0 && tid == 0) S->sort_result_in_alt = (kin != keys0);
 }
 
@@ -1106,8 +1109,8 @@ ga_bsort_scatter_kernel(const double * __restrict__ F, long long N, const unsign
 // good children of a generation pile up below the old 10 % mark). Every CTA looks at its bucket's size and leaves if it is not its.
 template <int kThreads, int kPer>
 __global__ void __launch_bounds__(kThreads)
-ga_bsort_bucket_kernel(const unsigned long long * __restrict__ keys, const unsigned * __restrict__ vals, const unsigned * __restrict__ bstart,
-                       const GaDevStatus * __restrict__ S, double * __restrict__ Fsorted, unsigned * __restrict__ perm_out, unsigned min_cnt,
+ga_bsort_bucket_kernel(const double * __restrict__ F, const unsigned long long * __restrict__ keys, const unsigned * __restrict__ vals,
+                       const unsigned * __restrict__ bstart, const GaDevStatus * __restrict__ S, double * __restrict__ Fsorted, unsigned * __restrict__ perm_out, unsigned min_cnt,
                        const unsigned * __restrict__ list /* nullptr: bucket = blockIdx.x; else [0] = count, buckets follow */)
 {
 	constexpr int kCap = kThreads * kPer;
@@ -1194,7 +1197,7 @@ ga_bsort_bucket_kernel(const unsigned long long * __restrict__ keys, const unsig
 				const unsigned long long kj = sk[j];
 				smaller += (kj < k[q] || (kj == k[q] && sv[j] < v[q])) ? 1u : 0u;
 			}
-			Fsorted[b0 + s0 + smaller] = key_to_double(k[q]);
+			Fsorted[b0 + s0 + smaller] = sorted_value(k[q], v[q], F);
 			perm_out[b0 + s0 + smaller] = v[q];
 		}
 	}
@@ -1517,8 +1520,6 @@ int ga_pipe_reset(pnol_ga * ga)
 		PNOL_CUDA(ctx, cudaMemcpyAsync(P->XL[0], ga->Xpop + P->lo * n, (size_t) (P->hi - P->lo) * n * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
 	PNOL_CUDA(ctx, cudaMemcpyAsync(P->Fs[0], ga->F, (size_t) Npop * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
 	PNOL_LAUNCH(ctx, ga_iota_kernel, blocks_for(Npop, 256), 256, 0, P->perm[0], Npop);
-	// hashes of all rows (the full sorted population is at hand on every rank right now)
-	PNOL_LAUNCH(ctx, ga_rows_hash_kernel, blocks_for(Npop * kRowLanes, 256), 256, 0, ga->Xpop, 0LL, 0LL, Npop, n, P->hash[0], (unsigned *) nullptr);
 	PNOL_CHECK(pipe_refresh_replica(ga, 0));
 	P->elite_idx_complete = true;
 	return PNOL_OK;
@@ -1559,7 +1560,7 @@ static int pipe_enqueue(pnol_ga * ga, double window_scale)
 		            (unsigned long long) ga->pos);
 		long long a, b;
 		clampr(0, Nelite, a, b);
-		if (b > a) PNOL_LAUNCH(ctx, ga_elite_copy_kernel, blocks_for((b - a) * kRowLanes, 256), 256, 0, T, P->perm[cur], P->hash[cur], a, b, n,
+		if (b > a) PNOL_LAUNCH(ctx, ga_elite_copy_kernel, blocks_for((b - a) * kRowLanes, 256), 256, 0, T, P->perm[cur], a, b, n,
 		                       Xloc + (a - lo) * n, P->hash[nxt], P->bcount);
 	}
 	// 1. crossover
@@ -1716,10 +1717,10 @@ static int pipe_enqueue(pnol_ga * ga, double window_scale)
 			PNOL_LAUNCH(ctx, ga_bsort_count_kernel, P->bs_grid, kBsCountThreads, kBsBuckets * 12, Fc, N, (const double *) P->Fs[cur], P->bs_tag, P->bs_totals);
 			PNOL_LAUNCH(ctx, ga_bsort_scan_kernel, 1, 1024, 0, P->bs_totals, P->bs_start, P->bs_cursor, S, P->bs_large);
 			PNOL_LAUNCH(ctx, ga_bsort_scatter_kernel, P->bs_grid, kBsCountThreads, 0, Fc, N, (const unsigned *) P->bs_tag, P->bs_cursor, k0, v0);
-			PNOL_LAUNCH(ctx, (ga_bsort_bucket_kernel<128, 8>), kBsBuckets, 128, bsort_bucket_smem(kBsCap), (const unsigned long long *) k0, (const unsigned *) v0,
+			PNOL_LAUNCH(ctx, (ga_bsort_bucket_kernel<128, 8>), kBsBuckets, 128, bsort_bucket_smem(kBsCap), Fc, (const unsigned long long *) k0, (const unsigned *) v0,
 			            (const unsigned *) P->bs_start, (const GaDevStatus *) S, Fo, po, 0u, (const unsigned *) nullptr);
 			// the large buckets from the list the scan kernel made (4096 CTAs of 131 KB that only look and leave took 20 us)
-			PNOL_LAUNCH(ctx, (ga_bsort_bucket_kernel<512, 16>), ctx->sm_count, 512, bsort_bucket_smem(kBsCapLarge), (const unsigned long long *) k0, (const unsigned *) v0,
+			PNOL_LAUNCH(ctx, (ga_bsort_bucket_kernel<512, 16>), ctx->sm_count, 512, bsort_bucket_smem(kBsCapLarge), Fc, (const unsigned long long *) k0, (const unsigned *) v0,
 			            (const unsigned *) P->bs_start, (const GaDevStatus *) S, Fo, po, (unsigned) kBsCap, (const unsigned *) P->bs_large);
 		}
 		void * args[] = {(void *) &Fc, (void *) &N, (void *) &range, (void *) &k0, (void *) &v0, (void *) &k1, (void *) &v1, (void *) &sc, (void *) &S,
