@@ -409,7 +409,10 @@ int pnol_ga_get_population(pnol_ga * ga, double * xpop, double * F);
  * (n_elite_mut x n); any may be NULL. These are the "selection/crossover indices" of the parity bar. */
 int pnol_ga_get_indices(pnol_ga * ga, int * cross_idx, int * mut_idx, int * elite_idx);
 
-/* stand-alone GA stages on caller data (per-stage parity at full size) */
+/* stand-alone GA stages on caller data (per-stage parity at full size). The check functions set indicator[i] = 1 for every row
+ * they modify and leave the other entries as passed (indicator may be NULL), and advance *stream_pos by the draws they take.
+ * Limits: npop <= 2^32 for pnol_ga_pop_sort, npop <= 2^24 for pnol_ga_check_identical, npop * n < 2^40 for pnol_ga_check_bounds;
+ * larger calls return PNOL_ERR_INVALID. */
 int pnol_ga_pop_sort(pnol_ctx * ctx, double * xpop, double * F, long long npop, int n);             /* GeneticAlgorithm.cpp:370-412 */
 int pnol_ga_check_bounds(pnol_ctx * ctx, double * xpop, long long npop, int n, const double * xlb, const double * xub,
                          unsigned char * indicator, const pnol_stream_desc * stream, uint64_t * stream_pos); /* :347-365 */

@@ -520,21 +520,23 @@ class Context:
         self.check(self.lib.pnol_ga_pop_sort(self.h, _ptr(xpop), _ptr(F), C.c_longlong(xpop.shape[0]), int(xpop.shape[1])))
         return xpop, F
 
-    def _ga_stage(self, fn, xpop, lb, ub, stream, pos):
+    def _ga_stage(self, fn, xpop, lb, ub, stream, pos, ind):
         xpop = _f64(xpop).copy()
         lb, ub = _f64(lb), _f64(ub)
-        ind = np.zeros(xpop.shape[0], dtype=np.uint8)
+        ind = np.zeros(xpop.shape[0], dtype=np.uint8) if ind is None else np.array(ind, dtype=np.uint8)
         sd, keep = self._stream_desc(stream)
         p = C.c_uint64(pos)
         self.check(fn(self.h, _ptr(xpop), C.c_longlong(xpop.shape[0]), int(xpop.shape[1]), _ptr(lb), _ptr(ub), _ptr(ind), C.byref(sd),
                       C.byref(p)))
         return xpop, ind, int(p.value)
 
-    def ga_check_bounds(self, xpop, lb, ub, stream, pos=0):
-        return self._ga_stage(self.lib.pnol_ga_check_bounds, xpop, lb, ub, stream, pos)
+    def ga_check_bounds(self, xpop, lb, ub, stream, pos=0, ind=None):
+        """-> (population, evaluation flags, stream position). The flags start as ind (zeros when None); repaired rows are set to 1."""
+        return self._ga_stage(self.lib.pnol_ga_check_bounds, xpop, lb, ub, stream, pos, ind)
 
-    def ga_check_identical(self, xpop, lb, ub, stream, pos=0):
-        return self._ga_stage(self.lib.pnol_ga_check_identical, xpop, lb, ub, stream, pos)
+    def ga_check_identical(self, xpop, lb, ub, stream, pos=0, ind=None):
+        """-> (population, evaluation flags, stream position). The flags start as ind (zeros when None); replaced rows are set to 1."""
+        return self._ga_stage(self.lib.pnol_ga_check_identical, xpop, lb, ub, stream, pos, ind)
 
 
 class GA:

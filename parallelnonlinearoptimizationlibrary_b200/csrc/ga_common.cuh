@@ -1,5 +1,5 @@
-// ga_common.cuh -- pieces shared by the genetic-algorithm translation units (ga.cu: state object, initial population and
-// stand-alone stages; ga_pipeline.cu: the fused, sync-free generation).
+// ga_common.cuh -- pieces shared by the genetic-algorithm translation units (ga.cu: the C-ABI layer and the start population;
+// ga_pipeline.cu: the generation's kernels and stages, which pnol_ga_init and the stand-alone stages run too).
 #pragma once
 
 #include "common.cuh"
@@ -14,13 +14,11 @@ struct StreamDev {
 	unsigned long long n_values;
 	unsigned long long seed;
 	double scale;
-	int * exhausted;            // set to 1 when an explicit stream is read past its end
+	// A read past the end of an explicit stream gives 0.0: kernels read speculatively (trial windows), and the host decides
+	// exhaustion from the draws the sequential algorithm consumed
 	__device__ __forceinline__ double u(unsigned long long k) const
 	{
-		if (values) {
-			if (k >= n_values) { if (exhausted) *exhausted = 1; return 0.0; }    // exhausted == nullptr: speculative reads (ga_pipeline.cu)
-			return values[k];
-		}
+		if (values) return k < n_values ? values[k] : 0.0;
 		return from_state(state(k));
 	}
 	// counter mode in two steps, for loops over equally spaced positions: state(k + d) = state(k) + d * kGamma saves the 64-bit
@@ -90,46 +88,6 @@ struct RowTable {
 	}
 };
 
-constexpr int kScanTile = 2048;      // elements per block of the three-kernel prefix sum (256 threads x 8)
-constexpr int kSortTile = 2048;      // keys per block of the radix sort of ga.cu's stages: 8 warps x 8 rounds x 32 lanes
-constexpr int kSortWarps = 8;
-
-struct SortScratch {
-	unsigned long long * keys_alt;
-	unsigned * vals_alt;
-	unsigned * counts;              // [8][256][nblocks]
-	unsigned long long * offsets;   // [256][nblocks]
-	unsigned long long * scan_tmp;
-	int * skip;                     // [8]
-	static size_t bytes(long long n)
-	{
-		long long nb = (n + kSortTile - 1) / kSortTile;
-		if (nb < 1) nb = 1;
-		size_t s = 0;
-		s += (size_t) n * 8 + 256;                 // keys_alt
-		s += (size_t) n * 4 + 256;                 // vals_alt
-		s += (size_t) 8 * 256 * nb * 4 + 256;      // counts
-		s += (size_t) 256 * nb * 8 + 256;          // offsets
-		s += (size_t) ((256 * nb + kScanTile - 1) / kScanTile + 1) * 8 + 256;
-		s += 256;
-		return s;
-	}
-	void carve(void * base, long long n)
-	{
-		long long nb = (n + kSortTile - 1) / kSortTile;
-		if (nb < 1) nb = 1;
-		unsigned char * p = (unsigned char *) base;
-		auto take = [&](size_t b) { void * r = p; p += (b + 255) & ~(size_t) 255; return r; };
-		keys_alt = (unsigned long long *) take((size_t) n * 8);
-		vals_alt = (unsigned *) take((size_t) n * 4);
-		counts = (unsigned *) take((size_t) 8 * 256 * nb * 4);
-		offsets = (unsigned long long *) take((size_t) 256 * nb * 8);
-		scan_tmp = (unsigned long long *) take((size_t) ((256 * nb + kScanTile - 1) / kScanTile + 1) * 8);
-		skip = (int *) take(64);
-	}
-};
-
-
 } // namespace pnol
 
 // state object of the C-ABI (pnol_ga_create ... pnol_ga_destroy)
@@ -140,17 +98,11 @@ struct pnol_ga {
 	int n;
 	int nelite, nelmut, ncross, nrand;
 	// device state
-	double * Xpop, * Xnew, * F, * Fnew, * fitness, * lb, * ub, * x0;
-	unsigned char * indicator;
+	double * Xnew;                       // Npop x n, replicated: pnol_ga_init's start population, pnol_ga_get_population's staging
+	double * fitness, * lb, * ub, * x0;
 	int * cross_idx, * mut_idx, * elite_idx;
 	long long * mut_pos;
 	double * stream_values;
-	int * exhausted;
-	// scratch
-	void * sort_mem; pnol::SortScratch sort;
-	unsigned long long * keys; unsigned * perm;
-	unsigned * u32a; unsigned long long * u64a; unsigned long long * scan_tmp; unsigned long long * total_dev;
-	double * gather = nullptr;           // all-gather buffer of the sharded fitness sweep (multi-GPU)
 	// host state
 	pnol_stream_desc stream;
 	uint64_t pos;
@@ -163,14 +115,25 @@ struct pnol_ga {
 
 
 namespace pnol {
+// the GA's random stream as the kernels read it
+inline StreamDev ga_stream(const pnol_ga * ga)
+{
+	StreamDev st;
+	st.values = ga->stream_values; st.n_values = ga->stream.n_values; st.seed = ga->stream.seed; st.scale = ga->stream.scale;
+	return st;
+}
 // ga_pipeline.cu
-int ga_pipe_create(pnol_ga * ga);                 // allocates the pipeline state (after the buffers of pnol_ga_init exist)
+int ga_pipe_create(pnol_ga * ga);
 void ga_pipe_destroy(pnol_ga * ga);
-int ga_pipe_reset(pnol_ga * ga);                  // after pnol_ga_init: sorted population -> pipeline representation
+int ga_pipe_init(pnol_ga * ga, double * f0_out);  // pnol_ga_init after the start population is in ga->Xnew (see there)
 int ga_pipe_generation(pnol_ga * ga);
 int ga_pipe_get_population(pnol_ga * ga, double * xpop, double * F);
 int ga_pipe_get_indices(pnol_ga * ga, int * cross_idx, int * mut_idx, int * elite_idx);
 int ga_pipe_peer_mode(pnol_ga * ga);
+// stand-alone stages on device arrays (pnol_ga_pop_sort, pnol_ga_check_identical, pnol_ga_check_bounds)
+int ga_stage_pop_sort(pnol_ctx * ctx, double * X, double * F, long long npop, int n);
+int ga_stage_repair(pnol_ctx * ctx, bool identical, double * X, long long npop, int n, const double * lb, const double * ub,
+                    unsigned char * indicator, const StreamDev & st, unsigned long long pos, unsigned long long * pos_end);
 // comm.cu
 int comm_allgather_bytes_dev(pnol_ctx * ctx, const void * send, void * recv, size_t bytes_per_rank);
 }

@@ -1,7 +1,9 @@
 // ga_pipeline.cu -- one generation of GeneticAlgorithmMPI::findMinBnd (Source/GeneticAlgorithmMPI.cpp:87-249) as a fused,
 // sync-free kernel pipeline: every stage reads the stream position it starts from out of a status block in device memory, so the
 // host enqueues the whole generation and synchronises ONCE at its end to read that block (stream position, best objective, error
-// bits). Bit-exact with the oracle (tests/test_gpu_ga.py).
+// bits). Bit-exact with the oracle (tests/test_gpu_ga.py). The population stages 4 - 7 are host functions over plain buffer views
+// (StageBufs): pnol_ga_init (a generation whose children are the start population, ga_pipe_init) and the stand-alone popSort /
+// duplicate / bounds calls (ga_stage_pop_sort, ga_stage_repair) run the same launch sequences.
 //
 // What changed against the stage-by-stage generation of round 1 (2.25 ms at 1M x 32, ~105 launches, 8 host round trips):
 //   * the population is never physically sorted. Rows stay where the generation that made them wrote them ("child order");
@@ -346,21 +348,29 @@ ga_cross_kernel(StreamDev st, GaDevStatus * __restrict__ S, const double * __res
 	if (cta == 0 && tid == 0) atomicOr(&S->error, kGaErrCrossWindow);
 }
 
-// row hash (and a zero box count: every gene of a crossover child is a parent's gene, which is inside the box) of rows [lo, hi)
+// row hash and out-of-box gene count of rows [lo, hi). Without lb / ub the count is zero: every gene of a crossover child is a
+// parent's gene, which is inside the box
 __global__ void __launch_bounds__(256)
-ga_rows_hash_kernel(const double * __restrict__ Xloc, long long own_lo, long long lo, long long hi, int n,
-                    unsigned long long * __restrict__ hash_new, unsigned * __restrict__ bcount)
+ga_rows_hash_kernel(const double * __restrict__ Xloc, long long own_lo, long long lo, long long hi, int n, const double * __restrict__ lb,
+                    const double * __restrict__ ub, unsigned long long * __restrict__ hash_new, unsigned * __restrict__ bcount)
 {
 	const long long row = lo + (((long long) blockIdx.x * blockDim.x + threadIdx.x) / kRowLanes);
 	const int g = threadIdx.x % kRowLanes;
 	const bool live = row < hi;
 	unsigned long long h = 0;
+	unsigned oob = 0;
 	if (live) {
 		const double * x = Xloc + (row - own_lo) * n;
-		for (int j = g; j < n; j += kRowLanes) h += gene_hash(x[j], j);
+		if (!lb) {
+			for (int j = g; j < n; j += kRowLanes) h += gene_hash(x[j], j);
+		} else {
+#pragma unroll 1      // (stand-alone stages and pnol_ga_init only; unrolled, the kernel took 38 registers instead of 32)
+			for (int j = g; j < n; j += kRowLanes) { const double v = x[j]; h += gene_hash(v, j); oob += (v > ub[j] || v < lb[j]) ? 1u : 0u; }
+		}
 	}
 	h = group_sum(h);
-	if (live && g == 0) { hash_new[row] = h; if (bcount) bcount[row] = 0; }
+	if (lb) oob = group_sum(oob);
+	if (live && g == 0) { hash_new[row] = h; bcount[row] = oob; }
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -806,7 +816,8 @@ __global__ void __launch_bounds__(256)
 ga_fix_kernel(StreamDev st, const GaDevStatus * __restrict__ S, long long own_lo, long long own_hi, int n, int Nelite,
               long long NeliteMutGenes, const double * __restrict__ lb, const double * __restrict__ ub,
               const unsigned char * __restrict__ dupflag, const unsigned * __restrict__ bcount,
-              const unsigned long long * __restrict__ offs, double * __restrict__ Xloc, unsigned char * __restrict__ indicator)
+              const unsigned long long * __restrict__ offs, double * __restrict__ Xloc, unsigned char * __restrict__ indicator,
+              int mark_modified)
 {
 	if (S->error) return;
 	const long long row = own_lo + (((long long) blockIdx.x * blockDim.x + threadIdx.x) / kRowLanes);
@@ -814,8 +825,13 @@ ga_fix_kernel(StreamDev st, const GaDevStatus * __restrict__ S, long long own_lo
 	const bool live = row < own_hi;
 	const bool dup = live && dupflag[row] != 0;
 	const unsigned cnt = live ? bcount[row] : 0;
-	if (live && g == 0) indicator[row - own_lo] = (row >= Nelite || dup) ? 1 : 0;      // elites keep their value unless replaced (:116, :220)
 	const bool work = dup || cnt != 0;
+	// evaluation flags. A generation writes every row: elites keep their value unless replaced (:116, :220). A stand-alone stage
+	// (mark_modified) sets the rows it modifies and leaves the others as the caller passed them
+	if (live && g == 0) {
+		if (!mark_modified) indicator[row - own_lo] = (row >= Nelite || dup) ? 1 : 0;
+		else if (work) indicator[row - own_lo] = 1;
+	}
 	if (!__any_sync(0xffffffffu, work)) return;
 	const unsigned long long P3 = S->pos_elite + 2ULL * (unsigned long long) NeliteMutGenes;       // after the elite mutations
 	const unsigned long long o = work ? offs[row] : 0;
@@ -1232,12 +1248,6 @@ ga_gather_sorted_kernel(RowTable cur, const unsigned * __restrict__ perm, long l
 	for (int j = g; j < n; j += kRowLanes) d[j] = __ldcg(s + j);
 }
 
-__global__ void ga_iota_kernel(unsigned * __restrict__ perm, long long n)
-{
-	const long long i = (long long) blockIdx.x * blockDim.x + threadIdx.x;
-	if (i < n) perm[i] = (unsigned) i;
-}
-
 } // namespace pnol
 
 using namespace pnol;
@@ -1245,6 +1255,26 @@ using namespace pnol;
 // ---------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------
+// The buffers of the population stages 4 (identical children), 5 (stream offsets, replacement and repair) and 7 (popSort): the
+// generation's, or a stand-alone call's, sized by its npop. Per row in row order: hash, bcount, dupflag, offs
+struct StageBufs {
+	GaDevStatus * S = nullptr;
+	unsigned long long * hash = nullptr;
+	unsigned * bcount = nullptr;                                       // out-of-box genes
+	unsigned char * dupflag = nullptr;
+	unsigned long long * offs = nullptr, * block_sums = nullptr;        // packed stream offsets, their per-tile sums
+	unsigned * suspects = nullptr;                                     // rows the duplicate query leaves to ga_dup_resolve_kernel
+	unsigned long long * tkeys = nullptr; unsigned * tmax = nullptr; unsigned tmask = 0;      // duplicate table of tmask + 1 slots
+	unsigned long long * skeys[2] = {nullptr, nullptr}; unsigned * svals[2] = {nullptr, nullptr}; unsigned * scounts = nullptr;
+	int sort_grid = 0; long long sort_range = 0;                       // radix kernel: cooperative grid, keys per CTA
+};
+
+// the bucket sort in front of the radix kernel at large Npop (generations only: it needs the previous sorted values)
+struct BucketBufs {
+	unsigned * tag = nullptr, * totals = nullptr, * start = nullptr, * cursor = nullptr, * large = nullptr;
+	int grid = 0;
+};
+
 struct GaPipe {
 	// population rows of THIS rank, double-buffered: XL[cur] holds rows [lo, hi) of the current population in child order
 	double * XL[2] = {nullptr, nullptr};
@@ -1257,15 +1287,13 @@ struct GaPipe {
 	int R = 1;                                        // row partitions: the communicator's ranks (rows sharded) or 1 (rows replicated, sweep sharded)
 	long long eper = 0;                               // rows replicated: rows of the fitness sweep per rank
 	bool shard_sweep = true;                          // rows replicated: split the sweep and all-gather F (false: every rank sweeps everything)
-	// replicated per-row arrays (sorted order: Fs, ratio, perm; child order: hash, bcount, dupflag, Fchild, offs)
+	// replicated per-row arrays (sorted order: Fs, ratio, perm; child order: hash, Fchild and the stage buffers)
 	unsigned * perm[2] = {nullptr, nullptr};
 	double * Fs[2] = {nullptr, nullptr};
 	unsigned long long * hash[2] = {nullptr, nullptr};
 	double * ratio = nullptr, * Fchild = nullptr;
-	unsigned * bcount = nullptr;
-	unsigned char * dupflag = nullptr, * indicator = nullptr;
-	unsigned long long * offs = nullptr, * block_sums = nullptr;
-	unsigned * suspects = nullptr;
+	unsigned char * indicator = nullptr;
+	StageBufs B;                                      // B.hash is hash[] of the population being made
 	// gather staging (several ranks): [hash (8) | bcount (4)] per row, per rank slots
 	unsigned char * hb_send = nullptr, * hb_recv = nullptr;
 	double * f_recv = nullptr;
@@ -1273,14 +1301,10 @@ struct GaPipe {
 	unsigned long long * cross_counts = nullptr; int cross_grid = 0;
 	// mutation
 	void * mut_mem = nullptr; size_t mut_bytes = 0;
-	// duplicate table
-	unsigned long long * tkeys = nullptr; unsigned * tmax = nullptr; unsigned tmask = 0;
 	// sort
-	unsigned long long * skeys[2] = {nullptr, nullptr}; unsigned * svals[2] = {nullptr, nullptr}; unsigned * scounts = nullptr;
-	int sort_grid = 0; long long sort_range = 0;
-	unsigned * bs_tag = nullptr, * bs_totals = nullptr, * bs_start = nullptr, * bs_cursor = nullptr, * bs_large = nullptr; bool bs_on = false; int bs_grid = 0;
+	BucketBufs bs; bool bs_on = false;
 	// status
-	GaDevStatus * status = nullptr; GaDevStatus * status_host = nullptr;
+	GaDevStatus * status_host = nullptr;
 	unsigned long long pos_elite_last = 0;           // start of the last generation's elite-mutation stage (for get_indices)
 	bool elite_idx_complete = true;
 	double accept_rate = 0.25;
@@ -1289,24 +1313,68 @@ struct GaPipe {
 
 namespace {
 
-template <class T> int pipe_alloc(pnol_ga * ga, T ** p, size_t count)
+// device memory freed with the list that owns it (GaPipe::owned, CallMem::owned)
+template <class T> int owned_alloc(pnol_ctx * ctx, std::vector<void *> & owned, T ** p, size_t count)
 {
 	void * d = nullptr;
-	PNOL_CUDA(ga->ctx, cudaMalloc(&d, (count ? count : 1) * sizeof(T)));
-	ga->pipe->owned.push_back(d);
+	PNOL_CUDA(ctx, cudaMalloc(&d, (count ? count : 1) * sizeof(T)));
+	owned.push_back(d);
 	*p = (T *) d;
 	return PNOL_OK;
 }
+template <class T> int pipe_alloc(pnol_ga * ga, T ** p, size_t count) { return owned_alloc(ga->ctx, ga->pipe->owned, p, count); }
 
-StreamDev pipe_stream(pnol_ga * ga)
-{
-	StreamDev st;
-	st.values = ga->stream_values; st.n_values = ga->stream.n_values; st.seed = ga->stream.seed; st.scale = ga->stream.scale;
-	st.exhausted = nullptr;            // speculative reads past the end are fine; ga_finish_kernel decides exhaustion
-	return st;
-}
+// device memory of one stand-alone call, freed when the call returns
+struct CallMem {
+	pnol_ctx * ctx;
+	std::vector<void *> owned;
+	explicit CallMem(pnol_ctx * c) : ctx(c) {}
+	~CallMem() { cudaStreamSynchronize(ctx->stream); for (void * p : owned) cudaFree(p); }
+	template <class T> int operator()(T ** p, size_t count) { return owned_alloc(ctx, owned, p, count); }
+};
 
 unsigned blocks_for(long long threads, int per_block) { return (unsigned) std::max<long long>(1, (threads + per_block - 1) / per_block); }
+
+// duplicate table: at least 2 slots per row, power of two
+unsigned dup_table_slots(long long Npop)
+{
+	unsigned slots = 1024;
+	while ((long long) slots < 2 * Npop) slots <<= 1;
+	return slots;
+}
+
+// radix sort of N keys: one CTA per SM at most (cooperative launch), contiguous ranges that are multiples of the ranking chunk
+int sort_geometry(pnol_ctx * ctx, long long N, StageBufs & B)
+{
+	int per_sm = 0;
+	PNOL_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ga_sort_kernel, kSortThreads, 0));
+	PNOL_REQUIRE(ctx, per_sm >= 1, "ga: the sort kernel does not fit an SM");
+	const int maxg = ctx->sm_count * per_sm;
+	long long range = (N + maxg - 1) / maxg;
+	range = (range + kSortChunk - 1) / kSortChunk * kSortChunk;
+	B.sort_range = range;
+	B.sort_grid = (int) ((N + range - 1) / range);
+	return PNOL_OK;
+}
+
+// status of stages run outside a generation: no error, draws from pos on, no suspects, the radix kernel sorts
+int status_reset(pnol_ctx * ctx, GaDevStatus * S, unsigned long long pos)
+{
+	GaDevStatus h = {};
+	h.pos_elite = pos;
+	h.sort_fallback = 1;
+	PNOL_CUDA(ctx, cudaMemcpyAsync(S, &h, sizeof h, cudaMemcpyHostToDevice, ctx->stream));
+	return PNOL_OK;
+}
+
+// a population whose rows all lie in one array
+RowTable one_table(const double * X, long long npop, int n)
+{
+	RowTable T;
+	for (int r = 0; r < kGaMaxRanks; r++) T.base[r] = nullptr;
+	T.base[0] = X; T.per = npop; T.n = n; T.nranks = 1;
+	return T;
+}
 
 // peer mappings of the ranks' row blocks (CUDA IPC over NVLink); false when any step fails (the caller falls back to replicas)
 bool pipe_open_peers(pnol_ga * ga)
@@ -1410,21 +1478,21 @@ int ga_pipe_create(pnol_ga * ga)
 		PNOL_CHECK(pipe_alloc(ga, &P->perm[b], (size_t) Npop));
 		PNOL_CHECK(pipe_alloc(ga, &P->Fs[b], (size_t) Npop));
 		PNOL_CHECK(pipe_alloc(ga, &P->hash[b], (size_t) P->per * R));
-		PNOL_CHECK(pipe_alloc(ga, &P->skeys[b], (size_t) Npop));
-		PNOL_CHECK(pipe_alloc(ga, &P->svals[b], (size_t) Npop));
+		PNOL_CHECK(pipe_alloc(ga, &P->B.skeys[b], (size_t) Npop));
+		PNOL_CHECK(pipe_alloc(ga, &P->B.svals[b], (size_t) Npop));
 		P->table[b].per = P->per; P->table[b].n = n; P->table[b].nranks = R;
 		for (int r = 0; r < kGaMaxRanks; r++) P->table[b].base[r] = nullptr;
 		P->table[b].base[0] = P->XL[b];
 	}
 	PNOL_CHECK(pipe_alloc(ga, &P->ratio, (size_t) Npop + kAccBuckets / 2 + 2));      // + the acceptance thresholds K[0 .. kAccBuckets] (pipe_accept)
 	PNOL_CHECK(pipe_alloc(ga, &P->Fchild, std::max((size_t) P->per * R, (size_t) P->eper * ctx->nranks)));
-	PNOL_CHECK(pipe_alloc(ga, &P->bcount, (size_t) P->per * R));
-	PNOL_CHECK(pipe_alloc(ga, &P->dupflag, (size_t) Npop));
 	PNOL_CHECK(pipe_alloc(ga, &P->indicator, (size_t) P->per));
-	PNOL_CHECK(pipe_alloc(ga, &P->offs, (size_t) Npop));
-	PNOL_CHECK(pipe_alloc(ga, &P->block_sums, (size_t) (Npop + kPackTile - 1) / kPackTile + 1));
-	PNOL_CHECK(pipe_alloc(ga, &P->suspects, (size_t) Npop));
-	PNOL_CHECK(pipe_alloc(ga, &P->status, 1));
+	PNOL_CHECK(pipe_alloc(ga, &P->B.bcount, (size_t) P->per * R));
+	PNOL_CHECK(pipe_alloc(ga, &P->B.dupflag, (size_t) Npop));
+	PNOL_CHECK(pipe_alloc(ga, &P->B.offs, (size_t) Npop));
+	PNOL_CHECK(pipe_alloc(ga, &P->B.block_sums, (size_t) (Npop + kPackTile - 1) / kPackTile + 1));
+	PNOL_CHECK(pipe_alloc(ga, &P->B.suspects, (size_t) Npop));
+	PNOL_CHECK(pipe_alloc(ga, &P->B.S, 1));
 	PNOL_CUDA(ctx, cudaMallocHost((void **) &P->status_host, sizeof(GaDevStatus)));
 	// crossover: cooperative grid (all CTAs resident), one count per CTA
 	{
@@ -1436,37 +1504,27 @@ int ga_pipe_create(pnol_ga * ga)
 		P->cross_grid = ctx->sm_count * std::min(per_sm, 4);
 		PNOL_CHECK(pipe_alloc(ga, &P->cross_counts, (size_t) P->cross_grid));
 	}
-	// duplicate table: at least 2 slots per row, power of two
 	{
-		unsigned slots = 1024;
-		while ((long long) slots < 2 * Npop) slots <<= 1;
-		P->tmask = slots - 1;
-		PNOL_CHECK(pipe_alloc(ga, &P->tkeys, (size_t) slots));
-		PNOL_CHECK(pipe_alloc(ga, &P->tmax, (size_t) slots));
+		const unsigned slots = dup_table_slots(Npop);
+		P->B.tmask = slots - 1;
+		PNOL_CHECK(pipe_alloc(ga, &P->B.tkeys, (size_t) slots));
+		PNOL_CHECK(pipe_alloc(ga, &P->B.tmax, (size_t) slots));
 	}
-	// sort: one CTA per SM at most (cooperative launch), contiguous ranges that are multiples of the ranking chunk
 	{
-		int per_sm = 0;
-		PNOL_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ga_sort_kernel, kSortThreads, 0));
-		PNOL_REQUIRE(ctx, per_sm >= 1, "ga: the sort kernel does not fit an SM");
-		const int maxg = ctx->sm_count * per_sm;
-		long long range = (Npop + maxg - 1) / maxg;
-		range = (range + kSortChunk - 1) / kSortChunk * kSortChunk;
-		P->sort_range = range;
-		P->sort_grid = (int) ((Npop + range - 1) / range);
-		PNOL_CHECK(pipe_alloc(ga, &P->scounts, (size_t) 256 * P->sort_grid));
+		PNOL_CHECK(sort_geometry(ctx, Npop, P->B));
+		PNOL_CHECK(pipe_alloc(ga, &P->B.scounts, (size_t) 256 * P->B.sort_grid));
 		// bucket sort in front of it at large Npop (PNOL_GA_SORT=radix: radix kernel only -- A/B runs and the equivalence test)
 		const char * sort_env = getenv("PNOL_GA_SORT");              // read per pnol_ga_create
 		const bool radix_only = sort_env && strcmp(sort_env, "radix") == 0;
 		P->bs_on = !radix_only && Npop >= 65536;
 		if (P->bs_on) {
-			P->bs_grid = 2 * ctx->sm_count;                          // two 1024-thread CTAs per SM (count: 48 KB, scatter: 16 KB of shared memory)
-			PNOL_CHECK(pipe_alloc(ga, &P->bs_tag, (size_t) Npop));
-			PNOL_CHECK(pipe_alloc(ga, &P->bs_totals, (size_t) kBsBuckets));
-			PNOL_CHECK(pipe_alloc(ga, &P->bs_start, (size_t) kBsBuckets + 1));
-			PNOL_CHECK(pipe_alloc(ga, &P->bs_cursor, (size_t) kBsBuckets));
-			PNOL_CHECK(pipe_alloc(ga, &P->bs_large, (size_t) kBsBuckets + 1));
-			PNOL_CUDA(ctx, cudaMemsetAsync(P->bs_totals, 0, kBsBuckets * sizeof(unsigned), ctx->stream));
+			P->bs.grid = 2 * ctx->sm_count;                          // two 1024-thread CTAs per SM (count: 48 KB, scatter: 16 KB of shared memory)
+			PNOL_CHECK(pipe_alloc(ga, &P->bs.tag, (size_t) Npop));
+			PNOL_CHECK(pipe_alloc(ga, &P->bs.totals, (size_t) kBsBuckets));
+			PNOL_CHECK(pipe_alloc(ga, &P->bs.start, (size_t) kBsBuckets + 1));
+			PNOL_CHECK(pipe_alloc(ga, &P->bs.cursor, (size_t) kBsBuckets));
+			PNOL_CHECK(pipe_alloc(ga, &P->bs.large, (size_t) kBsBuckets + 1));
+			PNOL_CUDA(ctx, cudaMemsetAsync(P->bs.totals, 0, kBsBuckets * sizeof(unsigned), ctx->stream));
 			PNOL_CUDA(ctx, cudaFuncSetAttribute(ga_bsort_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kBsBuckets * 12));
 			PNOL_CUDA(ctx, cudaFuncSetAttribute(ga_bsort_bucket_kernel<512, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bsort_bucket_smem(kBsCapLarge)));
 		}
@@ -1508,20 +1566,186 @@ static int pipe_refresh_replica(pnol_ga * ga, int b)
 	return comm_allgather_dev(ga->ctx, P->XL[b], P->replica[b], (size_t) P->per * ga->n);
 }
 
-// after pnol_ga_init: ga->Xpop / ga->F hold the sorted start population (replicated). Rows -> this rank's block, perm = identity.
-int ga_pipe_reset(pnol_ga * ga)
+// ---- the population stages. A generation runs them on its child rows; pnol_ga_init and the stand-alone calls run the same ones ----
+
+// 4. identical children: dupflag of rows [0, Npop) of X from their hashes (B.hash). S->nsuspect must be 0
+static int stage_identical(pnol_ctx * ctx, const StageBufs & B, long long Npop, const RowTable & X, int n)
+{
+	TimerScope ts(ctx, "ga_check_identical");
+	PNOL_CUDA(ctx, cudaMemsetAsync(B.tkeys, 0, ((size_t) B.tmask + 1) * 8, ctx->stream));
+	PNOL_CUDA(ctx, cudaMemsetAsync(B.tmax, 0, ((size_t) B.tmask + 1) * 4, ctx->stream));
+	PNOL_LAUNCH(ctx, ga_dup_insert_kernel, blocks_for(Npop, 256), 256, 0, B.hash, Npop, B.tkeys, B.tmax, B.tmask);
+	PNOL_LAUNCH(ctx, ga_dup_query_kernel, blocks_for(Npop, 256), 256, 0, B.hash, Npop, B.tkeys, B.tmax, B.tmask, X, n, B.dupflag, B.S,
+	            B.suspects);
+	PNOL_LAUNCH(ctx, ga_dup_resolve_kernel, 64, 256, 0, B.hash, Npop, X, n, B.dupflag, B.S, B.suspects);
+	return PNOL_OK;
+}
+
+// 5. stream offsets of all Npop rows from dupflag and bcount, then replacement and repair of rows [own_lo, own_hi) (Xloc holds row
+// own_lo first) and their evaluation flags (ga_fix_kernel). The draws start at S->pos_elite + 2 NeliteMutGenes. The packed offsets
+// hold the replaced rows above bit 40: fewer than 2^24 of them, and fewer than 2^40 repaired genes
+static int stage_fix(pnol_ctx * ctx, const StageBufs & B, const StreamDev & st, long long Npop, long long own_lo, long long own_hi, int n,
+                     int Nelite, long long NeliteMutGenes, const double * lb, const double * ub, double * Xloc, unsigned char * indicator,
+                     int mark_modified)
+{
+	TimerScope ts(ctx, "ga_check_bounds");
+	const int nb = (int) blocks_for(Npop, kPackTile);
+	PNOL_LAUNCH(ctx, ga_pack_sums_kernel, nb, 256, 0, B.dupflag, B.bcount, Npop, B.block_sums);
+	PNOL_LAUNCH(ctx, ga_pack_scan_kernel, nb, 256, 0, B.dupflag, B.bcount, Npop, B.block_sums, nb, B.offs, B.S, NeliteMutGenes, n);
+	if (own_hi > own_lo)
+		PNOL_LAUNCH(ctx, ga_fix_kernel, blocks_for((own_hi - own_lo) * kRowLanes, 256), 256, 0, st, B.S, own_lo, own_hi, n, Nelite,
+		            NeliteMutGenes, lb, ub, B.dupflag, B.bcount, B.offs, Xloc, indicator, mark_modified);
+	return PNOL_OK;
+}
+
+// 7. popSort (:220): sorted objective values Fs and the permutation perm (sorted position -> row) of F[0, N). With bs, the bucket
+// sort on the previous generation's sorted values (splitters) runs first and the radix kernel only when it falls back; without,
+// S->sort_fallback must be 1
+static int stage_sort(pnol_ctx * ctx, const StageBufs & B, const double * F, long long N, double * Fs, unsigned * perm,
+                      const BucketBufs * bs, const double * splitters)
+{
+	TimerScope ts(ctx, "ga_pop_sort");
+	GaDevStatus * S = B.S;
+	if (bs) {
+		PNOL_LAUNCH(ctx, ga_bsort_count_kernel, bs->grid, kBsCountThreads, kBsBuckets * 12, F, N, splitters, bs->tag, bs->totals);
+		PNOL_LAUNCH(ctx, ga_bsort_scan_kernel, 1, 1024, 0, bs->totals, bs->start, bs->cursor, S, bs->large);
+		PNOL_LAUNCH(ctx, ga_bsort_scatter_kernel, bs->grid, kBsCountThreads, 0, F, N, (const unsigned *) bs->tag, bs->cursor, B.skeys[0], B.svals[0]);
+		PNOL_LAUNCH(ctx, (ga_bsort_bucket_kernel<128, 8>), kBsBuckets, 128, bsort_bucket_smem(kBsCap), F, (const unsigned long long *) B.skeys[0],
+		            (const unsigned *) B.svals[0], (const unsigned *) bs->start, (const GaDevStatus *) S, Fs, perm, 0u, (const unsigned *) nullptr);
+		// the large buckets from the list the scan kernel made (4096 CTAs of 131 KB that only look and leave took 20 us)
+		PNOL_LAUNCH(ctx, (ga_bsort_bucket_kernel<512, 16>), ctx->sm_count, 512, bsort_bucket_smem(kBsCapLarge), F, (const unsigned long long *) B.skeys[0],
+		            (const unsigned *) B.svals[0], (const unsigned *) bs->start, (const GaDevStatus *) S, Fs, perm, (unsigned) kBsCap,
+		            (const unsigned *) bs->large);
+	}
+	long long range = B.sort_range;
+	unsigned long long * k0 = B.skeys[0], * k1 = B.skeys[1];
+	unsigned * v0 = B.svals[0], * v1 = B.svals[1], * sc = B.scounts;
+	void * args[] = {(void *) &F, (void *) &N, (void *) &range, (void *) &k0, (void *) &v0, (void *) &k1, (void *) &v1, (void *) &sc, (void *) &S,
+	                 (void *) &Fs, (void *) &perm};
+	PNOL_CUDA(ctx, cudaLaunchCooperativeKernel((const void *) ga_sort_kernel, dim3(B.sort_grid), dim3(kSortThreads), args, 0, ctx->stream));
+	ctx->launches++;
+	return PNOL_OK;
+}
+
+// 6. the fitness sweep (:217) of the population in buffer b into P->Fchild on every rank; rows sharded: the repaired rows into the
+// replicas too. indicator == nullptr: every row is evaluated
+static int pipe_sweep(pnol_ga * ga, int b, const unsigned char * indicator)
 {
 	pnol_ctx * ctx = ga->ctx;
 	GaPipe * P = ga->pipe;
-	const long long Npop = ga->prm.npop;
+	const long long Npop = ga->prm.npop, lo = P->lo, hi = P->hi;
 	const int n = ga->n;
+	const double * Xloc = P->XL[b];
+	if (P->R == 1 && ctx->nranks > 1 && P->shard_sweep) {
+		// rows replicated: this rank sweeps individuals [r eper, (r+1) eper) and the objective values are all-gathered
+		// (GeneticAlgorithmMPI::evaluatePopulationParallel, Source/GeneticAlgorithmMPI.cpp:283-414)
+		const long long elo = std::min<long long>(P->eper * ctx->rank, Npop), ehi = std::min<long long>(elo + P->eper, Npop);
+		if (ehi > elo) PNOL_CHECK(launch_eval_batch(ctx, ga->f, Xloc + elo * n, ehi - elo, n, n, indicator ? indicator + elo : nullptr, P->Fchild + elo));
+		TimerScope ts(ctx, "ga_gather_f");
+		PNOL_CHECK(comm_allgather_dev(ctx, P->Fchild + elo, P->f_recv, (size_t) P->eper));
+		PNOL_CUDA(ctx, cudaMemcpyAsync(P->Fchild, P->f_recv, (size_t) Npop * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+	} else if (hi > lo) PNOL_CHECK(launch_eval_batch(ctx, ga->f, Xloc, hi - lo, n, n, indicator, P->Fchild + lo));
+	if (P->R > 1) {
+		TimerScope ts(ctx, "ga_gather_f");
+		// rows that were not evaluated (elites) already hold the same value on every rank, so gathering whole blocks is exact
+		PNOL_CHECK(comm_allgather_dev(ctx, P->Fchild + lo, P->f_recv, (size_t) P->per));
+		PNOL_CUDA(ctx, cudaMemcpyAsync(P->Fchild, P->f_recv, (size_t) P->per * P->R * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+		PNOL_CHECK(pipe_refresh_replica(ga, b));      // repaired / replaced genes
+	}
+	return PNOL_OK;
+}
+
+// pnol_ga_init (Source/GeneticAlgorithmMPI.cpp:55-81) as a generation whose children are the start population: ga->Xnew holds it
+// (replicated) and ga->pos counts the draws it and the duplicate check took. Bounds repair (:74), the fitness sweep (:77) and popSort
+// (:81) into buffer 0: XL[0] in row order, perm[0] sorted position -> row, Fs[0] sorted
+int ga_pipe_init(pnol_ga * ga, double * f0_out)
+{
+	pnol_ctx * ctx = ga->ctx;
+	GaPipe * P = ga->pipe;
+	const long long Npop = ga->prm.npop, lo = P->lo, hi = P->hi;
+	const int n = ga->n;
+	StageBufs B = P->B;
+	B.hash = P->hash[0];
+	PNOL_CHECK(status_reset(ctx, B.S, ga->pos));
+	// box counts of all rows (the stream offsets need every row); no row is a duplicate
+	PNOL_LAUNCH(ctx, ga_rows_hash_kernel, blocks_for(Npop * kRowLanes, 256), 256, 0, (const double *) ga->Xnew, 0LL, 0LL, Npop, n, ga->lb, ga->ub,
+	            B.hash, B.bcount);
+	PNOL_CUDA(ctx, cudaMemsetAsync(B.dupflag, 0, (size_t) Npop, ctx->stream));
+	PNOL_CHECK(stage_fix(ctx, B, ga_stream(ga), Npop, lo, hi, n, 0, 0, ga->lb, ga->ub, ga->Xnew + lo * n, P->indicator, 0));
+	if (hi > lo)
+		PNOL_CUDA(ctx, cudaMemcpyAsync(P->XL[0], ga->Xnew + lo * n, (size_t) (hi - lo) * n * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+	PNOL_CHECK(pipe_sweep(ga, 0, nullptr));
+	PNOL_CHECK(stage_sort(ctx, B, P->Fchild, Npop, P->Fs[0], P->perm[0], nullptr, nullptr));
+	double f0 = 0, fb = 0;
+	PNOL_CUDA(ctx, cudaMemcpyAsync(&f0, P->Fchild, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));        // (:78) row 0
+	PNOL_CUDA(ctx, cudaMemcpyAsync(&fb, P->Fs[0], sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+	PNOL_CUDA(ctx, cudaMemcpyAsync(P->status_host, B.S, sizeof(GaDevStatus), cudaMemcpyDeviceToHost, ctx->stream));
+	PNOL_CHECK(finish(ctx));
 	P->cur = 0;
-	if (P->hi > P->lo)
-		PNOL_CUDA(ctx, cudaMemcpyAsync(P->XL[0], ga->Xpop + P->lo * n, (size_t) (P->hi - P->lo) * n * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-	PNOL_CUDA(ctx, cudaMemcpyAsync(P->Fs[0], ga->F, (size_t) Npop * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-	PNOL_LAUNCH(ctx, ga_iota_kernel, blocks_for(Npop, 256), 256, 0, P->perm[0], Npop);
-	PNOL_CHECK(pipe_refresh_replica(ga, 0));
 	P->elite_idx_complete = true;
+	ga->pos += P->status_host->noob;
+	if (ga->stream_values && ga->pos > ga->stream.n_values) {
+		PNOL_SET_ERR(ctx, "ga: the explicit random stream (%llu values) is exhausted", (unsigned long long) ga->stream.n_values);
+		return PNOL_ERR_STREAM;
+	}
+	ga->f_best_prev = fb; ga->f_best = fb;
+	if (f0_out) *f0_out = f0;
+	return PNOL_OK;
+}
+
+// pnol_ga_pop_sort: the radix kernel (no previous sorted values, so no bucket sort), then the rows in sorted order
+int ga_stage_pop_sort(pnol_ctx * ctx, double * X, double * F, long long npop, int n)
+{
+	CallMem M(ctx);
+	StageBufs B;
+	double * Xs, * Fs;
+	unsigned * perm;
+	PNOL_CHECK(sort_geometry(ctx, npop, B));
+	PNOL_CHECK(M(&B.S, 1));
+	for (int b = 0; b < 2; b++) { PNOL_CHECK(M(&B.skeys[b], (size_t) npop)); PNOL_CHECK(M(&B.svals[b], (size_t) npop)); }
+	PNOL_CHECK(M(&B.scounts, (size_t) 256 * B.sort_grid));
+	PNOL_CHECK(M(&Fs, (size_t) npop));
+	PNOL_CHECK(M(&perm, (size_t) npop));
+	PNOL_CHECK(M(&Xs, (size_t) npop * n));
+	PNOL_CHECK(status_reset(ctx, B.S, 0));
+	PNOL_CHECK(stage_sort(ctx, B, F, npop, Fs, perm, nullptr, nullptr));
+	PNOL_LAUNCH(ctx, ga_gather_sorted_kernel, blocks_for(npop * kRowLanes, 256), 256, 0, one_table(X, npop, n), (const unsigned *) perm, 0LL, npop, n, Xs);
+	PNOL_CUDA(ctx, cudaMemcpyAsync(X, Xs, (size_t) npop * n * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+	PNOL_CUDA(ctx, cudaMemcpyAsync(F, Fs, (size_t) npop * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+	return PNOL_OK;
+}
+
+// pnol_ga_check_identical (identical: stages 4 and 5 with the box counts zeroed) and pnol_ga_check_bounds (stage 5 with no
+// duplicates): rows modified are flagged in indicator (nullptr: no flags), the draws start at pos; *pos_end = the position after them
+int ga_stage_repair(pnol_ctx * ctx, bool identical, double * X, long long npop, int n, const double * lb, const double * ub,
+                    unsigned char * indicator, const StreamDev & st, unsigned long long pos, unsigned long long * pos_end)
+{
+	CallMem M(ctx);
+	StageBufs B;
+	PNOL_CHECK(M(&B.S, 1));
+	PNOL_CHECK(M(&B.hash, (size_t) npop));
+	PNOL_CHECK(M(&B.bcount, (size_t) npop));
+	PNOL_CHECK(M(&B.dupflag, (size_t) npop));
+	PNOL_CHECK(M(&B.offs, (size_t) npop));
+	PNOL_CHECK(M(&B.block_sums, (size_t) (npop + kPackTile - 1) / kPackTile + 1));
+	if (identical) {
+		const unsigned slots = dup_table_slots(npop);
+		B.tmask = slots - 1;
+		PNOL_CHECK(M(&B.tkeys, (size_t) slots));
+		PNOL_CHECK(M(&B.tmax, (size_t) slots));
+		PNOL_CHECK(M(&B.suspects, (size_t) npop));
+	}
+	if (!indicator) PNOL_CHECK(M(&indicator, (size_t) npop));
+	PNOL_CHECK(status_reset(ctx, B.S, pos));
+	PNOL_LAUNCH(ctx, ga_rows_hash_kernel, blocks_for(npop * kRowLanes, 256), 256, 0, (const double *) X, 0LL, 0LL, npop, n,
+	            identical ? nullptr : lb, identical ? nullptr : ub, B.hash, B.bcount);
+	if (identical) PNOL_CHECK(stage_identical(ctx, B, npop, one_table(X, npop, n), n));
+	else PNOL_CUDA(ctx, cudaMemsetAsync(B.dupflag, 0, (size_t) npop, ctx->stream));
+	PNOL_CHECK(stage_fix(ctx, B, st, npop, 0, npop, n, 0, 0, lb, ub, X, indicator, 1));
+	GaDevStatus h;
+	PNOL_CUDA(ctx, cudaMemcpyAsync(&h, B.S, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+	PNOL_CHECK(finish(ctx));
+	*pos_end = pos + h.ndup * (unsigned long long) n + h.noob;
 	return PNOL_OK;
 }
 
@@ -1545,8 +1769,10 @@ static int pipe_enqueue(pnol_ga * ga, double window_scale)
 	const int cur = P->cur, nxt = cur ^ 1;
 	const RowTable & T = P->table[cur];
 	const RowTable & Tn = P->table[nxt];
-	StreamDev st = pipe_stream(ga);
-	GaDevStatus * S = P->status;
+	StreamDev st = ga_stream(ga);
+	StageBufs B = P->B;
+	B.hash = P->hash[nxt];
+	GaDevStatus * S = B.S;
 	double * Xloc = P->XL[nxt];
 	const long long lo = P->lo, hi = P->hi;
 	auto clampr = [&](long long a, long long b, long long & x0, long long & x1) {   // [a, b) cut to the own rows
@@ -1561,7 +1787,7 @@ static int pipe_enqueue(pnol_ga * ga, double window_scale)
 		long long a, b;
 		clampr(0, Nelite, a, b);
 		if (b > a) PNOL_LAUNCH(ctx, ga_elite_copy_kernel, blocks_for((b - a) * kRowLanes, 256), 256, 0, T, P->perm[cur], a, b, n,
-		                       Xloc + (a - lo) * n, P->hash[nxt], P->bcount);
+		                       Xloc + (a - lo) * n, B.hash, B.bcount);
 	}
 	// 1. crossover
 	if (Ncross > 0) {
@@ -1584,7 +1810,8 @@ static int pipe_enqueue(pnol_ga * ga, double window_scale)
 		ctx->launches++;
 		long long a, b;
 		clampr(Nelite, Nelite + Ncross, a, b);
-		if (b > a) PNOL_LAUNCH(ctx, ga_rows_hash_kernel, blocks_for((b - a) * kRowLanes, 256), 256, 0, Xloc, lo, a, b, n, P->hash[nxt], P->bcount);
+		if (b > a) PNOL_LAUNCH(ctx, ga_rows_hash_kernel, blocks_for((b - a) * kRowLanes, 256), 256, 0, Xloc, lo, a, b, n, (const double *) nullptr,
+		                       (const double *) nullptr, B.hash, B.bcount);
 	}
 	// 2. mutation
 	{
@@ -1639,7 +1866,7 @@ static int pipe_enqueue(pnol_ga * ga, double window_scale)
 		clampr(Nelite + Ncross, Nelite + Ncross + Nrand, a, b);
 		if (b > a)
 			PNOL_LAUNCH(ctx, ga_mut_apply_kernel, blocks_for((b - a) * kRowLanes, 256), 256, 0, st, S, T, P->perm[cur], ga->mut_pos, ga->mut_idx,
-			            a - (Nelite + Ncross), b - (Nelite + Ncross), Nelite + Ncross, lo, n, ga->lb, ga->ub, spreadRatio, Xloc, P->hash[nxt], P->bcount);
+			            a - (Nelite + Ncross), b - (Nelite + Ncross), Nelite + Ncross, lo, n, ga->lb, ga->ub, spreadRatio, Xloc, B.hash, B.bcount);
 	}
 	// 3. elite mutations
 	if (NeliteMut > 0) {
@@ -1649,7 +1876,7 @@ static int pipe_enqueue(pnol_ga * ga, double window_scale)
 		clampr(row0, row0 + NeliteMut, a, b);
 		if (b > a)
 			PNOL_LAUNCH(ctx, ga_elite_mut_kernel, blocks_for((b - a) * kRowLanes, 256), 256, 0, st, S, T, P->perm[cur], a - row0, b - row0, row0, lo, n,
-			            (int) Nelite, ga->lb, ga->ub, ga->prm.elite_mutation_size, Xloc, P->hash[nxt], P->bcount, ga->elite_idx);
+			            (int) Nelite, ga->lb, ga->ub, ga->prm.elite_mutation_size, Xloc, B.hash, B.bcount, ga->elite_idx);
 	}
 	// hashes and box counts of all rows on every rank; the new rows where the duplicate check of another rank may look at them
 	if (R > 1) {
@@ -1657,77 +1884,25 @@ static int pipe_enqueue(pnol_ga * ga, double window_scale)
 		const size_t own = (size_t) (hi - lo);
 		PNOL_CUDA(ctx, cudaMemsetAsync(P->hb_send, 0, (size_t) P->per * 12, ctx->stream));
 		if (own) {
-			PNOL_CUDA(ctx, cudaMemcpyAsync(P->hb_send, P->hash[nxt] + lo, own * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-			PNOL_CUDA(ctx, cudaMemcpyAsync(P->hb_send + (size_t) P->per * 8, P->bcount + lo, own * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+			PNOL_CUDA(ctx, cudaMemcpyAsync(P->hb_send, B.hash + lo, own * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+			PNOL_CUDA(ctx, cudaMemcpyAsync(P->hb_send + (size_t) P->per * 8, B.bcount + lo, own * 4, cudaMemcpyDeviceToDevice, ctx->stream));
 		}
 		PNOL_CHECK(comm_allgather_bytes_dev(ctx, P->hb_send, P->hb_recv, (size_t) P->per * 12));
 		for (int r = 0; r < R; r++) {
 			const unsigned char * slot = P->hb_recv + (size_t) r * P->per * 12;
-			PNOL_CUDA(ctx, cudaMemcpyAsync(P->hash[nxt] + (size_t) r * P->per, slot, (size_t) P->per * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-			PNOL_CUDA(ctx, cudaMemcpyAsync(P->bcount + (size_t) r * P->per, slot + (size_t) P->per * 8, (size_t) P->per * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+			PNOL_CUDA(ctx, cudaMemcpyAsync(B.hash + (size_t) r * P->per, slot, (size_t) P->per * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+			PNOL_CUDA(ctx, cudaMemcpyAsync(B.bcount + (size_t) r * P->per, slot + (size_t) P->per * 8, (size_t) P->per * 4, cudaMemcpyDeviceToDevice, ctx->stream));
 		}
 		PNOL_CHECK(pipe_refresh_replica(ga, nxt));
 	}
 	// 4. identical children
-	{
-		TimerScope ts(ctx, "ga_check_identical");
-		PNOL_CUDA(ctx, cudaMemsetAsync(P->tkeys, 0, ((size_t) P->tmask + 1) * 8, ctx->stream));
-		PNOL_CUDA(ctx, cudaMemsetAsync(P->tmax, 0, ((size_t) P->tmask + 1) * 4, ctx->stream));
-		PNOL_LAUNCH(ctx, ga_dup_insert_kernel, blocks_for(Npop, 256), 256, 0, P->hash[nxt], (long long) Npop, P->tkeys, P->tmax, P->tmask);
-		PNOL_LAUNCH(ctx, ga_dup_query_kernel, blocks_for(Npop, 256), 256, 0, P->hash[nxt], (long long) Npop, P->tkeys, P->tmax, P->tmask, Tn, n,
-		            P->dupflag, S, P->suspects);
-		PNOL_LAUNCH(ctx, ga_dup_resolve_kernel, 64, 256, 0, P->hash[nxt], (long long) Npop, Tn, n, P->dupflag, S, P->suspects);
-	}
+	PNOL_CHECK(stage_identical(ctx, B, Npop, Tn, n));
 	// 5. stream offsets, replacement and repair, evaluation flags
-	{
-		TimerScope ts(ctx, "ga_check_bounds");
-		const int nb = (int) blocks_for(Npop, kPackTile);
-		PNOL_LAUNCH(ctx, ga_pack_sums_kernel, nb, 256, 0, P->dupflag, P->bcount, (long long) Npop, P->block_sums);
-		PNOL_LAUNCH(ctx, ga_pack_scan_kernel, nb, 256, 0, P->dupflag, P->bcount, (long long) Npop, P->block_sums, nb, P->offs, S, NeliteMut * n, n);
-		if (hi > lo)
-			PNOL_LAUNCH(ctx, ga_fix_kernel, blocks_for((hi - lo) * kRowLanes, 256), 256, 0, st, S, lo, hi, n, (int) Nelite, NeliteMut * n, ga->lb, ga->ub,
-			            P->dupflag, P->bcount, P->offs, Xloc, P->indicator);
-	}
+	PNOL_CHECK(stage_fix(ctx, B, st, Npop, lo, hi, n, (int) Nelite, NeliteMut * n, ga->lb, ga->ub, Xloc, P->indicator, 0));
 	// 6. the fitness sweep over this rank's rows (:217)
-	if (R == 1 && ctx->nranks > 1 && P->shard_sweep) {
-		// rows replicated: this rank sweeps individuals [r eper, (r+1) eper) and the objective values are all-gathered
-		// (GeneticAlgorithmMPI::evaluatePopulationParallel, Source/GeneticAlgorithmMPI.cpp:283-414)
-		const long long elo = std::min<long long>(P->eper * ctx->rank, Npop), ehi = std::min<long long>(elo + P->eper, Npop);
-		if (ehi > elo) PNOL_CHECK(launch_eval_batch(ctx, ga->f, Xloc + elo * n, ehi - elo, n, n, P->indicator + elo, P->Fchild + elo));
-		TimerScope ts(ctx, "ga_gather_f");
-		PNOL_CHECK(comm_allgather_dev(ctx, P->Fchild + elo, P->f_recv, (size_t) P->eper));
-		PNOL_CUDA(ctx, cudaMemcpyAsync(P->Fchild, P->f_recv, (size_t) Npop * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-	} else if (hi > lo) PNOL_CHECK(launch_eval_batch(ctx, ga->f, Xloc, hi - lo, n, n, P->indicator, P->Fchild + lo));
-	if (R > 1) {
-		TimerScope ts(ctx, "ga_gather_f");
-		// rows that were not evaluated (elites) already hold the same value on every rank, so gathering whole blocks is exact
-		PNOL_CHECK(comm_allgather_dev(ctx, P->Fchild + lo, P->f_recv, (size_t) P->per));
-		PNOL_CUDA(ctx, cudaMemcpyAsync(P->Fchild, P->f_recv, (size_t) P->per * R * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
-		PNOL_CHECK(pipe_refresh_replica(ga, nxt));      // repaired / replaced genes
-	}
+	PNOL_CHECK(pipe_sweep(ga, nxt, P->indicator));
 	// 7. popSort (:220): sorted objective values and the permutation, rows stay where they are
-	{
-		TimerScope ts(ctx, "ga_pop_sort");
-		const double * Fc = P->Fchild;
-		long long N = Npop, range = P->sort_range;
-		unsigned long long * k0 = P->skeys[0], * k1 = P->skeys[1];
-		unsigned * v0 = P->svals[0], * v1 = P->svals[1], * sc = P->scounts, * po = P->perm[nxt];
-		double * Fo = P->Fs[nxt];
-		if (P->bs_on) {
-			PNOL_LAUNCH(ctx, ga_bsort_count_kernel, P->bs_grid, kBsCountThreads, kBsBuckets * 12, Fc, N, (const double *) P->Fs[cur], P->bs_tag, P->bs_totals);
-			PNOL_LAUNCH(ctx, ga_bsort_scan_kernel, 1, 1024, 0, P->bs_totals, P->bs_start, P->bs_cursor, S, P->bs_large);
-			PNOL_LAUNCH(ctx, ga_bsort_scatter_kernel, P->bs_grid, kBsCountThreads, 0, Fc, N, (const unsigned *) P->bs_tag, P->bs_cursor, k0, v0);
-			PNOL_LAUNCH(ctx, (ga_bsort_bucket_kernel<128, 8>), kBsBuckets, 128, bsort_bucket_smem(kBsCap), Fc, (const unsigned long long *) k0, (const unsigned *) v0,
-			            (const unsigned *) P->bs_start, (const GaDevStatus *) S, Fo, po, 0u, (const unsigned *) nullptr);
-			// the large buckets from the list the scan kernel made (4096 CTAs of 131 KB that only look and leave took 20 us)
-			PNOL_LAUNCH(ctx, (ga_bsort_bucket_kernel<512, 16>), ctx->sm_count, 512, bsort_bucket_smem(kBsCapLarge), Fc, (const unsigned long long *) k0, (const unsigned *) v0,
-			            (const unsigned *) P->bs_start, (const GaDevStatus *) S, Fo, po, (unsigned) kBsCap, (const unsigned *) P->bs_large);
-		}
-		void * args[] = {(void *) &Fc, (void *) &N, (void *) &range, (void *) &k0, (void *) &v0, (void *) &k1, (void *) &v1, (void *) &sc, (void *) &S,
-		                 (void *) &Fo, (void *) &po};
-		PNOL_CUDA(ctx, cudaLaunchCooperativeKernel((const void *) ga_sort_kernel, dim3(P->sort_grid), dim3(kSortThreads), args, 0, ctx->stream));
-		ctx->launches++;
-	}
+	PNOL_CHECK(stage_sort(ctx, B, P->Fchild, Npop, P->Fs[nxt], P->perm[nxt], P->bs_on ? &P->bs : nullptr, P->Fs[cur]));
 	PNOL_LAUNCH(ctx, ga_finish_kernel, 1, 32, 0, S, P->Fs[nxt], NeliteMut * n, n,
 	            ga->stream_values ? (unsigned long long) ga->stream.n_values : ~0ULL);
 	PNOL_CUDA(ctx, cudaMemcpyAsync(P->status_host, S, sizeof(GaDevStatus), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1812,7 +1987,7 @@ int ga_pipe_get_indices(pnol_ga * ga, int * cross_idx, int * mut_idx, int * elit
 	GaPipe * P = ga->pipe;
 	if (elite_idx && !P->elite_idx_complete && ga->nelmut > 0) {
 		const long long count = (long long) ga->nelmut * ga->n;
-		PNOL_LAUNCH(ctx, ga_elite_idx_kernel, blocks_for(count, 256), 256, 0, pipe_stream(ga), P->pos_elite_last, count, ga->nelite, ga->elite_idx);
+		PNOL_LAUNCH(ctx, ga_elite_idx_kernel, blocks_for(count, 256), 256, 0, ga_stream(ga), P->pos_elite_last, count, ga->nelite, ga->elite_idx);
 		P->elite_idx_complete = true;
 	}
 	if (cross_idx) PNOL_CUDA(ctx, cudaMemcpyAsync(cross_idx, ga->cross_idx, (size_t) ga->ncross * ga->n * sizeof(int), cudaMemcpyDefault, ctx->stream));

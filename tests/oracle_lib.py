@@ -234,19 +234,19 @@ def _stream_args(stream):
             C.c_double(stream.get("scale", 1.0)))
 
 
-def ga_check_bounds(xpop, lb, ub, stream, pos=0):
+def ga_check_bounds(xpop, lb, ub, stream, pos=0, ind=None):
     xpop = f64(xpop).copy()
     lb, ub = f64(lb), f64(ub)
-    ind = np.zeros(xpop.shape[0], dtype=np.uint8)
+    ind = np.zeros(xpop.shape[0], dtype=np.uint8) if ind is None else np.array(ind, dtype=np.uint8)
     newpos = lib().oracle_ga_check_bounds(_p(xpop), C.c_longlong(xpop.shape[0]), C.c_int(xpop.shape[1]), _p(lb), _p(ub), _p(ind),
                                           *_stream_args(stream), C.c_uint64(pos))
     return xpop, ind, int(newpos)
 
 
-def ga_check_identical(xpop, lb, ub, stream, pos=0):
+def ga_check_identical(xpop, lb, ub, stream, pos=0, ind=None):
     xpop = f64(xpop).copy()
     lb, ub = f64(lb), f64(ub)
-    ind = np.zeros(xpop.shape[0], dtype=np.uint8)
+    ind = np.zeros(xpop.shape[0], dtype=np.uint8) if ind is None else np.array(ind, dtype=np.uint8)
     newpos = lib().oracle_ga_check_identical(_p(xpop), C.c_longlong(xpop.shape[0]), C.c_int(xpop.shape[1]), _p(lb), _p(ub),
                                              _p(ind), *_stream_args(stream), C.c_uint64(pos))
     return xpop, ind, int(newpos)

@@ -38,9 +38,12 @@ def test_check_bounds_stage(ctx):
     X = rng.uniform(-1.5, 2.2, size=(npop, n))
     X[10] = 0.0                                                # fully inside
     stream = dict(seed=99, scale=1.0)
-    Xg, ig, pg = ctx.ga_check_bounds(X, lb, ub, stream, pos=17)
-    Xw, iw, pw = O.ga_check_bounds(X, lb, ub, stream, pos=17)
-    assert pg == pw and np.array_equal(ig, iw) and np.array_equal(Xg, Xw)
+    # evaluation flags: repaired rows are set, the others keep what the caller passed
+    for ind in (None, rng.integers(0, 2, npop, dtype=np.uint8)):
+        Xg, ig, pg = ctx.ga_check_bounds(X, lb, ub, stream, pos=17, ind=ind)
+        Xw, iw, pw = O.ga_check_bounds(X, lb, ub, stream, pos=17, ind=ind)
+        assert pg == pw and np.array_equal(ig, iw) and np.array_equal(Xg, Xw)
+    assert ig[10] == ind[10] and np.any(ig == 0)
     # explicit stream, exhausted -> error
     with pytest.raises(capi.PnolError):
         ctx.ga_check_bounds(X, lb, ub, dict(values=np.linspace(0, 0.9, 5)), pos=0)
@@ -58,16 +61,29 @@ def test_check_identical_stage(ctx):
     X[300, 0] = 0.0
     X[301] = X[300]
     X[301, 0] = -0.0                                           # -0 == +0 in the reference's comparison
+    X[400, 1] = np.nan
+    X[401] = X[400]                                            # bit-identical, but NaN != NaN: not duplicates
     stream = dict(seed=5, scale=1.0)
-    Xg, ig, pg = ctx.ga_check_identical(X, lb, ub, stream, pos=3)
-    Xw, iw, pw = O.ga_check_identical(X, lb, ub, stream, pos=3)
-    assert pw == 3 + 5 * n
-    assert pg == pw and np.array_equal(ig, iw) and np.array_equal(Xg, Xw)
+    # evaluation flags: replaced rows are set, the others keep what the caller passed
+    for ind in (None, rng.integers(0, 2, npop, dtype=np.uint8)):
+        Xg, ig, pg = ctx.ga_check_identical(X, lb, ub, stream, pos=3, ind=ind)
+        Xw, iw, pw = O.ga_check_identical(X, lb, ub, stream, pos=3, ind=ind)
+        assert pw == 3 + 5 * n
+        assert pg == pw and np.array_equal(ig, iw) and np.array_equal(Xg, Xw, equal_nan=True)
+        assert np.array_equal(Xg[400:402], X[400:402], equal_nan=True)
+    assert np.any(ig == 0)
     # all rows identical (the reference's call on the zero-initialised XpopNew, GeneticAlgorithmMPI.cpp:71)
     Z = np.zeros((500, n))
     Xg, ig, pg = ctx.ga_check_identical(Z, lb, ub, stream, pos=0)
     Xw, iw, pw = O.ga_check_identical(Z, lb, ub, stream, pos=0)
     assert pg == pw == 499 * n and np.array_equal(Xg, Xw) and np.array_equal(ig, iw)
+
+
+def test_stage_size_limits(ctx):
+    """the stand-alone duplicate check counts replaced rows in 24 bits: a larger population is refused, not miscounted"""
+    X = np.zeros(((1 << 24) + 1, 1))
+    with pytest.raises(capi.PnolError):
+        ctx.ga_check_identical(X, [-1.0], [1.0], dict(seed=1, scale=1.0))
 
 
 GA_CASES = [

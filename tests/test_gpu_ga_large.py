@@ -304,7 +304,7 @@ def test_signed_zero_pop_sort(ctx):
 
 
 def test_signed_zero_init(ctx, ga_objectives):
-    """pnol_ga_init sorts the start population through ga.cu's radix sort"""
+    """pnol_ga_init sorts the start population with the radix kernel alone (the bucket sort needs a previous generation's values)"""
     n, npop, box = 8, 3000, 0.5
     want = reference(R.MY_F_SIGNED_ZERO, n, npop, 5, dict(seed=21, scale=SCALE), np.zeros(n), box, stop_after=0)
     f = ctx.functor(R.MY_F_SIGNED_ZERO)
