@@ -67,6 +67,13 @@ class Runtime {
 	// (SURVEY.md 8(f) item 2: work space 512 MB instead of m*n*8 bytes; same iterates up to the summation order of J^T J)
 	bool storeJacobian() const { return storeJ_; }
 	void setStoreJacobian(bool on) { storeJ_ = on; }
+	// Gradients of Objective::gradientApproximation[MPI][Recur] (hence of BFGS, BFGS_MPI, BFGS_Bnd, BFGS_Bnd_MPI_SW, BFGSBnd_MPI): the
+	// forward difference (false, default) or the objective's own derivative (true: pnol_gradient[_recur] from F::partial,
+	// include/pnol/functors.hpp; dX is ignored, an objective without one makes the call fail with PNOL_ERR_NO_FUNCTOR). In the analytic
+	// mode a gradient evaluates no objective value, so the evaluation counts the classes report (getEvals(), "function evaluations")
+	// count objective evaluations only.
+	bool analyticGradient() const { return gradAnalytic_; }
+	void setAnalyticGradient(bool on) { gradAnalytic_ = on; }
 	void check(int status) const;             // throws pnol::Error with pnol_last_error() text
   private:
 	Runtime();
@@ -80,6 +87,7 @@ class Runtime {
 	int jacMode_;
 	bool jacCache_;
 	bool storeJ_ = true;
+	bool gradAnalytic_ = false;
 };
 
 // RAII local (non-collective) mode for the serial classes: the reference's BFGS, BFGS_Bnd, LevMarq, GeneticAlgorithm and the

@@ -6,16 +6,17 @@
  * The reference lets a user plug any objective into every stencil and algorithm by subclassing Objective / MultiObjective and
  * implementing objEval (Source/PNOL_Objective.hpp:29, :57). Here the device side of that plug-in point is:
  *
- *   1. write the functor once, __host__ __device__, to the concept of include/pnol/functors.hpp (scalar: eval(P, X, n);
- *      residual model: residual(P, X, n, i), optionally jacobian(P, X, n, i, Ji) for PNOL_JAC_ANALYTIC; optionally kSeparable /
- *      sep_init / sep_term for the fast population sweep);
+ *   1. write the functor once, __host__ __device__, to the concept of include/pnol/functors.hpp (scalar: eval(P, X, n), optionally
+ *      partial(P, X, n, j) for pnol_gradient[_recur]; residual model: residual(P, X, n, i), optionally jacobian(P, X, n, i, Ji) for
+ *      PNOL_JAC_ANALYTIC; optionally kSeparable / sep_init / sep_term for the fast population sweep);
  *   2. in ONE .cu file of your own, compiled with
  *        nvcc -gencode arch=compute_100a,code=sm_100a -fmad=false -Xcompiler -ffp-contract=off -I<repo>/include ...
  *      write   PNOL_REGISTER_SCALAR_FUNCTOR(kind, MyFunctor, n_columns)   or   PNOL_REGISTER_RESIDUAL_FUNCTOR(kind, MyModel, n_columns)
  *      with a kind in [PNOL_F_USER_SCALAR_BASE, +1000) resp. [PNOL_F_USER_RESIDUAL_BASE, +1000);
  *   3. link that object into your program / shared library next to libpnol_b200.so. The macro registers a launch table
- *      (pnol_functor_vtable, include/pnol_b200.h) at load time; pnol_functor_create(kind) and every entry point that takes a
- *      functor -- pnol_eval_batch, pnol_fd_gradient[_recur], pnol_fd_hessian, pnol_alpha_pool, the GA, pnol_residual_eval,
+ *      (pnol_functor_vtable, include/pnol_b200.h) at load time, and for a scalar functor with partial() also its gradient launcher
+ *      (pnol_register_functor_gradient); pnol_functor_create(kind) and every entry point that takes a functor -- pnol_eval_batch,
+ *      pnol_fd_gradient[_recur], pnol_gradient[_recur], pnol_fd_hessian, pnol_alpha_pool, the GA, pnol_residual_eval,
  *      pnol_fd_jacobian, pnol_lm_step / pnol_lm_iterate -- then launch YOUR instantiations of the kernels below on the
  *      context's stream. The built-in objectives run through exactly these templates (csrc/eval_kernels.cu, residual_kernels.cu).
  *
@@ -363,6 +364,50 @@ int fd_points(const pnol_launch_env * env, const FunctorParams & P, const double
 }
 
 // ---------------------------------------------------------------------------------------------------
+// a3 / a5, analytic: g[i] = F::partial(x, pos[i]) for i in [i0, i1) (pos == nullptr: i itself) of a scalar functor that defines partial
+// (functors.hpp: has_partial). One coordinate per thread, so the depth of a gradient is that of ONE partial (O(1) for a locally coupled
+// objective) where the forward difference runs a whole evaluation per thread. The base point is staged in shared memory with coalesced
+// loads; each thread writes its entry straight to g, coalesced. pos[i] < 0 (a reduced entry without a slot, see fd_points_kernel) gives
+// 0.0, what the forward difference gives there. f0 (f(x)) only when f0_out != nullptr: one extra thread runs F::eval, the one long
+// dependent chain of the kernel, so it is not run when nobody asks for it.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kGradThreads = 128;
+
+template <class F>
+__global__ void __launch_bounds__(kGradThreads)
+gradient_kernel(FunctorParams P, const double * __restrict__ xfull, int nfull, const int * __restrict__ pos, int i0, int i1,
+                double * __restrict__ g_out, double * __restrict__ f0_out)
+{
+	extern __shared__ double xs[];
+#pragma unroll 4
+	for (int j = threadIdx.x; j < nfull; j += blockDim.x) xs[j] = xfull[j];
+	__syncthreads();
+	const PtrAcc acc{xs};
+	const int i = i0 + blockIdx.x * blockDim.x + threadIdx.x;
+	if (i < i1) {
+		const int pi = pos ? pos[i] : i;
+		g_out[i] = pi >= 0 ? F::partial(P, acc, nfull, pi) : 0.0;
+	} else if (i == i1 && f0_out) {
+		*f0_out = F::eval(P, acc, nfull);
+	}
+}
+
+template <class F>
+int gradient(const pnol_launch_env * env, const FunctorParams & P, const double * xfull, int nfull, const int * pos, int i0, int i1,
+             double * g_out, double * f0_out)
+{
+	const int nthreads = (i1 - i0) + (f0_out ? 1 : 0);
+	if (nthreads <= 0) return PNOL_OK;
+	size_t smem = (size_t) nfull * sizeof(double);
+	PNOL_DEV_REQUIRE(env, smem <= env->smem_optin, "gradient: n = %d does not fit in shared memory", nfull);
+	auto kern = gradient_kernel<F>;
+	PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+	PNOL_DEV_LAUNCH(env, kern, (unsigned) ((nthreads + kGradThreads - 1) / kGradThreads), kGradThreads, smem, P, xfull, nfull, pos, i0, i1,
+	                g_out, f0_out);
+	return PNOL_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
 // a6: forward-difference Hessian (Objective::hessianApproximation, Source/PNOL_Objective.cpp:38-85).
 // One thread per pair (i <= j): B_ij = (f_ij - f_i - f_j + f) / (dx_i dx_j), mirrored. f_i are the n stencil
 // values already produced by fd_points_kernel (the reference recomputes the same value for every pair).
@@ -653,6 +698,8 @@ template <class F> struct ScalarTable {
 	                       const unsigned char * is_const, int nfull, const double * alpha, int npool, double dalpha,
 	                       const unsigned char * eval_ind, int want_shifted, double * vals)
 	{ return alpha_pool<F>(env, *P, xfull, pfull, is_const, nfull, alpha, npool, dalpha, eval_ind, want_shifted, vals); }
+	static int gradient_(const pnol_launch_env * env, const pnol_functor_params * P, const double * xfull, int nfull, const int * pos, int i0,
+	                     int i1, double * g, double * f0) { return gradient<F>(env, *P, xfull, nfull, pos, i0, i1, g, f0); }
 	static pnol_functor_vtable make(int n_columns)
 	{
 		pnol_functor_vtable vt = {};
@@ -663,6 +710,15 @@ template <class F> struct ScalarTable {
 		vt.fd_hessian = fd_hessian_;
 		vt.alpha_pool = alpha_pool_;
 		return vt;
+	}
+	/* registers the table, then (F defines partial) its gradient launcher, in this order: a gradient attaches to the registered table */
+	static int register_as(int kind, const pnol_functor_vtable * vt)
+	{
+		int st = pnol_register_functor(kind, vt);
+		if constexpr (has_partial<F>::value) {
+			if (st == PNOL_OK) st = pnol_register_functor_gradient(kind, gradient_);
+		}
+		return st;
 	}
 };
 template <class R> struct ResidualTable {
@@ -689,7 +745,7 @@ template <class R> struct ResidualTable {
 /* Registration at load time of the translation unit (one per functor). KIND: an integer constant in the user ranges of pnol_b200.h. */
 #define PNOL_REGISTER_SCALAR_FUNCTOR(KIND, F, NCOLS)                                                              \
 	static const pnol_functor_vtable pnol_vt_##F = pnol::dev::ScalarTable<F>::make(NCOLS);                        \
-	static const int pnol_reg_##F = pnol_register_functor((KIND), &pnol_vt_##F);
+	static const int pnol_reg_##F = pnol::dev::ScalarTable<F>::register_as((KIND), &pnol_vt_##F);
 #define PNOL_REGISTER_RESIDUAL_FUNCTOR(KIND, R, NCOLS)                                                            \
 	static const pnol_functor_vtable pnol_vt_##R = pnol::dev::ResidualTable<R>::make(NCOLS);                      \
 	static const int pnol_reg_##R = pnol_register_functor((KIND), &pnol_vt_##R);

@@ -19,6 +19,10 @@
  *     template<class Acc> static void jacobian(const FunctorParams&, const Acc& X, int n, long long i, double * Ji);
  * which writes all n entries Ji[j] = d r_i / d x_j. That one definition is the specification: the kernels (the generic template of
  * device/functor_kernels.cuh and any specialised kernel of a built-in model) return its bits, host and device alike.
+ * A scalar functor MAY likewise define one partial derivative per coordinate (pnol_gradient; detected by has_partial below):
+ *     template<class Acc> static double partial(const FunctorParams&, const Acc& X, int n, int j);      // d f / d x_j
+ * gradient_kernel (device/functor_kernels.cuh) runs one coordinate per thread and returns its bits. Every built-in scalar objective
+ * defines one; each states its operation order, which the tests restate.
  */
 #ifndef PNOL_FUNCTORS_HPP_
 #define PNOL_FUNCTORS_HPP_
@@ -65,6 +69,23 @@ struct RosenbrockFunctor {
 		}
 		return value;
 	}
+	/* [j >= 1] 200 (x_j - x_{j-1}^2)  +  [j <= n-2] (-400 x_j (x_{j+1} - x_j^2) - 2 (1 - x_j)), in this order; a term whose condition
+	 * fails is left out (not added as 0), so n = 1 gives 0 */
+	template <class Acc> PNOL_HD static double partial(const FunctorParams &, const Acc & X, int n, int j)
+	{
+		const double xj = X[j];
+		double a = 0.0, b = 0.0;
+		if (j >= 1) {
+			const double xp = X[j - 1];
+			a = 200.0 * (xj - xp * xp);
+		}
+		if (j <= n - 2) {
+			const double xn = X[j + 1];
+			b = -400.0 * xj * (xn - xj * xj) - 2.0 * (1 - xj);
+		}
+		if (j >= 1 && j <= n - 2) return a + b;
+		return j >= 1 ? a : b;
+	}
 };
 
 /* Source/ExampleObjectives.hpp:214-224 with the runtime pow(X[k], power) replaced by repeated
@@ -87,6 +108,16 @@ struct PowerFunctor {
 		for (int k = 0; k < n; k++) value = value + sep_term(P, X[k]);
 		return value;
 	}
+	/* p x^(p-1): v = x^(p-1) by the same repeated multiplication ((x*x)*x...), then p * v; 0 for p <= 0 (f is then the constant n) */
+	template <class Acc> PNOL_HD static double partial(const FunctorParams & P, const Acc & X, int, int j)
+	{
+		const int power = (int) P.ints[0];
+		if (power <= 0) return 0.0;
+		const double x = X[j];
+		double v = 1.0;
+		for (int q = 0; q < power - 1; q++) v = v * x;
+		return (double) power * v;
+	}
 };
 
 /* Source/ExampleObjectives.hpp:58-69 */
@@ -98,6 +129,15 @@ struct BoothFunctor {
 		double a = x + 2 * y - 7;
 		double b = 2 * x + y - 5;
 		return a * a + b * b;
+	}
+	/* a, b as in eval: d/dx = 2 a + 4 b, d/dy = 4 a + 2 b; 0 for j >= 2 */
+	template <class Acc> PNOL_HD static double partial(const FunctorParams &, const Acc & X, int, int j)
+	{
+		if (j >= 2) return 0.0;
+		double x = X[0], y = X[1];
+		double a = x + 2 * y - 7;
+		double b = 2 * x + y - 5;
+		return j == 0 ? 2 * a + 4 * b : 4 * a + 2 * b;
 	}
 };
 
@@ -111,6 +151,24 @@ struct GoldsteinFunctor {
 		double d = 2 * x - 3 * y;
 		return (1 + (s * s) * (19 - 14 * x + 3 * (x * x) - 14 * y + 6 * x * y + 3 * (y * y))) *
 		       (30 + (d * d) * (18 - 32 * x + 12 * (x * x) + 48 * y - 36 * x * y + 27 * (y * y)));
+	}
+	/* product rule on f = A B, A = 1 + s^2 U, B = 30 + d^2 V (U, V the two polynomials of eval, in eval's order):
+	 *   dA = (2 s) U + s^2 (-14 + 6 x + 6 y)                 (the same for x and y)
+	 *   dB = (4 d) V + d^2 (-32 + 24 x - 36 y)     for x,    (-6 d) V + d^2 (48 - 36 x + 54 y)   for y
+	 *   df = dA B + A dB;  0 for j >= 2 */
+	template <class Acc> PNOL_HD static double partial(const FunctorParams &, const Acc & X, int, int j)
+	{
+		if (j >= 2) return 0.0;
+		double x = X[0], y = X[1];
+		double s = x + y + 1;
+		double d = 2 * x - 3 * y;
+		double U = 19 - 14 * x + 3 * (x * x) - 14 * y + 6 * x * y + 3 * (y * y);
+		double V = 18 - 32 * x + 12 * (x * x) + 48 * y - 36 * x * y + 27 * (y * y);
+		double s2 = s * s, d2 = d * d;
+		double A = 1 + s2 * U, B = 30 + d2 * V;
+		double dA = (2 * s) * U + s2 * (-14 + 6 * x + 6 * y);
+		double dB = j == 0 ? (4 * d) * V + d2 * (-32 + 24 * x - 36 * y) : (-6 * d) * V + d2 * (48 - 36 * x + 54 * y);
+		return dA * B + A * dB;
 	}
 };
 
@@ -131,6 +189,12 @@ struct RastriginFunctor {
 		for (int k = 0; k < n; k++) value = value + sep_term(P, X[k]);
 		return value;
 	}
+	/* 2 x + 20 pi sin(2 pi x), as 2 * x + RN(20 pi) * sin2pi(x) (pnol_math.h) */
+	template <class Acc> PNOL_HD static double partial(const FunctorParams &, const Acc & X, int, int j)
+	{
+		const double x = X[j];
+		return 2 * x + 62.83185307179586 * sin2pi(x);
+	}
 };
 
 /* Source/ExampleObjectives.hpp:287-298 with exp -> exp_hd; columns {x, y} */
@@ -146,6 +210,24 @@ struct ExpCurveSingleFunctor {
 			Fnorm = Fnorm + d * d;
 		}
 		return Fnorm;
+	}
+	/* with e, func, d as in eval and c = -(d + d): the terms c e (x0), c ((x0 e) t) (x1), c (x2), summed sequentially in row order
+	 * from 0; 0 for j >= 3 */
+	template <class Acc> PNOL_HD static double partial(const FunctorParams & P, const Acc & X, int, int j)
+	{
+		if (j >= 3) return 0.0;
+		double g = 0;
+		double x0 = X[0], x1 = X[1], x2 = X[2];
+		for (long long k = 0; k < P.m; k++) {
+			double t = P.col[0][k];
+			double e = exp_hd(x1 * t);
+			double func = x0 * e + x2;
+			double d = P.col[1][k] - func;
+			double c = -(d + d);
+			double term = j == 0 ? c * e : (j == 1 ? c * ((x0 * e) * t) : c);
+			g = g + term;
+		}
+		return g;
 	}
 };
 
@@ -253,6 +335,14 @@ template <class R> struct has_jacobian {
 	static constexpr bool test(decltype(&T::template jacobian<PtrAcc>)) { return true; }
 	template <class T> static constexpr bool test(...) { return false; }
 	static constexpr bool value = test<R>(nullptr);
+};
+
+/* has_partial<F>::value: F defines the per-coordinate analytic gradient of the concept above */
+template <class F> struct has_partial {
+	template <class T>
+	static constexpr bool test(decltype(&T::template partial<PtrAcc>)) { return true; }
+	template <class T> static constexpr bool test(...) { return false; }
+	static constexpr bool value = test<F>(nullptr);
 };
 
 } // namespace pnol

@@ -127,7 +127,8 @@ typedef struct {
 /* ---- open functor table: objectives that are not built in (Source/PNOL_Objective.hpp:29, :57 let a user plug in any objEval) ----
  * A user objective brings its own instantiations of the library's kernel templates (include/pnol/device/functor_kernels.cuh, compiled
  * out of tree by the user's nvcc) and registers their launchers under a kind of its choice:
- *     kinds [PNOL_F_USER_SCALAR_BASE, +1000)   scalar objectives  (eval_batch, fd_points, fd_hessian, alpha_pool)
+ *     kinds [PNOL_F_USER_SCALAR_BASE, +1000)   scalar objectives  (eval_batch, fd_points, fd_hessian, alpha_pool; optionally a gradient
+ *                                              launcher attached with pnol_register_functor_gradient: pnol_gradient[_recur])
  *     kinds [PNOL_F_USER_RESIDUAL_BASE, +1000) residual models    (residual, fd_jacobian; optionally jacobian: PNOL_JAC_ANALYTIC)
  * pnol_functor_create and every entry point that takes a functor then work for that kind as for the built-ins; libpnol_b200.so is not
  * rebuilt. PNOL_REGISTER_SCALAR_FUNCTOR / PNOL_REGISTER_RESIDUAL_FUNCTOR in that header fill the table and call pnol_register_functor
@@ -182,6 +183,19 @@ typedef struct pnol_functor_vtable {
 int pnol_register_functor(int kind, const pnol_functor_vtable * vt);
 int pnol_functor_registered(int kind);                     /* 1 for built-in and registered kinds */
 
+/* Analytic gradient of a user scalar kind (pnol_gradient[_recur]), kept beside its launch table so that the table's layout and
+ * PNOL_FUNCTOR_ABI stay as they are. The launcher writes g[i] = df/dx_{pos[i]} for i in [i0, i1) (pos NULL: pos[i] = i; pos[i] < 0:
+ * g[i] = 0) and, when f0_out != NULL, f(xfull) into *f0_out; every pointer is a DEVICE pointer, the call only enqueues on env->stream.
+ * pnol::dev::ScalarTable<F>::gradient_ (include/pnol/device/functor_kernels.cuh) is one; PNOL_REGISTER_SCALAR_FUNCTOR attaches it for
+ * a functor that defines partial(). */
+typedef int (*pnol_gradient_launcher)(const pnol_launch_env *, const pnol_functor_params *, const double * xfull, int nfull,
+                                      const int * pos, int i0, int i1, double * g_out, double * f0_out);
+/* attaches fn to the table currently registered for a SCALAR user kind; pnol_register_functor replacing that table drops it. Returns
+ * PNOL_OK, or PNOL_ERR_INVALID for a residual kind, a kind without a registered table, or fn == NULL. Thread-safe. */
+int pnol_register_functor_gradient(int kind, pnol_gradient_launcher fn);
+/* 1 when pnol_gradient accepts the kind: every built-in scalar objective, and user scalar kinds with a gradient attached */
+int pnol_functor_has_gradient(int kind);
+
 int pnol_functor_create(pnol_ctx * ctx, const pnol_functor_desc * desc, pnol_functor ** out);
 void pnol_functor_destroy(pnol_functor * f);
 int pnol_functor_is_residual(const pnol_functor * f);     /* 1 for the built-in kinds >= 100 and the user residual range */
@@ -212,6 +226,17 @@ int pnol_eval_recur(pnol_ctx * ctx, const pnol_functor * f, const double * xr, i
 int pnol_fd_gradient_recur(pnol_ctx * ctx, const pnol_functor * f, const double * xr, const double * dxr, int nr,
                            const double * const_x, const unsigned char * const_ind, int nfull, double * g_out,
                            double * f0_out);
+
+/* a3 / a4 / a5, analytic: g[i] = df/dx_i from the functor's own derivative (F::partial, include/pnol/functors.hpp; for a user kind the
+ * launcher attached with pnol_register_functor_gradient), one coordinate per GPU thread. Same arguments as the forward-difference calls
+ * above without dx, same communicator split (contiguous column blocks, all-gathered), same n range (the point must fit in shared
+ * memory). f0_out (optional) receives f(x) with the bits of pnol_eval_batch; it is computed only when requested. A scalar functor without
+ * a derivative is refused with PNOL_ERR_NO_FUNCTOR (never a silent forward difference), a residual model as the calls above refuse it.
+ * All six built-in scalar objectives have one. The _recur variant gives 0 for reduced entries beyond the free variables, as the
+ * forward difference does. */
+int pnol_gradient(pnol_ctx * ctx, const pnol_functor * f, const double * x, int n, double * g_out, double * f0_out);
+int pnol_gradient_recur(pnol_ctx * ctx, const pnol_functor * f, const double * xr, int nr, const double * const_x,
+                        const unsigned char * const_ind, int nfull, double * g_out, double * f0_out);
 
 /* a6: forward-difference Hessian, upper triangle computed and mirrored
  * (Objective::hessianApproximation, Source/PNOL_Objective.cpp:38-85). B_out is n x n. */

@@ -83,9 +83,10 @@ EXPORTS = [
     "pnol_ctx_create", "pnol_ctx_destroy", "pnol_last_error", "pnol_ctx_device", "pnol_ctx_stream", "pnol_ctx_sync",
     "pnol_ctx_sm_count", "pnol_ctx_launches", "pnol_version", "pnol_malloc", "pnol_free", "pnol_memcpy", "pnol_copy_start", "pnol_copy_wait", "pnol_memset",
     "pnol_host_alloc", "pnol_host_free", "pnol_comm_unique_id", "pnol_comm_init", "pnol_comm_rank", "pnol_comm_size",
-    "pnol_comm_set_local", "pnol_comm_allreduce_sum", "pnol_comm_allgather", "pnol_comm_broadcast", "pnol_register_functor", "pnol_functor_registered", "pnol_functor_create",
+    "pnol_comm_set_local", "pnol_comm_allreduce_sum", "pnol_comm_allgather", "pnol_comm_broadcast", "pnol_register_functor", "pnol_functor_registered",
+    "pnol_register_functor_gradient", "pnol_functor_has_gradient", "pnol_functor_create",
     "pnol_functor_destroy", "pnol_functor_is_residual", "pnol_functor_rows", "pnol_eval_batch", "pnol_fd_gradient",
-    "pnol_eval_recur", "pnol_fd_gradient_recur", "pnol_fd_hessian", "pnol_alpha_pool", "pnol_residual_eval",
+    "pnol_eval_recur", "pnol_fd_gradient_recur", "pnol_gradient", "pnol_gradient_recur", "pnol_fd_hessian", "pnol_alpha_pool", "pnol_residual_eval",
     "pnol_fd_jacobian", "pnol_lm_normal_eq", "pnol_lm_damp", "pnol_lm_step", "pnol_lm_iterate", "pnol_lm_last_run", "pnol_lm_exchange_mode", "pnol_lm_normal_eq_fused", "pnol_spd_solve", "pnol_lu_inverse",
     "pnol_matvec_neg", "pnol_bfgs_update_hinv", "pnol_dgemm_nn", "pnol_check_box_bounds", "pnol_compute_alpha_bnd",
     "pnol_stream_uniform", "pnol_ga_create", "pnol_ga_destroy", "pnol_ga_init", "pnol_ga_generation",
@@ -361,6 +362,27 @@ class Context:
         self.check(self.lib.pnol_fd_gradient_recur(self.h, f.handle, _ptr(xr), _ptr(dxr), xr.size, _ptr(const_x), _ptr(ind),
                                                    const_x.size, _ptr(g), C.byref(f0)))
         return g, f0.value
+
+    def gradient(self, f, x, want_f0=False, g=None, n=None):
+        """analytic gradient (pnol_gradient) from the functor's own derivative: returns (g, f0), f0 None unless want_f0. x and g may be
+        numpy arrays or raw device pointers (then pass n=); g defaults to a new host array"""
+        x = _f64(x)
+        n = _len(x, n)
+        if g is None:
+            g = np.empty(n, dtype=np.float64)
+        f0 = C.c_double()
+        self.check(self.lib.pnol_gradient(self.h, f.handle, _ptr(x), n, _ptr(g), C.byref(f0) if want_f0 else None))
+        return g, (f0.value if want_f0 else None)
+
+    def gradient_recur(self, f, xr, const_x, const_ind, want_f0=False):
+        """analytic gradient over the free variables (pnol_gradient_recur): returns (g, f0), f0 None unless want_f0"""
+        xr, const_x = _f64(xr), _f64(const_x)
+        ind = np.ascontiguousarray(const_ind, dtype=np.uint8)
+        g = np.empty(xr.size, dtype=np.float64)
+        f0 = C.c_double()
+        self.check(self.lib.pnol_gradient_recur(self.h, f.handle, _ptr(xr), xr.size, _ptr(const_x), _ptr(ind), const_x.size, _ptr(g),
+                                                C.byref(f0) if want_f0 else None))
+        return g, (f0.value if want_f0 else None)
 
     def fd_hessian(self, f, x, dx):
         x, dx = _f64(x), _f64(dx)

@@ -328,6 +328,7 @@ struct FunctorRegistry {
 	std::mutex mu;
 	std::map<int, const pnol_functor_vtable *> table;
 	std::vector<std::unique_ptr<pnol_functor_vtable> > copies;
+	std::map<int, pnol_gradient_launcher> gradient;      // pnol_register_functor_gradient: belongs to the table registered at the time
 };
 FunctorRegistry & registry()
 {
@@ -343,6 +344,14 @@ const pnol_functor_vtable * pnol::user_vtable(int kind)
 	std::lock_guard<std::mutex> lock(r.mu);
 	auto it = r.table.find(kind);
 	return it == r.table.end() ? nullptr : it->second;
+}
+
+pnol_gradient_launcher pnol::user_gradient(int kind)
+{
+	FunctorRegistry & r = registry();
+	std::lock_guard<std::mutex> lock(r.mu);
+	auto it = r.gradient.find(kind);
+	return it == r.gradient.end() ? nullptr : it->second;
 }
 
 extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
@@ -362,7 +371,26 @@ extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
 	std::lock_guard<std::mutex> lock(r.mu);
 	r.table[kind] = c;
 	r.copies.push_back(std::move(copy));
+	r.gradient.erase(kind);                                     // a gradient attached to the replaced table does not carry over
 	return PNOL_OK;
+}
+
+extern "C" int pnol_register_functor_gradient(int kind, pnol_gradient_launcher fn)
+{
+	if (!fn || !pnol::is_user_kind(kind) || pnol::is_residual_kind(kind)) return PNOL_ERR_INVALID;
+	FunctorRegistry & r = registry();
+	std::lock_guard<std::mutex> lock(r.mu);
+	if (r.table.find(kind) == r.table.end()) return PNOL_ERR_INVALID;
+	r.gradient[kind] = fn;
+	return PNOL_OK;
+}
+
+extern "C" int pnol_functor_has_gradient(int kind)
+{
+	switch (kind) {
+		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE: return 1;
+		default: return pnol::user_gradient(kind) != nullptr;
+	}
 }
 
 extern "C" int pnol_functor_registered(int kind)
@@ -450,11 +478,14 @@ extern "C" int pnol_eval_batch(pnol_ctx * ctx, const pnol_functor * f, const dou
 	return finish(ctx);
 }
 
-// shared tail of the FD-gradient entry points: evaluate points [i0, i1) (+ base), gather across ranks, quotient
-static int fd_gradient_common(pnol_ctx * ctx, const pnol_functor * f, const double * xfull_dev, int nfull, const int * pos_dev,
-                              const double * dx_dev, int nvar, double * g_out, double * f0_out)
+// shared tail of the gradient entry points: coordinates [i0, i1) of this rank, gathered across ranks. Forward difference (dx_dev):
+// stencil points (+ base), then the quotient. Analytic (dx_dev == nullptr): the functor's partials, written straight to the output
+// on one rank, through the gather buffer on several; the base value only when f0_out asks for it.
+static int gradient_common(pnol_ctx * ctx, const pnol_functor * f, const double * xfull_dev, int nfull, const int * pos_dev,
+                           const double * dx_dev, int nvar, double * g_out, double * f0_out)
 {
-	// scratch: fdx[nvar_padded] | f0 | g
+	const bool analytic = dx_dev == nullptr;
+	// scratch: fdx[nvar_padded] (analytic: the gathered partials) | f0 | g
 	const int R = ctx->nranks;
 	const int per = (nvar + R - 1) / R;            // coordinates per rank (contiguous column blocks)
 	const int padded = per * R;
@@ -465,12 +496,22 @@ static int fd_gradient_common(pnol_ctx * ctx, const pnol_functor * f, const doub
 	int i0 = ctx->rank * per, i1 = i0 + per;
 	if (i0 > nvar) i0 = nvar;
 	if (i1 > nvar) i1 = nvar;
-	// every rank also evaluates the base point (the reference gives it to one rank and sums; SURVEY 3.4)
-	PNOL_CHECK(launch_fd_points(ctx, f, xfull_dev, nfull, pos_dev, dx_dev, i0, i1, fdx, f0));
-	if (R > 1) PNOL_CHECK(comm_allgather_dev(ctx, fdx + (size_t) ctx->rank * per, fdx, (size_t) per));
 	DevOut<double> dg;
-	PNOL_CHECK(dg.init(ctx, g_out, (size_t) nvar));
-	PNOL_CHECK(launch_fd_quotient(ctx, fdx, f0, dx_dev, nvar, dg.get() ? dg.get() : gtmp));
+	if (analytic) {
+		PNOL_CHECK(dg.init(ctx, g_out, (size_t) nvar));
+		double * g = dg.get() ? dg.get() : gtmp;
+		PNOL_CHECK(launch_gradient(ctx, f, xfull_dev, nfull, pos_dev, i0, i1, R > 1 ? fdx : g, f0_out ? f0 : nullptr));
+		if (R > 1) {
+			PNOL_CHECK(comm_allgather_dev(ctx, fdx + (size_t) ctx->rank * per, fdx, (size_t) per));
+			PNOL_CUDA(ctx, cudaMemcpyAsync(g, fdx, (size_t) nvar * sizeof(double), cudaMemcpyDeviceToDevice, ctx->stream));
+		}
+	} else {
+		// every rank also evaluates the base point (the reference gives it to one rank and sums; SURVEY 3.4)
+		PNOL_CHECK(launch_fd_points(ctx, f, xfull_dev, nfull, pos_dev, dx_dev, i0, i1, fdx, f0));
+		if (R > 1) PNOL_CHECK(comm_allgather_dev(ctx, fdx + (size_t) ctx->rank * per, fdx, (size_t) per));
+		PNOL_CHECK(dg.init(ctx, g_out, (size_t) nvar));
+		PNOL_CHECK(launch_fd_quotient(ctx, fdx, f0, dx_dev, nvar, dg.get() ? dg.get() : gtmp));
+	}
 	PNOL_CHECK(dg.commit());
 	if (f0_out) PNOL_CUDA(ctx, cudaMemcpyAsync(f0_out, f0, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
 	return finish(ctx);
@@ -484,7 +525,16 @@ extern "C" int pnol_fd_gradient(pnol_ctx * ctx, const pnol_functor * f, const do
 	DevIn<double> dxp, ddx;
 	PNOL_CHECK(dxp.init(ctx, x, n));
 	PNOL_CHECK(ddx.init(ctx, dx, n));
-	return fd_gradient_common(ctx, f, dxp.get(), n, nullptr, ddx.get(), n, g_out, f0_out);
+	return gradient_common(ctx, f, dxp.get(), n, nullptr, ddx.get(), n, g_out, f0_out);
+}
+
+extern "C" int pnol_gradient(pnol_ctx * ctx, const pnol_functor * f, const double * x, int n, double * g_out, double * f0_out)
+{
+	if (!ctx || !f) return PNOL_ERR_INVALID;
+	PNOL_REQUIRE(ctx, x && g_out && n >= 1, "gradient: bad arguments");
+	DevIn<double> dxp;
+	PNOL_CHECK(dxp.init(ctx, x, n));
+	return gradient_common(ctx, f, dxp.get(), n, nullptr, nullptr, n, g_out, f0_out);
 }
 
 static int recur_assemble(pnol_ctx * ctx, const double * xr, int nr, const double * const_x, const unsigned char * const_ind,
@@ -530,7 +580,18 @@ extern "C" int pnol_fd_gradient_recur(pnol_ctx * ctx, const pnol_functor * f, co
 	double * xfull; int * pos;
 	PNOL_CHECK(recur_assemble(ctx, xr, nr, const_x, const_ind, nfull, dx_r, dcx, dci, &xfull, &pos));
 	PNOL_CHECK(ddx.init(ctx, dxr, nr));
-	return fd_gradient_common(ctx, f, xfull, nfull, pos, ddx.get(), nr, g_out, f0_out);
+	return gradient_common(ctx, f, xfull, nfull, pos, ddx.get(), nr, g_out, f0_out);
+}
+
+extern "C" int pnol_gradient_recur(pnol_ctx * ctx, const pnol_functor * f, const double * xr, int nr, const double * const_x,
+                                   const unsigned char * const_ind, int nfull, double * g_out, double * f0_out)
+{
+	if (!ctx || !f) return PNOL_ERR_INVALID;
+	PNOL_REQUIRE(ctx, xr && const_x && const_ind && g_out && nfull >= 1 && nr >= 1 && nr <= nfull, "gradient_recur: bad arguments");
+	DevIn<double> dx_r, dcx; DevIn<unsigned char> dci;
+	double * xfull; int * pos;
+	PNOL_CHECK(recur_assemble(ctx, xr, nr, const_x, const_ind, nfull, dx_r, dcx, dci, &xfull, &pos));
+	return gradient_common(ctx, f, xfull, nfull, pos, nullptr, nr, g_out, f0_out);
 }
 
 extern "C" int pnol_fd_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * dx, int n, double * B_out)

@@ -224,6 +224,7 @@ class TimerScope {
 
 // ---- open functor table (pnol_register_functor): launch table of a user kind, nullptr for the built-ins / unknown kinds ----
 const pnol_functor_vtable * user_vtable(int kind);
+pnol_gradient_launcher user_gradient(int kind);    // gradient launcher attached to a user kind's table, nullptr when none
 inline bool is_user_kind(int kind) { return kind >= PNOL_F_USER_SCALAR_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000; }
 inline bool is_residual_kind(int kind) { return (kind >= 100 && kind < PNOL_F_USER_SCALAR_BASE) || (kind >= PNOL_F_USER_RESIDUAL_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000); }
 inline pnol_launch_env make_env(pnol_ctx * ctx)
@@ -267,6 +268,8 @@ int launch_eval_batch(pnol_ctx * ctx, const pnol_functor * f, const double * pts
 int launch_fd_points(pnol_ctx * ctx, const pnol_functor * f, const double * xfull, int nfull, const int * pos,
                      const double * dx, int i0, int i1, double * fdx_out, double * f0_out);
 int launch_fd_quotient(pnol_ctx * ctx, const double * fdx, const double * f0, const double * dx, int n, double * g);
+int launch_gradient(pnol_ctx * ctx, const pnol_functor * f, const double * xfull, int nfull, const int * pos, int i0, int i1,
+                    double * g_out, double * f0_out);
 int launch_assemble_recur(pnol_ctx * ctx, const double * xr, int nr, const double * const_x,
                           const unsigned char * const_ind, int nfull, double * xfull, int * pos, int * nr_found);
 int launch_fd_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * dx, int n,

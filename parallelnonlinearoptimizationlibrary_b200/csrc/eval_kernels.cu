@@ -1,5 +1,5 @@
 // eval_kernels.cu -- scalar-objective launchers: population / batch sweep, forward-difference point evaluation (gradient, Recur
-// gradient, Hessian) and the alpha-pool evaluation of the pooled line searches.
+// gradient, Hessian), the analytic gradient and the alpha-pool evaluation of the pooled line searches.
 //
 // The kernels themselves are templates over the device functor in include/pnol/device/functor_kernels.cuh -- the SAME templates an
 // out-of-tree objective instantiates (open functor table, pnol_register_functor). This file instantiates them for the built-in
@@ -38,6 +38,24 @@ int launch_fd_points(pnol_ctx * ctx, const pnol_functor * f, const double * xful
 		return vt->fd_points(&env, &f->params, xfull, nfull, pos, dx, i0, i1, fdx_out, f0_out);
 	}
 	return dispatch_scalar(ctx, f->kind, [&](auto tag) -> int { return dev::fd_points<decltype(tag)>(&env, f->params, xfull, nfull, pos, dx, i0, i1, fdx_out, f0_out); });
+}
+
+// a3 / a4 / a5, analytic: the functor's partial derivatives, one coordinate per thread (pnol_gradient[_recur])
+int launch_gradient(pnol_ctx * ctx, const pnol_functor * f, const double * xfull, int nfull, const int * pos, int i0, int i1,
+                    double * g_out, double * f0_out)
+{
+	TimerScope ts(ctx, "gradient");
+	const pnol_launch_env env = make_env(ctx);
+	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
+		PNOL_REQUIRE(ctx, vt->fd_points, "functor kind %d is not a scalar objective", f->kind);
+		const pnol_gradient_launcher gl = user_gradient(f->kind);
+		if (!gl) {
+			PNOL_SET_ERR(ctx, "functor kind %d has no analytic gradient: its functor defines no partial() (pnol_register_functor_gradient)", f->kind);
+			return PNOL_ERR_NO_FUNCTOR;
+		}
+		return gl(&env, &f->params, xfull, nfull, pos, i0, i1, g_out, f0_out);
+	}
+	return dispatch_scalar(ctx, f->kind, [&](auto tag) -> int { return dev::gradient<decltype(tag)>(&env, f->params, xfull, nfull, pos, i0, i1, g_out, f0_out); });
 }
 
 // g[i] = (fdx[i] - f0) / dx[i]     (Source/PNOL_Objective.cpp:31, :150-153, :451-454)

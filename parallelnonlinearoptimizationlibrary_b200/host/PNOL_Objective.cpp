@@ -6,6 +6,21 @@
 
 #include <string>
 
+// Weak references: these sources are also linked against C-ABI implementations other than libpnol_b200.so -- the CPU stand-in of the
+// host-logic tests (oracle/host_logic_device.cpp) and programs built with it -- that need not provide the analytic gradient. There the
+// two symbols are null and the analytic mode fails with PNOL_ERR_NO_FUNCTOR (requireGradient) instead of the program failing to link.
+extern "C" int pnol_gradient( pnol_ctx *, const pnol_functor *, const double *, int, double *, double * ) __attribute__(( weak ));
+extern "C" int pnol_gradient_recur( pnol_ctx *, const pnol_functor *, const double *, int, const double *, const unsigned char *, int,
+		double *, double * ) __attribute__(( weak ));
+
+namespace {
+void requireGradient( bool available, const char * who )
+{
+	if( !available ) throw pnol::Error( PNOL_ERR_NO_FUNCTOR, std::string(who) + ": analytic gradients (Runtime::setAnalyticGradient) "
+			"are not provided by the C-ABI implementation this program is linked against" );
+}
+}
+
 pnol_functor * Objective::requireFunctor( const char * who )
 {
 	pnol_functor * f = deviceFunctor();
@@ -32,10 +47,17 @@ void Objective::gradientApproximation( vector <double> & X, vector <double> & dX
 
 // Source/PNOL_Objective.cpp:88-159: the reference deals the N+1 evaluations out to MPI ranks and sums; the values are
 // the same as the serial stencil. With a communicator attached the C-ABI splits the coordinates across GPUs (collective call).
+// Runtime::setAnalyticGradient(true): the functor's own partial derivatives instead (dX unused, no objective value evaluated).
 void Objective::gradientApproximationMPI( vector <double> & X, vector <double> & dX, vector <double> & dFdX )
 {
 	pnol::Runtime & rt = pnol::Runtime::instance();
 	pnol_functor * f = requireFunctor( "Objective::gradientApproximation" );
+	if( rt.analyticGradient() )
+	{
+		requireGradient( pnol_gradient != nullptr, "Objective::gradientApproximation" );
+		rt.check( pnol_gradient( rt.ctx(), f, X.data(), (int) X.size(), dFdX.data(), nullptr ) );
+		return;
+	}
 	rt.check( pnol_fd_gradient( rt.ctx(), f, X.data(), dX.data(), (int) X.size(), dFdX.data(), nullptr ) );
 	noteDeviceEvaluations( (long long) X.size() + 1 );                        // N + 1 points (:19-32)
 }
@@ -84,6 +106,13 @@ void Objective::gradientApproximationMPIRecur( vector <double> & X, vector <doub
 	pnol_functor * f = requireFunctor( "Objective::gradientApproximationRecur" );
 	vector<unsigned char> ind( constantIndicator.size() );
 	for( size_t i = 0; i < ind.size(); i++ ) ind[i] = constantIndicator[i] ? 1 : 0;
+	if( rt.analyticGradient() )
+	{
+		requireGradient( pnol_gradient_recur != nullptr, "Objective::gradientApproximationRecur" );
+		rt.check( pnol_gradient_recur( rt.ctx(), f, X.data(), (int) X.size(), constantX.data(), ind.data(), (int) constantX.size(),
+				dFdX.data(), nullptr ) );
+		return;
+	}
 	rt.check( pnol_fd_gradient_recur( rt.ctx(), f, X.data(), dX.data(), (int) X.size(), constantX.data(), ind.data(),
 			(int) constantX.size(), dFdX.data(), nullptr ) );
 	noteDeviceEvaluations( (long long) X.size() + 1 );                        // (:345-358)

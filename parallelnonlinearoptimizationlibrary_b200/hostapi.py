@@ -71,6 +71,12 @@ def set_jac_mode(mode):
     lib().pnolhost_set_jac_mode(int(mode))
 
 
+def set_analytic_gradient(on):
+    """True: the plugin classes' gradients (Objective::gradientApproximation*, hence the BFGS family) come from the objective's own
+    derivative (pnol_gradient[_recur]) instead of the forward difference (pnol::Runtime::setAnalyticGradient)"""
+    lib().pnolhost_set_analytic_gradient(int(bool(on)))
+
+
 def set_jacobian_cache(on):
     lib().pnolhost_set_jacobian_cache(int(bool(on)))
 
