@@ -74,6 +74,12 @@ class Runtime {
 	// count objective evaluations only.
 	bool analyticGradient() const { return gradAnalytic_; }
 	void setAnalyticGradient(bool on) { gradAnalytic_ = on; }
+	// Hessians of Objective::hessianApproximation (hence initHessFD of the five BFGS classes): the forward difference (false, default)
+	// or the objective's own second derivative (true: pnol_hessian from F::partial2, include/pnol/functors.hpp; dX is ignored, an
+	// objective without one makes the call fail with PNOL_ERR_NO_FUNCTOR). A switch of its own: a functor may define partial() without
+	// partial2(). In the analytic mode a Hessian evaluates no objective value and adds nothing to the evaluation counts.
+	bool analyticHessian() const { return hessAnalytic_; }
+	void setAnalyticHessian(bool on) { hessAnalytic_ = on; }
 	void check(int status) const;             // throws pnol::Error with pnol_last_error() text
   private:
 	Runtime();
@@ -88,6 +94,7 @@ class Runtime {
 	bool jacCache_;
 	bool storeJ_ = true;
 	bool gradAnalytic_ = false;
+	bool hessAnalytic_ = false;
 };
 
 // RAII local (non-collective) mode for the serial classes: the reference's BFGS, BFGS_Bnd, LevMarq, GeneticAlgorithm and the

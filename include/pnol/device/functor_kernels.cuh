@@ -7,16 +7,17 @@
  * implementing objEval (Source/PNOL_Objective.hpp:29, :57). Here the device side of that plug-in point is:
  *
  *   1. write the functor once, __host__ __device__, to the concept of include/pnol/functors.hpp (scalar: eval(P, X, n), optionally
- *      partial(P, X, n, j) for pnol_gradient[_recur]; residual model: residual(P, X, n, i), optionally jacobian(P, X, n, i, Ji) for
+ *      partial(P, X, n, j) for pnol_gradient[_recur] and partial2(P, X, n, i, j) for pnol_hessian; residual model: residual(P, X, n, i), optionally jacobian(P, X, n, i, Ji) for
  *      PNOL_JAC_ANALYTIC; optionally kSeparable / sep_init / sep_term for the fast population sweep);
  *   2. in ONE .cu file of your own, compiled with
  *        nvcc -gencode arch=compute_100a,code=sm_100a -fmad=false -Xcompiler -ffp-contract=off -I<repo>/include ...
  *      write   PNOL_REGISTER_SCALAR_FUNCTOR(kind, MyFunctor, n_columns)   or   PNOL_REGISTER_RESIDUAL_FUNCTOR(kind, MyModel, n_columns)
  *      with a kind in [PNOL_F_USER_SCALAR_BASE, +1000) resp. [PNOL_F_USER_RESIDUAL_BASE, +1000);
  *   3. link that object into your program / shared library next to libpnol_b200.so. The macro registers a launch table
- *      (pnol_functor_vtable, include/pnol_b200.h) at load time, and for a scalar functor with partial() also its gradient launcher
- *      (pnol_register_functor_gradient); pnol_functor_create(kind) and every entry point that takes a functor -- pnol_eval_batch,
- *      pnol_fd_gradient[_recur], pnol_gradient[_recur], pnol_fd_hessian, pnol_alpha_pool, the GA, pnol_residual_eval,
+ *      (pnol_functor_vtable, include/pnol_b200.h) at load time, and for a scalar functor with partial() / partial2() also its gradient /
+ *      Hessian launcher (pnol_register_functor_gradient / _hessian); pnol_functor_create(kind) and every entry point that takes a
+ *      functor -- pnol_eval_batch, pnol_fd_gradient[_recur], pnol_gradient[_recur], pnol_fd_hessian, pnol_hessian, pnol_alpha_pool,
+ *      the GA, pnol_residual_eval,
  *      pnol_fd_jacobian, pnol_lm_step / pnol_lm_iterate -- then launch YOUR instantiations of the kernels below on the
  *      context's stream. The built-in objectives run through exactly these templates (csrc/eval_kernels.cu, residual_kernels.cu).
  *
@@ -407,6 +408,20 @@ int gradient(const pnol_launch_env * env, const FunctorParams & P, const double 
 	return PNOL_OK;
 }
 
+// pair -> (i, j), i <= j, row-major over the upper triangle of an n x n matrix: row i starts at s(i) = i*n - i*(i-1)/2; solved by a
+// floating estimate, then fixed up
+__device__ __forceinline__ void unrank_upper(long long pair, int n, int & i, int & j)
+{
+	double nn = (double) n;
+	double est = (2.0 * nn + 1.0 - sqrt((2.0 * nn + 1.0) * (2.0 * nn + 1.0) - 8.0 * (double) pair)) * 0.5;
+	i = (int) est;
+	if (i < 0) i = 0;
+	if (i > n - 1) i = n - 1;
+	while (i > 0 && (long long) i * n - (long long) i * (i - 1) / 2 > pair) i--;
+	while ((long long) (i + 1) * n - (long long) (i + 1) * i / 2 <= pair) i++;
+	j = i + (int) (pair - ((long long) i * n - (long long) i * (i - 1) / 2));
+}
+
 // ---------------------------------------------------------------------------------------------------
 // a6: forward-difference Hessian (Objective::hessianApproximation, Source/PNOL_Objective.cpp:38-85).
 // One thread per pair (i <= j): B_ij = (f_ij - f_i - f_j + f) / (dx_i dx_j), mirrored. f_i are the n stencil
@@ -423,19 +438,8 @@ fd_hessian_kernel(FunctorParams P, const double * __restrict__ x, const double *
 	long long pair = (long long) blockIdx.x * blockDim.x + threadIdx.x;
 	long long npairs = (long long) n * (n + 1) / 2;
 	if (pair >= npairs) return;
-	// unrank pair -> (i, j), i <= j, row-major over the upper triangle
-	int i = 0;
-	{
-		// row i starts at s(i) = i*n - i*(i-1)/2 ; solve by floating estimate then fix up
-		double nn = (double) n;
-		double est = (2.0 * nn + 1.0 - sqrt((2.0 * nn + 1.0) * (2.0 * nn + 1.0) - 8.0 * (double) pair)) * 0.5;
-		i = (int) est;
-		if (i < 0) i = 0;
-		if (i > n - 1) i = n - 1;
-		while (i > 0 && (long long) i * n - (long long) i * (i - 1) / 2 > pair) i--;
-		while ((long long) (i + 1) * n - (long long) (i + 1) * i / 2 <= pair) i++;
-	}
-	int j = i + (int) (pair - ((long long) i * n - (long long) i * (i - 1) / 2));
+	int i, j;
+	unrank_upper(pair, n, i, j);
 	double fij;
 	if (i == j) {
 		// XdXij[i] = (X[i] + dX[i]) + dX[i]   (Source/PNOL_Objective.cpp:61-62 with i == j)
@@ -461,6 +465,84 @@ int fd_hessian(const pnol_launch_env * env, const FunctorParams & P, const doubl
 	PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
 	long long npairs = (long long) n * (n + 1) / 2;
 	PNOL_DEV_LAUNCH(env, kern, (unsigned) ((npairs + kFdThreads - 1) / kFdThreads), kFdThreads, smem, P, x, dx, n, fdx, f0, B);
+	return PNOL_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// a6, analytic: H[i][j] = F::partial2(x, i, j) of a scalar functor that defines partial2 (functors.hpp: has_partial2), n x n row-major.
+// The upper triangle is cut into 32 x 32 tiles (bi, bj), bi <= bj, numbered row-major and unranked as fd_hessian_kernel unranks its
+// pairs. A tile is 8 warps, each warp one row of 32 columns at a time, so that every store is one coalesced 256-byte row segment:
+//   - off-diagonal tile: partial2 of its 32 x 32 pairs, stored to rows i / columns j, and parked in a shared tile of odd pitch (33: the
+//     transposed read below is free of bank conflicts), from which the block stores the transpose to rows j / columns i;
+//   - diagonal tile: partial2 for r <= c only; r > c is filled from the shared tile, so each unordered pair is evaluated exactly once
+//     and H[j][i] has the bits of H[i][j].
+// Edge tiles mask rows and columns >= n. For a locally coupled objective partial2 is a few compares, so the kernel is bound by the n^2
+// store. The point is staged in shared memory once per BLOCK with coalesced loads, and a block then walks tiles blockIdx.x,
+// blockIdx.x + gridDim.x, ... (the grid is one wave): staging it once per tile would read n * 8 bytes from L2 for every 16 KB of
+// output, as much as the tile writes at n = 2048 and twice as much at n = 4096. 256 threads a block: 1024 (one tile row per warp, 32
+// warps between two barriers) measured 5-6 % faster at n >= 16384 but 37 % slower a call at n = 4096 (NVIDIA B200, DESIGN 4.3).
+// n range: x and the tile both fit in the opt-in shared memory, n <= (smem_optin - 32 * 33 * 8) / 8 (28000 on a B200).
+// ---------------------------------------------------------------------------------------------------
+constexpr int kHessTile = 32;
+constexpr int kHessPitch = kHessTile + 1;
+constexpr int kHessThreads = 256;
+
+template <class F>
+__global__ void __launch_bounds__(kHessThreads)
+hessian_kernel(FunctorParams P, const double * __restrict__ x, int n, double * __restrict__ H)
+{
+	extern __shared__ double sm[];
+	double * tile = sm;                          // kHessTile x kHessPitch
+	double * xs = sm + kHessTile * kHessPitch;   // n
+#pragma unroll 4
+	for (int j = threadIdx.x; j < n; j += blockDim.x) xs[j] = x[j];
+	__syncthreads();
+	const PtrAcc acc{xs};
+	const int tx = threadIdx.x & (kHessTile - 1), ty = threadIdx.x / kHessTile;
+	constexpr int kRowStep = kHessThreads / kHessTile;
+	const int T = (n + kHessTile - 1) / kHessTile;
+	const long long ntiles = (long long) T * (T + 1) / 2;
+	for (long long t = blockIdx.x; t < ntiles; t += gridDim.x) {
+		int bi, bj;
+		unrank_upper(t, T, bi, bj);
+		const int r0 = bi * kHessTile, c0 = bj * kHessTile;
+		const bool diag = bi == bj;
+		const int j = c0 + tx;
+#pragma unroll 4
+		for (int r = ty; r < kHessTile; r += kRowStep) {
+			const int i = r0 + r;
+			const bool in = i < n && j < n;
+			double v = 0.0;
+			if (in && (!diag || r <= tx)) v = F::partial2(P, acc, n, i, j);
+			if (in && !diag) H[(long long) i * n + j] = v;
+			tile[r * kHessPitch + tx] = v;
+		}
+		__syncthreads();
+		// diagonal tile: row r0 + r, column c0 + tx;  off-diagonal: the transpose, row c0 + r, column r0 + tx
+#pragma unroll 4
+		for (int r = ty; r < kHessTile; r += kRowStep) {
+			const int i = (diag ? r0 : c0) + r, jj = (diag ? c0 : r0) + tx;
+			if (i < n && jj < n) H[(long long) i * n + jj] = diag && r <= tx ? tile[r * kHessPitch + tx] : tile[tx * kHessPitch + r];
+		}
+		__syncthreads();
+	}
+}
+
+template <class F>
+int hessian(const pnol_launch_env * env, const FunctorParams & P, const double * x, int n, double * H)
+{
+	const size_t smem = ((size_t) kHessTile * kHessPitch + (size_t) n) * sizeof(double);
+	PNOL_DEV_REQUIRE(env, n >= 1 && smem <= env->smem_optin, "hessian: n = %d is outside 1 .. %d (the point and one %d x %d tile must fit "
+	                 "in shared memory)", n, (int) ((env->smem_optin / sizeof(double)) - kHessTile * kHessPitch), kHessTile, kHessTile);
+	auto kern = hessian_kernel<F>;
+	PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+	int per_sm = 1;
+	PNOL_DEV_CUDA(env, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kHessThreads, smem));
+	if (per_sm < 1) per_sm = 1;
+	const long long T = (n + kHessTile - 1) / kHessTile;
+	const long long ntiles = T * (T + 1) / 2;
+	const long long cap = (long long) env->sm_count * per_sm;
+	PNOL_DEV_LAUNCH(env, kern, (unsigned) (ntiles < cap ? ntiles : cap), kHessThreads, smem, P, x, n, H);
 	return PNOL_OK;
 }
 
@@ -700,6 +782,8 @@ template <class F> struct ScalarTable {
 	{ return alpha_pool<F>(env, *P, xfull, pfull, is_const, nfull, alpha, npool, dalpha, eval_ind, want_shifted, vals); }
 	static int gradient_(const pnol_launch_env * env, const pnol_functor_params * P, const double * xfull, int nfull, const int * pos, int i0,
 	                     int i1, double * g, double * f0) { return gradient<F>(env, *P, xfull, nfull, pos, i0, i1, g, f0); }
+	static int hessian_(const pnol_launch_env * env, const pnol_functor_params * P, const double * x, int n, double * H)
+	{ return hessian<F>(env, *P, x, n, H); }
 	static pnol_functor_vtable make(int n_columns)
 	{
 		pnol_functor_vtable vt = {};
@@ -711,12 +795,16 @@ template <class F> struct ScalarTable {
 		vt.alpha_pool = alpha_pool_;
 		return vt;
 	}
-	/* registers the table, then (F defines partial) its gradient launcher, in this order: a gradient attaches to the registered table */
+	/* registers the table, then (F defines partial / partial2) its gradient / Hessian launcher, in this order: a derivative attaches to
+	 * the registered table */
 	static int register_as(int kind, const pnol_functor_vtable * vt)
 	{
 		int st = pnol_register_functor(kind, vt);
 		if constexpr (has_partial<F>::value) {
 			if (st == PNOL_OK) st = pnol_register_functor_gradient(kind, gradient_);
+		}
+		if constexpr (has_partial2<F>::value) {
+			if (st == PNOL_OK) st = pnol_register_functor_hessian(kind, hessian_);
 		}
 		return st;
 	}

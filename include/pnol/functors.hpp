@@ -23,6 +23,10 @@
  *     template<class Acc> static double partial(const FunctorParams&, const Acc& X, int n, int j);      // d f / d x_j
  * gradient_kernel (device/functor_kernels.cuh) runs one coordinate per thread and returns its bits. Every built-in scalar objective
  * defines one; each states its operation order, which the tests restate.
+ * And one second derivative per pair (pnol_hessian; detected by has_partial2 below):
+ *     template<class Acc> static double partial2(const FunctorParams&, const Acc& X, int n, int i, int j);   // d2 f / dx_i dx_j
+ * It is only ever called with i <= j: hessian_kernel (device/functor_kernels.cuh) evaluates each unordered pair once and mirrors it,
+ * so H[j][i] has the bits of H[i][j] by construction. Every built-in scalar objective defines one; each states its operation order.
  */
 #ifndef PNOL_FUNCTORS_HPP_
 #define PNOL_FUNCTORS_HPP_
@@ -86,6 +90,20 @@ struct RosenbrockFunctor {
 		if (j >= 1 && j <= n - 2) return a + b;
 		return j >= 1 ? a : b;
 	}
+	/* H_jj = [j >= 1] 200  +  [j <= n-2] (1200 (x_j x_j) - 400 x_{j+1} + 2), in this order, a term whose condition fails left out (n = 1
+	 * gives 0); H_{j,j+1} = -400 x_j; every other entry 0 */
+	template <class Acc> PNOL_HD static double partial2(const FunctorParams &, const Acc & X, int n, int i, int j)
+	{
+		if (j == i + 1) return -400.0 * X[i];
+		if (j != i) return 0.0;
+		double b = 0.0;
+		if (j <= n - 2) {
+			const double xj = X[j], xn = X[j + 1];
+			b = 1200.0 * (xj * xj) - 400.0 * xn + 2.0;
+		}
+		if (j >= 1 && j <= n - 2) return 200.0 + b;
+		return j >= 1 ? 200.0 : b;
+	}
 };
 
 /* Source/ExampleObjectives.hpp:214-224 with the runtime pow(X[k], power) replaced by repeated
@@ -118,6 +136,17 @@ struct PowerFunctor {
 		for (int q = 0; q < power - 1; q++) v = v * x;
 		return (double) power * v;
 	}
+	/* diagonal p (p-1) x^(p-2): v = x^(p-2) by the same repeated multiplication, then (double) (p (p-1)) * v; 0 for p <= 1 and off the
+	 * diagonal */
+	template <class Acc> PNOL_HD static double partial2(const FunctorParams & P, const Acc & X, int, int i, int j)
+	{
+		const int power = (int) P.ints[0];
+		if (i != j || power <= 1) return 0.0;
+		const double x = X[j];
+		double v = 1.0;
+		for (int q = 0; q < power - 2; q++) v = v * x;
+		return (double) (power * (power - 1)) * v;
+	}
 };
 
 /* Source/ExampleObjectives.hpp:58-69 */
@@ -138,6 +167,12 @@ struct BoothFunctor {
 		double a = x + 2 * y - 7;
 		double b = 2 * x + y - 5;
 		return j == 0 ? 2 * a + 4 * b : 4 * a + 2 * b;
+	}
+	/* the constant [[10, 8], [8, 10]]; 0 when i or j >= 2 */
+	template <class Acc> PNOL_HD static double partial2(const FunctorParams &, const Acc &, int, int i, int j)
+	{
+		if (i >= 2 || j >= 2) return 0.0;
+		return i == j ? 10.0 : 8.0;
 	}
 };
 
@@ -170,6 +205,30 @@ struct GoldsteinFunctor {
 		double dB = j == 0 ? (4 * d) * V + d2 * (-32 + 24 * x - 36 * y) : (-6 * d) * V + d2 * (48 - 36 * x + 54 * y);
 		return dA * B + A * dB;
 	}
+	/* product rule on f = A B:  f_ij = A_ij B + A_i B_j + A_j B_i + A B_ij, in this order, with partial()'s names and order for s, d, U, V,
+	 * A, B, dA (= A_x = A_y) and dB (B_x, B_y), and Ux = -14 + 6 x + 6 y, Vx = -32 + 24 x - 36 y, Vy = 48 - 36 x + 54 y:
+	 *   A_ij = 2 U + (4 s) Ux + 6 s2                                   (the same for every pair: U_xx = U_xy = U_yy = 6)
+	 *   B_xx = 8 V + (8 d) Vx + 24 d2,   B_xy = -12 V + (4 d) Vy - (6 d) Vx - 36 d2,   B_yy = 18 V - (12 d) Vy + 54 d2
+	 * 0 when i or j >= 2 */
+	template <class Acc> PNOL_HD static double partial2(const FunctorParams &, const Acc & X, int, int i, int j)
+	{
+		if (i >= 2 || j >= 2) return 0.0;
+		double x = X[0], y = X[1];
+		double s = x + y + 1;
+		double d = 2 * x - 3 * y;
+		double U = 19 - 14 * x + 3 * (x * x) - 14 * y + 6 * x * y + 3 * (y * y);
+		double V = 18 - 32 * x + 12 * (x * x) + 48 * y - 36 * x * y + 27 * (y * y);
+		double s2 = s * s, d2 = d * d;
+		double A = 1 + s2 * U, B = 30 + d2 * V;
+		double Ux = -14 + 6 * x + 6 * y;
+		double Vx = -32 + 24 * x - 36 * y, Vy = 48 - 36 * x + 54 * y;
+		double dA = (2 * s) * U + s2 * Ux;
+		double Bx = (4 * d) * V + d2 * Vx, By = (-6 * d) * V + d2 * Vy;
+		double A2 = 2 * U + (4 * s) * Ux + 6 * s2;
+		double Bi = i == 0 ? Bx : By, Bj = j == 0 ? Bx : By;
+		double B2 = i != j ? -12 * V + (4 * d) * Vy - (6 * d) * Vx - 36 * d2 : (i == 0 ? 8 * V + (8 * d) * Vx + 24 * d2 : 18 * V - (12 * d) * Vy + 54 * d2);
+		return A2 * B + dA * Bj + dA * Bi + A * B2;
+	}
 };
 
 /* ours (BASELINE.json config 4): f = 10 n + sum_k (x_k^2 - 10 cos(2 pi x_k)), sequential sum.
@@ -194,6 +253,12 @@ struct RastriginFunctor {
 	{
 		const double x = X[j];
 		return 2 * x + 62.83185307179586 * sin2pi(x);
+	}
+	/* diagonal 2 + 40 pi^2 cos(2 pi x), as 2 + RN(40 pi^2) * cos2pi(x) (pnol_math.h); 0 off the diagonal */
+	template <class Acc> PNOL_HD static double partial2(const FunctorParams &, const Acc & X, int, int i, int j)
+	{
+		if (i != j) return 0.0;
+		return 2 + 394.78417604357435 * cos2pi(X[j]);
 	}
 };
 
@@ -228,6 +293,28 @@ struct ExpCurveSingleFunctor {
 			g = g + term;
 		}
 		return g;
+	}
+	/* with e, func, d as in eval: the terms 2 (g_i g_j) - (2 d) h_ij, summed sequentially in row order from 0, where g = (e, (x0 e) t, 1)
+	 * is the derivative of func and h its second derivative: h_01 = e t, h_11 = ((x0 e) t) t, every other h_ij = 0 (still multiplied
+	 * and subtracted); 0 when i or j >= 3 */
+	template <class Acc> PNOL_HD static double partial2(const FunctorParams & P, const Acc & X, int, int i, int j)
+	{
+		if (i >= 3 || j >= 3) return 0.0;
+		double H = 0;
+		double x0 = X[0], x1 = X[1], x2 = X[2];
+		for (long long k = 0; k < P.m; k++) {
+			double t = P.col[0][k];
+			double e = exp_hd(x1 * t);
+			double func = x0 * e + x2;
+			double d = P.col[1][k] - func;
+			double g1 = (x0 * e) * t;
+			double gi = i == 0 ? e : (i == 1 ? g1 : 1.0);
+			double gj = j == 0 ? e : (j == 1 ? g1 : 1.0);
+			double h = i == 0 && j == 1 ? e * t : (i == 1 && j == 1 ? g1 * t : 0.0);
+			double term = 2.0 * (gi * gj) - (2.0 * d) * h;
+			H = H + term;
+		}
+		return H;
 	}
 };
 
@@ -341,6 +428,14 @@ template <class R> struct has_jacobian {
 template <class F> struct has_partial {
 	template <class T>
 	static constexpr bool test(decltype(&T::template partial<PtrAcc>)) { return true; }
+	template <class T> static constexpr bool test(...) { return false; }
+	static constexpr bool value = test<F>(nullptr);
+};
+
+/* has_partial2<F>::value: F defines the per-pair analytic Hessian of the concept above */
+template <class F> struct has_partial2 {
+	template <class T>
+	static constexpr bool test(decltype(&T::template partial2<PtrAcc>)) { return true; }
 	template <class T> static constexpr bool test(...) { return false; }
 	static constexpr bool value = test<F>(nullptr);
 };

@@ -128,7 +128,8 @@ typedef struct {
  * A user objective brings its own instantiations of the library's kernel templates (include/pnol/device/functor_kernels.cuh, compiled
  * out of tree by the user's nvcc) and registers their launchers under a kind of its choice:
  *     kinds [PNOL_F_USER_SCALAR_BASE, +1000)   scalar objectives  (eval_batch, fd_points, fd_hessian, alpha_pool; optionally a gradient
- *                                              launcher attached with pnol_register_functor_gradient: pnol_gradient[_recur])
+ *                                              launcher attached with pnol_register_functor_gradient: pnol_gradient[_recur], and
+ *                                              a Hessian launcher attached with pnol_register_functor_hessian: pnol_hessian)
  *     kinds [PNOL_F_USER_RESIDUAL_BASE, +1000) residual models    (residual, fd_jacobian; optionally jacobian: PNOL_JAC_ANALYTIC)
  * pnol_functor_create and every entry point that takes a functor then work for that kind as for the built-ins; libpnol_b200.so is not
  * rebuilt. PNOL_REGISTER_SCALAR_FUNCTOR / PNOL_REGISTER_RESIDUAL_FUNCTOR in that header fill the table and call pnol_register_functor
@@ -196,6 +197,17 @@ int pnol_register_functor_gradient(int kind, pnol_gradient_launcher fn);
 /* 1 when pnol_gradient accepts the kind: every built-in scalar objective, and user scalar kinds with a gradient attached */
 int pnol_functor_has_gradient(int kind);
 
+/* Analytic Hessian of a user scalar kind (pnol_hessian), kept beside its launch table as the gradient launcher is. The launcher writes
+ * all n x n entries H[i * n + j] = d2f/dx_i dx_j (row-major); x and H are DEVICE pointers, the call only enqueues on env->stream.
+ * pnol::dev::ScalarTable<F>::hessian_ (include/pnol/device/functor_kernels.cuh) is one; PNOL_REGISTER_SCALAR_FUNCTOR attaches it for a
+ * functor that defines partial2(). */
+typedef int (*pnol_hessian_launcher)(const pnol_launch_env *, const pnol_functor_params *, const double * x, int n, double * H);
+/* attaches fn to the table currently registered for a SCALAR user kind; pnol_register_functor replacing that table drops it. Returns
+ * PNOL_OK, or PNOL_ERR_INVALID for a residual kind, a kind without a registered table, or fn == NULL. Thread-safe. */
+int pnol_register_functor_hessian(int kind, pnol_hessian_launcher fn);
+/* 1 when pnol_hessian accepts the kind: every built-in scalar objective, and user scalar kinds with a Hessian attached */
+int pnol_functor_has_hessian(int kind);
+
 int pnol_functor_create(pnol_ctx * ctx, const pnol_functor_desc * desc, pnol_functor ** out);
 void pnol_functor_destroy(pnol_functor * f);
 int pnol_functor_is_residual(const pnol_functor * f);     /* 1 for the built-in kinds >= 100 and the user residual range */
@@ -241,6 +253,15 @@ int pnol_gradient_recur(pnol_ctx * ctx, const pnol_functor * f, const double * x
 /* a6: forward-difference Hessian, upper triangle computed and mirrored
  * (Objective::hessianApproximation, Source/PNOL_Objective.cpp:38-85). B_out is n x n. */
 int pnol_fd_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * dx, int n, double * B_out);
+
+/* a6, analytic: H_out[i * n + j] = d2f/dx_i dx_j (n x n, row-major) from the functor's own second derivative (F::partial2,
+ * include/pnol/functors.hpp; for a user kind the launcher attached with pnol_register_functor_hessian). Each unordered pair is evaluated
+ * once and mirrored, so H_out is symmetric bit for bit; every entry is written. x and H_out may be host or device pointers. n range:
+ * 1 .. (opt-in shared memory per block - 32 * 33 * 8) / 8 (28000 on a B200), beyond it PNOL_ERR_INVALID. No collective: with a
+ * communicator attached every rank computes the whole matrix, as pnol_fd_hessian does. A scalar functor without a second derivative is
+ * refused with PNOL_ERR_NO_FUNCTOR (never a silent forward difference), a residual model as pnol_fd_hessian refuses it. All six
+ * built-in scalar objectives have one. */
+int pnol_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, int n, double * H_out);
 
 /* a13: alpha-pool evaluation for the pooled line searches. For k < npool with eval_ind[k] != 0
  * (eval_ind == NULL: all):  phi[k] = f(x + alpha[k] p)  and, when dphi != NULL,

@@ -84,9 +84,9 @@ EXPORTS = [
     "pnol_ctx_sm_count", "pnol_ctx_launches", "pnol_version", "pnol_malloc", "pnol_free", "pnol_memcpy", "pnol_copy_start", "pnol_copy_wait", "pnol_memset",
     "pnol_host_alloc", "pnol_host_free", "pnol_comm_unique_id", "pnol_comm_init", "pnol_comm_rank", "pnol_comm_size",
     "pnol_comm_set_local", "pnol_comm_allreduce_sum", "pnol_comm_allgather", "pnol_comm_broadcast", "pnol_register_functor", "pnol_functor_registered",
-    "pnol_register_functor_gradient", "pnol_functor_has_gradient", "pnol_functor_create",
+    "pnol_register_functor_gradient", "pnol_functor_has_gradient", "pnol_register_functor_hessian", "pnol_functor_has_hessian", "pnol_functor_create",
     "pnol_functor_destroy", "pnol_functor_is_residual", "pnol_functor_rows", "pnol_eval_batch", "pnol_fd_gradient",
-    "pnol_eval_recur", "pnol_fd_gradient_recur", "pnol_gradient", "pnol_gradient_recur", "pnol_fd_hessian", "pnol_alpha_pool", "pnol_residual_eval",
+    "pnol_eval_recur", "pnol_fd_gradient_recur", "pnol_gradient", "pnol_gradient_recur", "pnol_fd_hessian", "pnol_hessian", "pnol_alpha_pool", "pnol_residual_eval",
     "pnol_fd_jacobian", "pnol_lm_normal_eq", "pnol_lm_damp", "pnol_lm_step", "pnol_lm_iterate", "pnol_lm_last_run", "pnol_lm_exchange_mode", "pnol_lm_normal_eq_fused", "pnol_spd_solve", "pnol_lu_inverse",
     "pnol_matvec_neg", "pnol_bfgs_update_hinv", "pnol_dgemm_nn", "pnol_check_box_bounds", "pnol_compute_alpha_bnd",
     "pnol_stream_uniform", "pnol_ga_create", "pnol_ga_destroy", "pnol_ga_init", "pnol_ga_generation",
@@ -389,6 +389,16 @@ class Context:
         B = np.empty((x.size, x.size), dtype=np.float64)
         self.check(self.lib.pnol_fd_hessian(self.h, f.handle, _ptr(x), _ptr(dx), x.size, _ptr(B)))
         return B
+
+    def hessian(self, f, x, H=None, n=None):
+        """analytic Hessian (pnol_hessian) from the functor's own second derivative: returns H (n x n). x and H may be numpy arrays,
+        torch tensors or raw device pointers (then pass n=); H defaults to a new host array"""
+        x = _f64(x)
+        n = _len(x, n)
+        if H is None:
+            H = np.empty((n, n), dtype=np.float64)
+        self.check(self.lib.pnol_hessian(self.h, f.handle, _ptr(x), n, _ptr(H)))
+        return H
 
     def alpha_pool(self, f, x, p, alpha, dalpha, want_dphi=True, eval_ind=None, const_x=None, const_ind=None):
         x, p, alpha = _f64(x), _f64(p), _f64(alpha)

@@ -329,6 +329,7 @@ struct FunctorRegistry {
 	std::map<int, const pnol_functor_vtable *> table;
 	std::vector<std::unique_ptr<pnol_functor_vtable> > copies;
 	std::map<int, pnol_gradient_launcher> gradient;      // pnol_register_functor_gradient: belongs to the table registered at the time
+	std::map<int, pnol_hessian_launcher> hessian;        // pnol_register_functor_hessian: likewise
 };
 FunctorRegistry & registry()
 {
@@ -354,6 +355,14 @@ pnol_gradient_launcher pnol::user_gradient(int kind)
 	return it == r.gradient.end() ? nullptr : it->second;
 }
 
+pnol_hessian_launcher pnol::user_hessian(int kind)
+{
+	FunctorRegistry & r = registry();
+	std::lock_guard<std::mutex> lock(r.mu);
+	auto it = r.hessian.find(kind);
+	return it == r.hessian.end() ? nullptr : it->second;
+}
+
 extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
 {
 	if (!vt || !pnol::is_user_kind(kind)) return PNOL_ERR_INVALID;
@@ -371,7 +380,8 @@ extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
 	std::lock_guard<std::mutex> lock(r.mu);
 	r.table[kind] = c;
 	r.copies.push_back(std::move(copy));
-	r.gradient.erase(kind);                                     // a gradient attached to the replaced table does not carry over
+	r.gradient.erase(kind);                                     // a derivative attached to the replaced table does not carry over
+	r.hessian.erase(kind);
 	return PNOL_OK;
 }
 
@@ -390,6 +400,24 @@ extern "C" int pnol_functor_has_gradient(int kind)
 	switch (kind) {
 		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE: return 1;
 		default: return pnol::user_gradient(kind) != nullptr;
+	}
+}
+
+extern "C" int pnol_register_functor_hessian(int kind, pnol_hessian_launcher fn)
+{
+	if (!fn || !pnol::is_user_kind(kind) || pnol::is_residual_kind(kind)) return PNOL_ERR_INVALID;
+	FunctorRegistry & r = registry();
+	std::lock_guard<std::mutex> lock(r.mu);
+	if (r.table.find(kind) == r.table.end()) return PNOL_ERR_INVALID;
+	r.hessian[kind] = fn;
+	return PNOL_OK;
+}
+
+extern "C" int pnol_functor_has_hessian(int kind)
+{
+	switch (kind) {
+		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE: return 1;
+		default: return pnol::user_hessian(kind) != nullptr;
 	}
 }
 
@@ -608,6 +636,18 @@ extern "C" int pnol_fd_hessian(pnol_ctx * ctx, const pnol_functor * f, const dou
 	PNOL_CHECK(launch_fd_points(ctx, f, dxp.get(), n, nullptr, ddx.get(), 0, n, fdx, f0));
 	PNOL_CHECK(launch_fd_hessian(ctx, f, dxp.get(), ddx.get(), n, fdx, f0, dB.get()));
 	PNOL_CHECK(dB.commit());
+	return finish(ctx);
+}
+
+extern "C" int pnol_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, int n, double * H_out)
+{
+	if (!ctx || !f) return PNOL_ERR_INVALID;
+	PNOL_REQUIRE(ctx, x && H_out && n >= 1, "hessian: bad arguments");
+	DevIn<double> dxp; DevOut<double> dH;
+	PNOL_CHECK(dxp.init(ctx, x, n));
+	PNOL_CHECK(dH.init(ctx, H_out, (size_t) n * n));
+	PNOL_CHECK(launch_hessian(ctx, f, dxp.get(), n, dH.get()));
+	PNOL_CHECK(dH.commit());
 	return finish(ctx);
 }
 

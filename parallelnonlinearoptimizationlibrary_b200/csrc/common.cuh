@@ -225,6 +225,7 @@ class TimerScope {
 // ---- open functor table (pnol_register_functor): launch table of a user kind, nullptr for the built-ins / unknown kinds ----
 const pnol_functor_vtable * user_vtable(int kind);
 pnol_gradient_launcher user_gradient(int kind);    // gradient launcher attached to a user kind's table, nullptr when none
+pnol_hessian_launcher user_hessian(int kind);      // Hessian launcher attached to a user kind's table, nullptr when none
 inline bool is_user_kind(int kind) { return kind >= PNOL_F_USER_SCALAR_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000; }
 inline bool is_residual_kind(int kind) { return (kind >= 100 && kind < PNOL_F_USER_SCALAR_BASE) || (kind >= PNOL_F_USER_RESIDUAL_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000); }
 inline pnol_launch_env make_env(pnol_ctx * ctx)
@@ -274,6 +275,7 @@ int launch_assemble_recur(pnol_ctx * ctx, const double * xr, int nr, const doubl
                           const unsigned char * const_ind, int nfull, double * xfull, int * pos, int * nr_found);
 int launch_fd_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * dx, int n,
                       const double * fdx, const double * f0, double * B);
+int launch_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, int n, double * H);
 int launch_alpha_pool(pnol_ctx * ctx, const pnol_functor * f, const double * xfull, const double * pfull,
                       const unsigned char * is_const, int nfull, const double * alpha, int npool, double dalpha,
                       const unsigned char * eval_ind, double * phi, double * dphi, int * bad_dev);

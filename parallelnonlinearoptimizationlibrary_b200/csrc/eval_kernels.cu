@@ -1,5 +1,5 @@
 // eval_kernels.cu -- scalar-objective launchers: population / batch sweep, forward-difference point evaluation (gradient, Recur
-// gradient, Hessian), the analytic gradient and the alpha-pool evaluation of the pooled line searches.
+// gradient, Hessian), the analytic gradient and Hessian, and the alpha-pool evaluation of the pooled line searches.
 //
 // The kernels themselves are templates over the device functor in include/pnol/device/functor_kernels.cuh -- the SAME templates an
 // out-of-tree objective instantiates (open functor table, pnol_register_functor). This file instantiates them for the built-in
@@ -132,6 +132,23 @@ int launch_fd_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, 
 		return vt->fd_hessian(&env, &f->params, x, dx, n, fdx, f0, B);
 	}
 	return dispatch_scalar(ctx, f->kind, [&](auto tag) -> int { return dev::fd_hessian<decltype(tag)>(&env, f->params, x, dx, n, fdx, f0, B); });
+}
+
+// a6, analytic: the functor's second derivatives, one 32 x 32 tile of the upper triangle at a time, mirrored (pnol_hessian)
+int launch_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, int n, double * H)
+{
+	TimerScope ts(ctx, "hessian");
+	const pnol_launch_env env = make_env(ctx);
+	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
+		PNOL_REQUIRE(ctx, vt->fd_hessian, "functor kind %d is not a scalar objective", f->kind);
+		const pnol_hessian_launcher hl = user_hessian(f->kind);
+		if (!hl) {
+			PNOL_SET_ERR(ctx, "functor kind %d has no analytic Hessian: its functor defines no partial2() (pnol_register_functor_hessian)", f->kind);
+			return PNOL_ERR_NO_FUNCTOR;
+		}
+		return hl(&env, &f->params, x, n, H);
+	}
+	return dispatch_scalar(ctx, f->kind, [&](auto tag) -> int { return dev::hessian<decltype(tag)>(&env, f->params, x, n, H); });
 }
 
 // a13: alpha pool: phi, the forward-difference slope and the NaN/inf -> 1e10 sentinel of evaluateAlphaPoolAndDerivatives

@@ -7,18 +7,20 @@
 #include <string>
 
 // Weak references: these sources are also linked against C-ABI implementations other than libpnol_b200.so -- the CPU stand-in of the
-// host-logic tests (oracle/host_logic_device.cpp) and programs built with it -- that need not provide the analytic gradient. There the
-// two symbols are null and the analytic mode fails with PNOL_ERR_NO_FUNCTOR (requireGradient) instead of the program failing to link.
+// host-logic tests (oracle/host_logic_device.cpp) and programs built with it -- that need not provide the analytic derivatives. There
+// these symbols are null and the analytic modes fail with PNOL_ERR_NO_FUNCTOR (requireDerivative) instead of the program failing to link.
 extern "C" int pnol_gradient( pnol_ctx *, const pnol_functor *, const double *, int, double *, double * ) __attribute__(( weak ));
 extern "C" int pnol_gradient_recur( pnol_ctx *, const pnol_functor *, const double *, int, const double *, const unsigned char *, int,
 		double *, double * ) __attribute__(( weak ));
+extern "C" int pnol_hessian( pnol_ctx *, const pnol_functor *, const double *, int, double * ) __attribute__(( weak ));
 
 namespace {
-void requireGradient( bool available, const char * who )
+void requireDerivative( bool available, const char * who, const char * what )
 {
-	if( !available ) throw pnol::Error( PNOL_ERR_NO_FUNCTOR, std::string(who) + ": analytic gradients (Runtime::setAnalyticGradient) "
+	if( !available ) throw pnol::Error( PNOL_ERR_NO_FUNCTOR, std::string(who) + ": " + what + " "
 			"are not provided by the C-ABI implementation this program is linked against" );
 }
+void requireGradient( bool available, const char * who ) { requireDerivative( available, who, "analytic gradients (Runtime::setAnalyticGradient)" ); }
 }
 
 pnol_functor * Objective::requireFunctor( const char * who )
@@ -62,15 +64,24 @@ void Objective::gradientApproximationMPI( vector <double> & X, vector <double> &
 	noteDeviceEvaluations( (long long) X.size() + 1 );                        // N + 1 points (:19-32)
 }
 
-// Source/PNOL_Objective.cpp:38-85
+// Source/PNOL_Objective.cpp:38-85. Runtime::setAnalyticHessian(true): the functor's own second derivatives instead (dX unused, no
+// objective value evaluated).
 void Objective::hessianApproximation( vector <double> & X, vector <double> & dX, vector<vector<double> > & H )
 {
 	pnol::Runtime & rt = pnol::Runtime::instance();
 	pnol_functor * f = requireFunctor( "Objective::hessianApproximation" );
 	int N = (int) X.size();
 	vector<double> flat( (size_t) N*N );
-	rt.check( pnol_fd_hessian( rt.ctx(), f, X.data(), dX.data(), N, flat.data() ) );
-	noteDeviceEvaluations( 3LL*N*(N + 1)/2 + 1 );                            // what the reference evaluates (:47-71); the kernels reuse f_i
+	if( rt.analyticHessian() )
+	{
+		requireDerivative( pnol_hessian != nullptr, "Objective::hessianApproximation", "analytic Hessians (Runtime::setAnalyticHessian)" );
+		rt.check( pnol_hessian( rt.ctx(), f, X.data(), N, flat.data() ) );
+	}
+	else
+	{
+		rt.check( pnol_fd_hessian( rt.ctx(), f, X.data(), dX.data(), N, flat.data() ) );
+		noteDeviceEvaluations( 3LL*N*(N + 1)/2 + 1 );                        // what the reference evaluates (:47-71); the kernels reuse f_i
+	}
 	for( int i = 0; i < N; i++ )
 		for( int j = 0; j < N; j++ )
 			H[i][j] = flat[(size_t) i*N + j];

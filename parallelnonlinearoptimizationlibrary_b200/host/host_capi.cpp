@@ -65,6 +65,7 @@ int pnolhost_set_jacobian_cache( int on ) { pnol::Runtime::instance().setJacobia
 int pnolhost_set_store_jacobian( int on ) { pnol::Runtime::instance().setStoreJacobian( on != 0 ); return PNOL_OK; }
 int pnolhost_set_jac_mode( int m ) { pnol::Runtime::instance().setJacobianMode( m ); return PNOL_OK; }
 int pnolhost_set_analytic_gradient( int on ) { pnol::Runtime::instance().setAnalyticGradient( on != 0 ); return PNOL_OK; }
+int pnolhost_set_analytic_hessian( int on ) { pnol::Runtime::instance().setAnalyticHessian( on != 0 ); return PNOL_OK; }
 int pnolhost_set_stream( const double * values, unsigned long long n_values, unsigned long long seed, double scale )
 {
 	pnol_stream_desc s;

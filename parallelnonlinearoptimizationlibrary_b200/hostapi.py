@@ -77,6 +77,12 @@ def set_analytic_gradient(on):
     lib().pnolhost_set_analytic_gradient(int(bool(on)))
 
 
+def set_analytic_hessian(on):
+    """True: the plugin classes' Hessians (Objective::hessianApproximation, hence initHessFD of the BFGS family) come from the
+    objective's own second derivative (pnol_hessian) instead of the forward difference (pnol::Runtime::setAnalyticHessian)"""
+    lib().pnolhost_set_analytic_hessian(int(bool(on)))
+
+
 def set_jacobian_cache(on):
     lib().pnolhost_set_jacobian_cache(int(bool(on)))
 
