@@ -50,6 +50,9 @@ class BFGS_Bnd_MPI_SW : public AlgorithmBnd {
 	void serialZoomBnd( double alpha_a, double alpha_b, double phi_a, double phi_b, double dphi_a_dalpha, double dphi_b_dalpha,
 			double phi0, double dphi0dalpha, vector <double> & X, vector <double> & p, vector<double> & constantX, vector<bool> & constantIndicator,
 			int & iter_ls, double & alphaOpt, double & phiOpt, double & dphiOptdalpha );
+	// phi(alpha) and its slope for the serial line search: forward difference, or analytic (Runtime::setAnalyticSlope)
+	void serialPhiAndSlope( double alpha, vector <double> & X, vector <double> & p, vector<double> & constantX,
+			vector<bool> & constantIndicator, double & phi, double & dphi );
 
   public:
 	void findMinBnd( vector <double> & X, vector <double> & Xlb, vector <double> & Xub, double & f0, double & fOpt );

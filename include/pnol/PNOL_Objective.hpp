@@ -73,4 +73,12 @@ class MultiObjective {
 	pnol_functor * requireFunctor( const char * who );
 };
 
+namespace pnol {
+// phi[k] = f(X + alpha[k] p) and its analytic slope p . grad f(X + alpha[k] p) for the BFGS line searches in the mode
+// Runtime::setAnalyticSlope(true): pnol_alpha_pool_analytic on the runtime's context (constInd NULL: no active set). Throws pnol::Error
+// with PNOL_ERR_NO_FUNCTOR when the C-ABI implementation the program is linked against does not provide it.
+void alphaPoolAnalytic( const char * who, pnol_functor * f, const double * X, const double * p, int n, const double * alpha, int npool,
+		const double * constX, const unsigned char * constInd, int nfull, double * phi, double * dphi, int * bad );
+}
+
 #endif /* PNOL_OBJECTIVE_HPP_ */

@@ -80,6 +80,15 @@ class Runtime {
 	// partial2(). In the analytic mode a Hessian evaluates no objective value and adds nothing to the evaluation counts.
 	bool analyticHessian() const { return hessAnalytic_; }
 	void setAnalyticHessian(bool on) { hessAnalytic_ = on; }
+	// Line-search slopes phi'(alpha) = d/dalpha f(X + alpha p) of BFGS, BFGS_Bnd and BFGS_Bnd_MPI_SW: the forward difference with their
+	// dalpha (false, default) or p . grad f(X + alpha p) from the objective's own derivative (true: pnol_alpha_pool_analytic from
+	// F::partial, include/pnol/functors.hpp; dalpha is ignored, an objective without one makes the call fail with PNOL_ERR_NO_FUNCTOR).
+	// Meant to be used together with setAnalyticGradient(true): the strong-Wolfe tests compare every phi'(alpha) with the slope at 0,
+	// p . dFdX, which then has the same bits as the analytic slope at alpha = 0. A switch of its own, so that the analytic gradient alone
+	// keeps its iterates. In the analytic mode a pool entry counts one objective evaluation instead of two. BFGS_MPI and BFGSBnd_MPI
+	// use values only and are not affected.
+	bool analyticSlope() const { return slopeAnalytic_; }
+	void setAnalyticSlope(bool on) { slopeAnalytic_ = on; }
 	void check(int status) const;             // throws pnol::Error with pnol_last_error() text
   private:
 	Runtime();
@@ -95,6 +104,7 @@ class Runtime {
 	bool storeJ_ = true;
 	bool gradAnalytic_ = false;
 	bool hessAnalytic_ = false;
+	bool slopeAnalytic_ = false;
 };
 
 // RAII local (non-collective) mode for the serial classes: the reference's BFGS, BFGS_Bnd, LevMarq, GeneticAlgorithm and the

@@ -7,17 +7,18 @@
  * implementing objEval (Source/PNOL_Objective.hpp:29, :57). Here the device side of that plug-in point is:
  *
  *   1. write the functor once, __host__ __device__, to the concept of include/pnol/functors.hpp (scalar: eval(P, X, n), optionally
- *      partial(P, X, n, j) for pnol_gradient[_recur] and partial2(P, X, n, i, j) for pnol_hessian; residual model: residual(P, X, n, i), optionally jacobian(P, X, n, i, Ji) for
+ *      partial(P, X, n, j) for pnol_gradient[_recur] and pnol_alpha_pool_analytic, and partial2(P, X, n, i, j) for pnol_hessian; residual
+ *      model: residual(P, X, n, i), optionally jacobian(P, X, n, i, Ji) for
  *      PNOL_JAC_ANALYTIC; optionally kSeparable / sep_init / sep_term for the fast population sweep);
  *   2. in ONE .cu file of your own, compiled with
  *        nvcc -gencode arch=compute_100a,code=sm_100a -fmad=false -Xcompiler -ffp-contract=off -I<repo>/include ...
  *      write   PNOL_REGISTER_SCALAR_FUNCTOR(kind, MyFunctor, n_columns)   or   PNOL_REGISTER_RESIDUAL_FUNCTOR(kind, MyModel, n_columns)
  *      with a kind in [PNOL_F_USER_SCALAR_BASE, +1000) resp. [PNOL_F_USER_RESIDUAL_BASE, +1000);
  *   3. link that object into your program / shared library next to libpnol_b200.so. The macro registers a launch table
- *      (pnol_functor_vtable, include/pnol_b200.h) at load time, and for a scalar functor with partial() / partial2() also its gradient /
- *      Hessian launcher (pnol_register_functor_gradient / _hessian); pnol_functor_create(kind) and every entry point that takes a
- *      functor -- pnol_eval_batch, pnol_fd_gradient[_recur], pnol_gradient[_recur], pnol_fd_hessian, pnol_hessian, pnol_alpha_pool,
- *      the GA, pnol_residual_eval,
+ *      (pnol_functor_vtable, include/pnol_b200.h) at load time, and for a scalar functor with partial() also its gradient and slope
+ *      launchers (pnol_register_functor_gradient / _slope), with partial2() its Hessian launcher (pnol_register_functor_hessian);
+ *      pnol_functor_create(kind) and every entry point that takes a functor -- pnol_eval_batch, pnol_fd_gradient[_recur],
+ *      pnol_gradient[_recur], pnol_fd_hessian, pnol_hessian, pnol_alpha_pool, pnol_alpha_pool_analytic, the GA, pnol_residual_eval,
  *      pnol_fd_jacobian, pnol_lm_step / pnol_lm_iterate -- then launch YOUR instantiations of the kernels below on the
  *      context's stream. The built-in objectives run through exactly these templates (csrc/eval_kernels.cu, residual_kernels.cu).
  *
@@ -604,6 +605,73 @@ int alpha_pool(const pnol_launch_env * env, const FunctorParams & P, const doubl
 }
 
 // ---------------------------------------------------------------------------------------------------
+// a13, analytic slope: point k gives phi = f(x + alpha_k p) and phi' = sum_r p_r * df/dx_{pos[r]}(x + alpha_k p) of a scalar functor that
+// defines partial (functors.hpp: has_partial), in place of alpha_pool's forward-difference slope (pnol_alpha_pool_analytic).
+// One block per pool entry. The block stages the trial point xa[j] = is_const[j] ? x[j] : x[j] + alpha_k p[j] in shared memory once --
+// LineAcc's expression, so phi has the bits of alpha_pool's phi. Right after that barrier lane 0 of warp 0 starts the block's long chain,
+// F::eval on xa, while the other warps form prod[r] = g_r * p_r for the reduced coordinates, g_r = F::partial(xa, pos[r]) (pos ==
+// nullptr: r itself; pos[r] < 0, a reduced entry without a slot: 0, as gradient_kernel gives, so that entry contributes 0 * p_r). Those
+// warps then meet on a named barrier of their own, and lane 0 of warp 1 sums the products sequentially in r order, s = 0;
+// s = s + prod[0]; ... That is dotProd's order (include/pnol/UtilityFunctions.hpp), so at alpha = 0 the slope is bit for bit
+// dotProd(pnol_gradient_recur(x), p), the host's dphi0dalpha, and the strong-Wolfe tests compare like with like. A tree reduction
+// would be shorter but would lose that equality; the products and their sequential sum run beside the eval chain and are no longer
+// than it. Starting the eval before the partials rather than after one common barrier measured 54.6 instead of 60.8 us a pool of 9 for
+// Rosenbrock at n = 4096 (NVIDIA B200, DESIGN 4.4).
+// Raw values out, as alpha_pool: vals[k] = phi, vals[npool + k] = phi' (the library applies the 1e10 sentinel to phi only).
+// n range: xa (nfull doubles) and prod (n <= nfull doubles) in shared memory, 16 nfull bytes, less than alpha_pool's 17 nfull + 16.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kSlopeThreads = 256;
+
+template <class F>
+__global__ void __launch_bounds__(kSlopeThreads)
+alpha_slope_kernel(FunctorParams P, const double * __restrict__ xfull, const double * __restrict__ pfull,
+                   const unsigned char * __restrict__ is_const, int nfull, const int * __restrict__ pos, const double * __restrict__ p,
+                   int n, const double * __restrict__ alpha, int npool, const unsigned char * __restrict__ eval_ind,
+                   double * __restrict__ vals /* 2*npool */)
+{
+	const int k = blockIdx.x;
+	if (eval_ind && !eval_ind[k]) return;
+	extern __shared__ double sm[];
+	double * xa = sm;              // nfull
+	double * prod = sm + nfull;    // n
+	const double a = alpha[k];
+	for (int j = threadIdx.x; j < nfull; j += blockDim.x) xa[j] = is_const && is_const[j] ? xfull[j] : xfull[j] + a * pfull[j];
+	__syncthreads();
+	const PtrAcc acc{xa};
+	if (threadIdx.x < 32) {
+		if (threadIdx.x == 0) vals[k] = F::eval(P, acc, nfull);
+		return;
+	}
+	for (int r = threadIdx.x - 32; r < n; r += kSlopeThreads - 32) {
+		const int pr = pos ? pos[r] : r;
+		const double g = pr >= 0 ? F::partial(P, acc, nfull, pr) : 0.0;
+		prod[r] = g * p[r];
+	}
+	asm volatile("bar.sync 1, %0;" :: "n"(kSlopeThreads - 32) : "memory");    // the product warps only: warp 0 is in the eval chain
+	if (threadIdx.x == 32) {
+		double s = 0.0;
+		for (int r = 0; r < n; r++) s = s + prod[r];
+		vals[npool + k] = s;
+	}
+}
+
+/* vals[k] = f(x + alpha_k p), vals[npool + k] = its analytic slope along p (raw: the library applies the sentinel to phi) */
+template <class F>
+int alpha_slope(const pnol_launch_env * env, const FunctorParams & P, const double * xfull, const double * pfull, const unsigned char * is_const,
+                int nfull, const int * pos, const double * p, int n, const double * alpha, int npool, const unsigned char * eval_ind,
+                double * vals)
+{
+	const size_t smem = ((size_t) nfull + (size_t) n) * sizeof(double);
+	PNOL_DEV_REQUIRE(env, n >= 1 && n <= nfull && smem <= env->smem_optin, "alpha slope: n = %d, nfull = %d: needs 1 <= n <= nfull and the "
+	                 "trial point and the products, (nfull + n) * 8 bytes, within %zu bytes of shared memory", n, nfull, env->smem_optin);
+	if (npool <= 0) return PNOL_OK;
+	auto kern = alpha_slope_kernel<F>;
+	PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+	PNOL_DEV_LAUNCH(env, kern, (unsigned) npool, kSlopeThreads, smem, P, xfull, pfull, is_const, nfull, pos, p, n, alpha, npool, eval_ind, vals);
+	return PNOL_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
 // generic residual evaluation: F[i] = r_i(x)        (MultiObjective::objEval, Source/PNOL_Objective.hpp:57)
 // ---------------------------------------------------------------------------------------------------
 template <class R>
@@ -784,6 +852,10 @@ template <class F> struct ScalarTable {
 	                     int i1, double * g, double * f0) { return gradient<F>(env, *P, xfull, nfull, pos, i0, i1, g, f0); }
 	static int hessian_(const pnol_launch_env * env, const pnol_functor_params * P, const double * x, int n, double * H)
 	{ return hessian<F>(env, *P, x, n, H); }
+	static int alpha_slope_(const pnol_launch_env * env, const pnol_functor_params * P, const double * xfull, const double * pfull,
+	                        const unsigned char * is_const, int nfull, const int * pos, const double * p, int n, const double * alpha, int npool,
+	                        const unsigned char * eval_ind, double * vals)
+	{ return alpha_slope<F>(env, *P, xfull, pfull, is_const, nfull, pos, p, n, alpha, npool, eval_ind, vals); }
 	static pnol_functor_vtable make(int n_columns)
 	{
 		pnol_functor_vtable vt = {};
@@ -795,13 +867,14 @@ template <class F> struct ScalarTable {
 		vt.alpha_pool = alpha_pool_;
 		return vt;
 	}
-	/* registers the table, then (F defines partial / partial2) its gradient / Hessian launcher, in this order: a derivative attaches to
-	 * the registered table */
+	/* registers the table, then (F defines partial) its gradient and line-search slope launchers and (F defines partial2) its Hessian
+	 * launcher, in this order: a derivative attaches to the registered table */
 	static int register_as(int kind, const pnol_functor_vtable * vt)
 	{
 		int st = pnol_register_functor(kind, vt);
 		if constexpr (has_partial<F>::value) {
 			if (st == PNOL_OK) st = pnol_register_functor_gradient(kind, gradient_);
+			if (st == PNOL_OK) st = pnol_register_functor_slope(kind, alpha_slope_);
 		}
 		if constexpr (has_partial2<F>::value) {
 			if (st == PNOL_OK) st = pnol_register_functor_hessian(kind, hessian_);

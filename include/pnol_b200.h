@@ -129,7 +129,8 @@ typedef struct {
  * out of tree by the user's nvcc) and registers their launchers under a kind of its choice:
  *     kinds [PNOL_F_USER_SCALAR_BASE, +1000)   scalar objectives  (eval_batch, fd_points, fd_hessian, alpha_pool; optionally a gradient
  *                                              launcher attached with pnol_register_functor_gradient: pnol_gradient[_recur], and
- *                                              a Hessian launcher attached with pnol_register_functor_hessian: pnol_hessian)
+ *                                              a Hessian launcher attached with pnol_register_functor_hessian: pnol_hessian, and
+ *                                              a slope launcher attached with pnol_register_functor_slope: pnol_alpha_pool_analytic)
  *     kinds [PNOL_F_USER_RESIDUAL_BASE, +1000) residual models    (residual, fd_jacobian; optionally jacobian: PNOL_JAC_ANALYTIC)
  * pnol_functor_create and every entry point that takes a functor then work for that kind as for the built-ins; libpnol_b200.so is not
  * rebuilt. PNOL_REGISTER_SCALAR_FUNCTOR / PNOL_REGISTER_RESIDUAL_FUNCTOR in that header fill the table and call pnol_register_functor
@@ -208,6 +209,21 @@ int pnol_register_functor_hessian(int kind, pnol_hessian_launcher fn);
 /* 1 when pnol_hessian accepts the kind: every built-in scalar objective, and user scalar kinds with a Hessian attached */
 int pnol_functor_has_hessian(int kind);
 
+/* Analytic line-search slopes of a user scalar kind (pnol_alpha_pool_analytic), kept beside its launch table as the gradient launcher
+ * is. For k < npool with eval_ind[k] != 0 (eval_ind NULL: all) the launcher writes the RAW values vals[k] = f(xa) and
+ * vals[npool + k] = sum_r p[r] * df/dx_{pos[r]}(xa), summed sequentially in r order, r < n (pos NULL: pos[r] = r; pos[r] < 0: the term is
+ * 0 * p[r]), at xa[j] = is_const[j] ? xfull[j] : xfull[j] + alpha[k] * pfull[j] (is_const NULL: never); p is the reduced direction, pfull
+ * its expansion. Every pointer is a DEVICE pointer, the call only enqueues on env->stream. pnol::dev::ScalarTable<F>::alpha_slope_
+ * (include/pnol/device/functor_kernels.cuh) is one; PNOL_REGISTER_SCALAR_FUNCTOR attaches it for a functor that defines partial(). */
+typedef int (*pnol_slope_launcher)(const pnol_launch_env *, const pnol_functor_params *, const double * xfull, const double * pfull,
+                                   const unsigned char * is_const, int nfull, const int * pos, const double * p, int n,
+                                   const double * alpha, int npool, const unsigned char * eval_ind, double * vals /* 2 * npool */);
+/* attaches fn to the table currently registered for a SCALAR user kind; pnol_register_functor replacing that table drops it. Returns
+ * PNOL_OK, or PNOL_ERR_INVALID for a residual kind, a kind without a registered table, or fn == NULL. Thread-safe. */
+int pnol_register_functor_slope(int kind, pnol_slope_launcher fn);
+/* 1 when pnol_alpha_pool_analytic accepts the kind: every built-in scalar objective, and user scalar kinds with a slope attached */
+int pnol_functor_has_slope(int kind);
+
 int pnol_functor_create(pnol_ctx * ctx, const pnol_functor_desc * desc, pnol_functor ** out);
 void pnol_functor_destroy(pnol_functor * f);
 int pnol_functor_is_residual(const pnol_functor * f);     /* 1 for the built-in kinds >= 100 and the user residual range */
@@ -272,6 +288,21 @@ int pnol_alpha_pool(pnol_ctx * ctx, const pnol_functor * f, const double * x, co
                     const double * alpha, int npool, double dalpha, const unsigned char * eval_ind,
                     const double * const_x, const unsigned char * const_ind, int nfull,
                     double * phi, double * dphi, int * bad_out);
+
+/* a13, analytic slope: pnol_alpha_pool with dphi[k] = d/dalpha f(x + alpha p) at alpha[k] from the functor's own partial derivatives
+ * (F::partial, include/pnol/functors.hpp; for a user kind the launcher attached with pnol_register_functor_slope) instead of a forward
+ * difference: dphi[k] = sum_r p[r] * g_r, summed sequentially in r order as dotProd sums (include/pnol/UtilityFunctions.hpp), where g is
+ * what pnol_gradient[_recur] returns at the trial point (with an active set: reduced entries beyond the free variables give 0 * p[r]).
+ * At alpha = 0 (no -0 in x, p finite) dphi is therefore dotProd(pnol_gradient_recur(x), p) bit for bit. phi[k] has the bits of
+ * pnol_alpha_pool's phi[k]; NaN/inf values of phi are replaced by the 1e10 sentinel and counted in *bad_out (bad_out may be NULL), the
+ * slope is left raw. One objective evaluation per entry. dphi is required; entries with eval_ind[k] == 0 keep the caller's phi[k] and
+ * dphi[k]. x, p, alpha, eval_ind, phi and dphi may be host or device pointers. n range: (nfull + n) * 8 bytes of shared memory, which
+ * covers every n pnol_alpha_pool accepts; beyond it PNOL_ERR_INVALID. No collective. A scalar functor without partial() is refused
+ * with PNOL_ERR_NO_FUNCTOR (never a silent forward difference), a residual model as pnol_alpha_pool refuses it. */
+int pnol_alpha_pool_analytic(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * p, int n,
+                             const double * alpha, int npool, const unsigned char * eval_ind,
+                             const double * const_x, const unsigned char * const_ind, int nfull,
+                             double * phi, double * dphi, int * bad_out);
 
 /* ---------------------------------------------------------------------------------------------------
  * a2 / a10: residual evaluation F = F(x) over this context's rows; sumsq_out (optional) receives the

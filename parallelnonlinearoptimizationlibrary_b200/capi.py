@@ -84,9 +84,11 @@ EXPORTS = [
     "pnol_ctx_sm_count", "pnol_ctx_launches", "pnol_version", "pnol_malloc", "pnol_free", "pnol_memcpy", "pnol_copy_start", "pnol_copy_wait", "pnol_memset",
     "pnol_host_alloc", "pnol_host_free", "pnol_comm_unique_id", "pnol_comm_init", "pnol_comm_rank", "pnol_comm_size",
     "pnol_comm_set_local", "pnol_comm_allreduce_sum", "pnol_comm_allgather", "pnol_comm_broadcast", "pnol_register_functor", "pnol_functor_registered",
-    "pnol_register_functor_gradient", "pnol_functor_has_gradient", "pnol_register_functor_hessian", "pnol_functor_has_hessian", "pnol_functor_create",
+    "pnol_register_functor_gradient", "pnol_functor_has_gradient", "pnol_register_functor_hessian", "pnol_functor_has_hessian",
+    "pnol_register_functor_slope", "pnol_functor_has_slope", "pnol_functor_create",
     "pnol_functor_destroy", "pnol_functor_is_residual", "pnol_functor_rows", "pnol_eval_batch", "pnol_fd_gradient",
-    "pnol_eval_recur", "pnol_fd_gradient_recur", "pnol_gradient", "pnol_gradient_recur", "pnol_fd_hessian", "pnol_hessian", "pnol_alpha_pool", "pnol_residual_eval",
+    "pnol_eval_recur", "pnol_fd_gradient_recur", "pnol_gradient", "pnol_gradient_recur", "pnol_fd_hessian", "pnol_hessian", "pnol_alpha_pool",
+    "pnol_alpha_pool_analytic", "pnol_residual_eval",
     "pnol_fd_jacobian", "pnol_lm_normal_eq", "pnol_lm_damp", "pnol_lm_step", "pnol_lm_iterate", "pnol_lm_last_run", "pnol_lm_exchange_mode", "pnol_lm_normal_eq_fused", "pnol_spd_solve", "pnol_lu_inverse",
     "pnol_matvec_neg", "pnol_bfgs_update_hinv", "pnol_dgemm_nn", "pnol_check_box_bounds", "pnol_compute_alpha_bnd",
     "pnol_stream_uniform", "pnol_ga_create", "pnol_ga_destroy", "pnol_ga_init", "pnol_ga_generation",
@@ -413,6 +415,27 @@ class Context:
         self.check(self.lib.pnol_alpha_pool(self.h, f.handle, _ptr(x), _ptr(p), x.size, _ptr(alpha), npool,
                                             C.c_double(dalpha), _ptr(ei), _ptr(cx), _ptr(ci), nfull, _ptr(phi), _ptr(dphi),
                                             C.byref(bad)))
+        return phi, dphi, bad.value
+
+    def alpha_pool_analytic(self, f, x, p, alpha, eval_ind=None, const_x=None, const_ind=None, phi=None, dphi=None, n=None, npool=None):
+        """phi = f(x + alpha p) and the analytic slope dphi = p . grad f(x + alpha p) for a pool of step lengths
+        (pnol_alpha_pool_analytic): returns (phi, dphi, bad). x, p, alpha, phi and dphi may be numpy arrays, torch tensors or raw device
+        pointers (then pass n= and npool=); phi and dphi default to new host arrays, and entries with eval_ind == 0 keep what they
+        held"""
+        x, p, alpha = _f64(x), _f64(p), _f64(alpha)
+        n = _len(x, n)
+        npool = _len(alpha, npool)
+        if phi is None:
+            phi = np.zeros(npool)
+        if dphi is None:
+            dphi = np.zeros(npool)
+        bad = C.c_int()
+        ei = None if eval_ind is None else np.ascontiguousarray(eval_ind, dtype=np.uint8)
+        cx = None if const_x is None else _f64(const_x)
+        ci = None if const_ind is None else np.ascontiguousarray(const_ind, dtype=np.uint8)
+        nfull = n if cx is None else cx.size
+        self.check(self.lib.pnol_alpha_pool_analytic(self.h, f.handle, _ptr(x), _ptr(p), n, _ptr(alpha), npool, _ptr(ei), _ptr(cx),
+                                                     _ptr(ci), nfull, _ptr(phi), _ptr(dphi), C.byref(bad)))
         return phi, dphi, bad.value
 
     # ---- residual models ----

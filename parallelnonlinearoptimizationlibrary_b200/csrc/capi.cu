@@ -330,6 +330,7 @@ struct FunctorRegistry {
 	std::vector<std::unique_ptr<pnol_functor_vtable> > copies;
 	std::map<int, pnol_gradient_launcher> gradient;      // pnol_register_functor_gradient: belongs to the table registered at the time
 	std::map<int, pnol_hessian_launcher> hessian;        // pnol_register_functor_hessian: likewise
+	std::map<int, pnol_slope_launcher> slope;            // pnol_register_functor_slope: likewise
 };
 FunctorRegistry & registry()
 {
@@ -363,6 +364,14 @@ pnol_hessian_launcher pnol::user_hessian(int kind)
 	return it == r.hessian.end() ? nullptr : it->second;
 }
 
+pnol_slope_launcher pnol::user_slope(int kind)
+{
+	FunctorRegistry & r = registry();
+	std::lock_guard<std::mutex> lock(r.mu);
+	auto it = r.slope.find(kind);
+	return it == r.slope.end() ? nullptr : it->second;
+}
+
 extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
 {
 	if (!vt || !pnol::is_user_kind(kind)) return PNOL_ERR_INVALID;
@@ -382,6 +391,7 @@ extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
 	r.copies.push_back(std::move(copy));
 	r.gradient.erase(kind);                                     // a derivative attached to the replaced table does not carry over
 	r.hessian.erase(kind);
+	r.slope.erase(kind);
 	return PNOL_OK;
 }
 
@@ -418,6 +428,24 @@ extern "C" int pnol_functor_has_hessian(int kind)
 	switch (kind) {
 		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE: return 1;
 		default: return pnol::user_hessian(kind) != nullptr;
+	}
+}
+
+extern "C" int pnol_register_functor_slope(int kind, pnol_slope_launcher fn)
+{
+	if (!fn || !pnol::is_user_kind(kind) || pnol::is_residual_kind(kind)) return PNOL_ERR_INVALID;
+	FunctorRegistry & r = registry();
+	std::lock_guard<std::mutex> lock(r.mu);
+	if (r.table.find(kind) == r.table.end()) return PNOL_ERR_INVALID;
+	r.slope[kind] = fn;
+	return PNOL_OK;
+}
+
+extern "C" int pnol_functor_has_slope(int kind)
+{
+	switch (kind) {
+		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE: return 1;
+		default: return pnol::user_slope(kind) != nullptr;
 	}
 }
 
@@ -651,17 +679,45 @@ extern "C" int pnol_hessian(pnol_ctx * ctx, const pnol_functor * f, const double
 	return finish(ctx);
 }
 
-extern "C" int pnol_alpha_pool(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * p, int n,
-                               const double * alpha, int npool, double dalpha, const unsigned char * eval_ind,
-                               const double * const_x, const unsigned char * const_ind, int nfull,
-                               double * phi, double * dphi, int * bad_out)
+// The points of a pool in the full space. With an active set (const_ind != NULL) x and p are expanded as objEvalRecur scatters them
+// (p = 0 on constants; the kernels never add alpha*p there) and pos[i] is the slot of reduced entry i; without one they are x and p
+// themselves and pos is NULL.
+struct PoolPoints {
+	DevIn<double> dx, dp, dcx; DevIn<unsigned char> dci;
+	const double * xfull = nullptr; const double * pfull = nullptr; const unsigned char * is_const = nullptr; const int * pos = nullptr;
+};
+static int pool_points(pnol_ctx * ctx, const double * x, const double * p, int n, const double * const_x, const unsigned char * const_ind,
+                       int nfull, PoolPoints & pp)
 {
-	if (!ctx || !f) return PNOL_ERR_INVALID;
-	PNOL_REQUIRE(ctx, x && p && alpha && phi && n >= 1 && npool >= 1, "alpha_pool: bad arguments");
+	if (!const_ind) {
+		PNOL_CHECK(pp.dx.init(ctx, x, n));
+		PNOL_CHECK(pp.dp.init(ctx, p, n));
+		pp.xfull = pp.dx.get(); pp.pfull = pp.dp.get();
+		return PNOL_OK;
+	}
+	PNOL_REQUIRE(ctx, const_x != nullptr, "alpha_pool: const_x missing");
+	double * xf; int * pos;
+	PNOL_CHECK(recur_assemble(ctx, x, n, const_x, const_ind, nfull, pp.dx, pp.dcx, pp.dci, &xf, &pos));
+	// second assembly for p (constants -> 0): reuse the kernel with const_x := zeros
+	PNOL_CHECK(ws_reserve(ctx, 0, (size_t) 2 * nfull * sizeof(double) + 64));
+	double * zeros = (double *) ctx->ws[0];
+	double * pf = zeros + nfull;
+	PNOL_CUDA(ctx, cudaMemsetAsync(zeros, 0, (size_t) nfull * sizeof(double), ctx->stream));
+	PNOL_CHECK(pp.dp.init(ctx, p, n));
+	PNOL_CHECK(launch_assemble_recur(ctx, pp.dp.get(), n, zeros, pp.dci.get(), nfull, pf, nullptr, nullptr));
+	pp.xfull = xf; pp.pfull = pf; pp.is_const = pp.dci.get(); pp.pos = pos;
+	return PNOL_OK;
+}
+
+// the pool's evaluation: the forward-difference slope (dalpha) or, analytic, the functor's own slope (dalpha unused)
+static int alpha_pool_common(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * p, int n, const double * alpha,
+                             int npool, double dalpha, bool analytic, const unsigned char * eval_ind, const double * const_x,
+                             const unsigned char * const_ind, int nfull, double * phi, double * dphi, int * bad_out)
+{
 	const bool recur = const_ind != nullptr;
 	if (!recur) nfull = n;
 	PNOL_REQUIRE(ctx, nfull >= n, "alpha_pool: nfull < n");
-	DevIn<double> dx_, dp_, da_, dcx; DevIn<unsigned char> de_, dci;
+	DevIn<double> da_; DevIn<unsigned char> de_;
 	DevOut<double> dphi_o, dph_o;
 	PNOL_CHECK(da_.init(ctx, alpha, npool));
 	PNOL_CHECK(de_.init(ctx, eval_ind, npool));
@@ -670,29 +726,14 @@ extern "C" int pnol_alpha_pool(pnol_ctx * ctx, const pnol_functor * f, const dou
 	PNOL_CHECK(ws_reserve(ctx, 2, 64));
 	int * bad_dev = (int *) ctx->ws[2];
 	PNOL_CUDA(ctx, cudaMemsetAsync(bad_dev, 0, sizeof(int), ctx->stream));
-	const double * xfull; const double * pfull; const unsigned char * isconst = nullptr;
-	if (recur) {
-		// expand x and p to the full space (p = 0 on constants; the kernel never adds alpha*p there)
-		PNOL_REQUIRE(ctx, const_x != nullptr, "alpha_pool: const_x missing");
-		DevIn<double> dxr;
-		double * xf; int * pos;
-		PNOL_CHECK(recur_assemble(ctx, x, n, const_x, const_ind, nfull, dxr, dcx, dci, &xf, &pos));
-		// second assembly for p (constants -> 0): reuse the kernel with const_x := zeros
-		PNOL_CHECK(ws_reserve(ctx, 0, (size_t) 2 * nfull * sizeof(double) + 64));
-		double * zeros = (double *) ctx->ws[0];
-		double * pf = zeros + nfull;
-		PNOL_CUDA(ctx, cudaMemsetAsync(zeros, 0, (size_t) nfull * sizeof(double), ctx->stream));
-		PNOL_CHECK(dp_.init(ctx, p, n));
-		PNOL_CHECK(launch_assemble_recur(ctx, dp_.get(), n, zeros, dci.get(), nfull, pf, nullptr, nullptr));
-		xfull = xf; pfull = pf; isconst = dci.get();
-		PNOL_CHECK(launch_alpha_pool(ctx, f, xfull, pfull, isconst, nfull, da_.get(), npool, dalpha, de_.get(), dph_o.get(),
+	PoolPoints pp;
+	PNOL_CHECK(pool_points(ctx, x, p, n, const_x, const_ind, nfull, pp));
+	if (analytic)
+		PNOL_CHECK(launch_alpha_slope(ctx, f, pp.xfull, pp.pfull, pp.is_const, nfull, pp.pos, pp.dp.get(), n, da_.get(), npool, de_.get(),
+		                              dph_o.get(), dphi_o.get(), bad_dev));
+	else
+		PNOL_CHECK(launch_alpha_pool(ctx, f, pp.xfull, pp.pfull, pp.is_const, nfull, da_.get(), npool, dalpha, de_.get(), dph_o.get(),
 		                             dphi_o.get(), bad_dev));
-	} else {
-		PNOL_CHECK(dx_.init(ctx, x, n));
-		PNOL_CHECK(dp_.init(ctx, p, n));
-		PNOL_CHECK(launch_alpha_pool(ctx, f, dx_.get(), dp_.get(), nullptr, n, da_.get(), npool, dalpha, de_.get(), dph_o.get(),
-		                             dphi_o.get(), bad_dev));
-	}
 	PNOL_CHECK(dph_o.commit());
 	PNOL_CHECK(dphi_o.commit());
 	int bad = 0;
@@ -700,6 +741,26 @@ extern "C" int pnol_alpha_pool(pnol_ctx * ctx, const pnol_functor * f, const dou
 	PNOL_CHECK(finish(ctx));
 	if (bad_out) *bad_out = bad;
 	return PNOL_OK;
+}
+
+extern "C" int pnol_alpha_pool(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * p, int n,
+                               const double * alpha, int npool, double dalpha, const unsigned char * eval_ind,
+                               const double * const_x, const unsigned char * const_ind, int nfull,
+                               double * phi, double * dphi, int * bad_out)
+{
+	if (!ctx || !f) return PNOL_ERR_INVALID;
+	PNOL_REQUIRE(ctx, x && p && alpha && phi && n >= 1 && npool >= 1, "alpha_pool: bad arguments");
+	return alpha_pool_common(ctx, f, x, p, n, alpha, npool, dalpha, false, eval_ind, const_x, const_ind, nfull, phi, dphi, bad_out);
+}
+
+extern "C" int pnol_alpha_pool_analytic(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * p, int n,
+                                        const double * alpha, int npool, const unsigned char * eval_ind,
+                                        const double * const_x, const unsigned char * const_ind, int nfull,
+                                        double * phi, double * dphi, int * bad_out)
+{
+	if (!ctx || !f) return PNOL_ERR_INVALID;
+	PNOL_REQUIRE(ctx, x && p && alpha && phi && dphi && n >= 1 && npool >= 1, "alpha_pool_analytic: bad arguments");
+	return alpha_pool_common(ctx, f, x, p, n, alpha, npool, 0.0, true, eval_ind, const_x, const_ind, nfull, phi, dphi, bad_out);
 }
 
 // ---------------------------------------------------------------------------------------------------

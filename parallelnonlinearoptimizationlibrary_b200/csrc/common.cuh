@@ -226,6 +226,7 @@ class TimerScope {
 const pnol_functor_vtable * user_vtable(int kind);
 pnol_gradient_launcher user_gradient(int kind);    // gradient launcher attached to a user kind's table, nullptr when none
 pnol_hessian_launcher user_hessian(int kind);      // Hessian launcher attached to a user kind's table, nullptr when none
+pnol_slope_launcher user_slope(int kind);          // line-search slope launcher attached to a user kind's table, nullptr when none
 inline bool is_user_kind(int kind) { return kind >= PNOL_F_USER_SCALAR_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000; }
 inline bool is_residual_kind(int kind) { return (kind >= 100 && kind < PNOL_F_USER_SCALAR_BASE) || (kind >= PNOL_F_USER_RESIDUAL_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000); }
 inline pnol_launch_env make_env(pnol_ctx * ctx)
@@ -279,6 +280,9 @@ int launch_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, int
 int launch_alpha_pool(pnol_ctx * ctx, const pnol_functor * f, const double * xfull, const double * pfull,
                       const unsigned char * is_const, int nfull, const double * alpha, int npool, double dalpha,
                       const unsigned char * eval_ind, double * phi, double * dphi, int * bad_dev);
+int launch_alpha_slope(pnol_ctx * ctx, const pnol_functor * f, const double * xfull, const double * pfull,
+                       const unsigned char * is_const, int nfull, const int * pos, const double * p, int n, const double * alpha,
+                       int npool, const unsigned char * eval_ind, double * phi, double * dphi, int * bad_dev);
 
 // sum of squares: deterministic, fixed 4096-row blocks -> partials -> one 1024-thread block (sumsq_final_sum). partials_out / np_out
 // (both): only the partials are produced and handed back, the caller's own kernel finishes with sumsq_final_sum

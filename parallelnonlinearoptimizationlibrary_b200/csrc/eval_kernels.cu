@@ -1,5 +1,6 @@
 // eval_kernels.cu -- scalar-objective launchers: population / batch sweep, forward-difference point evaluation (gradient, Recur
-// gradient, Hessian), the analytic gradient and Hessian, and the alpha-pool evaluation of the pooled line searches.
+// gradient, Hessian), the analytic gradient and Hessian, and the alpha-pool evaluation of the pooled line searches (forward-difference
+// or analytic slopes).
 //
 // The kernels themselves are templates over the device functor in include/pnol/device/functor_kernels.cuh -- the SAME templates an
 // out-of-tree objective instantiates (open functor table, pnol_register_functor). This file instantiates them for the built-in
@@ -187,6 +188,48 @@ int launch_alpha_pool(pnol_ctx * ctx, const pnol_functor * f, const double * xfu
 	}
 	PNOL_CHECK(st);
 	PNOL_LAUNCH(ctx, alpha_pool_finish_kernel, (npool + 63) / 64, 64, 0, vals, npool, dalpha, eval_ind, dphi != nullptr, phi, dphi, bad_dev);
+	return PNOL_OK;
+}
+
+// a13, analytic slope: the sentinel on phi only, the slope copied raw (as alpha_pool_finish_kernel leaves the forward difference raw).
+// A kernel of its own so that alpha_pool_finish_kernel's code stays as it is.
+__global__ void alpha_slope_finish_kernel(const double * __restrict__ vals, int npool, const unsigned char * __restrict__ eval_ind,
+                                          double * __restrict__ phi, double * __restrict__ dphi, int * __restrict__ bad)
+{
+	int k = blockIdx.x * blockDim.x + threadIdx.x;
+	if (k >= npool) return;
+	if (eval_ind && !eval_ind[k]) return;
+	double ph = vals[k];
+	dphi[k] = vals[npool + k];
+	if (ph != ph || isinf(ph)) { ph = 1e10; atomicAdd(bad, 1); }
+	phi[k] = ph;
+}
+
+// a13, analytic slope: phi and sum_r p_r df/dx_{pos[r]} at each trial point, one block per pool entry (pnol_alpha_pool_analytic)
+int launch_alpha_slope(pnol_ctx * ctx, const pnol_functor * f, const double * xfull, const double * pfull,
+                       const unsigned char * is_const, int nfull, const int * pos, const double * p, int n, const double * alpha,
+                       int npool, const unsigned char * eval_ind, double * phi, double * dphi, int * bad_dev)
+{
+	TimerScope ts(ctx, "alpha_slope");
+	PNOL_CHECK(ws_reserve(ctx, 3, (size_t) 2 * npool * sizeof(double)));
+	double * vals = (double *) ctx->ws[3];
+	const pnol_launch_env env = make_env(ctx);
+	int st;
+	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
+		PNOL_REQUIRE(ctx, vt->alpha_pool, "functor kind %d is not a scalar objective", f->kind);
+		const pnol_slope_launcher sl = user_slope(f->kind);
+		if (!sl) {
+			PNOL_SET_ERR(ctx, "functor kind %d has no analytic line-search slope: its functor defines no partial() (pnol_register_functor_slope)", f->kind);
+			return PNOL_ERR_NO_FUNCTOR;
+		}
+		st = sl(&env, &f->params, xfull, pfull, is_const, nfull, pos, p, n, alpha, npool, eval_ind, vals);
+	} else {
+		st = dispatch_scalar(ctx, f->kind, [&](auto tag) -> int {
+			return dev::alpha_slope<decltype(tag)>(&env, f->params, xfull, pfull, is_const, nfull, pos, p, n, alpha, npool, eval_ind, vals);
+		});
+	}
+	PNOL_CHECK(st);
+	PNOL_LAUNCH(ctx, alpha_slope_finish_kernel, (npool + 63) / 64, 64, 0, vals, npool, eval_ind, phi, dphi, bad_dev);
 	return PNOL_OK;
 }
 

@@ -325,8 +325,8 @@ void BFGS_Bnd_MPI_SW::serialLineSearchBnd( vector <double> & X, vector <double> 
 	int iter_ls = 0;
 	while( iter_ls < maxIterLineSearch )
 	{
-		phii = lineSearchObj( alphai, X, p, constantX, constantIndicator );
-		double dphiidalpha = lineSearchFDDerivative( alphai, phii, X, p, constantX, constantIndicator );
+		double dphiidalpha;
+		serialPhiAndSlope( alphai, X, p, constantX, constantIndicator, phii, dphiidalpha );
 
 		// 1. sufficient decrease violated, or no longer decreasing: the minimum is bracketed (:266-273)
 		if( ( phii > phi0 + c1*alphai*dphi0dalpha ) || ( phii >= phiim1 && iter_ls > 1 ) )
@@ -374,6 +374,29 @@ void BFGS_Bnd_MPI_SW::serialLineSearchBnd( vector <double> & X, vector <double> 
 		cout << "  Line search completed with alpha = " << alphaOpt << " and F = " << Fopt << " after " << iter_ls << " iterations. Note: alphaMax = " << alphaMax << endl;
 }
 
+// one trial step of the serial line search: lineSearchObj + lineSearchFDDerivative (host evaluations, as the reference), or with
+// Runtime::setAnalyticSlope(true) phi and its analytic slope from one device call, a bad phi recomputed on the host (the serial reference
+// lets NaN/inf flow into its comparisons), the device slope kept
+void BFGS_Bnd_MPI_SW::serialPhiAndSlope( double alpha, vector <double> & X, vector <double> & p, vector<double> & constantX,
+		vector<bool> & constantIndicator, double & phi, double & dphi )
+{
+	if( !pnol::Runtime::instance().analyticSlope() )
+	{
+		phi = lineSearchObj( alpha, X, p, constantX, constantIndicator );
+		dphi = lineSearchFDDerivative( alpha, phi, X, p, constantX, constantIndicator );
+		return;
+	}
+	pnol_functor * f = objPtr->deviceFunctor();
+	if( !f ) throw pnol::Error( PNOL_ERR_NO_FUNCTOR, "BFGS_Bnd: the objective has no device functor (no CPU fallback)" );
+	vector<unsigned char> ind( constantIndicator.size() );
+	for( size_t i = 0; i < ind.size(); i++ ) ind[i] = constantIndicator[i] ? 1 : 0;
+	int bad = 0;
+	pnol::alphaPoolAnalytic( "BFGS_Bnd", f, X.data(), p.data(), (int) X.size(), &alpha, 1, constantX.data(), ind.data(), (int) constantX.size(),
+			&phi, &dphi, &bad );
+	if( bad == 0 ) objPtr->noteDeviceEvaluations( 1 );
+	else phi = lineSearchObj( alpha, X, p, constantX, constantIndicator );
+}
+
 // Source/BFGS_bnd_linesearch.cpp:385-460
 void BFGS_Bnd_MPI_SW::serialZoomBnd( double alpha_a, double alpha_b, double phi_a, double phi_b, double dphi_a_dalpha, double dphi_b_dalpha,
 		double phi0, double dphi0dalpha, vector <double> & X, vector <double> & p, vector<double> & constantX, vector<bool> & constantIndicator,
@@ -384,8 +407,8 @@ void BFGS_Bnd_MPI_SW::serialZoomBnd( double alpha_a, double alpha_b, double phi_
 	{
 		// 0. new trial step by cubic interpolation (:396-398)
 		double alpha_c = cubicInterpMinSimple( alpha_a, alpha_b, phi_a, phi_b, dphi_a_dalpha, dphi_b_dalpha );
-		double phi_c = lineSearchObj( alpha_c, X, p, constantX, constantIndicator );
-		double dphi_c_dalpha = lineSearchFDDerivative( alpha_c, phi_c, X, p, constantX, constantIndicator );
+		double phi_c, dphi_c_dalpha;
+		serialPhiAndSlope( alpha_c, X, p, constantX, constantIndicator, phi_c, dphi_c_dalpha );
 
 		// 1. shrink the interval from the side with the larger value (:415-431)
 		double phi_min = phi_a;
@@ -490,9 +513,19 @@ void BFGS_Bnd_MPI_SW::evaluateAlphaPoolAndDerivatives( vector <double> & alphaPo
 	vector<unsigned char> ind( constantIndicator.size() );
 	for( size_t i = 0; i < ind.size(); i++ ) ind[i] = constantIndicator[i] ? 1 : 0;
 	int bad = 0;
-	rt.check( pnol_alpha_pool( rt.ctx(), f, X.data(), p.data(), (int) X.size(), alphaPool.data(), N, dalpha, nullptr,
-			constantX.data(), ind.data(), (int) constantX.size(), phiPool.data(), dphidalphaPool.data(), &bad ) );
-	objPtr->noteDeviceEvaluations( 2LL*N );                                  // lineSearchObj + lineSearchFDDerivative per entry (:629-640)
+	if( rt.analyticSlope() )
+	{
+		// Runtime::setAnalyticSlope(true): phi and its analytic slope, one evaluation per entry
+		pnol::alphaPoolAnalytic( "BFGS_Bnd_MPI_SW", f, X.data(), p.data(), (int) X.size(), alphaPool.data(), N, constantX.data(), ind.data(),
+				(int) constantX.size(), phiPool.data(), dphidalphaPool.data(), &bad );
+		objPtr->noteDeviceEvaluations( N );
+	}
+	else
+	{
+		rt.check( pnol_alpha_pool( rt.ctx(), f, X.data(), p.data(), (int) X.size(), alphaPool.data(), N, dalpha, nullptr,
+				constantX.data(), ind.data(), (int) constantX.size(), phiPool.data(), dphidalphaPool.data(), &bad ) );
+		objPtr->noteDeviceEvaluations( 2LL*N );                              // lineSearchObj + lineSearchFDDerivative per entry (:629-640)
+	}
 	for( int i = 0; i < N; i++ )
 		if( phiPool[i] == 1e10 )
 		{

@@ -121,6 +121,15 @@ void BFGS::evalPhiAndSlope( double alpha, vector <double> & X, vector <double> &
 	pnol_functor * f = objPtr->deviceFunctor();
 	if( !f ) throw pnol::Error( PNOL_ERR_NO_FUNCTOR, "BFGS: the objective has no device functor (no CPU fallback)" );
 	int bad = 0;
+	if( rt.analyticSlope() )
+	{
+		// Runtime::setAnalyticSlope(true): the slope p . grad f(X + alpha p), one evaluation; a bad phi is recomputed on the host, the
+		// device slope kept
+		pnol::alphaPoolAnalytic( "BFGS", f, X.data(), p.data(), (int) X.size(), &alpha, 1, nullptr, nullptr, (int) X.size(), &phi, &dphi, &bad );
+		if( bad == 0 ) objPtr->noteDeviceEvaluations( 1 );
+		else phi = lineSearchObj( alpha, X, p );
+		return;
+	}
 	rt.check( pnol_alpha_pool( rt.ctx(), f, X.data(), p.data(), (int) X.size(), &alpha, 1, dalpha, nullptr, nullptr, nullptr,
 			(int) X.size(), &phi, &dphi, &bad ) );
 	if( bad == 0 ) objPtr->noteDeviceEvaluations( 2 );                        // phi and the point of its forward-difference slope

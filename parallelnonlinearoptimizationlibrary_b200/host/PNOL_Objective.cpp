@@ -13,6 +13,8 @@ extern "C" int pnol_gradient( pnol_ctx *, const pnol_functor *, const double *, 
 extern "C" int pnol_gradient_recur( pnol_ctx *, const pnol_functor *, const double *, int, const double *, const unsigned char *, int,
 		double *, double * ) __attribute__(( weak ));
 extern "C" int pnol_hessian( pnol_ctx *, const pnol_functor *, const double *, int, double * ) __attribute__(( weak ));
+extern "C" int pnol_alpha_pool_analytic( pnol_ctx *, const pnol_functor *, const double *, const double *, int, const double *, int,
+		const unsigned char *, const double *, const unsigned char *, int, double *, double *, int * ) __attribute__(( weak ));
 
 namespace {
 void requireDerivative( bool available, const char * who, const char * what )
@@ -21,6 +23,14 @@ void requireDerivative( bool available, const char * who, const char * what )
 			"are not provided by the C-ABI implementation this program is linked against" );
 }
 void requireGradient( bool available, const char * who ) { requireDerivative( available, who, "analytic gradients (Runtime::setAnalyticGradient)" ); }
+}
+
+void pnol::alphaPoolAnalytic( const char * who, pnol_functor * f, const double * X, const double * p, int n, const double * alpha, int npool,
+		const double * constX, const unsigned char * constInd, int nfull, double * phi, double * dphi, int * bad )
+{
+	requireDerivative( pnol_alpha_pool_analytic != nullptr, who, "analytic line-search slopes (Runtime::setAnalyticSlope)" );
+	Runtime & rt = Runtime::instance();
+	rt.check( pnol_alpha_pool_analytic( rt.ctx(), f, X, p, n, alpha, npool, nullptr, constX, constInd, nfull, phi, dphi, bad ) );
 }
 
 pnol_functor * Objective::requireFunctor( const char * who )

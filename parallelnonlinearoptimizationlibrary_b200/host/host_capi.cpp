@@ -25,6 +25,7 @@
 namespace {
 
 std::string gErr;
+long long gLastEvals = 0;          // objective evaluations of the last pnolhost_bfgs run
 
 struct CoutSilencer {
 	std::streambuf * old;
@@ -51,6 +52,16 @@ std::unique_ptr<Objective> makeScalar( const std::string & spec )
 	throw pnol::Error( PNOL_ERR_INVALID, "unknown scalar objective " + spec );
 }
 
+// forwards to an objective and counts what it evaluates: host objEval calls and the points the device reports
+struct CountingObjective : public Objective {
+	Objective & o;
+	long long evals = 0;
+	explicit CountingObjective( Objective & obj ) : o( obj ) {}
+	double objEval( vector <double> & X ) { evals++; return o.objEval( X ); }
+	pnol_functor * deviceFunctor() { return o.deviceFunctor(); }
+	void noteDeviceEvaluations( long long count ) { evals += count; }
+};
+
 }
 
 extern "C" {
@@ -66,6 +77,7 @@ int pnolhost_set_store_jacobian( int on ) { pnol::Runtime::instance().setStoreJa
 int pnolhost_set_jac_mode( int m ) { pnol::Runtime::instance().setJacobianMode( m ); return PNOL_OK; }
 int pnolhost_set_analytic_gradient( int on ) { pnol::Runtime::instance().setAnalyticGradient( on != 0 ); return PNOL_OK; }
 int pnolhost_set_analytic_hessian( int on ) { pnol::Runtime::instance().setAnalyticHessian( on != 0 ); return PNOL_OK; }
+int pnolhost_set_analytic_slope( int on ) { pnol::Runtime::instance().setAnalyticSlope( on != 0 ); return PNOL_OK; }
 int pnolhost_set_stream( const double * values, unsigned long long n_values, unsigned long long seed, double scale )
 {
 	pnol_stream_desc s;
@@ -191,6 +203,27 @@ int pnolhost_hessian( const char * objective, const double * X, const double * d
 	} );
 }
 
+// BFGS_Bnd_MPI_SW::evaluateAlphaPoolAndDerivatives on one pool (constInd NULL: no frozen members, nfull = n); *evals = the objective
+// evaluations it reports
+int pnolhost_alpha_pool_sw( const char * objective, const double * X, const double * p, int n, const double * alpha, int npool,
+		const double * constX, const unsigned char * constInd, int nfull, double * phi, double * dphi, long long * evals )
+{
+	return guarded( [&] {
+		CoutSilencer quiet( true );
+		std::unique_ptr<Objective> obj = makeScalar( objective );
+		CountingObjective counted( *obj );
+		BFGS_Bnd_MPI_SW alg; alg.setObjPtr( counted );
+		vector<double> Xv( X, X + n ), pv( p, p + n ), av( alpha, alpha + npool ), phiv( npool ), dphiv( npool );
+		vector<double> cx( constInd ? constX : X, ( constInd ? constX : X ) + nfull );
+		vector<bool> ci( nfull, false );
+		if( constInd ) for( int i = 0; i < nfull; i++ ) ci[i] = constInd[i] != 0;
+		alg.evaluateAlphaPoolAndDerivatives( av, Xv, pv, cx, ci, phiv, dphiv );
+		memcpy( phi, phiv.data(), npool*sizeof(double) );
+		memcpy( dphi, dphiv.data(), npool*sizeof(double) );
+		if( evals ) *evals = counted.evals;
+	} );
+}
+
 double pnolhost_obj_eval( const char * objective, const double * X, int n )
 {
 	double v = NAN;
@@ -226,7 +259,9 @@ int pnolhost_bfgs( const char * variant, const char * objective, double * X, int
 {
 	return guarded( [&] {
 		CoutSilencer quiet( verbose == 0 );
-		std::unique_ptr<Objective> obj = makeScalar( objective );
+		std::unique_ptr<Objective> made = makeScalar( objective );
+		CountingObjective counted( *made );
+		Objective * obj = &counted;
 		vector<double> Xv( X, X + n );
 		std::string v( variant );
 		double a = 0, b = 0;
@@ -272,8 +307,12 @@ int pnolhost_bfgs( const char * variant, const char * objective, double * X, int
 		if( f0 ) *f0 = a;
 		if( fOpt ) *fOpt = b;
 		if( iters ) *iters = it;
+		gLastEvals = counted.evals;
 	} );
 }
+
+// objective evaluations (host objEval calls and points evaluated on the device twin) of the last pnolhost_bfgs run
+long long pnolhost_last_evaluations() { return gLastEvals; }
 
 // SimplexSearch::findMin on one of the example objectives. p[7] = alpha gamma rho sigma maxIter initRandMax xMinDiff; the start simplex
 // draws from the stream set with pnolhost_set_stream(). report[2] = iterations, stream position

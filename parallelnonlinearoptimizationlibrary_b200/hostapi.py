@@ -83,6 +83,13 @@ def set_analytic_hessian(on):
     lib().pnolhost_set_analytic_hessian(int(bool(on)))
 
 
+def set_analytic_slope(on):
+    """True: the line-search slopes of BFGS, BFGS_Bnd and BFGS_Bnd_MPI_SW come from the objective's own derivative
+    (pnol_alpha_pool_analytic) instead of the forward difference with their dalpha (pnol::Runtime::setAnalyticSlope); meant to be used
+    together with set_analytic_gradient(True)"""
+    lib().pnolhost_set_analytic_slope(int(bool(on)))
+
+
 def set_jacobian_cache(on):
     lib().pnolhost_set_jacobian_cache(int(bool(on)))
 
