@@ -30,6 +30,7 @@ struct LMReport {            // what the last findMin did (the reference only pr
 	double chiSq = 0;
 	double lambda = 0;
 	double xdiff2Norm = 0;
+	int stopped = 0;         // LevMarqBatch: 1 when the x_min_diff rule ended the problem's loop
 };
 void lmFindMin( MultiObjective * obj, double lambda0, double lambdaFactor, double dXGrad, int maxIter, double xMinDiff,
 		int verbose, vector <double> & X, vector <double> & F0, vector <double> & FOpt, LMReport & report );

@@ -16,10 +16,11 @@
  *      with a kind in [PNOL_F_USER_SCALAR_BASE, +1000) resp. [PNOL_F_USER_RESIDUAL_BASE, +1000);
  *   3. link that object into your program / shared library next to libpnol_b200.so. The macro registers a launch table
  *      (pnol_functor_vtable, include/pnol_b200.h) at load time, and for a scalar functor with partial() also its gradient and slope
- *      launchers (pnol_register_functor_gradient / _slope), with partial2() its Hessian launcher (pnol_register_functor_hessian);
+ *      launchers (pnol_register_functor_gradient / _slope), with partial2() its Hessian launcher (pnol_register_functor_hessian), for
+ *      a residual model its batched LM launcher (pnol_register_functor_lm_batch);
  *      pnol_functor_create(kind) and every entry point that takes a functor -- pnol_eval_batch, pnol_fd_gradient[_recur],
  *      pnol_gradient[_recur], pnol_fd_hessian, pnol_hessian, pnol_alpha_pool, pnol_alpha_pool_analytic, the GA, pnol_residual_eval,
- *      pnol_fd_jacobian, pnol_lm_step / pnol_lm_iterate -- then launch YOUR instantiations of the kernels below on the
+ *      pnol_fd_jacobian, pnol_lm_step / pnol_lm_iterate, pnol_lm_batch -- then launch YOUR instantiations of the kernels below on the
  *      context's stream. The built-in objectives run through exactly these templates (csrc/eval_kernels.cu, residual_kernels.cu).
  *
  * Everything here is header-only device / launch code; it needs nothing from the library but pnol_register_functor.
@@ -836,6 +837,271 @@ int jacobian(const pnol_launch_env * env, const FunctorParams & P, const double 
 	return PNOL_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------
+// batched Levenberg-Marquardt (pnol_lm_batch): problem b owns rows [row_off[b], row_off[b+1]) of the functor and row b of X (B x n).
+// One CTA runs one problem's whole LevMarq::findMin (Source/LevenbergMarquardtMPI.cpp:12-173), operation for operation oracle_lm
+// (oracle/pnol_oracle.cpp) restricted to the problem's rows, so every problem returns the bits the reference returns on it alone:
+//   - chi^2 = r * r, r = sqrt(s), s = s + F_k F_k over the rows in ascending order (pow(vector2Norm(F), 2)): thread 0 walks the tile.
+//   - J pass, per tile of TR rows: r0 (column n of the tile) by R::residual; the forward difference (r_i(X + dx_j e_j) - r0) / dx_j with
+//     the IEEE quotient (div_exact) over (row, column) items, or the row of R::jacobian. The owners then add the tile's rows in row
+//     order to their sums, held in registers: pair (i, j <= i) is JTJ[i][j], pair (i, n) is (J^T F)_i, each from 0, never fused.
+//   - A = JTJ (mirrored) with A_ii = (1 + lambda) JTJ_ii, rhs = -(J^T F); the shim's LU with partial pivoting (whole-row swaps, first
+//     largest |entry|, a zero pivot left to IEEE arithmetic) in shared memory: the pivot search, the substitutions and every sequential
+//     sum by thread 0, the row swap and the elimination over the block (each entry still sees its updates in k order).
+//   - X + sigma, its chi^2, the accept / reject rule, the stop ||sigma||_2 < x_min_diff after an accepted step.
+// After a rejected step X is restored, so J, J^T J and J^T F are what they were: the sums are kept (the reference recomputes the
+// same values). No global scratch: the residuals at X are recomputed in each J pass, as gradientApproximation recomputes F.
+// A problem's bits depend on nothing but its own rows, X row, dx and the scalars: not on B, its position or the other problems.
+// Configurations by n (threads, sums per owner thread, tile rows): n <= 8: 32/2/32, <= 16: 64/3/32, <= 32: 128/5/64, <= 64: 256/9/64.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kLmBatchMaxN = 64;
+
+__host__ __device__ inline int lm_batch_pitch(int n) { return (n + 1) | 1; }
+__host__ __device__ inline int lm_batch_nsums(int n) { return n * (n + 1) / 2 + n; }
+// shared memory of one problem: xs, xt, dx, 1/dx, sigma, y (6n), the sums, A (n x (n+1)), the tile, 2 broadcast slots; then n ints
+__host__ __device__ inline size_t lm_batch_smem(int n, int tile_rows)
+{
+	return ((size_t) 6 * n + lm_batch_nsums(n) + (size_t) n * (n + 1) + (size_t) tile_rows * lm_batch_pitch(n) + 2) * sizeof(double) +
+	       (size_t) n * sizeof(int);
+}
+
+template <class R, bool kAnalytic, int T, int OWN, int TR>
+__global__ void __launch_bounds__(T)
+lm_batch_kernel(FunctorParams P, const long long * __restrict__ row_off, int n, double * __restrict__ X, const double * __restrict__ dx,
+                double lambda0, double lambda_factor, double x_min_diff, int max_iter, double * __restrict__ chisq_out,
+                double * __restrict__ lambda_out, int * __restrict__ iters_out, int * __restrict__ stopped_out, double * __restrict__ F_out)
+{
+	extern __shared__ double sm[];
+	const int tid = threadIdx.x;
+	const long long b = blockIdx.x;
+	const long long base = row_off[b];
+	const long long mb = row_off[b + 1] - base;
+	const int pitch = lm_batch_pitch(n);
+	const int NL = n * (n + 1) / 2, NS = NL + n;
+	const int ap = n + 1;
+	double * xs = sm;                 // X
+	double * xt = xs + n;             // trial X
+	double * dxs = xt + n;
+	double * rdx = dxs + n;           // RN(1/dx) or 0 (exact_div.cuh)
+	double * sig = rdx + n;           // sigma
+	double * yv = sig + n;            // forward substitution
+	double * G = yv + n;              // the NS sums of the last J pass
+	double * A = G + NS;              // n x ap
+	double * tile = A + (size_t) n * ap;   // TR x pitch
+	double * bc = tile + (size_t) TR * pitch;   // broadcast slots
+	int * piv = reinterpret_cast<int *>(bc + 2);
+
+	for (int j = tid; j < n; j += T) {
+		xs[j] = X[b * n + j];
+		if (!kAnalytic) { dxs[j] = dx[j]; rdx[j] = make_recip(dx[j]).r; }
+	}
+	// the pairs this thread owns: slot s < NL is (i, j <= i) of the lower triangle row by row, slot NL + i is (i, n)
+	int pa[OWN], pb[OWN];
+#pragma unroll
+	for (int q = 0; q < OWN; q++) {
+		const int s = tid + q * T;
+		pa[q] = -1; pb[q] = 0;
+		if (s < NL) {
+			int i = 0;
+			while ((i + 1) * (i + 2) / 2 <= s) i++;
+			pa[q] = i; pb[q] = s - i * (i + 1) / 2;
+		} else if (s < NS) {
+			pa[q] = s - NL; pb[q] = n;
+		}
+	}
+	__syncthreads();
+
+	// chi^2 at x: tiles of residuals, thread 0 adds their squares in row order
+	auto chisq_at = [&](const double * x) -> double {
+		const PtrAcc acc{x};
+		double s = 0.0;
+		for (long long row0 = 0; row0 < mb; row0 += TR) {
+			const int rows = (int) min((long long) TR, mb - row0);
+			if (tid < rows) tile[tid] = R::residual(P, acc, n, base + row0 + tid);
+			__syncthreads();
+			if (tid == 0)
+				for (int r = 0; r < rows; r++) s = s + tile[r] * tile[r];
+			__syncthreads();
+		}
+		if (tid == 0) { const double root = sqrt(s); bc[0] = root * root; }
+		__syncthreads();
+		const double c = bc[0];
+		__syncthreads();
+		return c;
+	};
+
+	double lambda = lambda0;
+	double chi = chisq_at(xs);
+	int iter = 0, stopped = 0;
+	bool fresh = false;            // G holds the sums at the current X
+	while (iter < max_iter) {
+		if (!fresh) {
+			double acc[OWN];
+#pragma unroll
+			for (int q = 0; q < OWN; q++) acc[q] = 0.0;
+			const PtrAcc ax{xs};
+			for (long long row0 = 0; row0 < mb; row0 += TR) {
+				const int rows = (int) min((long long) TR, mb - row0);
+				if (tid < rows) {
+					const long long i = base + row0 + tid;
+					tile[tid * pitch + n] = R::residual(P, ax, n, i);
+					if constexpr (kAnalytic) R::jacobian(P, ax, n, i, tile + tid * pitch);
+				}
+				if constexpr (!kAnalytic) {
+					__syncthreads();
+					for (int e = tid; e < rows * n; e += T) {
+						const int j = e / rows, r = e - j * rows;
+						const PerturbAcc acc1{xs, j, xs[j] + dxs[j]};       // XdX[j] = XdX[j] + dX[j]   (PNOL_Objective.cpp:186)
+						const double rj = R::residual(P, acc1, n, base + row0 + r);
+						RecipDiv rd; rd.d = dxs[j]; rd.r = rdx[j];
+						tile[r * pitch + j] = div_exact(rj - tile[r * pitch + n], rd);   // (FdX[i] - F[i]) / dX[j]   (:192)
+					}
+				}
+				__syncthreads();
+#pragma unroll
+				for (int q = 0; q < OWN; q++) {
+					if (pa[q] < 0) continue;
+					const double * ci = tile + pa[q];
+					const double * cj = tile + pb[q];
+					double a = acc[q];
+					for (int r = 0; r < rows; r++) a = a + ci[r * pitch] * cj[r * pitch];
+					acc[q] = a;
+				}
+				__syncthreads();
+			}
+#pragma unroll
+			for (int q = 0; q < OWN; q++)
+				if (pa[q] >= 0) G[tid + q * T] = acc[q];
+			fresh = true;
+		}
+		__syncthreads();
+		// damped normal matrix (Source/LevenbergMarquardtMPI.cpp:64-85); piv = identity
+		for (int e = tid; e < n * n; e += T) {
+			const int i = e / n, j = e - i * n;
+			const double s = i >= j ? G[i * (i + 1) / 2 + j] : G[j * (j + 1) / 2 + i];
+			A[i * ap + j] = i == j ? (1 + lambda) * s : s;
+		}
+		for (int i = tid; i < n; i += T) piv[i] = i;
+		__syncthreads();
+		// LU with partial pivoting (oracle/shim/shim_impl.cpp:63-80)
+		for (int k = 0; k < n; k++) {
+			if (tid == 0) {
+				int p = k;
+				double best = fabs(A[k * ap + k]);
+				for (int i = k + 1; i < n; i++)
+					if (fabs(A[i * ap + k]) > best) { best = fabs(A[i * ap + k]); p = i; }
+				if (p != k) { const int t = piv[p]; piv[p] = piv[k]; piv[k] = t; }
+				reinterpret_cast<int *>(bc)[0] = p;
+			}
+			__syncthreads();
+			const int p = reinterpret_cast<const int *>(bc)[0];
+			if (p != k)
+				for (int j = tid; j < n; j += T) { const double t = A[p * ap + j]; A[p * ap + j] = A[k * ap + j]; A[k * ap + j] = t; }
+			__syncthreads();
+			for (int i = k + 1 + tid; i < n; i += T) A[i * ap + k] = A[i * ap + k] / A[k * ap + k];
+			__syncthreads();
+			const int w = n - k - 1;
+			for (int e = tid; e < w * w; e += T) {
+				const int i = k + 1 + e / w, j = k + 1 + e % w;
+				A[i * ap + j] = A[i * ap + j] - A[i * ap + k] * A[k * ap + j];
+			}
+			__syncthreads();
+		}
+		// substitutions (shim_impl.cpp:82-98) with rhs = -(J^T F)
+		if (tid == 0) {
+			for (int i = 0; i < n; i++) {
+				double s = -G[NL + piv[i]];
+				for (int k = 0; k < i; k++) s = s - A[i * ap + k] * yv[k];
+				yv[i] = s;
+			}
+			for (int i = n - 1; i >= 0; i--) {
+				double s = yv[i];
+				for (int k = i + 1; k < n; k++) s = s - A[i * ap + k] * sig[k];
+				sig[i] = s / A[i * ap + i];
+			}
+		}
+		__syncthreads();
+		for (int j = tid; j < n; j += T) xt[j] = xs[j] + sig[j];   // (:97-100)
+		__syncthreads();
+		const double chi_t = chisq_at(xt);                           // (:103-108)
+		if (chi_t >= chi || chi_t != chi_t) {                        // (:110-129)
+			lambda = lambda * lambda_factor;
+		} else {                                                     // (:132-141)
+			lambda = lambda / lambda_factor;
+			chi = chi_t;
+			for (int j = tid; j < n; j += T) xs[j] = xt[j];
+			fresh = false;
+			double s2 = 0.0;
+			for (int j = 0; j < n; j++) s2 = s2 + sig[j] * sig[j];
+			__syncthreads();
+			if (sqrt(s2) < x_min_diff) { stopped = 1; break; }
+		}
+		iter++;
+	}
+	for (int j = tid; j < n; j += T) X[b * n + j] = xs[j];
+	if (tid == 0) {
+		chisq_out[b] = chi;
+		lambda_out[b] = lambda;
+		iters_out[b] = iter;
+		stopped_out[b] = stopped;
+	}
+	if (F_out) {
+		const PtrAcc acc{xs};
+		for (long long r = tid; r < mb; r += T) F_out[base + r] = R::residual(P, acc, n, base + r);
+	}
+}
+
+template <class R, bool kAnalytic, int T, int OWN, int TR>
+int lm_batch_launch(const pnol_launch_env * env, const FunctorParams & P, const long long * row_off, long long B, int n, double * X,
+                    const double * dx, double lambda0, double lambda_factor, double x_min_diff, int max_iter, double * chisq_out,
+                    double * lambda_out, int * iters_out, int * stopped_out, double * F_out)
+{
+	const size_t smem = lm_batch_smem(n, TR);
+	PNOL_DEV_REQUIRE(env, lm_batch_nsums(n) <= OWN * T && smem <= env->smem_optin, "lm batch: n = %d needs %zu bytes of shared memory", n, smem);
+	auto kern = lm_batch_kernel<R, kAnalytic, T, OWN, TR>;
+	PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+	PNOL_DEV_LAUNCH(env, kern, (unsigned) B, T, smem, P, row_off, n, X, dx, lambda0, lambda_factor, x_min_diff, max_iter, chisq_out,
+	                lambda_out, iters_out, stopped_out, F_out);
+	return PNOL_OK;
+}
+
+template <class R, bool kAnalytic>
+int lm_batch_mode(const pnol_launch_env * env, const FunctorParams & P, const long long * row_off, long long B, int n, double * X,
+                  const double * dx, double lambda0, double lambda_factor, double x_min_diff, int max_iter, double * chisq_out,
+                  double * lambda_out, int * iters_out, int * stopped_out, double * F_out)
+{
+#define PNOL_LM_BATCH_CFG(T, OWN, TR) \
+	lm_batch_launch<R, kAnalytic, T, OWN, TR>(env, P, row_off, B, n, X, dx, lambda0, lambda_factor, x_min_diff, max_iter, chisq_out, \
+	                                          lambda_out, iters_out, stopped_out, F_out)
+	if (n <= 8) return PNOL_LM_BATCH_CFG(32, 2, 32);
+	if (n <= 16) return PNOL_LM_BATCH_CFG(64, 3, 32);
+	if (n <= 32) return PNOL_LM_BATCH_CFG(128, 5, 64);
+	return PNOL_LM_BATCH_CFG(256, 9, 64);
+#undef PNOL_LM_BATCH_CFG
+}
+
+/* pnol_lm_batch on device pointers: row_off (B + 1), X (B x n, in/out), dx (n; unused with PNOL_JAC_ANALYTIC), the four per-problem
+ * outputs (B), F_out (rows, may be NULL). The caller has checked row_off. n in 1 .. 64; PNOL_JAC_ANALYTIC needs R::jacobian. */
+template <class R>
+int lm_batch(const pnol_launch_env * env, const FunctorParams & P, const long long * row_off, long long B, int n, double * X, const double * dx,
+             double lambda0, double lambda_factor, double x_min_diff, int max_iter, int jac_mode, double * chisq_out, double * lambda_out,
+             int * iters_out, int * stopped_out, double * F_out)
+{
+	PNOL_DEV_REQUIRE(env, n >= 1 && n <= kLmBatchMaxN, "lm batch: n = %d is outside 1 .. %d", n, kLmBatchMaxN);
+	PNOL_DEV_REQUIRE(env, B >= 0 && B <= 0x7fffffffLL, "lm batch: B = %lld is outside 0 .. 2^31 - 1", B);
+	if (B == 0) return PNOL_OK;
+	if (jac_mode == PNOL_JAC_ANALYTIC) {
+		if constexpr (has_jacobian<R>::value)
+			return lm_batch_mode<R, true>(env, P, row_off, B, n, X, dx, lambda0, lambda_factor, x_min_diff, max_iter, chisq_out, lambda_out,
+			                              iters_out, stopped_out, F_out);
+		PNOL_DEV_ERR(env, "lm batch: the residual model has no analytic Jacobian (jacobian()): PNOL_JAC_ANALYTIC refused");
+		return PNOL_ERR_NO_FUNCTOR;
+	}
+	PNOL_DEV_REQUIRE(env, dx != nullptr, "lm batch: dx is required for a forward-difference Jacobian");
+	return lm_batch_mode<R, false>(env, P, row_off, B, n, X, dx, lambda0, lambda_factor, x_min_diff, max_iter, chisq_out, lambda_out,
+	                               iters_out, stopped_out, F_out);
+}
+
 /* ---- launch tables (pnol_functor_vtable) of a functor type ---- */
 template <class F> struct ScalarTable {
 	static int eval_batch_(const pnol_launch_env * env, const pnol_functor_params * P, const double * pts, long long B, int n, long long ld,
@@ -888,6 +1154,13 @@ template <class R> struct ResidualTable {
 	                        double * F) { return fd_jacobian<R>(env, *P, x, dx, n, J, F); }
 	static int jacobian_(const pnol_launch_env * env, const pnol_functor_params * P, const double * x, int n, double * J, double * F)
 	{ return jacobian<R>(env, *P, x, n, J, F); }
+	static int lm_batch_(const pnol_launch_env * env, const pnol_functor_params * P, const long long * row_off, long long B, int n, double * X,
+	                     const double * dx, double lambda0, double lambda_factor, double x_min_diff, int max_iter, int jac_mode,
+	                     double * chisq_out, double * lambda_out, int * iters_out, int * stopped_out, double * F_out)
+	{
+		return lm_batch<R>(env, *P, row_off, B, n, X, dx, lambda0, lambda_factor, x_min_diff, max_iter, jac_mode, chisq_out, lambda_out,
+		                   iters_out, stopped_out, F_out);
+	}
 	static pnol_functor_vtable make(int n_columns)
 	{
 		pnol_functor_vtable vt = {};
@@ -897,6 +1170,13 @@ template <class R> struct ResidualTable {
 		vt.fd_jacobian = fd_jacobian_;
 		if constexpr (has_jacobian<R>::value) vt.jacobian = jacobian_;      // NULL otherwise: PNOL_JAC_ANALYTIC is refused
 		return vt;
+	}
+	/* registers the table, then attaches its batched LM launcher (it serves PNOL_JAC_ANALYTIC only when R defines jacobian()) */
+	static int register_as(int kind, const pnol_functor_vtable * vt)
+	{
+		int st = pnol_register_functor(kind, vt);
+		if (st == PNOL_OK) st = pnol_register_functor_lm_batch(kind, lm_batch_);
+		return st;
 	}
 };
 
@@ -909,6 +1189,6 @@ template <class R> struct ResidualTable {
 	static const int pnol_reg_##F = pnol::dev::ScalarTable<F>::register_as((KIND), &pnol_vt_##F);
 #define PNOL_REGISTER_RESIDUAL_FUNCTOR(KIND, R, NCOLS)                                                            \
 	static const pnol_functor_vtable pnol_vt_##R = pnol::dev::ResidualTable<R>::make(NCOLS);                      \
-	static const int pnol_reg_##R = pnol_register_functor((KIND), &pnol_vt_##R);
+	static const int pnol_reg_##R = pnol::dev::ResidualTable<R>::register_as((KIND), &pnol_vt_##R);
 
 #endif /* PNOL_DEVICE_FUNCTOR_KERNELS_CUH_ */

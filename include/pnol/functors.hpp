@@ -15,6 +15,8 @@
  * Residual functor concept (row i of the residual vector, data columns in FunctorParams::col):
  *     struct R { static constexpr int kKind;  template<class Acc> static double residual(const FunctorParams&, const Acc& X, int n, long long i); };
  * Acc needs only `double operator[](int) const`.
+ * Batch contract (pnol_lm_batch, which fits many problems whose rows lie back to back in one functor): residual row i reads only row i
+ * of each data column and does not use P.m. All three built-in models below keep it.
  * A residual functor MAY also define its analytic Jacobian row (PNOL_JAC_ANALYTIC; detected by has_jacobian below):
  *     template<class Acc> static void jacobian(const FunctorParams&, const Acc& X, int n, long long i, double * Ji);
  * which writes all n entries Ji[j] = d r_i / d x_j. That one definition is the specification: the kernels (the generic template of

@@ -131,7 +131,8 @@ typedef struct {
  *                                              launcher attached with pnol_register_functor_gradient: pnol_gradient[_recur], and
  *                                              a Hessian launcher attached with pnol_register_functor_hessian: pnol_hessian, and
  *                                              a slope launcher attached with pnol_register_functor_slope: pnol_alpha_pool_analytic)
- *     kinds [PNOL_F_USER_RESIDUAL_BASE, +1000) residual models    (residual, fd_jacobian; optionally jacobian: PNOL_JAC_ANALYTIC)
+ *     kinds [PNOL_F_USER_RESIDUAL_BASE, +1000) residual models    (residual, fd_jacobian; optionally jacobian: PNOL_JAC_ANALYTIC; a batch
+ *                                              LM launcher attached with pnol_register_functor_lm_batch: pnol_lm_batch)
  * pnol_functor_create and every entry point that takes a functor then work for that kind as for the built-ins; libpnol_b200.so is not
  * rebuilt. PNOL_REGISTER_SCALAR_FUNCTOR / PNOL_REGISTER_RESIDUAL_FUNCTOR in that header fill the table and call pnol_register_functor
  * at load time. INTEGRATION.md section A shows the whole recipe; tests/test_gpu_user_functor.py does it end to end. */
@@ -223,6 +224,21 @@ typedef int (*pnol_slope_launcher)(const pnol_launch_env *, const pnol_functor_p
 int pnol_register_functor_slope(int kind, pnol_slope_launcher fn);
 /* 1 when pnol_alpha_pool_analytic accepts the kind: every built-in scalar objective, and user scalar kinds with a slope attached */
 int pnol_functor_has_slope(int kind);
+
+/* Batched Levenberg-Marquardt of a user residual kind (pnol_lm_batch), kept beside its launch table as the gradient launcher is. The
+ * launcher runs the whole fit of every problem with pnol_lm_batch's arguments and semantics (row_off already checked, B >= 1); every
+ * pointer is a DEVICE pointer, the call only enqueues on env->stream. pnol::dev::ResidualTable<R>::lm_batch_
+ * (include/pnol/device/functor_kernels.cuh) is one; PNOL_REGISTER_RESIDUAL_FUNCTOR attaches it, and it serves PNOL_JAC_ANALYTIC only
+ * when R defines jacobian() (else PNOL_ERR_NO_FUNCTOR). */
+typedef int (*pnol_lm_batch_launcher)(const pnol_launch_env *, const pnol_functor_params *, const long long * row_off, long long B, int n,
+                                      double * X, const double * dx, double lambda0, double lambda_factor, double x_min_diff, int max_iter,
+                                      int jac_mode, double * chisq_out, double * lambda_out, int * iters_out, int * stopped_out,
+                                      double * F_out);
+/* attaches fn to the table currently registered for a RESIDUAL user kind; pnol_register_functor replacing that table drops it. Returns
+ * PNOL_OK, or PNOL_ERR_INVALID for a scalar kind, a kind without a registered table, or fn == NULL. Thread-safe. */
+int pnol_register_functor_lm_batch(int kind, pnol_lm_batch_launcher fn);
+/* 1 when pnol_lm_batch accepts the kind: the three built-in residual models, and user residual kinds with a batch launcher attached */
+int pnol_functor_has_lm_batch(int kind);
 
 int pnol_functor_create(pnol_ctx * ctx, const pnol_functor_desc * desc, pnol_functor ** out);
 void pnol_functor_destroy(pnol_functor * f);
@@ -362,6 +378,30 @@ int pnol_lm_step(pnol_ctx * ctx, const pnol_functor * f, const double * x, const
 int pnol_lm_iterate(pnol_ctx * ctx, const pnol_functor * f, double * x, const double * dx, int n, double * J, double * F, double * Ftrial,
                     double * JTJ, double * lambda_inout, double * chisq_inout, double lambda_factor, double x_min_diff, int iterations,
                     int jac_mode, int * accepted_out, int * rejected_out, int * swapped_out);
+
+/* Batched LM: B independent small fits in ONE kernel launch, each problem's whole LevMarq::findMin (Source/LevenbergMarquardtMPI.cpp:
+ * 12-173) on the device without a host round trip. Problem b owns rows [row_off[b], row_off[b+1]) of the functor's rows and row b of X
+ * (B x n, row-major, in/out); it starts from lambda0 and uses dx (n entries, shared by all problems) for the forward difference.
+ * Batch contract of the residual functor: residual row i reads only row i of each data column and does not use P.m (all three
+ * built-in models and every functor written to include/pnol/functors.hpp's concept this way).
+ * Every problem returns, bit for bit, what the reference's findMin returns on that problem alone with the shim's dense helpers
+ * (oracle_lm): chi^2 = pow(vector2Norm(F), 2) summed sequentially in row order; J by the forward difference with the IEEE quotient,
+ * or from R::jacobian with jac_mode = PNOL_JAC_ANALYTIC (any other mode is the forward difference); J^T J and J^T F summed
+ * sequentially in row order from 0, unfused; A_ii = (1 + lambda) JTJ_ii; the LU solve with partial pivoting (a rank-deficient problem
+ * gets a NaN step, which the chi^2 test rejects); accept / reject with lambda * / lambda_factor; the stop ||sigma||_2 < x_min_diff after
+ * an accepted step, or max_iter passes. A problem's bits depend neither on B nor on its position nor on the other problems.
+ * Outputs per problem: X, chisq_out (final chi^2), lambda_out, iters_out (the reference's iteration counter: the pass that stops the
+ * loop is not counted), stopped_out (1 when the x_min_diff rule fired); F_out (may be NULL, one entry per row of the functor) the
+ * residuals at the final X of the problem owning each row (rows outside every problem are left as they are).
+ *   - n in 1 .. 64 (larger problems: pnol_lm_iterate); any row count per problem, 0 and fewer rows than parameters included.
+ *   - Every array may be a host or a device pointer. No collective: under a communicator each rank fits the problems of its rows.
+ *   - B = 0 is a no-op; max_iter = 0 returns the initial chi^2, lambda0 and X unchanged.
+ *   - PNOL_ERR_INVALID: a scalar functor, n outside 1 .. 64, B < 0, row_off not non-decreasing within [0, m], dx == NULL in a
+ *     forward-difference mode, the sum-of-Lorentzians model with n not 2 * 2^j. PNOL_ERR_NO_FUNCTOR: PNOL_JAC_ANALYTIC for a model
+ *     without jacobian(), or a user kind without a batch launcher (pnol_register_functor_lm_batch). */
+int pnol_lm_batch(pnol_ctx * ctx, const pnol_functor * f, const long long * row_off, long long B, int n, double * X, const double * dx,
+                  double lambda0, double lambda_factor, double x_min_diff, int max_iter, int jac_mode, double * chisq_out, double * lambda_out,
+                  int * iters_out, int * stopped_out, double * F_out);
 
 /* Which way the sums of the row-sharded LM step (J^T J | J^T F and the trial chi^2, Source/LevenbergMarquardtMPI.cpp:60-108) travel on
  * this context: 0 one rank, 1 NVLink peer memory inside the step's own kernels (csrc/peer.cu), 2 NCCL all-reduce (a peer mapping

@@ -85,11 +85,12 @@ EXPORTS = [
     "pnol_host_alloc", "pnol_host_free", "pnol_comm_unique_id", "pnol_comm_init", "pnol_comm_rank", "pnol_comm_size",
     "pnol_comm_set_local", "pnol_comm_allreduce_sum", "pnol_comm_allgather", "pnol_comm_broadcast", "pnol_register_functor", "pnol_functor_registered",
     "pnol_register_functor_gradient", "pnol_functor_has_gradient", "pnol_register_functor_hessian", "pnol_functor_has_hessian",
-    "pnol_register_functor_slope", "pnol_functor_has_slope", "pnol_functor_create",
+    "pnol_register_functor_slope", "pnol_functor_has_slope", "pnol_register_functor_lm_batch", "pnol_functor_has_lm_batch",
+    "pnol_functor_create",
     "pnol_functor_destroy", "pnol_functor_is_residual", "pnol_functor_rows", "pnol_eval_batch", "pnol_fd_gradient",
     "pnol_eval_recur", "pnol_fd_gradient_recur", "pnol_gradient", "pnol_gradient_recur", "pnol_fd_hessian", "pnol_hessian", "pnol_alpha_pool",
     "pnol_alpha_pool_analytic", "pnol_residual_eval",
-    "pnol_fd_jacobian", "pnol_lm_normal_eq", "pnol_lm_damp", "pnol_lm_step", "pnol_lm_iterate", "pnol_lm_last_run", "pnol_lm_exchange_mode", "pnol_lm_normal_eq_fused", "pnol_spd_solve", "pnol_lu_inverse",
+    "pnol_fd_jacobian", "pnol_lm_normal_eq", "pnol_lm_damp", "pnol_lm_step", "pnol_lm_iterate", "pnol_lm_last_run", "pnol_lm_exchange_mode", "pnol_lm_batch", "pnol_lm_normal_eq_fused", "pnol_spd_solve", "pnol_lu_inverse",
     "pnol_matvec_neg", "pnol_bfgs_update_hinv", "pnol_dgemm_nn", "pnol_check_box_bounds", "pnol_compute_alpha_bnd",
     "pnol_stream_uniform", "pnol_ga_create", "pnol_ga_destroy", "pnol_ga_init", "pnol_ga_generation",
     "pnol_ga_status_get", "pnol_ga_set_sharding", "pnol_ga_peer_mode", "pnol_ga_get_population", "pnol_ga_get_indices", "pnol_ga_pop_sort", "pnol_ga_check_bounds",
@@ -501,6 +502,36 @@ class Context:
                                             C.byref(lam_c), C.byref(chi_c), C.c_double(factor), C.c_double(x_min_diff), int(iterations),
                                             int(jac_mode), C.byref(acc), C.byref(rej), C.byref(sw)))
         return x, lam_c.value, chi_c.value, acc.value, rej.value, sw.value
+
+    def lm_batch(self, f, row_off, X, dx=None, lambda0=0.001, factor=10.0, x_min_diff=1e-7, max_iter=100, jac_mode=JAC_AUTO,
+                 want_F=False, n=None, B=None, out=None):
+        """Batched LM (pnol_lm_batch): problem b owns rows [row_off[b], row_off[b+1]) of the functor and row b of X (B x n).
+        Returns dict(X, chisq, lam, iters, stopped, F). X is fitted in place when it is a float64 numpy array, torch tensor or raw
+        device pointer (then pass n= and B=); otherwise a fitted copy is returned. dx: n entries (None with jac_mode=JAC_ANALYTIC).
+        out (optional): dict of preallocated outputs under the same names (host or device), e.g. prefilled arrays."""
+        if isinstance(X, np.ndarray) and X.dtype == np.float64 and X.flags["C_CONTIGUOUS"]:
+            Xa = X
+        else:
+            Xa = _f64(X) if not isinstance(X, np.ndarray) else np.array(X, dtype=np.float64)
+        if isinstance(Xa, np.ndarray) and Xa.ndim == 2:
+            B, n = Xa.shape if B is None or n is None else (B, n)
+        ro = row_off if (isinstance(row_off, (int, np.integer)) or hasattr(row_off, "data_ptr")) else \
+            np.ascontiguousarray(row_off, dtype=np.int64)
+        if B is None:
+            B = _len(ro, None) - 1
+        if n is None:
+            n = _len(Xa, None) // max(B, 1)
+        dx = _f64(dx)
+        out = dict(out or {})
+        chisq = out.get("chisq", np.empty(B))
+        lam = out.get("lam", np.empty(B))
+        iters = out.get("iters", np.empty(B, dtype=np.int32))
+        stopped = out.get("stopped", np.empty(B, dtype=np.int32))
+        F = out.get("F", np.empty(f.m) if want_F else None)
+        self.check(self.lib.pnol_lm_batch(self.h, f.handle, _ptr(ro), C.c_longlong(B), int(n), _ptr(Xa), _ptr(dx), C.c_double(lambda0),
+                                          C.c_double(factor), C.c_double(x_min_diff), int(max_iter), int(jac_mode), _ptr(chisq),
+                                          _ptr(lam), _ptr(iters), _ptr(stopped), _ptr(F)))
+        return dict(X=Xa, chisq=chisq, lam=lam, iters=iters, stopped=stopped, F=F)
 
     def lm_exchange_mode(self):
         """0 one rank, 1 NVLink peer memory, 2 NCCL, -1 not decided yet"""

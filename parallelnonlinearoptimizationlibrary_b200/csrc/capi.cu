@@ -331,6 +331,7 @@ struct FunctorRegistry {
 	std::map<int, pnol_gradient_launcher> gradient;      // pnol_register_functor_gradient: belongs to the table registered at the time
 	std::map<int, pnol_hessian_launcher> hessian;        // pnol_register_functor_hessian: likewise
 	std::map<int, pnol_slope_launcher> slope;            // pnol_register_functor_slope: likewise
+	std::map<int, pnol_lm_batch_launcher> lm_batch;      // pnol_register_functor_lm_batch: likewise
 };
 FunctorRegistry & registry()
 {
@@ -372,6 +373,14 @@ pnol_slope_launcher pnol::user_slope(int kind)
 	return it == r.slope.end() ? nullptr : it->second;
 }
 
+pnol_lm_batch_launcher pnol::user_lm_batch(int kind)
+{
+	FunctorRegistry & r = registry();
+	std::lock_guard<std::mutex> lock(r.mu);
+	auto it = r.lm_batch.find(kind);
+	return it == r.lm_batch.end() ? nullptr : it->second;
+}
+
 extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
 {
 	if (!vt || !pnol::is_user_kind(kind)) return PNOL_ERR_INVALID;
@@ -392,6 +401,7 @@ extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
 	r.gradient.erase(kind);                                     // a derivative attached to the replaced table does not carry over
 	r.hessian.erase(kind);
 	r.slope.erase(kind);
+	r.lm_batch.erase(kind);
 	return PNOL_OK;
 }
 
@@ -446,6 +456,24 @@ extern "C" int pnol_functor_has_slope(int kind)
 	switch (kind) {
 		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE: return 1;
 		default: return pnol::user_slope(kind) != nullptr;
+	}
+}
+
+extern "C" int pnol_register_functor_lm_batch(int kind, pnol_lm_batch_launcher fn)
+{
+	if (!fn || !pnol::is_user_kind(kind) || !pnol::is_residual_kind(kind)) return PNOL_ERR_INVALID;
+	FunctorRegistry & r = registry();
+	std::lock_guard<std::mutex> lock(r.mu);
+	if (r.table.find(kind) == r.table.end()) return PNOL_ERR_INVALID;
+	r.lm_batch[kind] = fn;
+	return PNOL_OK;
+}
+
+extern "C" int pnol_functor_has_lm_batch(int kind)
+{
+	switch (kind) {
+		case PNOL_F_EXPCURVE: case PNOL_F_CUBIC: case PNOL_F_LORENTZ_SUM: return 1;
+		default: return pnol::user_lm_batch(kind) != nullptr;
 	}
 }
 

@@ -227,6 +227,7 @@ const pnol_functor_vtable * user_vtable(int kind);
 pnol_gradient_launcher user_gradient(int kind);    // gradient launcher attached to a user kind's table, nullptr when none
 pnol_hessian_launcher user_hessian(int kind);      // Hessian launcher attached to a user kind's table, nullptr when none
 pnol_slope_launcher user_slope(int kind);          // line-search slope launcher attached to a user kind's table, nullptr when none
+pnol_lm_batch_launcher user_lm_batch(int kind);    // batched LM launcher attached to a user residual kind's table, nullptr when none
 inline bool is_user_kind(int kind) { return kind >= PNOL_F_USER_SCALAR_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000; }
 inline bool is_residual_kind(int kind) { return (kind >= 100 && kind < PNOL_F_USER_SCALAR_BASE) || (kind >= PNOL_F_USER_RESIDUAL_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000); }
 inline pnol_launch_env make_env(pnol_ctx * ctx)
@@ -303,6 +304,8 @@ __device__ __forceinline__ double sumsq_final_sum(const double * __restrict__ pa
 	}
 	return red[0];
 }
+// PNOL_ERR_INVALID unless n = 2 * 2^j for the sum-of-Lorentzians model (its balanced tree); PNOL_OK for every other kind
+int lorentz_shape_ok(pnol_ctx * ctx, const pnol_functor * f, int n);
 int launch_fd_jacobian(pnol_ctx * ctx, const pnol_functor * f, const double * x, const double * dx, int n, double * J,
                        double * F, int mode, const double * Fw = nullptr, double * jtf_out = nullptr, bool * jtf_done = nullptr);
 

@@ -12,6 +12,7 @@
 #include "pnol/ExampleObjectives.hpp"
 #include "pnol/LevenbergMarquardt.hpp"
 #include "pnol/LevenbergMarquardtMPI.hpp"
+#include "pnol/LevenbergMarquardtBatch.hpp"
 #include "pnol/BFGS_with_linesearch.hpp"
 #include "pnol/BFGS_with_linesearch_MPI.hpp"
 #include "pnol/BFGS_bnd_linesearch_MPI_SW.hpp"
@@ -61,6 +62,25 @@ struct CountingObjective : public Objective {
 	pnol_functor * deviceFunctor() { return o.deviceFunctor(); }
 	void noteDeviceEvaluations( long long count ) { evals += count; }
 };
+
+// a built-in residual model over caller data (host arrays are copied): the objective LevMarqBatch fits
+template <class R> struct BatchModel : public pnol::FunctorMultiObjective<R> {
+	BatchModel( const double * scalars, const double * const * columns, int ncols, long long m )
+	{
+		for( int k = 0; k < PNOL_MAX_SCALARS; k++ ) this->P.scalars[k] = scalars ? scalars[k] : 0.0;
+		this->cols.resize( ncols );
+		for( int c = 0; c < ncols; c++ ) this->cols[c].assign( columns[c], columns[c] + m );
+		this->bindColumns();
+	}
+};
+
+std::unique_ptr<MultiObjective> makeResidual( int kind, const double * scalars, const double * const * columns, int ncols, long long m )
+{
+	if( kind == PNOL_F_EXPCURVE && ncols == 2 ) return std::unique_ptr<MultiObjective>( new BatchModel<pnol::ExpCurveFunctor>( scalars, columns, ncols, m ) );
+	if( kind == PNOL_F_CUBIC && ncols == 3 ) return std::unique_ptr<MultiObjective>( new BatchModel<pnol::CubicFunctor>( scalars, columns, ncols, m ) );
+	if( kind == PNOL_F_LORENTZ_SUM && ncols == 2 ) return std::unique_ptr<MultiObjective>( new BatchModel<pnol::LorentzSumFunctor>( scalars, columns, ncols, m ) );
+	throw pnol::Error( PNOL_ERR_INVALID, "unknown residual model / column count" );
+}
 
 }
 
@@ -164,6 +184,43 @@ int pnolhost_lm_example( const char * name, double * X, int n, double lambda0, d
 		if( F ) memcpy( F, Fv.data(), m*sizeof(double) );
 		const pnol::LMReport & rep = lm.lastReport();
 		if( report ) { report[0] = rep.iterations; report[1] = rep.accepted; report[2] = rep.rejected; report[3] = rep.chiSq; report[4] = rep.lambda; report[5] = rep.xdiff2Norm; }
+	} );
+}
+
+// LevMarqBatch::findMin(rowOffsets, X, reports) on a built-in residual model (kind, scalars[8], ncols columns of m rows). X is B x n
+// row-major (in/out); iters / stopped / chi / lam receive the per-problem reports
+int pnolhost_lm_batch( int kind, const double * scalars, const double * const * columns, int ncols, long long m, const long long * rowOff,
+		long long B, double * X, int n, double lambda0, double factor, double dxgrad, double maxiter, double xmindiff, int * iters, int * stopped,
+		double * chi, double * lam )
+{
+	return guarded( [&] {
+		std::unique_ptr<MultiObjective> obj = makeResidual( kind, scalars, columns, ncols, m );
+		vector<long long> ro( rowOff, rowOff + B + 1 );
+		vector<vector<double> > Xv( (size_t) B );
+		for( long long b = 0; b < B; b++ ) Xv[b].assign( X + b*n, X + (b + 1)*n );
+		vector<pnol::LMReport> rep;
+		LevMarqBatch lm; lm.setObjPtr( *obj ); lm.setParams( lambda0, factor, dxgrad, maxiter, xmindiff, -1 );
+		lm.findMin( ro, Xv, rep );
+		for( long long b = 0; b < B; b++ )
+		{
+			memcpy( X + b*n, Xv[b].data(), n*sizeof(double) );
+			iters[b] = rep[b].iterations; stopped[b] = rep[b].stopped; chi[b] = rep[b].chiSq; lam[b] = rep[b].lambda;
+		}
+	} );
+}
+
+// the base class's findMin(X, F0, FOpt) of LevMarqBatch: all m rows as one problem
+int pnolhost_lm_batch_single( int kind, const double * scalars, const double * const * columns, int ncols, long long m, double * X, int n,
+		double lambda0, double factor, double dxgrad, double maxiter, double xmindiff, double * F0, double * F )
+{
+	return guarded( [&] {
+		std::unique_ptr<MultiObjective> obj = makeResidual( kind, scalars, columns, ncols, m );
+		vector<double> Xv( X, X + n ), F0v( m ), Fv( m );
+		LevMarqBatch lm; lm.setObjPtr( *obj ); lm.setParams( lambda0, factor, dxgrad, maxiter, xmindiff, -1 );
+		lm.findMin( Xv, F0v, Fv );
+		memcpy( X, Xv.data(), n*sizeof(double) );
+		if( F0 ) memcpy( F0, F0v.data(), m*sizeof(double) );
+		if( F ) memcpy( F, Fv.data(), m*sizeof(double) );
 	} );
 }
 

@@ -137,6 +137,45 @@ def lm_lorentz(t, y, w, x0, lambda0=0.001, factor=10.0, dxgrad=1e-7, maxiter=10,
                 xdiff2Norm=rep[5])
 
 
+def _model_args(kind, scalars, columns):
+    sc = np.zeros(8)
+    sc[:len(scalars)] = scalars
+    cols = [_f64(c) for c in columns]
+    ptrs = (C.c_void_p * len(cols))(*[c.ctypes.data for c in cols])
+    return sc, cols, ptrs
+
+
+def lm_batch_model(kind, scalars, columns, row_off, X, lambda0=0.001, factor=10.0, dxgrad=1e-7, maxiter=100, xmindiff=1e-7):
+    """LevMarqBatch::findMin(rowOffsets, X, reports) on a built-in residual model (capi.F_EXPCURVE / F_CUBIC / F_LORENTZ_SUM) over the
+    columns; X is B x n. The Jacobian mode is the one set with set_jac_mode. Returns dict(X, iters, stopped, chisq, lam)."""
+    sc, cols, ptrs = _model_args(kind, scalars, columns)
+    Xv = np.array(X, dtype=np.float64, order="C")
+    B, n = Xv.shape
+    ro = np.ascontiguousarray(row_off, dtype=np.int64)
+    it, stp = np.zeros(B, dtype=np.int32), np.zeros(B, dtype=np.int32)
+    chi, lam = np.zeros(B), np.zeros(B)
+    _check(lib().pnolhost_lm_batch(int(kind), _p(sc), ptrs, len(cols), C.c_longlong(cols[0].size), _p(ro), C.c_longlong(B), _p(Xv), int(n),
+                                   C.c_double(lambda0), C.c_double(factor), C.c_double(dxgrad), C.c_double(maxiter), C.c_double(xmindiff),
+                                   _p(it), _p(stp), _p(chi), _p(lam)))
+    return dict(X=Xv, iters=it, stopped=stp, chisq=chi, lam=lam)
+
+
+def lm_batch_lorentz(t, y, w, row_off, X, **kw):
+    """LevMarqBatch::findMin on LorentzSumObjective(t, y, w): every problem a spectrum of rows [row_off[b], row_off[b+1])"""
+    return lm_batch_model(capi.F_LORENTZ_SUM, (w,), (t, y), row_off, X, **kw)
+
+
+def lm_batch_single(kind, scalars, columns, x0, lambda0=0.001, factor=10.0, dxgrad=1e-7, maxiter=100, xmindiff=1e-7):
+    """LevMarqBatch::findMin(X, F0, FOpt): all rows as one problem. Returns dict(X, F0, F)."""
+    sc, cols, ptrs = _model_args(kind, scalars, columns)
+    m = cols[0].size
+    Xv = _f64(x0).copy()
+    F0, F = np.empty(m), np.empty(m)
+    _check(lib().pnolhost_lm_batch_single(int(kind), _p(sc), ptrs, len(cols), C.c_longlong(m), _p(Xv), int(Xv.size), C.c_double(lambda0),
+                                          C.c_double(factor), C.c_double(dxgrad), C.c_double(maxiter), C.c_double(xmindiff), _p(F0), _p(F)))
+    return dict(X=Xv, F0=F0, F=F)
+
+
 class LMProblem:
     """A LorentzSumObjective held the way a C++ user holds it (built once from host data); run() is
     `LevMarqMPI lm; lm.setObjPtr(obj); lm.setParams(...); lm.findMin(X, F0, F)` on vectors that live with the problem."""
