@@ -21,7 +21,7 @@
  *      pnol_functor_create(kind) and every entry point that takes a functor -- pnol_eval_batch, pnol_fd_gradient[_recur],
  *      pnol_gradient[_recur], pnol_fd_hessian, pnol_hessian, pnol_alpha_pool, pnol_alpha_pool_analytic, the GA, pnol_residual_eval,
  *      pnol_fd_jacobian, pnol_lm_step / pnol_lm_iterate, pnol_lm_batch -- then launch YOUR instantiations of the kernels below on the
- *      context's stream. The built-in objectives run through exactly these templates (csrc/eval_kernels.cu, residual_kernels.cu).
+ *      context's stream. The built-in objectives run through exactly these templates and tables (csrc/builtin_functors.cu).
  *
  * Everything here is header-only device / launch code; it needs nothing from the library but pnol_register_functor.
  */

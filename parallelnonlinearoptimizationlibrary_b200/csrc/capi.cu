@@ -3,7 +3,6 @@
 #include "common.cuh"
 #include "peer.cuh"
 
-#include <memory>
 #include <mutex>
 #include <vector>
 #include <thread>
@@ -323,62 +322,40 @@ extern "C" int pnol_timer_reset(pnol_ctx * ctx)
 // ---------------------------------------------------------------------------------------------------
 // ---- open functor table (include/pnol_b200.h: pnol_register_functor) ----
 namespace {
-// The library's own copies of the registered tables. A replaced table is kept (`copies`): a launch may still be using it.
+// the records of the registered user kinds: the library's own copy of each table and the side launchers attached to it
 struct FunctorRegistry {
 	std::mutex mu;
-	std::map<int, const pnol_functor_vtable *> table;
-	std::vector<std::unique_ptr<pnol_functor_vtable> > copies;
-	std::map<int, pnol_gradient_launcher> gradient;      // pnol_register_functor_gradient: belongs to the table registered at the time
-	std::map<int, pnol_hessian_launcher> hessian;        // pnol_register_functor_hessian: likewise
-	std::map<int, pnol_slope_launcher> slope;            // pnol_register_functor_slope: likewise
-	std::map<int, pnol_lm_batch_launcher> lm_batch;      // pnol_register_functor_lm_batch: likewise
+	std::map<int, KindTable> kinds;
 };
 FunctorRegistry & registry()
 {
 	static FunctorRegistry * r = new FunctorRegistry();      // never destroyed: registrations come from static initialisers of other modules
 	return *r;
 }
+
+// pnol_register_functor_*: attaches fn as member `slot` of the record registered for a user kind of the family (residual or scalar)
+template <class L> int attach(int kind, bool residual, L KindTable::*slot, L fn)
+{
+	if (!fn || !pnol::is_user_kind(kind) || pnol::is_residual_kind(kind) != residual) return PNOL_ERR_INVALID;
+	FunctorRegistry & r = registry();
+	std::lock_guard<std::mutex> lock(r.mu);
+	auto it = r.kinds.find(kind);
+	if (it == r.kinds.end()) return PNOL_ERR_INVALID;
+	it->second.*slot = fn;
+	return PNOL_OK;
+}
 } // namespace
 
-const pnol_functor_vtable * pnol::user_vtable(int kind)
+bool pnol::kind_table(int kind, KindTable * out)
 {
-	if (!is_user_kind(kind)) return nullptr;
+	if (const KindTable * b = builtin_kind_table(kind)) { *out = *b; return true; }
+	if (!is_user_kind(kind)) return false;
 	FunctorRegistry & r = registry();
 	std::lock_guard<std::mutex> lock(r.mu);
-	auto it = r.table.find(kind);
-	return it == r.table.end() ? nullptr : it->second;
-}
-
-pnol_gradient_launcher pnol::user_gradient(int kind)
-{
-	FunctorRegistry & r = registry();
-	std::lock_guard<std::mutex> lock(r.mu);
-	auto it = r.gradient.find(kind);
-	return it == r.gradient.end() ? nullptr : it->second;
-}
-
-pnol_hessian_launcher pnol::user_hessian(int kind)
-{
-	FunctorRegistry & r = registry();
-	std::lock_guard<std::mutex> lock(r.mu);
-	auto it = r.hessian.find(kind);
-	return it == r.hessian.end() ? nullptr : it->second;
-}
-
-pnol_slope_launcher pnol::user_slope(int kind)
-{
-	FunctorRegistry & r = registry();
-	std::lock_guard<std::mutex> lock(r.mu);
-	auto it = r.slope.find(kind);
-	return it == r.slope.end() ? nullptr : it->second;
-}
-
-pnol_lm_batch_launcher pnol::user_lm_batch(int kind)
-{
-	FunctorRegistry & r = registry();
-	std::lock_guard<std::mutex> lock(r.mu);
-	auto it = r.lm_batch.find(kind);
-	return it == r.lm_batch.end() ? nullptr : it->second;
+	auto it = r.kinds.find(kind);
+	if (it == r.kinds.end()) return false;
+	*out = it->second;
+	return true;
 }
 
 extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
@@ -387,103 +364,48 @@ extern "C" int pnol_register_functor(int kind, const pnol_functor_vtable * vt)
 	// abi_version leads every version of the table; a version-1 table ends before `jacobian`, so only that prefix may be read
 	const int abi = vt->abi_version;
 	if (abi != 1 && abi != PNOL_FUNCTOR_ABI) return PNOL_ERR_INVALID;
-	std::unique_ptr<pnol_functor_vtable> copy(new pnol_functor_vtable());
-	memcpy(copy.get(), vt, abi == 1 ? offsetof(pnol_functor_vtable, jacobian) : sizeof(pnol_functor_vtable));
-	const pnol_functor_vtable * c = copy.get();
+	KindTable k = {};
+	memcpy(&k.vt, vt, abi == 1 ? offsetof(pnol_functor_vtable, jacobian) : sizeof(pnol_functor_vtable));
+	const pnol_functor_vtable * c = &k.vt;
 	if (c->n_columns < 0 || c->n_columns > PNOL_MAX_COLUMNS) return PNOL_ERR_INVALID;
 	const bool residual = pnol::is_residual_kind(kind);
 	if (residual ? !(c->residual && c->fd_jacobian) : !(c->eval_batch && c->fd_points && c->fd_hessian && c->alpha_pool)) return PNOL_ERR_INVALID;
 	if (!residual && c->jacobian) return PNOL_ERR_INVALID;      // an analytic Jacobian belongs to a residual model
 	FunctorRegistry & r = registry();
 	std::lock_guard<std::mutex> lock(r.mu);
-	r.table[kind] = c;
-	r.copies.push_back(std::move(copy));
-	r.gradient.erase(kind);                                     // a derivative attached to the replaced table does not carry over
-	r.hessian.erase(kind);
-	r.slope.erase(kind);
-	r.lm_batch.erase(kind);
+	r.kinds[kind] = k;      // a new record: launchers attached to the replaced table do not carry over
 	return PNOL_OK;
 }
 
-extern "C" int pnol_register_functor_gradient(int kind, pnol_gradient_launcher fn)
-{
-	if (!fn || !pnol::is_user_kind(kind) || pnol::is_residual_kind(kind)) return PNOL_ERR_INVALID;
-	FunctorRegistry & r = registry();
-	std::lock_guard<std::mutex> lock(r.mu);
-	if (r.table.find(kind) == r.table.end()) return PNOL_ERR_INVALID;
-	r.gradient[kind] = fn;
-	return PNOL_OK;
-}
-
-extern "C" int pnol_functor_has_gradient(int kind)
-{
-	switch (kind) {
-		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE: return 1;
-		default: return pnol::user_gradient(kind) != nullptr;
-	}
-}
-
-extern "C" int pnol_register_functor_hessian(int kind, pnol_hessian_launcher fn)
-{
-	if (!fn || !pnol::is_user_kind(kind) || pnol::is_residual_kind(kind)) return PNOL_ERR_INVALID;
-	FunctorRegistry & r = registry();
-	std::lock_guard<std::mutex> lock(r.mu);
-	if (r.table.find(kind) == r.table.end()) return PNOL_ERR_INVALID;
-	r.hessian[kind] = fn;
-	return PNOL_OK;
-}
-
-extern "C" int pnol_functor_has_hessian(int kind)
-{
-	switch (kind) {
-		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE: return 1;
-		default: return pnol::user_hessian(kind) != nullptr;
-	}
-}
-
-extern "C" int pnol_register_functor_slope(int kind, pnol_slope_launcher fn)
-{
-	if (!fn || !pnol::is_user_kind(kind) || pnol::is_residual_kind(kind)) return PNOL_ERR_INVALID;
-	FunctorRegistry & r = registry();
-	std::lock_guard<std::mutex> lock(r.mu);
-	if (r.table.find(kind) == r.table.end()) return PNOL_ERR_INVALID;
-	r.slope[kind] = fn;
-	return PNOL_OK;
-}
-
-extern "C" int pnol_functor_has_slope(int kind)
-{
-	switch (kind) {
-		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE: return 1;
-		default: return pnol::user_slope(kind) != nullptr;
-	}
-}
-
-extern "C" int pnol_register_functor_lm_batch(int kind, pnol_lm_batch_launcher fn)
-{
-	if (!fn || !pnol::is_user_kind(kind) || !pnol::is_residual_kind(kind)) return PNOL_ERR_INVALID;
-	FunctorRegistry & r = registry();
-	std::lock_guard<std::mutex> lock(r.mu);
-	if (r.table.find(kind) == r.table.end()) return PNOL_ERR_INVALID;
-	r.lm_batch[kind] = fn;
-	return PNOL_OK;
-}
-
-extern "C" int pnol_functor_has_lm_batch(int kind)
-{
-	switch (kind) {
-		case PNOL_F_EXPCURVE: case PNOL_F_CUBIC: case PNOL_F_LORENTZ_SUM: return 1;
-		default: return pnol::user_lm_batch(kind) != nullptr;
-	}
-}
+extern "C" int pnol_register_functor_gradient(int kind, pnol_gradient_launcher fn) { return attach(kind, false, &KindTable::gradient, fn); }
+extern "C" int pnol_register_functor_hessian(int kind, pnol_hessian_launcher fn) { return attach(kind, false, &KindTable::hessian, fn); }
+extern "C" int pnol_register_functor_slope(int kind, pnol_slope_launcher fn) { return attach(kind, false, &KindTable::slope, fn); }
+extern "C" int pnol_register_functor_lm_batch(int kind, pnol_lm_batch_launcher fn) { return attach(kind, true, &KindTable::lm_batch, fn); }
 
 extern "C" int pnol_functor_registered(int kind)
 {
-	switch (kind) {
-		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: case PNOL_F_EXPCURVE_SINGLE:
-		case PNOL_F_EXPCURVE: case PNOL_F_CUBIC: case PNOL_F_LORENTZ_SUM: return 1;
-		default: return pnol::user_vtable(kind) != nullptr;
-	}
+	KindTable k;
+	return pnol::kind_table(kind, &k);
+}
+extern "C" int pnol_functor_has_gradient(int kind)
+{
+	KindTable k;
+	return pnol::kind_table(kind, &k) && k.gradient;
+}
+extern "C" int pnol_functor_has_hessian(int kind)
+{
+	KindTable k;
+	return pnol::kind_table(kind, &k) && k.hessian;
+}
+extern "C" int pnol_functor_has_slope(int kind)
+{
+	KindTable k;
+	return pnol::kind_table(kind, &k) && k.slope;
+}
+extern "C" int pnol_functor_has_lm_batch(int kind)
+{
+	KindTable k;
+	return pnol::kind_table(kind, &k) && k.lm_batch;
 }
 
 extern "C" int pnol_functor_create(pnol_ctx * ctx, const pnol_functor_desc * desc, pnol_functor ** out)
@@ -491,20 +413,12 @@ extern "C" int pnol_functor_create(pnol_ctx * ctx, const pnol_functor_desc * des
 	if (!ctx || !desc || !out) return PNOL_ERR_INVALID;
 	*out = nullptr;
 	PNOL_REQUIRE(ctx, desc->n_columns >= 0 && desc->n_columns <= PNOL_MAX_COLUMNS, "functor: bad column count %d", desc->n_columns);
-	int need_cols = 0;
-	switch (desc->kind) {
-		case PNOL_F_ROSENBROCK: case PNOL_F_POWER: case PNOL_F_BOOTH: case PNOL_F_GOLDSTEIN: case PNOL_F_RASTRIGIN: need_cols = 0; break;
-		case PNOL_F_EXPCURVE_SINGLE: case PNOL_F_EXPCURVE: case PNOL_F_LORENTZ_SUM: need_cols = 2; break;
-		case PNOL_F_CUBIC: need_cols = 3; break;
-		default: {
-			const pnol_functor_vtable * vt = user_vtable(desc->kind);
-			if (!vt) {
-				PNOL_SET_ERR(ctx, "unknown functor kind %d (user kinds must be registered first: pnol_register_functor)", desc->kind);
-				return PNOL_ERR_NO_FUNCTOR;
-			}
-			need_cols = vt->n_columns;
-		}
+	KindTable kt;
+	if (!kind_table(desc->kind, &kt)) {
+		PNOL_SET_ERR(ctx, "unknown functor kind %d (user kinds must be registered first: pnol_register_functor)", desc->kind);
+		return PNOL_ERR_NO_FUNCTOR;
 	}
+	const int need_cols = kt.vt.n_columns;
 	PNOL_REQUIRE(ctx, desc->n_columns == need_cols, "functor kind %d needs %d data columns, got %d", desc->kind, need_cols, desc->n_columns);
 	PNOL_REQUIRE(ctx, need_cols == 0 || desc->m >= 0, "functor: bad row count");
 	pnol_functor * f = new pnol_functor();

@@ -222,14 +222,27 @@ class TimerScope {
 	cudaEvent_t a_ = nullptr, b_ = nullptr;
 };
 
-// ---- open functor table (pnol_register_functor): launch table of a user kind, nullptr for the built-ins / unknown kinds ----
-const pnol_functor_vtable * user_vtable(int kind);
-pnol_gradient_launcher user_gradient(int kind);    // gradient launcher attached to a user kind's table, nullptr when none
-pnol_hessian_launcher user_hessian(int kind);      // Hessian launcher attached to a user kind's table, nullptr when none
-pnol_slope_launcher user_slope(int kind);          // line-search slope launcher attached to a user kind's table, nullptr when none
-pnol_lm_batch_launcher user_lm_batch(int kind);    // batched LM launcher attached to a user residual kind's table, nullptr when none
+// ---- functor kinds: everything the library can launch for one kind ----
+struct KindTable {
+	pnol_functor_vtable vt;               // the family's launchers, n_columns and (residual models, may be null) jacobian
+	pnol_gradient_launcher gradient;      // scalar objectives, may be null: pnol_gradient[_recur]
+	pnol_hessian_launcher hessian;        // scalar objectives, may be null: pnol_hessian
+	pnol_slope_launcher slope;            // scalar objectives, may be null: pnol_alpha_pool_analytic
+	pnol_lm_batch_launcher lm_batch;      // residual models, may be null: pnol_lm_batch
+};
+// copies out the record of a built-in or registered kind (capi.cu); false for any other kind. A copy, so that re-registering a kind
+// while a launch runs is safe.
+bool kind_table(int kind, KindTable * out);
+const KindTable * builtin_kind_table(int kind);      // builtin_functors.cu: nullptr unless the kind is built in
 inline bool is_user_kind(int kind) { return kind >= PNOL_F_USER_SCALAR_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000; }
 inline bool is_residual_kind(int kind) { return (kind >= 100 && kind < PNOL_F_USER_SCALAR_BASE) || (kind >= PNOL_F_USER_RESIDUAL_BASE && kind < PNOL_F_USER_RESIDUAL_BASE + 1000); }
+// a functor of the other family (family: "scalar objective" or "residual model"). The status differs by origin, as it always has:
+// PNOL_ERR_NO_FUNCTOR for a built-in kind, PNOL_ERR_INVALID for a user kind.
+inline int wrong_family(pnol_ctx * ctx, int kind, const char * family)
+{
+	PNOL_SET_ERR(ctx, "functor kind %d is not a %s", kind, family);
+	return is_user_kind(kind) ? PNOL_ERR_INVALID : PNOL_ERR_NO_FUNCTOR;
+}
 inline pnol_launch_env make_env(pnol_ctx * ctx)
 {
 	pnol_launch_env env;
@@ -240,29 +253,6 @@ inline pnol_launch_env make_env(pnol_ctx * ctx)
 	env.err = ctx->errbuf;
 	env.err_len = sizeof ctx->errbuf;
 	return env;
-}
-
-// ---- functor dispatch: calls fn(Functor{}) for the functor's kind ----
-template <class Fn> int dispatch_scalar(pnol_ctx * ctx, int kind, Fn && fn)
-{
-	switch (kind) {
-		case PNOL_F_ROSENBROCK: return fn(RosenbrockFunctor{});
-		case PNOL_F_POWER: return fn(PowerFunctor{});
-		case PNOL_F_BOOTH: return fn(BoothFunctor{});
-		case PNOL_F_GOLDSTEIN: return fn(GoldsteinFunctor{});
-		case PNOL_F_RASTRIGIN: return fn(RastriginFunctor{});
-		case PNOL_F_EXPCURVE_SINGLE: return fn(ExpCurveSingleFunctor{});
-		default: PNOL_SET_ERR(ctx, "functor kind %d is not a scalar objective", kind); return PNOL_ERR_NO_FUNCTOR;
-	}
-}
-template <class Fn> int dispatch_residual(pnol_ctx * ctx, int kind, Fn && fn)
-{
-	switch (kind) {
-		case PNOL_F_EXPCURVE: return fn(ExpCurveFunctor{});
-		case PNOL_F_CUBIC: return fn(CubicFunctor{});
-		case PNOL_F_LORENTZ_SUM: return fn(LorentzSumFunctor{});
-		default: PNOL_SET_ERR(ctx, "functor kind %d is not a residual model", kind); return PNOL_ERR_NO_FUNCTOR;
-	}
 }
 
 // ---- internal entry points implemented across the .cu files (device pointers only) ----

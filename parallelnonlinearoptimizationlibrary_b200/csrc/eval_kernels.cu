@@ -3,14 +3,13 @@
 // or analytic slopes).
 //
 // The kernels themselves are templates over the device functor in include/pnol/device/functor_kernels.cuh -- the SAME templates an
-// out-of-tree objective instantiates (open functor table, pnol_register_functor). This file instantiates them for the built-in
-// objectives and routes user kinds to their registered launch table.
+// out-of-tree objective instantiates (open functor table, pnol_register_functor). Every launcher here calls the record of the functor's
+// kind (kind_table): builtin_functors.cu instantiates the templates for the built-in objectives, a user kind brings its own.
 //
 // Mapping (north_star): one evaluation point per THREAD, the shared base point staged in shared memory;
 // population tiles are read from HBM with coalesced 16-byte loads and parked in shared memory with an odd row
 // pitch so that thread r walking row r is bank-conflict free. Functor code is compiled with -fmad=false.
 #include "common.cuh"
-#include "pnol/device/functor_kernels.cuh"
 
 namespace pnol {
 
@@ -20,12 +19,10 @@ int launch_eval_batch(pnol_ctx * ctx, const pnol_functor * f, const double * pts
 {
 	if (B <= 0) return PNOL_OK;
 	TimerScope ts(ctx, "eval_batch");
+	KindTable kt;
+	if (!kind_table(f->kind, &kt) || !kt.vt.eval_batch) return wrong_family(ctx, f->kind, "scalar objective");
 	const pnol_launch_env env = make_env(ctx);
-	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
-		PNOL_REQUIRE(ctx, vt->eval_batch, "functor kind %d is not a scalar objective", f->kind);
-		return vt->eval_batch(&env, &f->params, pts, B, n, ld, indicator, f_out);
-	}
-	return dispatch_scalar(ctx, f->kind, [&](auto tag) -> int { return dev::eval_batch<decltype(tag)>(&env, f->params, pts, B, n, ld, indicator, f_out); });
+	return kt.vt.eval_batch(&env, &f->params, pts, B, n, ld, indicator, f_out);
 }
 
 // a3 / a4 / a5: forward-difference stencil points (Source/PNOL_Objective.cpp:19-32, 125-145; Recur: :345-358, :399-420)
@@ -33,12 +30,10 @@ int launch_fd_points(pnol_ctx * ctx, const pnol_functor * f, const double * xful
                      const double * dx, int i0, int i1, double * fdx_out, double * f0_out)
 {
 	TimerScope ts(ctx, "fd_points");
+	KindTable kt;
+	if (!kind_table(f->kind, &kt) || !kt.vt.fd_points) return wrong_family(ctx, f->kind, "scalar objective");
 	const pnol_launch_env env = make_env(ctx);
-	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
-		PNOL_REQUIRE(ctx, vt->fd_points, "functor kind %d is not a scalar objective", f->kind);
-		return vt->fd_points(&env, &f->params, xfull, nfull, pos, dx, i0, i1, fdx_out, f0_out);
-	}
-	return dispatch_scalar(ctx, f->kind, [&](auto tag) -> int { return dev::fd_points<decltype(tag)>(&env, f->params, xfull, nfull, pos, dx, i0, i1, fdx_out, f0_out); });
+	return kt.vt.fd_points(&env, &f->params, xfull, nfull, pos, dx, i0, i1, fdx_out, f0_out);
 }
 
 // a3 / a4 / a5, analytic: the functor's partial derivatives, one coordinate per thread (pnol_gradient[_recur])
@@ -46,17 +41,14 @@ int launch_gradient(pnol_ctx * ctx, const pnol_functor * f, const double * xfull
                     double * g_out, double * f0_out)
 {
 	TimerScope ts(ctx, "gradient");
-	const pnol_launch_env env = make_env(ctx);
-	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
-		PNOL_REQUIRE(ctx, vt->fd_points, "functor kind %d is not a scalar objective", f->kind);
-		const pnol_gradient_launcher gl = user_gradient(f->kind);
-		if (!gl) {
-			PNOL_SET_ERR(ctx, "functor kind %d has no analytic gradient: its functor defines no partial() (pnol_register_functor_gradient)", f->kind);
-			return PNOL_ERR_NO_FUNCTOR;
-		}
-		return gl(&env, &f->params, xfull, nfull, pos, i0, i1, g_out, f0_out);
+	KindTable kt;
+	if (!kind_table(f->kind, &kt) || !kt.vt.fd_points) return wrong_family(ctx, f->kind, "scalar objective");
+	if (!kt.gradient) {
+		PNOL_SET_ERR(ctx, "functor kind %d has no analytic gradient: its functor defines no partial() (pnol_register_functor_gradient)", f->kind);
+		return PNOL_ERR_NO_FUNCTOR;
 	}
-	return dispatch_scalar(ctx, f->kind, [&](auto tag) -> int { return dev::gradient<decltype(tag)>(&env, f->params, xfull, nfull, pos, i0, i1, g_out, f0_out); });
+	const pnol_launch_env env = make_env(ctx);
+	return kt.gradient(&env, &f->params, xfull, nfull, pos, i0, i1, g_out, f0_out);
 }
 
 // g[i] = (fdx[i] - f0) / dx[i]     (Source/PNOL_Objective.cpp:31, :150-153, :451-454)
@@ -127,29 +119,24 @@ int launch_fd_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, 
                       const double * fdx, const double * f0, double * B)
 {
 	TimerScope ts(ctx, "fd_hessian");
+	KindTable kt;
+	if (!kind_table(f->kind, &kt) || !kt.vt.fd_hessian) return wrong_family(ctx, f->kind, "scalar objective");
 	const pnol_launch_env env = make_env(ctx);
-	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
-		PNOL_REQUIRE(ctx, vt->fd_hessian, "functor kind %d is not a scalar objective", f->kind);
-		return vt->fd_hessian(&env, &f->params, x, dx, n, fdx, f0, B);
-	}
-	return dispatch_scalar(ctx, f->kind, [&](auto tag) -> int { return dev::fd_hessian<decltype(tag)>(&env, f->params, x, dx, n, fdx, f0, B); });
+	return kt.vt.fd_hessian(&env, &f->params, x, dx, n, fdx, f0, B);
 }
 
 // a6, analytic: the functor's second derivatives, one 32 x 32 tile of the upper triangle at a time, mirrored (pnol_hessian)
 int launch_hessian(pnol_ctx * ctx, const pnol_functor * f, const double * x, int n, double * H)
 {
 	TimerScope ts(ctx, "hessian");
-	const pnol_launch_env env = make_env(ctx);
-	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
-		PNOL_REQUIRE(ctx, vt->fd_hessian, "functor kind %d is not a scalar objective", f->kind);
-		const pnol_hessian_launcher hl = user_hessian(f->kind);
-		if (!hl) {
-			PNOL_SET_ERR(ctx, "functor kind %d has no analytic Hessian: its functor defines no partial2() (pnol_register_functor_hessian)", f->kind);
-			return PNOL_ERR_NO_FUNCTOR;
-		}
-		return hl(&env, &f->params, x, n, H);
+	KindTable kt;
+	if (!kind_table(f->kind, &kt) || !kt.vt.fd_hessian) return wrong_family(ctx, f->kind, "scalar objective");
+	if (!kt.hessian) {
+		PNOL_SET_ERR(ctx, "functor kind %d has no analytic Hessian: its functor defines no partial2() (pnol_register_functor_hessian)", f->kind);
+		return PNOL_ERR_NO_FUNCTOR;
 	}
-	return dispatch_scalar(ctx, f->kind, [&](auto tag) -> int { return dev::hessian<decltype(tag)>(&env, f->params, x, n, H); });
+	const pnol_launch_env env = make_env(ctx);
+	return kt.hessian(&env, &f->params, x, n, H);
 }
 
 // a13: alpha pool: phi, the forward-difference slope and the NaN/inf -> 1e10 sentinel of evaluateAlphaPoolAndDerivatives
@@ -176,17 +163,10 @@ int launch_alpha_pool(pnol_ctx * ctx, const pnol_functor * f, const double * xfu
 	TimerScope ts(ctx, "alpha_pool");
 	PNOL_CHECK(ws_reserve(ctx, 3, (size_t) 2 * npool * sizeof(double)));
 	double * vals = (double *) ctx->ws[3];
+	KindTable kt;
+	if (!kind_table(f->kind, &kt) || !kt.vt.alpha_pool) return wrong_family(ctx, f->kind, "scalar objective");
 	const pnol_launch_env env = make_env(ctx);
-	int st;
-	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
-		PNOL_REQUIRE(ctx, vt->alpha_pool, "functor kind %d is not a scalar objective", f->kind);
-		st = vt->alpha_pool(&env, &f->params, xfull, pfull, is_const, nfull, alpha, npool, dalpha, eval_ind, dphi != nullptr, vals);
-	} else {
-		st = dispatch_scalar(ctx, f->kind, [&](auto tag) -> int {
-			return dev::alpha_pool<decltype(tag)>(&env, f->params, xfull, pfull, is_const, nfull, alpha, npool, dalpha, eval_ind, dphi != nullptr, vals);
-		});
-	}
-	PNOL_CHECK(st);
+	PNOL_CHECK(kt.vt.alpha_pool(&env, &f->params, xfull, pfull, is_const, nfull, alpha, npool, dalpha, eval_ind, dphi != nullptr, vals));
 	PNOL_LAUNCH(ctx, alpha_pool_finish_kernel, (npool + 63) / 64, 64, 0, vals, npool, dalpha, eval_ind, dphi != nullptr, phi, dphi, bad_dev);
 	return PNOL_OK;
 }
@@ -213,22 +193,14 @@ int launch_alpha_slope(pnol_ctx * ctx, const pnol_functor * f, const double * xf
 	TimerScope ts(ctx, "alpha_slope");
 	PNOL_CHECK(ws_reserve(ctx, 3, (size_t) 2 * npool * sizeof(double)));
 	double * vals = (double *) ctx->ws[3];
-	const pnol_launch_env env = make_env(ctx);
-	int st;
-	if (const pnol_functor_vtable * vt = user_vtable(f->kind)) {
-		PNOL_REQUIRE(ctx, vt->alpha_pool, "functor kind %d is not a scalar objective", f->kind);
-		const pnol_slope_launcher sl = user_slope(f->kind);
-		if (!sl) {
-			PNOL_SET_ERR(ctx, "functor kind %d has no analytic line-search slope: its functor defines no partial() (pnol_register_functor_slope)", f->kind);
-			return PNOL_ERR_NO_FUNCTOR;
-		}
-		st = sl(&env, &f->params, xfull, pfull, is_const, nfull, pos, p, n, alpha, npool, eval_ind, vals);
-	} else {
-		st = dispatch_scalar(ctx, f->kind, [&](auto tag) -> int {
-			return dev::alpha_slope<decltype(tag)>(&env, f->params, xfull, pfull, is_const, nfull, pos, p, n, alpha, npool, eval_ind, vals);
-		});
+	KindTable kt;
+	if (!kind_table(f->kind, &kt) || !kt.vt.alpha_pool) return wrong_family(ctx, f->kind, "scalar objective");
+	if (!kt.slope) {
+		PNOL_SET_ERR(ctx, "functor kind %d has no analytic line-search slope: its functor defines no partial() (pnol_register_functor_slope)", f->kind);
+		return PNOL_ERR_NO_FUNCTOR;
 	}
-	PNOL_CHECK(st);
+	const pnol_launch_env env = make_env(ctx);
+	PNOL_CHECK(kt.slope(&env, &f->params, xfull, pfull, is_const, nfull, pos, p, n, alpha, npool, eval_ind, vals));
 	PNOL_LAUNCH(ctx, alpha_slope_finish_kernel, (npool + 63) / 64, 64, 0, vals, npool, eval_ind, phi, dphi, bad_dev);
 	return PNOL_OK;
 }

@@ -1,7 +1,7 @@
 // lm_batch.cu -- pnol_lm_batch: many small independent Levenberg-Marquardt fits in one kernel launch, each problem bit for bit the
 // reference's LevMarq::findMin on its own rows. The kernel (lm_batch_kernel) is the header template of include/pnol/device/
-// functor_kernels.cuh, instantiated here for the three built-in residual models; a user residual kind brings its own instantiation
-// through the launcher attached with pnol_register_functor_lm_batch. Functor code is compiled with -fmad=false.
+// functor_kernels.cuh; the launcher comes from the record of the functor's kind (kind_table): builtin_residual_functors.cu instantiates
+// it for the three built-in residual models, a user residual kind attaches its own with pnol_register_functor_lm_batch.
 #include "common.cuh"
 #include "pnol/device/functor_kernels.cuh"
 
@@ -24,13 +24,11 @@ extern "C" int pnol_lm_batch(pnol_ctx * ctx, const pnol_functor * f, const long 
 	const bool analytic = jac_mode == PNOL_JAC_ANALYTIC;
 	PNOL_REQUIRE(ctx, analytic || dx, "lm_batch: dx is required for a forward-difference Jacobian");
 	PNOL_CHECK(lorentz_shape_ok(ctx, f, n));
-	pnol_lm_batch_launcher user = nullptr;
-	if (user_vtable(f->kind)) {
-		user = user_lm_batch(f->kind);
-		if (!user) {
-			PNOL_SET_ERR(ctx, "functor kind %d has no batched LM launcher (pnol_register_functor_lm_batch)", f->kind);
-			return PNOL_ERR_NO_FUNCTOR;
-		}
+	KindTable kt;
+	if (!kind_table(f->kind, &kt) || !kt.vt.residual) return wrong_family(ctx, f->kind, "residual model");
+	if (!kt.lm_batch) {
+		PNOL_SET_ERR(ctx, "functor kind %d has no batched LM launcher (pnol_register_functor_lm_batch)", f->kind);
+		return PNOL_ERR_NO_FUNCTOR;
 	}
 	// row_off: B + 1 non-decreasing offsets within [0, m] (read on the host: a device array is copied back first)
 	const long long m = f->params.m;
@@ -58,17 +56,8 @@ extern "C" int pnol_lm_batch(pnol_ctx * ctx, const pnol_functor * f, const long 
 	PNOL_CHECK(dstop.init(ctx, stopped_out, (size_t) B));
 	if (F_out) PNOL_CHECK(dF.init(ctx, F_out, (size_t) m, true));      // rows outside every problem keep what they held
 	const pnol_launch_env env = make_env(ctx);
-	int st;
-	if (user) {
-		st = user(&env, &f->params, dro.get(), B, n, dX.get(), ddx.get(), lambda0, lambda_factor, x_min_diff, max_iter, jac_mode, dchi.get(),
-		          dlam.get(), dit.get(), dstop.get(), dF.get());
-	} else {
-		st = dispatch_residual(ctx, f->kind, [&](auto tag) -> int {
-			return dev::lm_batch<decltype(tag)>(&env, f->params, dro.get(), B, n, dX.get(), ddx.get(), lambda0, lambda_factor, x_min_diff,
-			                                    max_iter, jac_mode, dchi.get(), dlam.get(), dit.get(), dstop.get(), dF.get());
-		});
-	}
-	PNOL_CHECK(st);
+	PNOL_CHECK(kt.lm_batch(&env, &f->params, dro.get(), B, n, dX.get(), ddx.get(), lambda0, lambda_factor, x_min_diff, max_iter, jac_mode,
+	                       dchi.get(), dlam.get(), dit.get(), dstop.get(), dF.get()));
 	PNOL_CHECK(dX.commit());
 	PNOL_CHECK(dchi.commit());
 	PNOL_CHECK(dlam.commit());
