@@ -856,6 +856,40 @@ int jacobian(const pnol_launch_env * env, const FunctorParams & P, const double 
 // ---------------------------------------------------------------------------------------------------
 constexpr int kLmBatchMaxN = 64;
 
+// In-place LU with partial pivoting of the n x n matrix A (row pitch ap) in shared memory by a block of T threads, the shim's luSolve
+// factorisation (oracle/shim/shim_impl.cpp:63-80): whole-row swaps, the first largest |entry| as pivot, a zero pivot left to IEEE
+// arithmetic. The pivot search is thread 0's (piv, which must hold the identity on entry, records the row order; slot is one int of
+// shared memory for the broadcast), the row swap, the column scaling and the elimination are spread over the block -- each entry still
+// sees its updates in k order, so the factors have the bits of the sequential loop. Used by lm_batch_kernel and bfgs_batch_kernel.
+template <int T>
+__device__ __forceinline__ void block_lu_factor(double * A, int ap, int n, int * piv, int * slot)
+{
+	const int tid = threadIdx.x;
+	for (int k = 0; k < n; k++) {
+		if (tid == 0) {
+			int p = k;
+			double best = fabs(A[k * ap + k]);
+			for (int i = k + 1; i < n; i++)
+				if (fabs(A[i * ap + k]) > best) { best = fabs(A[i * ap + k]); p = i; }
+			if (p != k) { const int t = piv[p]; piv[p] = piv[k]; piv[k] = t; }
+			slot[0] = p;
+		}
+		__syncthreads();
+		const int p = slot[0];
+		if (p != k)
+			for (int j = tid; j < n; j += T) { const double t = A[p * ap + j]; A[p * ap + j] = A[k * ap + j]; A[k * ap + j] = t; }
+		__syncthreads();
+		for (int i = k + 1 + tid; i < n; i += T) A[i * ap + k] = A[i * ap + k] / A[k * ap + k];
+		__syncthreads();
+		const int w = n - k - 1;
+		for (int e = tid; e < w * w; e += T) {
+			const int i = k + 1 + e / w, j = k + 1 + e % w;
+			A[i * ap + j] = A[i * ap + j] - A[i * ap + k] * A[k * ap + j];
+		}
+		__syncthreads();
+	}
+}
+
 __host__ __device__ inline int lm_batch_pitch(int n) { return (n + 1) | 1; }
 __host__ __device__ inline int lm_batch_nsums(int n) { return n * (n + 1) / 2 + n; }
 // shared memory of one problem: xs, xt, dx, 1/dx, sigma, y (6n), the sums, A (n x (n+1)), the tile, 2 broadcast slots; then n ints
@@ -983,30 +1017,7 @@ lm_batch_kernel(FunctorParams P, const long long * __restrict__ row_off, int n, 
 		}
 		for (int i = tid; i < n; i += T) piv[i] = i;
 		__syncthreads();
-		// LU with partial pivoting (oracle/shim/shim_impl.cpp:63-80)
-		for (int k = 0; k < n; k++) {
-			if (tid == 0) {
-				int p = k;
-				double best = fabs(A[k * ap + k]);
-				for (int i = k + 1; i < n; i++)
-					if (fabs(A[i * ap + k]) > best) { best = fabs(A[i * ap + k]); p = i; }
-				if (p != k) { const int t = piv[p]; piv[p] = piv[k]; piv[k] = t; }
-				reinterpret_cast<int *>(bc)[0] = p;
-			}
-			__syncthreads();
-			const int p = reinterpret_cast<const int *>(bc)[0];
-			if (p != k)
-				for (int j = tid; j < n; j += T) { const double t = A[p * ap + j]; A[p * ap + j] = A[k * ap + j]; A[k * ap + j] = t; }
-			__syncthreads();
-			for (int i = k + 1 + tid; i < n; i += T) A[i * ap + k] = A[i * ap + k] / A[k * ap + k];
-			__syncthreads();
-			const int w = n - k - 1;
-			for (int e = tid; e < w * w; e += T) {
-				const int i = k + 1 + e / w, j = k + 1 + e % w;
-				A[i * ap + j] = A[i * ap + j] - A[i * ap + k] * A[k * ap + j];
-			}
-			__syncthreads();
-		}
+		block_lu_factor<T>(A, ap, n, piv, reinterpret_cast<int *>(bc));
 		// substitutions (shim_impl.cpp:82-98) with rhs = -(J^T F)
 		if (tid == 0) {
 			for (int i = 0; i < n; i++) {
@@ -1102,6 +1113,381 @@ int lm_batch(const pnol_launch_env * env, const FunctorParams & P, const long lo
 	                               iters_out, stopped_out, F_out);
 }
 
+// ---------------------------------------------------------------------------------------------------
+// batched BFGS (pnol_bfgs_batch): problem b starts from row b of X (B x n) and minimises the functor's objective. One CTA runs one
+// problem's whole BFGS::findMin (Source/BFGS_with_linesearch.cpp:12-139) -- the strong-Wolfe line search with its zoom and
+// cubicInterpMin (:177-385) and the literal updateHessianInv (:389-432) included -- operation for operation what the unmodified host
+// BFGS controller computes on the C-ABI's CPU stand-in (oracle/host_logic_device.cpp, whose dense helpers are the reference's
+// sequential ones), so every problem returns the bits the reference returns on that start alone:
+//   - D: the identity, or (init_hess_fd) the inverse of the Hessian at X: B by the forward difference (n + 1 stencil values, then one
+//     thread per pair i <= j with (f_ij - f_i - f_j + f) / (dx dx), the diagonal point (x_i + dx) + dx) or by F::partial2, mirrored;
+//     then matrixInverse as the stand-in computes it, one LU with partial pivoting (block_lu_factor) and one pair of substitutions
+//     with b = e_j per column j, each column one thread.
+//   - gradient: n + 1 stencil points, one thread each (PerturbAcc: fd_points' bits), and the IEEE quotient; or n F::partial calls.
+//   - p = -D g, one row per thread, each a sequential k sum.
+//   - line search: every thread runs the same scalar control (Wolfe tests, zoom, cubicInterpMin with pow(d1, 2) as d1 * d1 and the
+//     reference's sign(), the `iter > 1` of the sufficient-decrease test) on values broadcast through shared memory, so the control
+//     flow is uniform and needs no extra barrier. A point is phi(alpha) and phi(alpha + dalpha) on lanes 0 and 1 (LineAcc: unfused
+//     x + alpha p), slope (phi2 - phi) / dalpha; or, analytic slope, phi on thread 0 while the threads of the other warps (lanes 1 ..
+//     n of a single-warp block) form p_r * df/dx_r at the staged point, summed in r order as alpha_slope_kernel sums them. Values are
+//     raw: the serial class has no 1e10 sentinel. An exhausted search leaves alpha = 0 and Fopt = F (and then rho = 1/0: D turns NaN,
+//     as in the reference).
+//   - update: A = M1 D, then D = A M2 + M3, each entry one thread's sequential k sum, M1 / M2 / M3 formed on the fly with
+//     oracle_update_hinv's expressions (never the RANK2 form, whose bits differ).
+//   - stop: sum |X - Xprev| and ||g||_2 sequentially; stop code 0 / 1 / 2 for the first false conjunct of the loop condition.
+// Scalar sums every thread needs (p . g, y . s, the stop norms) are computed by every thread from shared memory: same operations in the
+// same order, hence the same bits everywhere. Two shared buffers alternate for the line-search values so that a point's writes never
+// race the previous point's readers. A problem's bits depend on nothing but its start, the functor and the parameters.
+// Configurations by n (threads): n <= 8: 32, <= 16: 64, <= 32: 128, <= 64: 256.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kBfgsBatchMaxN = 64;
+
+// D and the update / LU scratch A (n x (n + 1) each), twelve n-vectors, four line-search values and four broadcast slots; n + 1 ints
+__host__ __device__ inline size_t bfgs_batch_smem(int n)
+{
+	return ((size_t) 2 * n * (n + 1) + (size_t) 12 * n + 8) * sizeof(double) + (size_t) (n + 1) * sizeof(int);
+}
+
+// the reference's sign() and cubicInterpMin (Source/BFGS_with_linesearch.cpp:359-385); pow(d1, 2) is d1 * d1 there (a literal square,
+// folded by the compiler)
+__device__ __forceinline__ double bfgs_sign(double x) { if (x > 0) return 1.0; if (x < 0) return -1.0; return 0.0; }
+__device__ __forceinline__ double bfgs_cubic_interp_min(double alo, double ahi, double plo, double phh, double dlo, double dhh)
+{
+	const double d1 = dlo + dhh - 3 * (plo - phh) / (alo - ahi);
+	const double d2 = bfgs_sign(ahi - alo) * sqrt(d1 * d1 - dlo * dhh);
+	double a = ahi - (ahi - alo) * (dhh + d2 - d1) / (dhh - dlo + 2 * d2);
+	if (alo < ahi) {
+		if (a < alo) a = (ahi + alo) / 2;
+	} else {
+		if (a < ahi) a = (ahi + alo) / 2;
+	}
+	return a;
+}
+
+template <class F, int T>
+__global__ void __launch_bounds__(T)
+bfgs_batch_kernel(FunctorParams P, int n, double * __restrict__ X, pnol_bfgs_params prm, int flags, double * __restrict__ f0_out,
+                  double * __restrict__ fopt_out, int * __restrict__ iters_out, int * __restrict__ stop_out)
+{
+	extern __shared__ double sm[];
+	const int tid = threadIdx.x;
+	const long long b = blockIdx.x;
+	const int ap = n + 1;
+	double * D = sm;                       // inverse Hessian, n x ap
+	double * A = D + (size_t) n * ap;      // M1 D, or the Hessian and its LU factors
+	double * xs = A + (size_t) n * ap;     // X
+	double * ps = xs + n;                  // p
+	double * g = ps + n;                   // dFdX
+	double * gp = g + n;                   // dFdX_prev
+	double * sv = gp + n;                  // s = alpha p
+	double * yv = sv + n;                  // g = dFdX - dFdX_prev (the reference's name for it)
+	double * rg = yv + n;                  // rho * yv
+	double * ad = rg + n;                  // |X - Xprev|
+	double * fdx = ad + n;                 // stencil values
+	double * xa = fdx + n;                 // staged trial point (analytic slope)
+	double * prod = xa + n;                // 2 x n slope products
+	double * vals = prod + 2 * n;          // 2 x 2 line-search values
+	double * bc = vals + 4;                // broadcast slots: [0] f(X) of the gradient, [1] f(X) of the FD Hessian
+	int * piv = reinterpret_cast<int *>(bc + 4);   // n pivots, then the LU's broadcast slot
+
+	bool agrad = false, aslope = false;
+	if constexpr (has_partial<F>::value) {
+		agrad = (flags & PNOL_BFGS_ANALYTIC_GRADIENT) != 0;
+		aslope = (flags & PNOL_BFGS_ANALYTIC_SLOPE) != 0;
+	}
+	const int max_ls = prm.max_iter_ls;
+	const double c1 = prm.c1, c2 = prm.c2;
+
+	for (int j = tid; j < n; j += T) xs[j] = X[b * n + j];
+	__syncthreads();
+
+	// ---- D (:35-57) ----
+	const int npairs = n * (n + 1) / 2;
+	auto unrank = [](int e, int & i, int & j) {      // pair e of the lower triangle row by row -> (i <= j)
+		int r = 0;
+		while ((r + 1) * (r + 2) / 2 <= e) r++;
+		i = e - r * (r + 1) / 2; j = r;
+	};
+	if (prm.init_hess_fd) {
+		bool analytic_b = false;
+		if constexpr (has_partial2<F>::value) {
+			if (flags & PNOL_BFGS_ANALYTIC_HESSIAN) {
+				analytic_b = true;
+				const PtrAcc ax{xs};
+				for (int e = tid; e < npairs; e += T) {
+					int i, j;
+					unrank(e, i, j);
+					const double v = F::partial2(P, ax, n, i, j);
+					A[i * ap + j] = v;
+					A[j * ap + i] = v;
+				}
+			}
+		}
+		if (!analytic_b) {
+			// Objective::hessianApproximation (Source/PNOL_Objective.cpp:38-85), f(X + dx e_i) computed once per i
+			const double dxh = prm.dx_hess;
+			for (int i = tid; i <= n; i += T) {
+				if (i < n) {
+					const PerturbAcc acc{xs, i, xs[i] + dxh};
+					fdx[i] = F::eval(P, acc, n);
+				} else {
+					const PtrAcc ax{xs};
+					bc[1] = F::eval(P, ax, n);
+				}
+			}
+			__syncthreads();
+			const double f = bc[1];
+			for (int e = tid; e < npairs; e += T) {
+				int i, j;
+				unrank(e, i, j);
+				double fij;
+				if (i == j) {
+					const PerturbAcc acc{xs, i, (xs[i] + dxh) + dxh};
+					fij = F::eval(P, acc, n);
+				} else {
+					const Perturb2Acc acc{xs, i, xs[i] + dxh, j, xs[j] + dxh};
+					fij = F::eval(P, acc, n);
+				}
+				const double v = (fij - fdx[i] - fdx[j] + f) / (dxh * dxh);
+				A[i * ap + j] = v;
+				A[j * ap + i] = v;
+			}
+		}
+		for (int i = tid; i < n; i += T) piv[i] = i;
+		__syncthreads();
+		block_lu_factor<T>(A, ap, n, piv, piv + n);
+		// matrixInverse: column j solves with b = e_j (oracle_lu_solve's substitutions), in place in column j of D
+		for (int j = tid; j < n; j += T) {
+			for (int i = 0; i < n; i++) {
+				double s = piv[i] == j ? 1.0 : 0.0;
+				for (int k = 0; k < i; k++) s = s - A[i * ap + k] * D[k * ap + j];
+				D[i * ap + j] = s;
+			}
+			for (int i = n - 1; i >= 0; i--) {
+				double s = D[i * ap + j];
+				for (int k = i + 1; k < n; k++) s = s - A[i * ap + k] * D[k * ap + j];
+				D[i * ap + j] = s / A[i * ap + i];
+			}
+		}
+	} else {
+		for (int e = tid; e < n * n; e += T) {
+			const int i = e / n, j = e - i * n;
+			D[i * ap + j] = i == j ? 1.0 : 0.0;
+		}
+	}
+	__syncthreads();
+
+	// ---- gradient at xs into g; with_f: bc[0] = f(xs) as well (the forward difference always evaluates it, for its quotient) ----
+	auto gradient_at_x = [&](bool with_f) {
+		const PtrAcc ax{xs};
+		if constexpr (has_partial<F>::value) {
+			if (agrad) {
+				for (int i = tid; i < n; i += T) g[i] = F::partial(P, ax, n, i);
+				if (with_f && tid == n) bc[0] = F::eval(P, ax, n);
+				__syncthreads();
+				return;
+			}
+		}
+		const double dxg = prm.dx_grad;
+		for (int i = tid; i <= n; i += T) {
+			if (i < n) {
+				const PerturbAcc acc{xs, i, xs[i] + dxg};      // XdX[i] = XdX[i] + dX[i]  (Source/PNOL_Objective.cpp:27)
+				fdx[i] = F::eval(P, acc, n);
+			} else {
+				bc[0] = F::eval(P, ax, n);
+			}
+		}
+		__syncthreads();
+		const double f = bc[0];
+		for (int i = tid; i < n; i += T) g[i] = (fdx[i] - f) / dxg;
+		__syncthreads();
+	};
+
+	// ---- phi(a) and its slope; every thread gets both ----
+	int parity = 0;
+	const int pofs = T > 32 ? 32 : 1;      // first product thread: the second warp, or lane 1 of a single-warp block
+	auto eval_phi = [&](double a, double & phi, double & dphi) {
+		double * v = vals + 2 * parity;
+		if constexpr (has_partial<F>::value) {
+			if (aslope) {
+				double * pr = prod + n * parity;
+				for (int j = tid; j < n; j += T) xa[j] = xs[j] + a * ps[j];
+				__syncthreads();
+				const PtrAcc acc{xa};
+				if (tid == 0) {
+					v[0] = F::eval(P, acc, n);
+				} else if (tid >= pofs && tid < pofs + n) {
+					const int r = tid - pofs;
+					pr[r] = F::partial(P, acc, n, r) * ps[r];
+				}
+				__syncthreads();
+				phi = v[0];
+				double s = 0.0;
+				for (int r = 0; r < n; r++) s = s + pr[r];
+				dphi = s;
+				parity ^= 1;
+				return;
+			}
+		}
+		if (tid < 2) {
+			// lineSearchObj / lineSearchFDDerivative (:144-172): X[i] + alpha*p[i], X[i] + (alpha+dalpha)*p[i]
+			const LineAcc acc{xs, ps, nullptr, tid == 0 ? a : a + prm.dalpha};
+			v[tid] = F::eval(P, acc, n);
+		}
+		__syncthreads();
+		phi = v[0];
+		dphi = (v[1] - v[0]) / prm.dalpha;
+		parity ^= 1;
+	};
+
+	// ---- lineSearchZoom (:296-356) ----
+	auto zoom = [&](double alo, double ahi, double plo, double phh, double dlo, double dhh, double phi0, double dphi0, double & aopt,
+	                double & fopt) {
+		for (int it = 0; it < max_ls; it++) {
+			const double aj = bfgs_cubic_interp_min(alo, ahi, plo, phh, dlo, dhh);
+			double pj, dj;
+			eval_phi(aj, pj, dj);
+			if (pj > phi0 + c1 * aj * dphi0 || pj >= plo) {
+				ahi = aj; phh = pj; dhh = dj;
+			} else {
+				if (fabs(dj) <= fabs(c2 * dphi0)) { aopt = aj; fopt = pj; break; }
+				if (dj * (ahi - alo) >= 0) { ahi = alo; phh = plo; dhh = dlo; }
+				alo = aj; plo = pj; dlo = dj;
+			}
+		}
+	};
+
+	// ---- findMin (:62-139) ----
+	gradient_at_x(true);
+	double Fc = bc[0];
+	const double f0 = Fc;
+	const int max_iter = prm.max_iter;
+	const double xmin = prm.x_min_diff, gmin = prm.min_grad_2norm;
+	int iter = 0;
+	double xdiff = xmin * 2;
+	double g2 = 2 * gmin;
+	while (iter < max_iter && xdiff > xmin && g2 > gmin) {
+		for (int i = tid; i < n; i += T) {                             // p = -D dFdX (:78-79)
+			double s = 0;
+			for (int k = 0; k < n; k++) s = s + D[i * ap + k] * g[k];
+			ps[i] = -s;
+			gp[i] = g[i];
+		}
+		__syncthreads();
+		// cubicInterpolationLineSearch (:177-291)
+		double alpha = 0, Fopt = Fc;
+		const double phi0 = Fc;
+		double dphi0 = 0;
+		for (int k = 0; k < n; k++) dphi0 = dphi0 + g[k] * ps[k];      // dotProd(dFdX, p)
+		double am1 = 0, phim1 = phi0, dm1 = dphi0;
+		double ai = prm.alpha_guess;
+		for (int it = 0; it < max_ls; it++) {
+			double phii, dphii;
+			eval_phi(ai, phii, dphii);
+			if ((phii > phi0 + c1 * ai * dphi0) || (phii >= phim1 && it > 1)) {
+				zoom(am1, ai, phim1, phii, dm1, dphii, phi0, dphi0, alpha, Fopt);
+				break;
+			}
+			if (fabs(dphii) <= fabs(c2 * dphi0)) { alpha = ai; Fopt = phii; break; }
+			if (dphii >= 0) {
+				zoom(ai, am1, phii, phim1, dphii, dm1, phi0, dphi0, alpha, Fopt);
+				break;
+			}
+			am1 = ai; phim1 = phii; dm1 = dphii;
+			ai = 2 * ai;
+		}
+		for (int i = tid; i < n; i += T) {                             // (:88-93), s (:100-105)
+			const double xo = xs[i];
+			const double xn = xo + alpha * ps[i];
+			xs[i] = xn;
+			sv[i] = alpha * ps[i];
+			ad[i] = fabs(xn - xo);
+		}
+		Fc = Fopt;
+		__syncthreads();
+		gradient_at_x(false);                                          // (:97)
+		for (int i = tid; i < n; i += T) yv[i] = g[i] - gp[i];
+		__syncthreads();
+		// updateHessianInv (:389-432): A = M1 D, D = A M2 + M3
+		double ys = 0;
+		for (int k = 0; k < n; k++) ys = ys + yv[k] * sv[k];
+		const double rho = 1 / ys;
+		for (int e = tid; e < n * n; e += T) {
+			const int i = e / n, j = e - i * n;
+			const double rs = rho * sv[i];
+			double acc = 0;
+			for (int k = 0; k < n; k++) {
+				const double m1 = (i == k ? 1.0 : 0.0) - rs * yv[k];
+				acc = acc + m1 * D[k * ap + j];
+			}
+			A[i * ap + j] = acc;
+		}
+		for (int i = tid; i < n; i += T) rg[i] = rho * yv[i];
+		__syncthreads();
+		for (int e = tid; e < n * n; e += T) {
+			const int i = e / n, j = e - i * n;
+			double acc = 0;
+			for (int k = 0; k < n; k++) {
+				const double m2 = (k == j ? 1.0 : 0.0) - rg[k] * sv[j];
+				acc = acc + A[i * ap + k] * m2;
+			}
+			D[i * ap + j] = acc + (rho * sv[i]) * sv[j];
+		}
+		xdiff = 0;
+		for (int i = 0; i < n; i++) xdiff = xdiff + ad[i];            // (:111-113)
+		double s2 = 0;
+		for (int i = 0; i < n; i++) s2 = s2 + g[i] * g[i];
+		g2 = sqrt(s2);                                                 // vector2Norm(dFdX)
+		__syncthreads();
+		iter = iter + 1;
+	}
+	for (int j = tid; j < n; j += T) X[b * n + j] = xs[j];
+	if (tid == 0) {
+		f0_out[b] = f0;
+		fopt_out[b] = Fc;
+		iters_out[b] = iter;
+		stop_out[b] = !(iter < max_iter) ? 0 : (!(xdiff > xmin) ? 1 : 2);
+	}
+}
+
+template <class F, int T>
+int bfgs_batch_launch(const pnol_launch_env * env, const FunctorParams & P, long long B, int n, double * X, const pnol_bfgs_params & prm,
+                      int flags, double * f0_out, double * fopt_out, int * iters_out, int * stop_out)
+{
+	const size_t smem = bfgs_batch_smem(n);
+	PNOL_DEV_REQUIRE(env, smem <= env->smem_optin, "bfgs batch: n = %d needs %zu bytes of shared memory", n, smem);
+	auto kern = bfgs_batch_kernel<F, T>;
+	PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+	PNOL_DEV_LAUNCH(env, kern, (unsigned) B, T, smem, P, n, X, prm, flags, f0_out, fopt_out, iters_out, stop_out);
+	return PNOL_OK;
+}
+
+/* pnol_bfgs_batch on device pointers: X (B x n, in/out), the four per-problem outputs (B). n in 1 .. 64. The analytic gradient and
+ * slope flags need F::partial, the analytic Hessian flag with init_hess_fd F::partial2 (PNOL_ERR_NO_FUNCTOR otherwise). */
+template <class F>
+int bfgs_batch(const pnol_launch_env * env, const FunctorParams & P, long long B, int n, double * X, const pnol_bfgs_params * prm, int flags,
+               double * f0_out, double * fopt_out, int * iters_out, int * stop_out)
+{
+	PNOL_DEV_REQUIRE(env, n >= 1 && n <= kBfgsBatchMaxN, "bfgs batch: n = %d is outside 1 .. %d", n, kBfgsBatchMaxN);
+	PNOL_DEV_REQUIRE(env, B >= 0 && B <= 0x7fffffffLL, "bfgs batch: B = %lld is outside 0 .. 2^31 - 1", B);
+	PNOL_DEV_REQUIRE(env, prm != nullptr, "bfgs batch: the parameters are required");
+	if (B == 0) return PNOL_OK;
+	if (!has_partial<F>::value && (flags & (PNOL_BFGS_ANALYTIC_GRADIENT | PNOL_BFGS_ANALYTIC_SLOPE))) {
+		PNOL_DEV_ERR(env, "bfgs batch: the objective has no analytic gradient (partial()): the analytic gradient / slope flags are refused");
+		return PNOL_ERR_NO_FUNCTOR;
+	}
+	if (!has_partial2<F>::value && (flags & PNOL_BFGS_ANALYTIC_HESSIAN) && prm->init_hess_fd) {
+		PNOL_DEV_ERR(env, "bfgs batch: the objective has no analytic Hessian (partial2()): the analytic Hessian flag is refused");
+		return PNOL_ERR_NO_FUNCTOR;
+	}
+#define PNOL_BFGS_BATCH_CFG(T) bfgs_batch_launch<F, T>(env, P, B, n, X, *prm, flags, f0_out, fopt_out, iters_out, stop_out)
+	if (n <= 8) return PNOL_BFGS_BATCH_CFG(32);
+	if (n <= 16) return PNOL_BFGS_BATCH_CFG(64);
+	if (n <= 32) return PNOL_BFGS_BATCH_CFG(128);
+	return PNOL_BFGS_BATCH_CFG(256);
+#undef PNOL_BFGS_BATCH_CFG
+}
+
 /* ---- launch tables (pnol_functor_vtable) of a functor type ---- */
 template <class F> struct ScalarTable {
 	static int eval_batch_(const pnol_launch_env * env, const pnol_functor_params * P, const double * pts, long long B, int n, long long ld,
@@ -1122,6 +1508,9 @@ template <class F> struct ScalarTable {
 	                        const unsigned char * is_const, int nfull, const int * pos, const double * p, int n, const double * alpha, int npool,
 	                        const unsigned char * eval_ind, double * vals)
 	{ return alpha_slope<F>(env, *P, xfull, pfull, is_const, nfull, pos, p, n, alpha, npool, eval_ind, vals); }
+	static int bfgs_batch_(const pnol_launch_env * env, const pnol_functor_params * P, long long B, int n, double * X, const pnol_bfgs_params * prm,
+	                       int flags, double * f0_out, double * fopt_out, int * iters_out, int * stop_out)
+	{ return bfgs_batch<F>(env, *P, B, n, X, prm, flags, f0_out, fopt_out, iters_out, stop_out); }
 	static pnol_functor_vtable make(int n_columns)
 	{
 		pnol_functor_vtable vt = {};
@@ -1133,11 +1522,12 @@ template <class F> struct ScalarTable {
 		vt.alpha_pool = alpha_pool_;
 		return vt;
 	}
-	/* registers the table, then (F defines partial) its gradient and line-search slope launchers and (F defines partial2) its Hessian
-	 * launcher, in this order: a derivative attaches to the registered table */
+	/* registers the table, then its batched BFGS launcher, (F defines partial) its gradient and line-search slope launchers and (F defines
+	 * partial2) its Hessian launcher, in this order: a launcher attaches to the registered table */
 	static int register_as(int kind, const pnol_functor_vtable * vt)
 	{
 		int st = pnol_register_functor(kind, vt);
+		if (st == PNOL_OK) st = pnol_register_functor_bfgs_batch(kind, bfgs_batch_);
 		if constexpr (has_partial<F>::value) {
 			if (st == PNOL_OK) st = pnol_register_functor_gradient(kind, gradient_);
 			if (st == PNOL_OK) st = pnol_register_functor_slope(kind, alpha_slope_);

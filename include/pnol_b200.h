@@ -130,7 +130,8 @@ typedef struct {
  *     kinds [PNOL_F_USER_SCALAR_BASE, +1000)   scalar objectives  (eval_batch, fd_points, fd_hessian, alpha_pool; optionally a gradient
  *                                              launcher attached with pnol_register_functor_gradient: pnol_gradient[_recur], and
  *                                              a Hessian launcher attached with pnol_register_functor_hessian: pnol_hessian, and
- *                                              a slope launcher attached with pnol_register_functor_slope: pnol_alpha_pool_analytic)
+ *                                              a slope launcher attached with pnol_register_functor_slope: pnol_alpha_pool_analytic,
+ *                                              and a batch BFGS launcher attached with pnol_register_functor_bfgs_batch: pnol_bfgs_batch)
  *     kinds [PNOL_F_USER_RESIDUAL_BASE, +1000) residual models    (residual, fd_jacobian; optionally jacobian: PNOL_JAC_ANALYTIC; a batch
  *                                              LM launcher attached with pnol_register_functor_lm_batch: pnol_lm_batch)
  * pnol_functor_create and every entry point that takes a functor then work for that kind as for the built-ins; libpnol_b200.so is not
@@ -239,6 +240,33 @@ typedef int (*pnol_lm_batch_launcher)(const pnol_launch_env *, const pnol_functo
 int pnol_register_functor_lm_batch(int kind, pnol_lm_batch_launcher fn);
 /* 1 when pnol_lm_batch accepts the kind: the three built-in residual models, and user residual kinds with a batch launcher attached */
 int pnol_functor_has_lm_batch(int kind);
+
+/* Parameters of the batched BFGS (pnol_bfgs_batch): BFGS::setParams' arguments in the same order and with the same meaning
+ * (include/pnol/BFGS_with_linesearch.hpp; verbose is not kept). init_hess_fd != 0: D starts as the inverse of the Hessian at X. */
+typedef struct pnol_bfgs_params {
+	double c1, c2, dalpha, alpha_guess;
+	int max_iter_ls;
+	double dx_grad, dx_hess;
+	int max_iter;
+	double x_min_diff, min_grad_2norm;
+	int init_hess_fd;
+} pnol_bfgs_params;
+/* deriv_flags of pnol_bfgs_batch: each derivative from the functor's own partial() / partial2() instead of a forward difference */
+enum { PNOL_BFGS_ANALYTIC_GRADIENT = 1, PNOL_BFGS_ANALYTIC_SLOPE = 2, PNOL_BFGS_ANALYTIC_HESSIAN = 4 };
+
+/* Batched BFGS of a user scalar kind (pnol_bfgs_batch), kept beside its launch table as the gradient launcher is. The launcher runs the
+ * whole minimisation of every start with pnol_bfgs_batch's arguments and semantics; X and the four outputs are DEVICE pointers, prm a
+ * host pointer, and the call only enqueues on env->stream. pnol::dev::ScalarTable<F>::bfgs_batch_ (include/pnol/device/
+ * functor_kernels.cuh) is one; PNOL_REGISTER_SCALAR_FUNCTOR attaches it for every scalar functor, and it serves the analytic flags only
+ * when F defines partial() (gradient, slope) and partial2() (Hessian with init_hess_fd), else PNOL_ERR_NO_FUNCTOR. */
+typedef int (*pnol_bfgs_batch_launcher)(const pnol_launch_env *, const pnol_functor_params *, long long B, int n, double * X,
+                                        const pnol_bfgs_params * prm, int deriv_flags, double * f0_out, double * fopt_out, int * iters_out,
+                                        int * stop_out);
+/* attaches fn to the table currently registered for a SCALAR user kind; pnol_register_functor replacing that table drops it. Returns
+ * PNOL_OK, or PNOL_ERR_INVALID for a residual kind, a kind without a registered table, or fn == NULL. Thread-safe. */
+int pnol_register_functor_bfgs_batch(int kind, pnol_bfgs_batch_launcher fn);
+/* 1 when pnol_bfgs_batch accepts the kind: the six built-in scalar objectives, and user scalar kinds with a batch launcher attached */
+int pnol_functor_has_bfgs_batch(int kind);
 
 int pnol_functor_create(pnol_ctx * ctx, const pnol_functor_desc * desc, pnol_functor ** out);
 void pnol_functor_destroy(pnol_functor * f);
@@ -402,6 +430,33 @@ int pnol_lm_iterate(pnol_ctx * ctx, const pnol_functor * f, double * x, const do
 int pnol_lm_batch(pnol_ctx * ctx, const pnol_functor * f, const long long * row_off, long long B, int n, double * X, const double * dx,
                   double lambda0, double lambda_factor, double x_min_diff, int max_iter, int jac_mode, double * chisq_out, double * lambda_out,
                   int * iters_out, int * stopped_out, double * F_out);
+
+/* Batched BFGS: B independent minimisations of ONE scalar objective in ONE kernel launch -- multiple starts, e.g. random points or a
+ * GA's best individuals -- each start's whole BFGS::findMin (Source/BFGS_with_linesearch.cpp:12-139: strong-Wolfe cubic-interpolation
+ * line search, the literal two-product updateHessianInv) on the device without a host round trip. Problem b starts from row b of X
+ * (B x n, row-major, in/out); all problems share the functor, its data columns and prm.
+ * Every problem returns, bit for bit, what the unmodified host BFGS::findMin returns on that start alone when the C-ABI's dense helpers
+ * are the reference's sequential ones (dotProd, matrixVectorMultiply, matrixMultiply, the LU of matrixInverse): X, f0_out and fopt_out
+ * (findMin's f0 and fOpt), iters_out (its iterationsDone) and stop_out, the first conjunct of the loop condition
+ * iter < maxIter && xdiff > xMinDiff && grad2Norm > minGrad2Norm that was false at the end: 0 max_iter, 1 xdiff (a NaN xdiff included),
+ * 2 the gradient norm. Line-search values are raw (no 1e10 sentinel); an exhausted line search leaves alpha = 0, and the update then
+ * turns D into NaN, as in the reference. A problem's bits depend neither on B nor on its position nor on the other problems. A NaN
+ * result is NaN in the same entries as on the host, with the GPU's NaN sign and payload (x86 encodes the NaN of an invalid operation
+ * differently).
+ * NOT the target: the BFGS classes of this library on the GPU (include/pnol/BFGS_with_linesearch.hpp) use the RANK2 update or the
+ * FP64 tensor-core products and agree with this call to about 1e-9 relative, not in every bit.
+ * deriv_flags: PNOL_BFGS_ANALYTIC_GRADIENT takes dFdX from partial() (dx_grad is not read), PNOL_BFGS_ANALYTIC_SLOPE the line-search slope
+ * p . grad f(x + alpha p) from partial() (dalpha is not read), PNOL_BFGS_ANALYTIC_HESSIAN the initial Hessian from partial2(); dx_hess
+ * is read only when the forward-difference Hessian initialises D.
+ *   - n in 1 .. 64 (larger problems: the BFGS class). B = 0 is a no-op.
+ *   - Every array may be a host or a device pointer, a misaligned one included. No collective: under a communicator each rank runs the
+ *     problems it was given.
+ *   - PNOL_ERR_INVALID: n outside 1 .. 64, B < 0 or B > 2^31 - 1, prm, X or an output NULL. A residual model is refused as the other
+ *     scalar entry points refuse it. PNOL_ERR_NO_FUNCTOR: a flag asks for a derivative the kind lacks (partial() for the gradient or
+ *     slope flags, partial2() for the Hessian flag with init_hess_fd), or a user kind without a batch launcher
+ *     (pnol_register_functor_bfgs_batch). */
+int pnol_bfgs_batch(pnol_ctx * ctx, const pnol_functor * f, long long B, int n, double * X, const pnol_bfgs_params * prm, int deriv_flags,
+                    double * f0_out, double * fopt_out, int * iters_out, int * stop_out);
 
 /* Which way the sums of the row-sharded LM step (J^T J | J^T F and the trial chi^2, Source/LevenbergMarquardtMPI.cpp:60-108) travel on
  * this context: 0 one rank, 1 NVLink peer memory inside the step's own kernels (csrc/peer.cu), 2 NCCL all-reduce (a peer mapping

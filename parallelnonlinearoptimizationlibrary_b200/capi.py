@@ -25,6 +25,7 @@ F_ROSENBROCK, F_POWER, F_BOOTH, F_GOLDSTEIN, F_RASTRIGIN, F_EXPCURVE_SINGLE = 1,
 F_EXPCURVE, F_CUBIC, F_LORENTZ_SUM = 101, 102, 103
 JAC_AUTO, JAC_BLACKBOX, JAC_STRUCTURED, JAC_ANALYTIC = 0, 1, 2, 3      # JAC_ANALYTIC: the model's own derivative, dx may be None
 HINV_LITERAL, HINV_RANK2 = 0, 1
+BFGS_ANALYTIC_GRADIENT, BFGS_ANALYTIC_SLOPE, BFGS_ANALYTIC_HESSIAN = 1, 2, 4      # pnol_bfgs_batch deriv_flags
 COMM_ID_BYTES = 128
 
 c_double_p = C.POINTER(C.c_double)
@@ -64,6 +65,23 @@ class GaParams(C.Structure):
     ]
 
 
+class BfgsParams(C.Structure):
+    """pnol_bfgs_params: BFGS::setParams' arguments in order"""
+    _fields_ = [
+        ("c1", C.c_double),
+        ("c2", C.c_double),
+        ("dalpha", C.c_double),
+        ("alpha_guess", C.c_double),
+        ("max_iter_ls", C.c_int),
+        ("dx_grad", C.c_double),
+        ("dx_hess", C.c_double),
+        ("max_iter", C.c_int),
+        ("x_min_diff", C.c_double),
+        ("min_grad_2norm", C.c_double),
+        ("init_hess_fd", C.c_int),
+    ]
+
+
 class GaStatus(C.Structure):
     _fields_ = [
         ("generation", C.c_int),
@@ -86,11 +104,12 @@ EXPORTS = [
     "pnol_comm_set_local", "pnol_comm_allreduce_sum", "pnol_comm_allgather", "pnol_comm_broadcast", "pnol_register_functor", "pnol_functor_registered",
     "pnol_register_functor_gradient", "pnol_functor_has_gradient", "pnol_register_functor_hessian", "pnol_functor_has_hessian",
     "pnol_register_functor_slope", "pnol_functor_has_slope", "pnol_register_functor_lm_batch", "pnol_functor_has_lm_batch",
+    "pnol_register_functor_bfgs_batch", "pnol_functor_has_bfgs_batch",
     "pnol_functor_create",
     "pnol_functor_destroy", "pnol_functor_is_residual", "pnol_functor_rows", "pnol_eval_batch", "pnol_fd_gradient",
     "pnol_eval_recur", "pnol_fd_gradient_recur", "pnol_gradient", "pnol_gradient_recur", "pnol_fd_hessian", "pnol_hessian", "pnol_alpha_pool",
     "pnol_alpha_pool_analytic", "pnol_residual_eval",
-    "pnol_fd_jacobian", "pnol_lm_normal_eq", "pnol_lm_damp", "pnol_lm_step", "pnol_lm_iterate", "pnol_lm_last_run", "pnol_lm_exchange_mode", "pnol_lm_batch", "pnol_lm_normal_eq_fused", "pnol_spd_solve", "pnol_lu_inverse",
+    "pnol_fd_jacobian", "pnol_lm_normal_eq", "pnol_lm_damp", "pnol_lm_step", "pnol_lm_iterate", "pnol_lm_last_run", "pnol_lm_exchange_mode", "pnol_lm_batch", "pnol_bfgs_batch", "pnol_lm_normal_eq_fused", "pnol_spd_solve", "pnol_lu_inverse",
     "pnol_matvec_neg", "pnol_bfgs_update_hinv", "pnol_dgemm_nn", "pnol_check_box_bounds", "pnol_compute_alpha_bnd",
     "pnol_stream_uniform", "pnol_ga_create", "pnol_ga_destroy", "pnol_ga_init", "pnol_ga_generation",
     "pnol_ga_status_get", "pnol_ga_set_sharding", "pnol_ga_peer_mode", "pnol_ga_get_population", "pnol_ga_get_indices", "pnol_ga_pop_sort", "pnol_ga_check_bounds",
@@ -532,6 +551,34 @@ class Context:
                                           C.c_double(factor), C.c_double(x_min_diff), int(max_iter), int(jac_mode), _ptr(chisq),
                                           _ptr(lam), _ptr(iters), _ptr(stopped), _ptr(F)))
         return dict(X=Xa, chisq=chisq, lam=lam, iters=iters, stopped=stopped, F=F)
+
+    def bfgs_batch(self, f, X, c1=1e-4, c2=0.9, dalpha=1e-6, alpha_guess=1.0, max_iter_ls=1000, dx_grad=1e-6, dx_hess=1e-3, max_iter=10000,
+                   x_min_diff=1e-5, min_grad_2norm=1e-5, init_hess_fd=False, flags=0, n=None, B=None, out=None, prm=None):
+        """Batched BFGS (pnol_bfgs_batch): start b is row b of X (B x n), every start minimises the scalar functor f. The keywords are
+        BFGS::setParams' (BFGS's defaults); prm (optional) a ready BfgsParams or None to pass NULL. flags: BFGS_ANALYTIC_* bits.
+        Returns dict(X, f0, fopt, iters, stop). X is minimised in place when it is a float64 numpy array, torch tensor or raw device
+        pointer (then pass n= and B=); otherwise a copy is returned. out (optional): dict of preallocated outputs under the same names."""
+        if isinstance(X, np.ndarray) and X.dtype == np.float64 and X.flags["C_CONTIGUOUS"]:
+            Xa = X
+        else:
+            Xa = _f64(X) if not isinstance(X, np.ndarray) else np.array(X, dtype=np.float64)
+        if B is None or n is None:
+            shape = tuple(Xa.shape)
+            B, n = (shape[0], shape[1]) if len(shape) == 2 else (1, shape[0])
+        if prm is None:
+            prm = BfgsParams(c1, c2, dalpha, alpha_guess, int(max_iter_ls), dx_grad, dx_hess, int(max_iter), x_min_diff, min_grad_2norm,
+                             int(bool(init_hess_fd)))
+        elif prm == "null":
+            prm = None
+        out = dict(out or {})
+        nb = max(int(B), 0)              # a negative B is the library's to refuse
+        f0 = out.get("f0", np.empty(nb))
+        fopt = out.get("fopt", np.empty(nb))
+        iters = out.get("iters", np.empty(nb, dtype=np.int32))
+        stop = out.get("stop", np.empty(nb, dtype=np.int32))
+        self.check(self.lib.pnol_bfgs_batch(self.h, f.handle, C.c_longlong(B), int(n), _ptr(Xa), C.byref(prm) if prm is not None else None,
+                                            int(flags), _ptr(f0), _ptr(fopt), _ptr(iters), _ptr(stop)))
+        return dict(X=Xa, f0=f0, fopt=fopt, iters=iters, stop=stop)
 
     def lm_exchange_mode(self):
         """0 one rank, 1 NVLink peer memory, 2 NCCL, -1 not decided yet"""

@@ -6,6 +6,11 @@
 #include "pnol/device/functor_kernels.cuh"
 
 namespace pnol {
+
+// builtin_bfgs_batch.cu: the batched BFGS launchers of the scalar objectives (bfgs_batch_kernel, 6 objectives x 4 configurations) take
+// long to compile; in a file of their own they build in parallel with the other kernels
+template <class F> pnol_bfgs_batch_launcher bfgs_batch_launcher();
+
 namespace {
 
 template <class F> KindTable scalar_kind(int n_columns)
@@ -16,6 +21,7 @@ template <class F> KindTable scalar_kind(int n_columns)
 	k.gradient = dev::ScalarTable<F>::gradient_;
 	k.hessian = dev::ScalarTable<F>::hessian_;
 	k.slope = dev::ScalarTable<F>::alpha_slope_;
+	k.bfgs_batch = bfgs_batch_launcher<F>();
 	return k;
 }
 

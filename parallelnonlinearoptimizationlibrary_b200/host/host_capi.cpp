@@ -14,6 +14,7 @@
 #include "pnol/LevenbergMarquardtMPI.hpp"
 #include "pnol/LevenbergMarquardtBatch.hpp"
 #include "pnol/BFGS_with_linesearch.hpp"
+#include "pnol/BFGSBatch.hpp"
 #include "pnol/BFGS_with_linesearch_MPI.hpp"
 #include "pnol/BFGS_bnd_linesearch_MPI_SW.hpp"
 #include "pnol/BFGS_bnd_linesearch.hpp"
@@ -365,6 +366,34 @@ int pnolhost_bfgs( const char * variant, const char * objective, double * X, int
 		if( fOpt ) *fOpt = b;
 		if( iters ) *iters = it;
 		gLastEvals = counted.evals;
+	} );
+}
+
+// BFGSBatch::findMin(X, reports) on one of the example objectives: X is B x n row-major (in/out), p[11] as for pnolhost_bfgs("bfgs");
+// single != 0: the base class's findMin(X, f0, fOpt) on the one start of X (B = 1; iters / stop are then not written)
+int pnolhost_bfgs_batch( const char * objective, double * X, long long B, int n, const double * p, int single, double * f0, double * fOpt,
+		int * iters, int * stop )
+{
+	return guarded( [&] {
+		std::unique_ptr<Objective> obj = makeScalar( objective );
+		BFGSBatch alg; alg.setObjPtr( *obj );
+		alg.setParams( p[0], p[1], p[2], p[3], (int) p[4], p[5], p[6], p[7], p[8], p[9], p[10] != 0, false );
+		if( single )
+		{
+			vector<double> Xv( X, X + n );
+			alg.findMin( Xv, f0[0], fOpt[0] );
+			memcpy( X, Xv.data(), n*sizeof(double) );
+			return;
+		}
+		vector<vector<double> > Xv( (size_t) B );
+		for( long long b = 0; b < B; b++ ) Xv[b].assign( X + b*n, X + (b + 1)*n );
+		vector<pnol::BFGSReport> rep;
+		alg.findMin( Xv, rep );
+		for( long long b = 0; b < B; b++ )
+		{
+			memcpy( X + b*n, Xv[b].data(), n*sizeof(double) );
+			f0[b] = rep[b].f0; fOpt[b] = rep[b].fOpt; iters[b] = rep[b].iterations; stop[b] = rep[b].stop;
+		}
 	} );
 }
 

@@ -265,6 +265,36 @@ def bfgs(variant, objective, x0, params, xlb=None, xub=None, pool_width=0, verbo
     return dict(X=Xv, f0=f0.value, fOpt=fopt.value, iterations=it.value)
 
 
+BFGS_DEFAULTS = dict(c1=1e-4, c2=0.9, dalpha=1e-6, alpha_guess=1.0, max_iter_ls=1000, dx_grad=1e-6, dx_hess=1e-3, max_iter=10000,
+                     x_min_diff=1e-5, min_grad_2norm=1e-5, init_hess_fd=0)
+
+
+def bfgs_params(**kw):
+    """BFGS::setParams' eleven numbers in order (pnolhost_bfgs("bfgs", ...) and bfgs_batch), BFGS's defaults for what kw leaves out"""
+    unknown = set(kw) - set(BFGS_DEFAULTS)
+    if unknown:
+        raise TypeError("unknown BFGS parameters %s" % sorted(unknown))
+    prm = dict(BFGS_DEFAULTS, **kw)
+    return np.array([float(prm[k]) for k in BFGS_DEFAULTS], dtype=np.float64)
+
+
+def bfgs_batch(objective, X, params=None, single=False):
+    """BFGSBatch::findMin(X, reports) on an example objective ("rosenbrock", "booth", "goldstein", "rastrigin", "expsingle", "power:k"):
+    X is B x n, one start per row; params: the eleven numbers of bfgs_params() (None: the defaults). The derivative modes are those set
+    with set_analytic_gradient / set_analytic_slope / set_analytic_hessian. Returns dict(X, f0, fOpt, iterations, stop). single=True:
+    the base class's findMin(X, f0, fOpt) on the one start of X (iterations and stop are then not reported: -1)."""
+    Xv = np.array(X, dtype=np.float64, order="C")
+    if Xv.ndim == 1:
+        Xv = Xv.reshape(1, -1)
+    B, n = Xv.shape
+    p = bfgs_params() if params is None else _f64(params)
+    f0, fopt = np.zeros(max(B, 1)), np.zeros(max(B, 1))
+    it, stop = np.full(max(B, 1), -1, dtype=np.int32), np.full(max(B, 1), -1, dtype=np.int32)
+    _check(lib().pnolhost_bfgs_batch(objective.encode(), _p(Xv), C.c_longlong(B), int(n), _p(p), int(bool(single)), _p(f0), _p(fopt), _p(it),
+                                     _p(stop)))
+    return dict(X=Xv, f0=f0[:B], fOpt=fopt[:B], iterations=it[:B], stop=stop[:B])
+
+
 def ga(objective, x0, xlb, xub, npop, maxgen, elite_frac=0.1, cross_frac=0.3, elite_mut_frac=0.2, mut_size=0.5,
        elite_mut_size=0.01, nstatic=50.0, serial=False):
     Xv, lb, ub = _f64(x0).copy(), _f64(xlb), _f64(xub)
