@@ -17,10 +17,11 @@
  *   3. link that object into your program / shared library next to libpnol_b200.so. The macro registers a launch table
  *      (pnol_functor_vtable, include/pnol_b200.h) at load time, and for a scalar functor with partial() also its gradient and slope
  *      launchers (pnol_register_functor_gradient / _slope), with partial2() its Hessian launcher (pnol_register_functor_hessian), for
- *      a residual model its batched LM launcher (pnol_register_functor_lm_batch);
+ *      a residual model its batched LM launcher (pnol_register_functor_lm_batch), for every scalar functor its batched BFGS and simplex
+ *      launchers (pnol_register_functor_bfgs_batch / _simplex_batch);
  *      pnol_functor_create(kind) and every entry point that takes a functor -- pnol_eval_batch, pnol_fd_gradient[_recur],
  *      pnol_gradient[_recur], pnol_fd_hessian, pnol_hessian, pnol_alpha_pool, pnol_alpha_pool_analytic, the GA, pnol_residual_eval,
- *      pnol_fd_jacobian, pnol_lm_step / pnol_lm_iterate, pnol_lm_batch -- then launch YOUR instantiations of the kernels below on the
+ *      pnol_fd_jacobian, pnol_lm_step / pnol_lm_iterate, pnol_lm_batch, pnol_bfgs_batch, pnol_simplex_batch -- then launch YOUR instantiations of the kernels below on the
  *      context's stream. The built-in objectives run through exactly these templates and tables (csrc/builtin_functors.cu).
  *
  * Everything here is header-only device / launch code; it needs nothing from the library but pnol_register_functor.
@@ -35,6 +36,8 @@
 #include "../../pnol_b200.h"
 #include "../functors.hpp"
 #include "exact_div.cuh"
+#include "random_stream.cuh"
+#include "simplex_sort.hpp"
 
 namespace pnol {
 namespace dev {
@@ -1488,6 +1491,291 @@ int bfgs_batch(const pnol_launch_env * env, const FunctorParams & P, long long B
 #undef PNOL_BFGS_BATCH_CFG
 }
 
+// ---------------------------------------------------------------------------------------------------
+// batched simplex search (pnol_simplex_batch): start b starts from row b of X (B x n) and runs SimplexSearch::findMin
+// (host/SimplexSearch.cpp, Source/SimplexSearch.cpp:13-349) on the functor's objective, operation for operation what the unmodified
+// host controller computes on the C-ABI's CPU stand-in, so every start returns the bits the reference returns on it alone:
+//   - start simplex: vertex 0 is the start, vertex i = 1 .. n is x0[j] + initRandMax*(u - 0.5)*2.0 with u the stream's value at
+//     stream_offset + b n^2 + (i - 1) n + j;
+//   - centroid: xbar[i] = xbar[i] + x[k][i]/n over the n best vertices in sorted order from k = 0, each term divided (x (1/n) when n is
+//     a power of two, else the IEEE quotient of div_exact: the divisor is loop-invariant); never a running centroid;
+//   - reflection xbar + alpha*(xbar - w), expansion xbar + gamma*(xbar - w), contraction xbar + rho*(w - xbar), shrink
+//     x0 + sigma*(xk - x0), all unfused, with the reference's accept rules; a shrink evaluates all n + 1 vertices, vertex 0 included
+//     (a sentinel of the sort can sit in f[0]);
+//   - simplexSort's permutation with both of its quirks (simplex_sort.hpp), and simplexDiff as a max with `>` (NaN skipped).
+// Mapping: one group of G lanes per start (G from n: 4, 8, 16 or 32), 32 * kSimplexBatchWarps / G starts per CTA, a start's state in
+// shared memory: the n + 1 vertex rows (physical storage), f and the sorted f, xbar, the candidate values, and idx (logical vertex k
+// lives in row idx[k]) with the sort's scratch. A sort permutes idx, not the rows. Outside simplexSort's regime a pass can take an
+// entry twice; the reference's rows are copies then, so the repeated entry gets the storage of the lost row and a copy of its content.
+// Every iteration lanes 0, 1 and 2 evaluate the reflection, the expansion and the contraction in one F::eval instruction stream
+// (SimplexCandAcc forms the coordinates on the fly), so that an iteration costs one evaluation latency; only the evaluations the
+// reference makes are counted (evals_out). The groups of a warp run independently: every barrier is the group's __syncwarp, every
+// reduction its shuffles, and a group that stopped idles until its warp ends.
+// ---------------------------------------------------------------------------------------------------
+constexpr int kSimplexBatchMaxN = 64;
+constexpr int kSimplexBatchWarps = 4;
+
+__host__ __device__ inline int simplex_batch_group(int n) { return n <= 4 ? 4 : (n <= 8 ? 8 : (n <= 16 ? 16 : 32)); }
+// shared memory of one start in doubles: the (n + 1) x n vertex rows, f and the sorted f (n + 1 each), xbar (n), the candidate values
+// (4), then five (n + 1)-int arrays (idx, the new idx, the pass order, the taken marks, the copy sources)
+__host__ __device__ inline int simplex_batch_stride(int n)
+{
+	const int N = n + 1;
+	return N * n + 2 * N + n + 4 + (5 * N + 1) / 2;
+}
+
+// a candidate from the centroid and the worst vertex w, formed on the fly: toward == 0 gives xbar + c*(xbar - w) (reflection,
+// expansion), toward == 1 xbar + c*(w - xbar) (contraction)
+struct SimplexCandAcc {
+	const double * xbar; const double * w; double c; int toward;
+	__device__ __forceinline__ double operator[](int j) const
+	{
+		const double xb = xbar[j], wj = w[j];
+		return xb + c * (toward ? wj - xb : xb - wj);
+	}
+};
+
+template <int G>
+__device__ __forceinline__ SimplexSortStats simplex_group_stats(const double * f, int N, int lane, unsigned gmask)
+{
+	SimplexSortStats s = simplex_stats_partial(f, N, lane, G);
+#pragma unroll
+	for (int o = G / 2; o > 0; o >>= 1) {
+		SimplexSortStats t;
+		t.M = __shfl_xor_sync(gmask, s.M, o, G);
+		t.m = __shfl_xor_sync(gmask, s.m, o, G);
+		t.iM = __shfl_xor_sync(gmask, s.iM, o, G);
+		t.im = __shfl_xor_sync(gmask, s.im, o, G);
+		t.nan = __shfl_xor_sync(gmask, s.nan, o, G);
+		s = simplex_stats_combine(s, t);
+	}
+	return s;
+}
+
+template <class F, int G>
+__global__ void __launch_bounds__(32 * kSimplexBatchWarps)
+simplex_batch_kernel(FunctorParams P, long long B, int n, double * __restrict__ X, pnol_simplex_params prm, StreamDev st,
+                     unsigned long long offset, double * __restrict__ f0_out, double * __restrict__ fopt_out, int * __restrict__ iters_out,
+                     int * __restrict__ stop_out, long long * __restrict__ evals_out)
+{
+	extern __shared__ double sm[];
+	constexpr int kGroups = 32 * kSimplexBatchWarps / G;
+	const int lane = threadIdx.x & (G - 1);
+	const int grp = threadIdx.x / G;
+	const long long b = (long long) blockIdx.x * kGroups + grp;
+	if (b >= B) return;
+	const unsigned gmask = G == 32 ? 0xffffffffu : (((1u << G) - 1u) << (threadIdx.x & 31 & ~(G - 1)));
+	const int N = n + 1;
+	double * V = sm + (size_t) grp * simplex_batch_stride(n);      // row r: V + r n
+	double * fv = V + N * n;                                        // f of logical vertex k
+	double * ft = fv + N;
+	double * xbar = ft + N;
+	double * cand = xbar + n;                                       // f of the reflection, expansion, contraction
+	int * idx = reinterpret_cast<int *>(cand + 4);
+	int * nidx = idx + N;
+	int * perm = nidx + N;
+	int * mark = perm + N;
+	int * csrc = mark + N;
+
+	// ---- simplexSort (:272-326): fv and idx in sorted order ----
+	auto sort = [&]() {
+		const SimplexSortStats s = simplex_group_stats<G>(fv, N, lane, gmask);
+		if (simplex_in_regime(fv, s)) {
+			const bool one_first = fv[1] == s.m;
+			for (int i = lane; i < N; i += G) {
+				const int r = simplex_rank(fv, N, i, one_first);
+				nidx[r] = idx[i];
+				ft[r] = fv[i];
+			}
+			__syncwarp(gmask);
+			for (int k = lane; k < N; k += G) { idx[k] = nidx[k]; fv[k] = ft[k]; }
+			__syncwarp(gmask);
+			return;
+		}
+		// the literal N passes, each a group argmin
+		const double S = 2 * simplex_first_max(fv, s);
+		int c = 1;
+		for (int k = 0; k < N; k++) {
+			const SimplexSortStats t = simplex_group_stats<G>(fv, N, lane, gmask);
+			c = simplex_pass_take(fv, c, t);
+			__syncwarp(gmask);
+			if (lane == 0) { perm[k] = c; ft[k] = fv[c]; fv[c] = S; }
+			__syncwarp(gmask);
+		}
+		// a repeated entry gets the storage of a lost one (exactly as many are lost as repeated) and a copy of its row
+		if (lane == 0) {
+			for (int l = 0; l < N; l++) mark[l] = 0;
+			for (int k = 0; k < N; k++) {
+				const int e = perm[k];
+				if (!mark[e]) { mark[e] = 1; nidx[k] = idx[e]; csrc[k] = -1; }
+				else { nidx[k] = -1; csrc[k] = idx[e]; }
+			}
+			int l = 0;
+			for (int k = 0; k < N; k++) {
+				if (nidx[k] >= 0) continue;
+				while (mark[l]) l++;
+				nidx[k] = idx[l++];
+			}
+		}
+		__syncwarp(gmask);
+		for (int k = 0; k < N; k++)
+			if (csrc[k] >= 0)
+				for (int j = lane; j < n; j += G) V[nidx[k] * n + j] = V[csrc[k] * n + j];
+		__syncwarp(gmask);
+		for (int k = lane; k < N; k += G) { idx[k] = nidx[k]; fv[k] = ft[k]; }
+		__syncwarp(gmask);
+	};
+
+	// ---- start simplex, its evaluation and sort (:47-73) ----
+	const unsigned long long base = offset + (unsigned long long) b * (unsigned long long) (n * n);
+	for (int e = lane; e < N * n; e += G) {
+		const int i = e / n, j = e - i * n;
+		double v = X[b * n + j];
+		if (i > 0) v = v + prm.init_rand_max * (st.u(base + (unsigned long long) (e - n)) - 0.5) * 2.0;
+		V[e] = v;
+	}
+	for (int k = lane; k < N; k += G) idx[k] = k;
+	__syncwarp(gmask);
+	for (int k = lane; k < N; k += G) {
+		const PtrAcc a{V + k * n};
+		fv[k] = F::eval(P, a, n);
+	}
+	__syncwarp(gmask);
+	const double f0 = fv[0];
+	long long evals = N;
+	sort();
+
+	const RecipDiv rd = make_recip((double) n);
+	const bool pow2 = (n & (n - 1)) == 0;
+	const bool three = recip_three_ok(rd) != 0;
+	const double rn = 1.0 / (double) n;
+	int iter = 0;
+	double xdiff = prm.x_min_diff * 2;
+	while (iter < prm.max_iter && xdiff > prm.x_min_diff) {
+		// centroid of the n best vertices (:86-98)
+		for (int i = lane; i < n; i += G) {
+			double s = 0.0;
+			for (int k = 0; k < n; k++) {
+				const double x = V[idx[k] * n + i];
+				double q;
+				if (pow2) q = x * rn;
+				else if (three && div_exact_x_ok_pz(x)) q = div_exact3_core(x, rd);
+				else q = div_exact(x, rd);
+				s = s + q;
+			}
+			xbar[i] = s;
+		}
+		__syncwarp(gmask);
+		// the three candidates at once (:100-172)
+		double * w = V + idx[n] * n;
+		if (lane < 3) {
+			const SimplexCandAcc acc{xbar, w, lane == 0 ? prm.alpha : (lane == 1 ? prm.gamma : prm.rho), lane == 2};
+			cand[lane] = F::eval(P, acc, n);
+		}
+		__syncwarp(gmask);
+		const double fr = cand[0], fe = cand[1], fc = cand[2];
+		int take;                                                   // 0 reflection, 1 expansion, 2 contraction, 3 shrink
+		evals += 1;
+		if (fr >= fv[0] && fr < fv[n - 1]) {
+			take = 0;
+		} else if (fr < fv[0]) {
+			evals += 1;
+			take = fe < fr ? 1 : 0;
+		} else {
+			evals += 1;
+			take = fc < fv[n] ? 2 : 3;
+		}
+		if (take < 3) {
+			const double c = take == 0 ? prm.alpha : (take == 1 ? prm.gamma : prm.rho);
+			for (int j = lane; j < n; j += G) {
+				const double xb = xbar[j], wj = w[j];
+				w[j] = xb + c * (take == 2 ? wj - xb : xb - wj);
+			}
+			__syncwarp(gmask);
+			if (lane == 0) fv[n] = take == 0 ? fr : (take == 1 ? fe : fc);
+		} else {
+			// shrink towards the best vertex, then evaluate all n + 1 vertices (:175-189)
+			const double * x0 = V + idx[0] * n;
+			for (int e = lane; e < n * n; e += G) {
+				const int k = 1 + e / n, j = e - (k - 1) * n;
+				double * xk = V + idx[k] * n;
+				xk[j] = x0[j] + prm.sigma * (xk[j] - x0[j]);
+			}
+			__syncwarp(gmask);
+			for (int k = lane; k < N; k += G) {
+				const PtrAcc a{V + idx[k] * n};
+				fv[k] = F::eval(P, a, n);
+			}
+			evals += N;
+		}
+		__syncwarp(gmask);
+		sort();
+		// simplexDiff (:330-349): the largest |x0[j] - xk[j]| found with `>`, NaN skipped
+		const double * x0 = V + idx[0] * n;
+		double mx = 0;
+		for (int e = lane; e < n * n; e += G) {
+			const int k = 1 + e / n, j = e - (k - 1) * n;
+			const double d = fabs(x0[j] - V[idx[k] * n + j]);
+			if (d > mx) mx = d;
+		}
+#pragma unroll
+		for (int o = G / 2; o > 0; o >>= 1) {
+			const double t = __shfl_xor_sync(gmask, mx, o, G);
+			if (t > mx) mx = t;
+		}
+		xdiff = mx;
+		iter = iter + 1;
+	}
+	for (int j = lane; j < n; j += G) X[b * n + j] = V[idx[0] * n + j];
+	if (lane == 0) {
+		f0_out[b] = f0;
+		fopt_out[b] = fv[0];
+		iters_out[b] = iter;
+		stop_out[b] = !(iter < prm.max_iter) ? 0 : 1;
+		if (evals_out) evals_out[b] = evals;
+	}
+}
+
+template <class F, int G>
+int simplex_batch_launch(const pnol_launch_env * env, const FunctorParams & P, long long B, int n, double * X, const pnol_simplex_params & prm,
+                         const StreamDev & st, unsigned long long offset, double * f0_out, double * fopt_out, int * iters_out, int * stop_out,
+                         long long * evals_out)
+{
+	constexpr int kGroups = 32 * kSimplexBatchWarps / G;
+	const size_t smem = (size_t) kGroups * simplex_batch_stride(n) * sizeof(double);
+	PNOL_DEV_REQUIRE(env, smem <= env->smem_optin, "simplex batch: n = %d needs %zu bytes of shared memory", n, smem);
+	auto kern = simplex_batch_kernel<F, G>;
+	PNOL_DEV_CUDA(env, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem));
+	const long long grid = (B + kGroups - 1) / kGroups;
+	PNOL_DEV_LAUNCH(env, kern, (unsigned) grid, 32 * kSimplexBatchWarps, smem, P, B, n, X, prm, st, offset, f0_out, fopt_out, iters_out,
+	                stop_out, evals_out);
+	return PNOL_OK;
+}
+
+/* pnol_simplex_batch on device pointers: X (B x n, in/out), the per-start outputs (B; evals_out may be NULL), stream->values (when set)
+ * a device array whose value at position p is values[p]. n in 1 .. 64. */
+template <class F>
+int simplex_batch(const pnol_launch_env * env, const FunctorParams & P, long long B, int n, double * X, const pnol_simplex_params * prm,
+                  const pnol_stream_desc * stream, uint64_t stream_offset, double * f0_out, double * fopt_out, int * iters_out, int * stop_out,
+                  long long * evals_out)
+{
+	PNOL_DEV_REQUIRE(env, n >= 1 && n <= kSimplexBatchMaxN, "simplex batch: n = %d is outside 1 .. %d", n, kSimplexBatchMaxN);
+	PNOL_DEV_REQUIRE(env, B >= 0 && B <= 0x7fffffffLL, "simplex batch: B = %lld is outside 0 .. 2^31 - 1", B);
+	PNOL_DEV_REQUIRE(env, prm != nullptr && stream != nullptr, "simplex batch: the parameters and the stream are required");
+	if (B == 0) return PNOL_OK;
+	StreamDev st;
+	st.values = stream->values; st.n_values = stream->n_values; st.seed = stream->seed; st.scale = stream->scale;
+#define PNOL_SIMPLEX_BATCH_CFG(G) \
+	simplex_batch_launch<F, G>(env, P, B, n, X, *prm, st, stream_offset, f0_out, fopt_out, iters_out, stop_out, evals_out)
+	switch (simplex_batch_group(n)) {
+		case 4: return PNOL_SIMPLEX_BATCH_CFG(4);
+		case 8: return PNOL_SIMPLEX_BATCH_CFG(8);
+		case 16: return PNOL_SIMPLEX_BATCH_CFG(16);
+		default: return PNOL_SIMPLEX_BATCH_CFG(32);
+	}
+#undef PNOL_SIMPLEX_BATCH_CFG
+}
+
 /* ---- launch tables (pnol_functor_vtable) of a functor type ---- */
 template <class F> struct ScalarTable {
 	static int eval_batch_(const pnol_launch_env * env, const pnol_functor_params * P, const double * pts, long long B, int n, long long ld,
@@ -1511,6 +1799,10 @@ template <class F> struct ScalarTable {
 	static int bfgs_batch_(const pnol_launch_env * env, const pnol_functor_params * P, long long B, int n, double * X, const pnol_bfgs_params * prm,
 	                       int flags, double * f0_out, double * fopt_out, int * iters_out, int * stop_out)
 	{ return bfgs_batch<F>(env, *P, B, n, X, prm, flags, f0_out, fopt_out, iters_out, stop_out); }
+	static int simplex_batch_(const pnol_launch_env * env, const pnol_functor_params * P, long long B, int n, double * X,
+	                          const pnol_simplex_params * prm, const pnol_stream_desc * stream, uint64_t stream_offset, double * f0_out,
+	                          double * fopt_out, int * iters_out, int * stop_out, long long * evals_out)
+	{ return simplex_batch<F>(env, *P, B, n, X, prm, stream, stream_offset, f0_out, fopt_out, iters_out, stop_out, evals_out); }
 	static pnol_functor_vtable make(int n_columns)
 	{
 		pnol_functor_vtable vt = {};
@@ -1522,12 +1814,13 @@ template <class F> struct ScalarTable {
 		vt.alpha_pool = alpha_pool_;
 		return vt;
 	}
-	/* registers the table, then its batched BFGS launcher, (F defines partial) its gradient and line-search slope launchers and (F defines
-	 * partial2) its Hessian launcher, in this order: a launcher attaches to the registered table */
+	/* registers the table, then its batched BFGS and simplex launchers, (F defines partial) its gradient and line-search slope launchers
+	 * and (F defines partial2) its Hessian launcher, in this order: a launcher attaches to the registered table */
 	static int register_as(int kind, const pnol_functor_vtable * vt)
 	{
 		int st = pnol_register_functor(kind, vt);
 		if (st == PNOL_OK) st = pnol_register_functor_bfgs_batch(kind, bfgs_batch_);
+		if (st == PNOL_OK) st = pnol_register_functor_simplex_batch(kind, simplex_batch_);
 		if constexpr (has_partial<F>::value) {
 			if (st == PNOL_OK) st = pnol_register_functor_gradient(kind, gradient_);
 			if (st == PNOL_OK) st = pnol_register_functor_slope(kind, alpha_slope_);

@@ -131,7 +131,9 @@ typedef struct {
  *                                              launcher attached with pnol_register_functor_gradient: pnol_gradient[_recur], and
  *                                              a Hessian launcher attached with pnol_register_functor_hessian: pnol_hessian, and
  *                                              a slope launcher attached with pnol_register_functor_slope: pnol_alpha_pool_analytic,
- *                                              and a batch BFGS launcher attached with pnol_register_functor_bfgs_batch: pnol_bfgs_batch)
+ *                                              a batch BFGS launcher attached with pnol_register_functor_bfgs_batch: pnol_bfgs_batch,
+ *                                              and a batch simplex launcher attached with pnol_register_functor_simplex_batch:
+ *                                              pnol_simplex_batch)
  *     kinds [PNOL_F_USER_RESIDUAL_BASE, +1000) residual models    (residual, fd_jacobian; optionally jacobian: PNOL_JAC_ANALYTIC; a batch
  *                                              LM launcher attached with pnol_register_functor_lm_batch: pnol_lm_batch)
  * pnol_functor_create and every entry point that takes a functor then work for that kind as for the built-ins; libpnol_b200.so is not
@@ -529,6 +531,55 @@ typedef struct {
 	double scale;               /* counter mode: values lie in [0, scale); use scale <= 1 - 0.5/Npop */
 } pnol_stream_desc;
 double pnol_stream_uniform(uint64_t seed, uint64_t k, double scale);
+
+/* ---------------------------------------------------------------------------------------------------
+ * Batched simplex search: B independent Nelder-Mead minimisations of ONE scalar objective in ONE kernel launch -- multiple starts of
+ * an objective without derivatives (no partial(), noisy, piecewise) -- each start's whole SimplexSearch::findMin
+ * (Source/SimplexSearch.cpp:13-349) on the device without a host round trip. Start b starts from row b of X (B x n, row-major,
+ * in/out); all starts share the functor, its data columns and prm.
+ * ------------------------------------------------------------------------------------------------- */
+/* SimplexSearch::setSimplexParams' arguments in the same order (verbose is not kept) */
+typedef struct pnol_simplex_params {
+	double alpha, gamma, rho, sigma;
+	int max_iter;
+	double init_rand_max, x_min_diff;
+} pnol_simplex_params;
+
+/* Batched simplex search of a user scalar kind (pnol_simplex_batch), kept beside its launch table as the batched BFGS launcher is. The
+ * launcher runs every start with pnol_simplex_batch's arguments and semantics, except that stream->values (when set) is a DEVICE array
+ * whose value at stream position p is values[p] (pnol_simplex_batch stages the slice it needs and passes stream_offset 0 with it); X
+ * and the outputs are DEVICE pointers (evals_out may be NULL), prm and stream host pointers, and the call only enqueues on env->stream.
+ * pnol::dev::ScalarTable<F>::simplex_batch_ (include/pnol/device/functor_kernels.cuh) is one; PNOL_REGISTER_SCALAR_FUNCTOR attaches it
+ * for every scalar functor (no derivative is needed). */
+typedef int (*pnol_simplex_batch_launcher)(const pnol_launch_env *, const pnol_functor_params *, long long B, int n, double * X,
+                                           const pnol_simplex_params * prm, const pnol_stream_desc * stream, uint64_t stream_offset,
+                                           double * f0_out, double * fopt_out, int * iters_out, int * stop_out, long long * evals_out);
+/* attaches fn to the table currently registered for a SCALAR user kind; pnol_register_functor replacing that table drops it. Returns
+ * PNOL_OK, or PNOL_ERR_INVALID for a residual kind, a kind without a registered table, or fn == NULL. Thread-safe. */
+int pnol_register_functor_simplex_batch(int kind, pnol_simplex_batch_launcher fn);
+/* 1 when pnol_simplex_batch accepts the kind: the six built-in scalar objectives, and user scalar kinds with a batch launcher attached */
+int pnol_functor_has_simplex_batch(int kind);
+
+/* Every start returns, bit for bit, what the unmodified host SimplexSearch::findMin returns on that start alone when its start simplex
+ * draws the same values: X (the best vertex), f0_out (f at the start point, findMin's f0), fopt_out (its fOpt), iters_out
+ * (iterations()), stop_out (the first false conjunct of iter < maxIter && xdiff > xMinDiff: 0 max_iter, 1 xdiff, a NaN xdiff
+ * included) and evals_out (may be NULL: the objective evaluations the reference makes, n + 1 at the start, then per iteration 1, plus
+ * 1 for an expansion or a contraction, plus n + 1 for a shrink). simplexSort's quirks are reproduced: outside 0 < max f < inf without
+ * NaN the sorted f can hold its 2 max f sentinels and a vertex can appear twice. A start's bits depend neither on B nor on its
+ * position nor on the other starts; a NaN result is NaN in the same entries as on the host, with the GPU's NaN sign and payload.
+ * Random draws: start b takes its n^2 start-simplex draws at stream positions stream_offset + b n^2 + (i - 1) n + j for vertex
+ * i = 1 .. n and coordinate j; with stream_offset = 0 and B = 1 that is exactly what SimplexSearch::findMin consumes. The offset lets
+ * a caller split one batch into chunks, or across ranks, with the same bits.
+ *   - n in 1 .. 64 (larger problems: the SimplexSearch class). B = 0 is a no-op.
+ *   - Every array may be a host or a device pointer, a misaligned one included. No collective: under a communicator each rank runs the
+ *     starts it was given.
+ *   - PNOL_ERR_INVALID: n outside 1 .. 64, B < 0 or B > 2^31 - 1, prm, stream, X or a required output NULL. A residual model is refused
+ *     as the other scalar entry points refuse it. PNOL_ERR_STREAM: an explicit stream with fewer than stream_offset + B n^2 values
+ *     (checked before anything runs: X and the outputs are left untouched). PNOL_ERR_NO_FUNCTOR: a user kind without a batch launcher
+ *     (pnol_register_functor_simplex_batch). */
+int pnol_simplex_batch(pnol_ctx * ctx, const pnol_functor * f, long long B, int n, double * X, const pnol_simplex_params * prm,
+                       const pnol_stream_desc * stream, uint64_t stream_offset, double * f0_out, double * fopt_out, int * iters_out,
+                       int * stop_out, long long * evals_out);
 
 /* ---------------------------------------------------------------------------------------------------
  * a15 / a16: genetic algorithm state machine (Source/GeneticAlgorithmMPI.cpp:12-276)

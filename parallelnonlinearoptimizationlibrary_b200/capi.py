@@ -82,6 +82,19 @@ class BfgsParams(C.Structure):
     ]
 
 
+class SimplexParams(C.Structure):
+    """pnol_simplex_params: SimplexSearch::setSimplexParams' arguments in order"""
+    _fields_ = [
+        ("alpha", C.c_double),
+        ("gamma", C.c_double),
+        ("rho", C.c_double),
+        ("sigma", C.c_double),
+        ("max_iter", C.c_int),
+        ("init_rand_max", C.c_double),
+        ("x_min_diff", C.c_double),
+    ]
+
+
 class GaStatus(C.Structure):
     _fields_ = [
         ("generation", C.c_int),
@@ -104,12 +117,12 @@ EXPORTS = [
     "pnol_comm_set_local", "pnol_comm_allreduce_sum", "pnol_comm_allgather", "pnol_comm_broadcast", "pnol_register_functor", "pnol_functor_registered",
     "pnol_register_functor_gradient", "pnol_functor_has_gradient", "pnol_register_functor_hessian", "pnol_functor_has_hessian",
     "pnol_register_functor_slope", "pnol_functor_has_slope", "pnol_register_functor_lm_batch", "pnol_functor_has_lm_batch",
-    "pnol_register_functor_bfgs_batch", "pnol_functor_has_bfgs_batch",
+    "pnol_register_functor_bfgs_batch", "pnol_functor_has_bfgs_batch", "pnol_register_functor_simplex_batch", "pnol_functor_has_simplex_batch",
     "pnol_functor_create",
     "pnol_functor_destroy", "pnol_functor_is_residual", "pnol_functor_rows", "pnol_eval_batch", "pnol_fd_gradient",
     "pnol_eval_recur", "pnol_fd_gradient_recur", "pnol_gradient", "pnol_gradient_recur", "pnol_fd_hessian", "pnol_hessian", "pnol_alpha_pool",
     "pnol_alpha_pool_analytic", "pnol_residual_eval",
-    "pnol_fd_jacobian", "pnol_lm_normal_eq", "pnol_lm_damp", "pnol_lm_step", "pnol_lm_iterate", "pnol_lm_last_run", "pnol_lm_exchange_mode", "pnol_lm_batch", "pnol_bfgs_batch", "pnol_lm_normal_eq_fused", "pnol_spd_solve", "pnol_lu_inverse",
+    "pnol_fd_jacobian", "pnol_lm_normal_eq", "pnol_lm_damp", "pnol_lm_step", "pnol_lm_iterate", "pnol_lm_last_run", "pnol_lm_exchange_mode", "pnol_lm_batch", "pnol_bfgs_batch", "pnol_simplex_batch", "pnol_lm_normal_eq_fused", "pnol_spd_solve", "pnol_lu_inverse",
     "pnol_matvec_neg", "pnol_bfgs_update_hinv", "pnol_dgemm_nn", "pnol_check_box_bounds", "pnol_compute_alpha_bnd",
     "pnol_stream_uniform", "pnol_ga_create", "pnol_ga_destroy", "pnol_ga_init", "pnol_ga_generation",
     "pnol_ga_status_get", "pnol_ga_set_sharding", "pnol_ga_peer_mode", "pnol_ga_get_population", "pnol_ga_get_indices", "pnol_ga_pop_sort", "pnol_ga_check_bounds",
@@ -579,6 +592,48 @@ class Context:
         self.check(self.lib.pnol_bfgs_batch(self.h, f.handle, C.c_longlong(B), int(n), _ptr(Xa), C.byref(prm) if prm is not None else None,
                                             int(flags), _ptr(f0), _ptr(fopt), _ptr(iters), _ptr(stop)))
         return dict(X=Xa, f0=f0, fopt=fopt, iters=iters, stop=stop)
+
+    def simplex_batch(self, f, X, alpha=1.0, gamma=2.0, rho=0.5, sigma=0.5, max_iter=10000, init_rand_max=1.0, x_min_diff=1e-7, stream=None,
+                      stream_offset=0, n=None, B=None, out=None, prm=None, want_evals=True):
+        """Batched simplex search (pnol_simplex_batch): start b is row b of X (B x n), every start minimises the scalar functor f. The
+        keywords are SimplexSearch::setSimplexParams' (SimplexSearch's defaults); prm (optional) a ready SimplexParams, or "null" to pass
+        NULL. stream: a StreamDesc, an array of explicit values (host or device), an int seed of the counter stream (scale 1), or "null";
+        None is the counter stream with seed 0. Returns dict(X, f0, fopt, iters, stop, evals). X is minimised in place when it is a
+        float64 numpy array, torch tensor or raw device pointer (then pass n= and B=); otherwise a copy is returned. out (optional): dict
+        of preallocated outputs under the same names; want_evals=False passes NULL for evals."""
+        if isinstance(X, np.ndarray) and X.dtype == np.float64 and X.flags["C_CONTIGUOUS"]:
+            Xa = X
+        else:
+            Xa = _f64(X) if not isinstance(X, np.ndarray) else np.array(X, dtype=np.float64)
+        if B is None or n is None:
+            shape = tuple(Xa.shape)
+            B, n = (shape[0], shape[1]) if len(shape) == 2 else (1, shape[0])
+        if prm is None:
+            prm = SimplexParams(alpha, gamma, rho, sigma, int(max_iter), init_rand_max, x_min_diff)
+        elif prm == "null":
+            prm = None
+        keep = None
+        if stream is None or isinstance(stream, (int, np.integer)):
+            sd = StreamDesc(None, 0, int(stream or 0), 1.0)
+        elif isinstance(stream, StreamDesc):
+            sd = stream
+        elif isinstance(stream, str) and stream == "null":
+            sd = None
+        else:
+            keep = stream if hasattr(stream, "data_ptr") else np.ascontiguousarray(stream, dtype=np.float64)
+            sd = StreamDesc(_ptr(keep).value, int(keep.numel() if hasattr(keep, "numel") else keep.size), 0, 1.0)
+        out = dict(out or {})
+        nb = max(int(B), 0)              # a negative B is the library's to refuse
+        f0 = out.get("f0", np.empty(nb))
+        fopt = out.get("fopt", np.empty(nb))
+        iters = out.get("iters", np.empty(nb, dtype=np.int32))
+        stop = out.get("stop", np.empty(nb, dtype=np.int32))
+        evals = out.get("evals", np.empty(nb, dtype=np.int64)) if want_evals else None
+        self.check(self.lib.pnol_simplex_batch(self.h, f.handle, C.c_longlong(B), int(n), _ptr(Xa), C.byref(prm) if prm is not None else None,
+                                               C.byref(sd) if sd is not None else None, C.c_uint64(int(stream_offset)), _ptr(f0), _ptr(fopt),
+                                               _ptr(iters), _ptr(stop), _ptr(evals)))
+        del keep
+        return dict(X=Xa, f0=f0, fopt=fopt, iters=iters, stop=stop, evals=evals)
 
     def lm_exchange_mode(self):
         """0 one rank, 1 NVLink peer memory, 2 NCCL, -1 not decided yet"""

@@ -10,6 +10,8 @@ namespace pnol {
 // builtin_bfgs_batch.cu: the batched BFGS launchers of the scalar objectives (bfgs_batch_kernel, 6 objectives x 4 configurations) take
 // long to compile; in a file of their own they build in parallel with the other kernels
 template <class F> pnol_bfgs_batch_launcher bfgs_batch_launcher();
+// builtin_simplex_batch.cu: the batched simplex launchers (simplex_batch_kernel, 6 objectives x 4 group sizes), for the same reason
+template <class F> pnol_simplex_batch_launcher simplex_batch_launcher();
 
 namespace {
 
@@ -22,6 +24,7 @@ template <class F> KindTable scalar_kind(int n_columns)
 	k.hessian = dev::ScalarTable<F>::hessian_;
 	k.slope = dev::ScalarTable<F>::alpha_slope_;
 	k.bfgs_batch = bfgs_batch_launcher<F>();
+	k.simplex_batch = simplex_batch_launcher<F>();
 	return k;
 }
 

@@ -382,6 +382,10 @@ extern "C" int pnol_register_functor_hessian(int kind, pnol_hessian_launcher fn)
 extern "C" int pnol_register_functor_slope(int kind, pnol_slope_launcher fn) { return attach(kind, false, &KindTable::slope, fn); }
 extern "C" int pnol_register_functor_lm_batch(int kind, pnol_lm_batch_launcher fn) { return attach(kind, true, &KindTable::lm_batch, fn); }
 extern "C" int pnol_register_functor_bfgs_batch(int kind, pnol_bfgs_batch_launcher fn) { return attach(kind, false, &KindTable::bfgs_batch, fn); }
+extern "C" int pnol_register_functor_simplex_batch(int kind, pnol_simplex_batch_launcher fn)
+{
+	return attach(kind, false, &KindTable::simplex_batch, fn);
+}
 
 extern "C" int pnol_functor_registered(int kind)
 {
@@ -412,6 +416,11 @@ extern "C" int pnol_functor_has_bfgs_batch(int kind)
 {
 	KindTable k;
 	return pnol::kind_table(kind, &k) && k.bfgs_batch;
+}
+extern "C" int pnol_functor_has_simplex_batch(int kind)
+{
+	KindTable k;
+	return pnol::kind_table(kind, &k) && k.simplex_batch;
 }
 
 extern "C" int pnol_functor_create(pnol_ctx * ctx, const pnol_functor_desc * desc, pnol_functor ** out)

@@ -230,6 +230,7 @@ struct KindTable {
 	pnol_slope_launcher slope;            // scalar objectives, may be null: pnol_alpha_pool_analytic
 	pnol_lm_batch_launcher lm_batch;      // residual models, may be null: pnol_lm_batch
 	pnol_bfgs_batch_launcher bfgs_batch;  // scalar objectives, may be null: pnol_bfgs_batch
+	pnol_simplex_batch_launcher simplex_batch;  // scalar objectives, may be null: pnol_simplex_batch
 };
 // copies out the record of a built-in or registered kind (capi.cu); false for any other kind. A copy, so that re-registering a kind
 // while a launch runs is safe.

@@ -23,11 +23,12 @@
 #include "pnol/GeneticAlgorithmMPI.hpp"
 #include "pnol/Box_boundary_functions.hpp"
 #include "pnol/SimplexSearch.hpp"
+#include "pnol/SimplexSearchBatch.hpp"
 
 namespace {
 
 std::string gErr;
-long long gLastEvals = 0;          // objective evaluations of the last pnolhost_bfgs run
+long long gLastEvals = 0;          // objective evaluations of the last pnolhost_bfgs / pnolhost_simplex[_batch] run
 
 struct CoutSilencer {
 	std::streambuf * old;
@@ -397,7 +398,8 @@ int pnolhost_bfgs_batch( const char * objective, double * X, long long B, int n,
 	} );
 }
 
-// objective evaluations (host objEval calls and points evaluated on the device twin) of the last pnolhost_bfgs run
+// objective evaluations (host objEval calls and points evaluated on the device twin) of the last pnolhost_bfgs, pnolhost_simplex or
+// pnolhost_simplex_batch run
 long long pnolhost_last_evaluations() { return gLastEvals; }
 
 // SimplexSearch::findMin on one of the example objectives. p[7] = alpha gamma rho sigma maxIter initRandMax xMinDiff; the start simplex
@@ -407,15 +409,53 @@ int pnolhost_simplex( const char * objective, double * X, int n, const double * 
 	return guarded( [&] {
 		CoutSilencer quiet( verbose == 0 );
 		std::unique_ptr<Objective> obj = makeScalar( objective );
+		CountingObjective counted( *obj );
+		gLastEvals = 0;
 		vector<double> Xv( X, X + n );
-		SimplexSearch alg; alg.setObjPtr( *obj );
+		SimplexSearch alg; alg.setObjPtr( counted );
 		alg.setSimplexParams( p[0], p[1], p[2], p[3], (int) p[4], p[5], p[6], verbose != 0 );
 		double a = 0, b = 0;
 		alg.findMin( Xv, a, b );
+		gLastEvals = counted.evals;
 		memcpy( X, Xv.data(), n*sizeof(double) );
 		if( f0 ) *f0 = a;
 		if( fOpt ) *fOpt = b;
 		if( report ) { report[0] = alg.iterations(); report[1] = (double) alg.streamPosition(); }
+	} );
+}
+
+// SimplexSearchBatch::findMin(X, reports) on one of the example objectives: X is B x n row-major (in/out), p[7] as for pnolhost_simplex;
+// the start simplices draw from the stream set with pnolhost_set_stream(). single != 0: the base class's findMin(X, f0, fOpt) on the
+// one start of X (B = 1; iters / stop / evals are then not written). report[1] (may be NULL): the stream position afterwards.
+int pnolhost_simplex_batch( const char * objective, double * X, long long B, int n, const double * p, int single, double * f0, double * fOpt,
+		int * iters, int * stop, long long * evals, double * report )
+{
+	return guarded( [&] {
+		std::unique_ptr<Objective> obj = makeScalar( objective );
+		CountingObjective counted( *obj );
+		gLastEvals = 0;
+		SimplexSearchBatch alg; alg.setObjPtr( counted );
+		alg.setSimplexParams( p[0], p[1], p[2], p[3], (int) p[4], p[5], p[6], false );
+		if( single )
+		{
+			vector<double> Xv( X, X + n );
+			alg.findMin( Xv, f0[0], fOpt[0] );
+			memcpy( X, Xv.data(), n*sizeof(double) );
+		}
+		else
+		{
+			vector<vector<double> > Xv( (size_t) B );
+			for( long long b = 0; b < B; b++ ) Xv[b].assign( X + b*n, X + (b + 1)*n );
+			vector<pnol::SimplexReport> rep;
+			alg.findMin( Xv, rep );
+			for( long long b = 0; b < B; b++ )
+			{
+				memcpy( X + b*n, Xv[b].data(), n*sizeof(double) );
+				f0[b] = rep[b].f0; fOpt[b] = rep[b].fOpt; iters[b] = rep[b].iterations; stop[b] = rep[b].stop; evals[b] = rep[b].evaluations;
+			}
+		}
+		gLastEvals = counted.evals;
+		if( report ) { report[0] = 0; report[1] = (double) alg.streamPosition(); }
 	} );
 }
 

@@ -317,6 +317,25 @@ def simplex(objective, x0, alpha=1.0, gamma=2.0, rho=0.5, sigma=0.5, maxiter=100
     return dict(X=Xv, f0=f0.value, fOpt=fopt.value, iterations=int(rep[0]), stream_pos=int(rep[1]))
 
 
+def simplex_batch(objective, X, alpha=1.0, gamma=2.0, rho=0.5, sigma=0.5, maxiter=10000, init_rand_max=1.0, xmindiff=1e-7, single=False):
+    """SimplexSearchBatch::findMin(X, reports) on an example objective ("rosenbrock", "booth", "goldstein", "rastrigin", "expsingle",
+    "power:k"): X is B x n, one start per row; start b draws its start simplex from position b n^2 of the stream of set_stream().
+    Returns dict(X, f0, fOpt, iterations, stop, evals, stream_pos). single=True: the base class's findMin(X, f0, fOpt) on the one start
+    of X (iterations, stop and evals are then not reported: -1)."""
+    Xv = np.array(X, dtype=np.float64, order="C")
+    if Xv.ndim == 1:
+        Xv = Xv.reshape(1, -1)
+    B, n = Xv.shape
+    p = _f64([alpha, gamma, rho, sigma, maxiter, init_rand_max, xmindiff])
+    f0, fopt = np.zeros(max(B, 1)), np.zeros(max(B, 1))
+    it, stop = np.full(max(B, 1), -1, dtype=np.int32), np.full(max(B, 1), -1, dtype=np.int32)
+    ev = np.full(max(B, 1), -1, dtype=np.int64)
+    rep = np.zeros(2)
+    _check(lib().pnolhost_simplex_batch(objective.encode(), _p(Xv), C.c_longlong(B), int(n), _p(p), int(bool(single)), _p(f0), _p(fopt),
+                                        _p(it), _p(stop), _p(ev), _p(rep)))
+    return dict(X=Xv, f0=f0[:B], fOpt=fopt[:B], iterations=it[:B], stop=stop[:B], evals=ev[:B], stream_pos=int(rep[1]))
+
+
 def check_box_bounds(x, xlb, xub):
     Xv, lb, ub = _f64(x).copy(), _f64(xlb), _f64(xub)
     _check(lib().pnolhost_check_box_bounds(_p(Xv), _p(lb), _p(ub), Xv.size))
