@@ -1,5 +1,5 @@
 """Shared cases of the batched BFGS tests: the objectives, their dimensions, seeded starts and parameters, and the runners of the CPU
-stand-in (tests/host_logic_bfgs_batch.cpp): oracle_bfgs per start through BFGSBatch, and the unmodified host BFGS controller per start."""
+stand-in (tests/host_logic_standin.cpp): oracle_bfgs per start through BFGSBatch, and the unmodified host BFGS controller per start."""
 import ctypes as C
 
 import numpy as np

@@ -1,5 +1,5 @@
 """Shared cases of the batched simplex tests: the objectives and their dimensions (those of tests/bfgs_batch_cases.py), seeded starts,
-parameters and streams, and the runners of the CPU stand-in (tests/host_logic_simplex_batch.cpp): oracle_simplex per start through
+parameters and streams, and the runners of the CPU stand-in (tests/host_logic_standin.cpp): oracle_simplex per start through
 SimplexSearchBatch or the stand-in's C-ABI, and the unmodified host SimplexSearch controller per start on exactly that start's draws."""
 import ctypes as C
 
@@ -68,8 +68,11 @@ def run_batch(lib, name, X, prm, stream):
     ev = np.zeros(B, dtype=np.int64)
     rep = np.zeros(2)
     keep = set_stream(lib, stream)
-    st = lib.pnolhost_simplex_batch(name.encode(), _p(Xv), C.c_longlong(B), int(n), _p(vec(prm)), 0, _p(f0), _p(fopt), _p(it), _p(stop),
-                                    _p(ev), _p(rep))
+    try:
+        st = lib.pnolhost_simplex_batch(name.encode(), _p(Xv), C.c_longlong(B), int(n), _p(vec(prm)), 0, _p(f0), _p(fopt), _p(it), _p(stop),
+                                        _p(ev), _p(rep))
+    finally:
+        lib.pnolhost_clear_stream()
     del keep
     return st, dict(X=Xv, f0=f0, fopt=fopt, iters=it, stop=stop, evals=ev, stream_pos=int(rep[1]), total_evals=int(lib.pnolhost_last_evaluations()))
 
@@ -80,7 +83,10 @@ def run_serial(lib, name, x0, prm, values):
     f0, fopt = C.c_double(), C.c_double()
     rep = np.zeros(2)
     keep = set_stream(lib, ("values", values))
-    st = lib.pnolhost_simplex(name.encode(), _p(Xv), Xv.size, _p(vec(prm)), 0, C.byref(f0), C.byref(fopt), _p(rep))
+    try:
+        st = lib.pnolhost_simplex(name.encode(), _p(Xv), Xv.size, _p(vec(prm)), 0, C.byref(f0), C.byref(fopt), _p(rep))
+    finally:
+        lib.pnolhost_clear_stream()
     del keep
     return st, dict(X=Xv, f0=f0.value, fopt=fopt.value, iters=int(rep[0]), stream_pos=int(rep[1]), evals=int(lib.pnolhost_last_evaluations()))
 

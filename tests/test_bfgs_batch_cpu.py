@@ -1,9 +1,8 @@
-"""Batched BFGS without a GPU: oracle_bfgs (tests/host_logic_bfgs_batch.cpp, the CPU stand-in's pnol_bfgs_batch, reached through
+"""Batched BFGS without a GPU: oracle_bfgs (tests/host_logic_standin.cpp, the CPU stand-in's pnol_bfgs_batch, reached through
 BFGSBatch) bit for bit against the unmodified host BFGS controller on the same stand-in, start by start, for the six built-in
 objectives, every derivative-flag combination, both initial inverse Hessians and the edge parameters; the base-class findMin; the
 refusal on a C-ABI without pnol_bfgs_batch; pnol_register_functor_bfgs_batch's rules and pnol_functor_has_bfgs_batch for every kind."""
 import ctypes as C
-import shutil
 import subprocess
 import sys
 
@@ -11,13 +10,13 @@ import numpy as np
 import pytest
 
 import bfgs_batch_cases as BC
-import host_logic_bfgs_batch_lib as HLB
+import host_standin
 from parallelnonlinearoptimizationlibrary_b200 import capi
 
 
 @pytest.fixture(scope="module")
 def standin():
-    hl = HLB.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     return hl
@@ -83,14 +82,9 @@ def test_base_class_find_min_is_one_start(standin):
 
 
 _REFUSAL = r"""
-import ctypes as C, glob, os, subprocess, sys
+import ctypes as C, sys
 import numpy as np
-root, so = sys.argv[1], sys.argv[2]
-host = os.path.join(root, "parallelnonlinearoptimizationlibrary_b200", "host")
-subprocess.check_call(["g++", "-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-w", "-shared", "-Wl,-Bsymbolic", "-I" + os.path.join(root, "include"),
-                       "-I" + host] + sorted(glob.glob(os.path.join(host, "*.cpp"))) +
-                      [os.path.join(root, "oracle", "host_logic_device.cpp"), os.path.join(root, "oracle", "pnol_oracle.cpp"), "-o", so])
-lib = C.CDLL(so, mode=C.RTLD_LOCAL)
+lib = C.CDLL(sys.argv[1], mode=C.RTLD_LOCAL)
 lib.pnolhost_last_error.restype = C.c_char_p
 p = lambda a: C.c_void_p(a.ctypes.data)
 X = np.array([[-1.2, 1.0]]); prm = np.array([1e-4, 0.9, 1e-6, 1.0, 40, 1e-6, 1e-3, 10, 1e-9, 1e-6, 0.0])
@@ -100,12 +94,13 @@ print(st, lib.pnolhost_last_error().decode())
 """
 
 
-def test_bfgs_batch_on_a_c_abi_without_it_is_refused(tmp_path):
+def test_bfgs_batch_on_a_c_abi_without_it_is_refused():
     """The host sources reference pnol_bfgs_batch weakly: linked against a C-ABI implementation without it (the unmodified stand-in) they
     still build and load, and BFGSBatch fails with PNOL_ERR_NO_FUNCTOR."""
-    if shutil.which("g++") is None:
+    so = host_standin.base_path()
+    if so is None:
         pytest.skip("no g++ on this box")
-    r = subprocess.run([sys.executable, "-c", _REFUSAL, HLB.ROOT, str(tmp_path / "libstandin.so")], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-c", _REFUSAL, so], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     st, msg = r.stdout.strip().split(" ", 1)
     assert int(st) == capi.ERR_NO_FUNCTOR and "pnol_bfgs_batch" in msg and "not provided by the C-ABI implementation" in msg, r.stdout
@@ -149,7 +144,7 @@ print(" ".join(str(k) for k in range(-1, 3101) if lib.pnol_functor_has_bfgs_batc
 
 
 def _scan(libraries):
-    r = subprocess.run([sys.executable, "-c", _SCAN, HLB.ROOT] + libraries, capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-c", _SCAN, host_standin.ROOT] + libraries, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     return [int(k) for k in r.stdout.split()]
 

@@ -1,7 +1,7 @@
 """GPU: analytic gradients (pnol_gradient[_recur]) against the host definition of every partial (include/pnol/functors.hpp, the
 user's tests/user_functor/my_gradients.hpp) bit for bit; the refusals; the plugin classes with Runtime::setAnalyticGradient(true),
 against the same controllers run on the CPU stand-in of tests/test_host_logic_cpu.py extended by the host partials
-(tests/host_logic_gradient.cpp); and the column split over 2+ GPUs."""
+(tests/host_logic_standin.cpp); and the column split over 2+ GPUs."""
 import ctypes as C
 import os
 import sys
@@ -9,7 +9,7 @@ import sys
 import numpy as np
 import pytest
 
-import host_logic_gradient_lib as HLG
+import host_standin
 import user_functor_lib as UF
 import user_gradient_lib as UG
 from parallelnonlinearoptimizationlibrary_b200 import capi
@@ -204,7 +204,7 @@ def test_bfgs_iterates_match_the_host_logic_stand_in(host, variant, obj, x0, ite
     """The stand-in runs the same host controllers with the partials and the dense algebra on the CPU, in the literal two-product
     updateHessianInv; the GPU is set to the same form. What remains is the summation order of the device's dense algebra."""
     import test_host_logic_cpu as TH
-    hl = HLG.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     host.set_hinv_mode(capi.HINV_LITERAL)

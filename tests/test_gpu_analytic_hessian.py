@@ -1,14 +1,14 @@
 """GPU: analytic Hessians (pnol_hessian) against the host definition of every partial2 (include/pnol/functors.hpp, the user's
 tests/user_functor/my_hessians.hpp) bit for bit, up to the largest n that fits; the refusals; the plugin member and the BFGS classes with
 initHessFD and Runtime::setAnalyticHessian(true), against the same controllers run on the CPU stand-in extended by the host partial2()
-(tests/host_logic_hessian.cpp); and every rank of a communicator returning the one-GPU bits."""
+(tests/host_logic_standin.cpp); and every rank of a communicator returning the one-GPU bits."""
 import os
 import sys
 
 import numpy as np
 import pytest
 
-import host_logic_hessian_lib as HLH
+import host_standin
 import test_user_hessian_cpu as HC
 import user_functor_lib as UF
 import user_gradient_lib as UG
@@ -228,7 +228,7 @@ def test_bfgs_iterates_match_the_host_logic_stand_in(host, variant, obj):
     partial2 and the dense algebra on the CPU (LU inverse included), in the literal two-product updateHessianInv; the GPU is set to the
     same form. What remains is the summation order of the device's dense algebra."""
     import test_host_logic_cpu as TH
-    hl = HLH.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     x0 = {p[0]: p[1] for p in HC.PROBLEMS}[obj]

@@ -1,5 +1,5 @@
 """GPU: analytic line-search slopes (pnol_alpha_pool_analytic) against the host restatement bit for bit -- phi from the CPU stand-in
-(tests/host_logic_slope.cpp) and from pnol_alpha_pool, the slope from the functor's host partial() summed as dotProd sums
+(tests/host_logic_standin.cpp) and from pnol_alpha_pool, the slope from the functor's host partial() summed as dotProd sums
 (tests/test_user_slope_cpu.py) -- for every built-in and both user kinds of tests/user_functor/my_gradients.hpp, up to the largest n
 pnol_alpha_pool accepts; the slope at alpha = 0 against dotProd(pnol_gradient[_recur], p); the sentinel; the refusals; and BFGS, BFGS_Bnd
 and BFGS_Bnd_MPI_SW with Runtime::setAnalyticSlope(true) against the same controllers on the stand-in."""
@@ -8,6 +8,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
+import host_standin
 import test_user_slope_cpu as SC
 import user_functor_lib as UF
 import user_gradient_lib as UG
@@ -30,7 +31,7 @@ def user():
 
 @pytest.fixture(scope="module")
 def standin():
-    hl = SC.HLS.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     return SC.Standin(hl)

@@ -1,5 +1,5 @@
 """Batched BFGS on the GPU (pnol_bfgs_batch): every field of every start bit for bit the CPU stand-in's oracle_bfgs
-(tests/host_logic_bfgs_batch.cpp), which tests/test_bfgs_batch_cpu.py pins bit for bit to the unmodified host BFGS controller, for the
+(tests/host_logic_standin.cpp), which tests/test_bfgs_batch_cpu.py pins bit for bit to the unmodified host BFGS controller, for the
 six built-in objectives, all eight derivative-flag combinations and both initial inverse Hessians; the user kinds; independence from
 B, position and order; random samples at 65 536 and 2^20 starts; host, device and misaligned pointers; the refusals; the plugin class;
 and a batch split over two GPUs."""
@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 import bfgs_batch_cases as BC
-import host_logic_bfgs_batch_lib as HLB
+import host_standin
 from parallelnonlinearoptimizationlibrary_b200 import capi, hostapi
 
 pytestmark = pytest.mark.gpu
@@ -24,7 +24,7 @@ def ctx():
 
 @pytest.fixture(scope="module")
 def standin():
-    hl = HLB.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     return hl

@@ -10,11 +10,7 @@ and asserts that the path ran:
     radix kernel. The bucket sizes depend only on the multiset of the new objective values, which is the next sorted F;
   * mutation: the geometry of generation 1 (the host's acceptance-rate estimate starts at 0.25) decides whether the compose
     kernel holds its tables in shared memory and over how many segments it composes them."""
-import ctypes as C
 import hashlib
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -33,17 +29,7 @@ SCALE = 1.0 - 2.0 ** -20
 @pytest.fixture(scope="module")
 def ga_objectives(ctx):
     """tests/user_functor/my_ga_objectives.cu compiled out of tree and loaded: registers the quantized and signed-zero objectives"""
-    from parallelnonlinearoptimizationlibrary_b200 import hostapi
-    capi.load_library()
-    hostapi.lib()
-    d = tempfile.mkdtemp(prefix="pnol_ga_objectives_")
-    out = os.path.join(d, "libmy_ga_objectives.so")
-    cmd = [user_functor_lib.nvcc(), "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-fmad=false", "-Xcompiler",
-           "-fPIC,-ffp-contract=off", "-I" + os.path.join(user_functor_lib.ROOT, "include"), "-I" + user_functor_lib.SRC, "-shared",
-           "-o", out, os.path.join(user_functor_lib.SRC, "my_ga_objectives.cu"), "-L" + user_functor_lib.LIBDIR, "-lpnol_b200",
-           "-Xlinker", "-rpath", "-Xlinker", user_functor_lib.LIBDIR]
-    subprocess.run(cmd, check=True, cwd=d, capture_output=True, text=True)
-    lib = C.CDLL(out, mode=C.RTLD_GLOBAL)
+    lib = user_functor_lib.build_user_library("my_ga_objectives.cu", with_host_lib=False)
     assert lib.my_ga_registration_status() == 0
     return lib
 

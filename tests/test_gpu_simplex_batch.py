@@ -1,5 +1,5 @@
 """Batched simplex search on the GPU (pnol_simplex_batch): every field of every start bit for bit the CPU stand-in's oracle_simplex
-(tests/host_logic_simplex_batch.cpp), which tests/test_simplex_batch_cpu.py pins bit for bit to the unmodified host SimplexSearch
+(tests/host_logic_standin.cpp), which tests/test_simplex_batch_cpu.py pins bit for bit to the unmodified host SimplexSearch
 controller, for the six built-in objectives with counter and explicit streams and for user objectives that drive simplexSort into its
 quirks; the plugin class on the verbatim reference's golden cases; independence from B, position and stream offset; random samples at
 65 536 and 2^20 starts; host, device and misaligned pointers; the refusals; and a batch split over two GPUs."""
@@ -9,7 +9,7 @@ import sys
 import numpy as np
 import pytest
 
-import host_logic_simplex_batch_lib as HLS
+import host_standin
 import simplex_batch_cases as SC
 from parallelnonlinearoptimizationlibrary_b200 import capi, hostapi
 
@@ -29,7 +29,7 @@ def ctx():
 
 @pytest.fixture(scope="module")
 def standin():
-    hl = HLS.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     return hl

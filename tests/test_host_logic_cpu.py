@@ -20,6 +20,8 @@ import sys
 import numpy as np
 import pytest
 
+import host_standin
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, os.path.join(HERE, "golden"))
@@ -32,16 +34,10 @@ def g(case, name):
 
 
 @pytest.fixture(scope="module")
-def hl(tmp_path_factory):
-    cxx = shutil.which("g++")
-    if cxx is None:
+def hl():
+    so = host_standin.base_path()
+    if so is None:
         pytest.skip("no g++ on this box")
-    so = str(tmp_path_factory.mktemp("host_logic") / "libpnol_host_logic_test.so")
-    host = os.path.join(ROOT, "parallelnonlinearoptimizationlibrary_b200", "host")
-    # -Bsymbolic: the library's own pnol_* definitions win over a product library another test may have loaded RTLD_GLOBAL
-    subprocess.check_call([cxx, "-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-w", "-shared", "-Wl,-Bsymbolic", "-I" + os.path.join(ROOT, "include"),
-                           "-I" + host] + sorted(glob.glob(os.path.join(host, "*.cpp"))) +
-                          [os.path.join(ROOT, "oracle", "host_logic_device.cpp"), os.path.join(ROOT, "oracle", "pnol_oracle.cpp"), "-o", so])
     lib = C.CDLL(so, mode=C.RTLD_LOCAL)
     lib.pnolhost_last_error.restype = C.c_char_p
     lib.pnolhost_set_hinv_mode(0)          # PNOL_HINV_LITERAL: the reference's two matrix products
@@ -128,7 +124,10 @@ def test_simplex_search_bit_for_bit(hl):
                       kw.get("initrandmax", 1.0), kw.get("xmindiff", 1e-7)], dtype=np.float64)
         f0, fo = C.c_double(), C.c_double()
         rep = np.zeros(2)
-        st = hl.pnolhost_simplex(obj.encode(), _p(X), X.size, _p(p), 0, C.byref(f0), C.byref(fo), _p(rep))
+        try:
+            st = hl.pnolhost_simplex(obj.encode(), _p(X), X.size, _p(p), 0, C.byref(f0), C.byref(fo), _p(rep))
+        finally:
+            hl.pnolhost_clear_stream()
         assert st == 0, hl.pnolhost_last_error()
         assert np.array_equal(X, S[name + "/X"]) and f0.value == S[name + "/f0"][0] and fo.value == S[name + "/fOpt"][0], name
         assert int(rep[1]) == int(S[name + "/stream_pos"][0])
@@ -186,8 +185,11 @@ def test_genetic_algorithm_host_class_bit_for_bit(hl, spec, obj, serial):
     lb, ub = g(c, "lb"), g(c, "ub")
     f0, fo = C.c_double(), C.c_double()
     rep = np.zeros(7)
-    st = hl.pnolhost_ga(obj.encode(), _p(X), X.size, _p(lb), _p(ub), int(g(c, "npop")), int(g(c, "gens")), C.c_double(0.1), C.c_double(0.3),
-                        C.c_double(0.2), C.c_double(0.5), C.c_double(0.01), C.c_double(50.0), serial, C.byref(f0), C.byref(fo), _p(rep))
+    try:
+        st = hl.pnolhost_ga(obj.encode(), _p(X), X.size, _p(lb), _p(ub), int(g(c, "npop")), int(g(c, "gens")), C.c_double(0.1), C.c_double(0.3),
+                            C.c_double(0.2), C.c_double(0.5), C.c_double(0.01), C.c_double(50.0), serial, C.byref(f0), C.byref(fo), _p(rep))
+    finally:
+        hl.pnolhost_clear_stream()
     assert st == 0, hl.pnolhost_last_error()
     assert np.array_equal(X, g(c, "X")) and f0.value == g(c, "f0")[0] and fo.value == g(c, "fOpt")[0]
     assert int(rep[0]) == int(g(c, "gens")) and int(rep[2]) == int(g(c, "stream_pos")[0])
@@ -235,8 +237,11 @@ def test_paths_outside_the_stand_in_fail_loudly(hl):
     f0, fo = C.c_double(), C.c_double()
     rep = np.zeros(7)
     hl.pnolhost_set_stream(C.c_void_p(0), C.c_ulonglong(0), C.c_ulonglong(1), C.c_double(0.99))
-    st = hl.pnolhost_ga(b"rosenbrock", _p(X), 4, _p(lb), _p(ub), 50, 3, C.c_double(0.6), C.c_double(0.6), C.c_double(0.2), C.c_double(0.5),
-                        C.c_double(0.01), C.c_double(50.0), 0, C.byref(f0), C.byref(fo), _p(rep))
+    try:
+        st = hl.pnolhost_ga(b"rosenbrock", _p(X), 4, _p(lb), _p(ub), 50, 3, C.c_double(0.6), C.c_double(0.6), C.c_double(0.2), C.c_double(0.5),
+                            C.c_double(0.01), C.c_double(50.0), 0, C.byref(f0), C.byref(fo), _p(rep))
+    finally:
+        hl.pnolhost_clear_stream()
     assert st != 0 and b"random children" in hl.pnolhost_last_error()
     st = hl.pnolhost_bfgs(b"bfgs", b"no_such_objective", _p(X), 4, _p(np.zeros(11)), None, None, 0, 0, C.byref(f0), C.byref(fo), C.byref(C.c_int()))
     assert st != 0

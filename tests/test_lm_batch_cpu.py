@@ -1,16 +1,15 @@
 """Batched Levenberg-Marquardt without a GPU: LevMarqBatch (include/pnol/LevenbergMarquardtBatch.hpp) on the CPU stand-in extended by
-pnol_lm_batch (tests/host_logic_lm_batch.cpp: oracle_lm per problem on its sliced columns), each problem bit for bit oracle_lib.lm on
+pnol_lm_batch (tests/host_logic_standin.cpp: oracle_lm per problem on its sliced columns), each problem bit for bit oracle_lib.lm on
 the problem alone; the refusal on a C-ABI implementation without pnol_lm_batch; and the registration rules of
 pnol_register_functor_lm_batch in the product library."""
 import ctypes as C
-import shutil
 import subprocess
 import sys
 
 import numpy as np
 import pytest
 
-import host_logic_lm_batch_lib as HLB
+import host_standin
 import lm_batch_cases as LC
 from parallelnonlinearoptimizationlibrary_b200 import capi
 
@@ -19,7 +18,7 @@ PRM = dict(lambda0=1e-3, factor=10.0, dxgrad=1e-7, maxiter=40, xmindiff=1e-9)
 
 @pytest.fixture(scope="module")
 def standin():
-    hl = HLB.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     return hl
@@ -105,14 +104,9 @@ def test_max_iter_zero_and_empty_batch(standin):
 
 
 _REFUSAL = r"""
-import ctypes as C, glob, os, subprocess, sys
+import ctypes as C, sys
 import numpy as np
-root, so = sys.argv[1], sys.argv[2]
-host = os.path.join(root, "parallelnonlinearoptimizationlibrary_b200", "host")
-subprocess.check_call(["g++", "-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-w", "-shared", "-Wl,-Bsymbolic", "-I" + os.path.join(root, "include"),
-                       "-I" + host] + sorted(glob.glob(os.path.join(host, "*.cpp"))) +
-                      [os.path.join(root, "oracle", "host_logic_device.cpp"), os.path.join(root, "oracle", "pnol_oracle.cpp"), "-o", so])
-lib = C.CDLL(so, mode=C.RTLD_LOCAL)
+lib = C.CDLL(sys.argv[1], mode=C.RTLD_LOCAL)
 lib.pnolhost_last_error.restype = C.c_char_p
 p = lambda a: C.c_void_p(a.ctypes.data)
 t = np.linspace(0, 1, 20); y = 2 * np.exp(0.5 * t) + 0.1
@@ -125,12 +119,13 @@ print(st, lib.pnolhost_last_error().decode())
 """
 
 
-def test_lm_batch_on_a_c_abi_without_it_is_refused(tmp_path):
+def test_lm_batch_on_a_c_abi_without_it_is_refused():
     """The host sources reference pnol_lm_batch weakly: linked against a C-ABI implementation without it (the unmodified stand-in, in a
     process where no libpnol_b200.so is loaded) they still build and load, and LevMarqBatch fails with PNOL_ERR_NO_FUNCTOR."""
-    if shutil.which("g++") is None:
+    so = host_standin.base_path()
+    if so is None:
         pytest.skip("no g++ on this box")
-    r = subprocess.run([sys.executable, "-c", _REFUSAL, LC.O.ROOT, str(tmp_path / "libstandin.so")], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-c", _REFUSAL, so], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     st, msg = r.stdout.strip().split(" ", 1)
     assert int(st) == capi.ERR_NO_FUNCTOR and "pnol_lm_batch" in msg and "not provided by the C-ABI implementation" in msg, r.stdout

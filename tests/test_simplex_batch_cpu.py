@@ -1,25 +1,24 @@
-"""Batched simplex search without a GPU: oracle_simplex (tests/host_logic_simplex_batch.cpp, the CPU stand-in's pnol_simplex_batch,
+"""Batched simplex search without a GPU: oracle_simplex (tests/host_logic_standin.cpp, the CPU stand-in's pnol_simplex_batch,
 reached through SimplexSearchBatch or the stand-in's C-ABI) bit for bit against the unmodified host SimplexSearch controller on the same
 stand-in, start by start, each start given exactly its slice of the stream, for the six built-in objectives, both stream kinds,
 offsets, non-default and edge parameters, with the evaluation counts; simplex_sort_perm (include/pnol/device/simplex_sort.hpp, the
 permutation logic the kernel runs) against the library's simplexSort on random arrays with ties, signed zeros, infinities and NaN; the
 refusals; pnol_register_functor_simplex_batch's rules and pnol_functor_has_simplex_batch for every kind."""
 import ctypes as C
-import shutil
 import subprocess
 import sys
 
 import numpy as np
 import pytest
 
-import host_logic_simplex_batch_lib as HLS
+import host_standin
 import simplex_batch_cases as SC
 from parallelnonlinearoptimizationlibrary_b200 import capi
 
 
 @pytest.fixture(scope="module")
 def standin():
-    hl = HLS.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     return hl
@@ -112,7 +111,10 @@ def test_base_class_find_min_is_one_start(standin):
     SC.set_stream(standin, ("values", vals))
     Xv, f0, fopt = x0.copy(), np.zeros(1), np.zeros(1)
     p = lambda a: C.c_void_p(a.ctypes.data)
-    assert standin.pnolhost_simplex_batch(b"rosenbrock", p(Xv), C.c_longlong(1), 3, p(SC.vec(prm)), 1, p(f0), p(fopt), None, None, None, None) == 0
+    try:
+        assert standin.pnolhost_simplex_batch(b"rosenbrock", p(Xv), C.c_longlong(1), 3, p(SC.vec(prm)), 1, p(f0), p(fopt), None, None, None, None) == 0
+    finally:
+        standin.pnolhost_clear_stream()
     st, want = SC.run_serial(standin, "rosenbrock", x0, prm, vals)
     assert st == 0 and SC.same(Xv, want["X"]) and SC.same(f0[0], want["f0"]) and SC.same(fopt[0], want["fopt"])
     assert np.max(np.abs(Xv - 1.0)) < 1e-3
@@ -172,14 +174,9 @@ def test_sort_permutation_is_simplex_sort(standin):
 
 
 _REFUSAL = r"""
-import ctypes as C, glob, os, subprocess, sys
+import ctypes as C, sys
 import numpy as np
-root, so = sys.argv[1], sys.argv[2]
-host = os.path.join(root, "parallelnonlinearoptimizationlibrary_b200", "host")
-subprocess.check_call(["g++", "-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-w", "-shared", "-Wl,-Bsymbolic", "-I" + os.path.join(root, "include"),
-                       "-I" + host] + sorted(glob.glob(os.path.join(host, "*.cpp"))) +
-                      [os.path.join(root, "oracle", "host_logic_device.cpp"), os.path.join(root, "oracle", "pnol_oracle.cpp"), "-o", so])
-lib = C.CDLL(so, mode=C.RTLD_LOCAL)
+lib = C.CDLL(sys.argv[1], mode=C.RTLD_LOCAL)
 lib.pnolhost_last_error.restype = C.c_char_p
 p = lambda a: C.c_void_p(a.ctypes.data)
 X = np.array([[-1.2, 1.0]]); prm = np.array([1.0, 2.0, 0.5, 0.5, 10, 1.0, 1e-7])
@@ -190,12 +187,13 @@ print(st, lib.pnolhost_last_error().decode())
 """
 
 
-def test_simplex_batch_on_a_c_abi_without_it_is_refused(tmp_path):
+def test_simplex_batch_on_a_c_abi_without_it_is_refused():
     """The host sources reference pnol_simplex_batch weakly: linked against a C-ABI implementation without it (the unmodified stand-in)
     they still build and load, and SimplexSearchBatch fails with PNOL_ERR_NO_FUNCTOR."""
-    if shutil.which("g++") is None:
+    so = host_standin.base_path()
+    if so is None:
         pytest.skip("no g++ on this box")
-    r = subprocess.run([sys.executable, "-c", _REFUSAL, HLS.ROOT, str(tmp_path / "libstandin.so")], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-c", _REFUSAL, so], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     st, msg = r.stdout.strip().split(" ", 1)
     assert int(st) == capi.ERR_NO_FUNCTOR and "pnol_simplex_batch" in msg and "not provided by the C-ABI implementation" in msg, r.stdout
@@ -239,7 +237,7 @@ print(" ".join(str(k) for k in range(-1, 3101) if lib.pnol_functor_has_simplex_b
 
 
 def _scan(libraries):
-    r = subprocess.run([sys.executable, "-c", _SCAN, HLS.ROOT] + libraries, capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-c", _SCAN, host_standin.ROOT] + libraries, capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     return [int(k) for k in r.stdout.split()]
 

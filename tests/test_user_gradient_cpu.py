@@ -8,7 +8,7 @@ import mpmath
 import numpy as np
 import pytest
 
-import host_logic_gradient_lib as HLG
+import host_standin
 import user_gradient_lib as UG
 from parallelnonlinearoptimizationlibrary_b200 import capi
 
@@ -233,9 +233,9 @@ def _bfgs(lib, variant, obj, x0, params, lb=None, ub=None, pool=0):
 
 
 def test_host_controllers_take_the_partials_in_the_analytic_mode(user):
-    """The unmodified host sources on the CPU stand-in extended by the host partials (tests/host_logic_gradient.cpp):
+    """The unmodified host sources on the CPU stand-in extended by the host partials (tests/host_logic_standin.cpp):
     Objective::gradientApproximation[MPI][Recur] return partial()'s bits and ignore dX, and BFGS / BFGS_Bnd_MPI_SW reach the optima."""
-    hl = HLG.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     p = lambda a: C.c_void_p(a.ctypes.data)                         # noqa: E731
@@ -265,14 +265,9 @@ def test_host_controllers_take_the_partials_in_the_analytic_mode(user):
 
 
 _REFUSAL = r"""
-import ctypes as C, glob, os, subprocess, sys
+import ctypes as C, sys
 import numpy as np
-root, so = sys.argv[1], sys.argv[2]
-host = os.path.join(root, "parallelnonlinearoptimizationlibrary_b200", "host")
-subprocess.check_call(["g++", "-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-w", "-shared", "-Wl,-Bsymbolic", "-I" + os.path.join(root, "include"),
-                       "-I" + host] + sorted(glob.glob(os.path.join(host, "*.cpp"))) +
-                      [os.path.join(root, "oracle", "host_logic_device.cpp"), os.path.join(root, "oracle", "pnol_oracle.cpp"), "-o", so])
-lib = C.CDLL(so, mode=C.RTLD_LOCAL)
+lib = C.CDLL(sys.argv[1], mode=C.RTLD_LOCAL)
 lib.pnolhost_last_error.restype = C.c_char_p
 x, dx, g = np.full(4, 0.5), np.full(4, 1e-7), np.empty(4)
 p = lambda a: C.c_void_p(a.ctypes.data)
@@ -283,16 +278,16 @@ print(st, lib.pnolhost_last_error().decode())
 """
 
 
-def test_analytic_mode_on_a_c_abi_without_the_gradient_is_refused(tmp_path):
+def test_analytic_mode_on_a_c_abi_without_the_gradient_is_refused():
     """The host sources reference pnol_gradient[_recur] weakly: linked against a C-ABI implementation without them (the unmodified
     stand-in, in a process where no libpnol_b200.so is loaded) they still build and load, and the analytic mode is refused with
     PNOL_ERR_NO_FUNCTOR instead of computing anything."""
-    import shutil
     import subprocess
     import sys
-    if shutil.which("g++") is None:
+    so = host_standin.base_path()
+    if so is None:
         pytest.skip("no g++ on this box")
-    r = subprocess.run([sys.executable, "-c", _REFUSAL, UG.ROOT, str(tmp_path / "libstandin.so")], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-c", _REFUSAL, so], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     st, msg = r.stdout.strip().split(" ", 1)
     assert int(st) == capi.ERR_NO_FUNCTOR and "not provided by the C-ABI implementation" in msg, r.stdout

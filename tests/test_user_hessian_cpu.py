@@ -2,14 +2,14 @@
 (include/pnol/functors.hpp, the user's tests/user_functor/my_hessians.hpp) against a numpy restatement of its stated operation order
 (bit for bit) and against a complex-step derivative of the gradient or an mpmath second derivative (to 32 ulp of the Hessian's largest
 entry); the registration rules of pnol_register_functor_hessian; and the BFGS controllers with initHessFD in the analytic mode on the CPU
-stand-in extended by the host partial2() (tests/host_logic_hessian.cpp)."""
+stand-in extended by the host partial2() (tests/host_logic_standin.cpp)."""
 import ctypes as C
 
 import mpmath
 import numpy as np
 import pytest
 
-import host_logic_hessian_lib as HLH
+import host_standin
 import user_gradient_lib as UG
 import user_hessian_lib as UH
 from parallelnonlinearoptimizationlibrary_b200 import capi
@@ -301,7 +301,7 @@ def run_bfgs(call, variant, obj, x0, iters):
 def test_host_hessian_member_takes_partial2_in_the_analytic_mode(user):
     """Objective::hessianApproximation on the stand-in extended by the host partial2(): partial2()'s bits, dX ignored; the forward
     difference when the switch is off."""
-    hl = HLH.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     p = lambda a: C.c_void_p(a.ctypes.data)                         # noqa: E731
@@ -324,7 +324,7 @@ def test_host_hessian_member_takes_partial2_in_the_analytic_mode(user):
 def test_bfgs_controllers_start_from_the_analytic_hessian(user, variant):
     """initHessFD = 1 with analytic gradient and Hessian: the five BFGS classes on the extended stand-in reach the known optima."""
     import test_host_logic_cpu as TH
-    hl = HLH.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     hl.pnolhost_set_analytic_gradient(1)
@@ -342,14 +342,9 @@ def test_bfgs_controllers_start_from_the_analytic_hessian(user, variant):
 
 
 _REFUSAL = r"""
-import ctypes as C, glob, os, subprocess, sys
+import ctypes as C, sys
 import numpy as np
-root, so = sys.argv[1], sys.argv[2]
-host = os.path.join(root, "parallelnonlinearoptimizationlibrary_b200", "host")
-subprocess.check_call(["g++", "-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-w", "-shared", "-Wl,-Bsymbolic", "-I" + os.path.join(root, "include"),
-                       "-I" + host] + sorted(glob.glob(os.path.join(host, "*.cpp"))) +
-                      [os.path.join(root, "oracle", "host_logic_device.cpp"), os.path.join(root, "oracle", "pnol_oracle.cpp"), "-o", so])
-lib = C.CDLL(so, mode=C.RTLD_LOCAL)
+lib = C.CDLL(sys.argv[1], mode=C.RTLD_LOCAL)
 lib.pnolhost_last_error.restype = C.c_char_p
 x, dx, H = np.full(4, 0.5), np.full(4, 1e-4), np.empty(16)
 p = lambda a: C.c_void_p(a.ctypes.data)
@@ -360,16 +355,16 @@ print(st, lib.pnolhost_last_error().decode())
 """
 
 
-def test_analytic_hessian_on_a_c_abi_without_it_is_refused(tmp_path):
+def test_analytic_hessian_on_a_c_abi_without_it_is_refused():
     """The host sources reference pnol_hessian weakly: linked against a C-ABI implementation without it (the unmodified stand-in, in a
     process where no libpnol_b200.so is loaded) they still build and load, and the analytic mode is refused with PNOL_ERR_NO_FUNCTOR
     instead of computing anything."""
-    import shutil
     import subprocess
     import sys
-    if shutil.which("g++") is None:
+    so = host_standin.base_path()
+    if so is None:
         pytest.skip("no g++ on this box")
-    r = subprocess.run([sys.executable, "-c", _REFUSAL, UH.ROOT, str(tmp_path / "libstandin.so")], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-c", _REFUSAL, so], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     st, msg = r.stdout.strip().split(" ", 1)
     assert int(st) == capi.ERR_NO_FUNCTOR and "analytic Hessians (Runtime::setAnalyticHessian)" in msg, r.stdout

@@ -1,5 +1,5 @@
 """Analytic line-search slopes (pnol_alpha_pool_analytic) without a GPU: the CPU stand-in extended by the slope
-(tests/host_logic_slope.cpp: the host eval() and partial() of include/pnol/functors.hpp with the kernel's point assembly, sequential sum
+(tests/host_logic_standin.cpp: the host eval() and partial() of include/pnol/functors.hpp with the kernel's point assembly, sequential sum
 and sentinel) against dotProd of its own pnol_gradient_recur at alpha = 0 (bit for bit), against a numpy restatement over the host
 partial() of every built-in and of the user's tests/user_functor/my_gradients.hpp (bit for bit), and against a complex-step or mpmath
 directional derivative; the registration rules of pnol_register_functor_slope; and the BFGS controllers with
@@ -10,7 +10,7 @@ import mpmath
 import numpy as np
 import pytest
 
-import host_logic_slope_lib as HLS
+import host_standin
 import user_gradient_lib as UG
 import user_hessian_lib as UH
 from parallelnonlinearoptimizationlibrary_b200 import capi
@@ -46,7 +46,7 @@ def user():
 
 @pytest.fixture(scope="module")
 def standin():
-    hl = HLS.build_and_load()
+    hl = host_standin.load()
     if hl is None:
         pytest.skip("no g++ on this box")
     return Standin(hl)
@@ -402,14 +402,9 @@ def test_pool_member_counts_one_evaluation_per_entry(standin):
 
 
 _REFUSAL = r"""
-import ctypes as C, glob, os, subprocess, sys
+import ctypes as C, sys
 import numpy as np
-root, so = sys.argv[1], sys.argv[2]
-host = os.path.join(root, "parallelnonlinearoptimizationlibrary_b200", "host")
-subprocess.check_call(["g++", "-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-w", "-shared", "-Wl,-Bsymbolic", "-I" + os.path.join(root, "include"),
-                       "-I" + host] + sorted(glob.glob(os.path.join(host, "*.cpp"))) +
-                      [os.path.join(root, "oracle", "host_logic_device.cpp"), os.path.join(root, "oracle", "pnol_oracle.cpp"), "-o", so])
-lib = C.CDLL(so, mode=C.RTLD_LOCAL)
+lib = C.CDLL(sys.argv[1], mode=C.RTLD_LOCAL)
 lib.pnolhost_last_error.restype = C.c_char_p
 p = lambda a: C.c_void_p(a.ctypes.data)
 x, prm = np.full(4, 3.0), np.array([1e-4, 0.9, 1e-6, 1.0, 1000, 1e-7, 1e-3, 5, 1e-5, 1e-5, 0])
@@ -422,16 +417,16 @@ print(st, lib.pnolhost_last_error().decode())
 """
 
 
-def test_analytic_slopes_on_a_c_abi_without_them_are_refused(tmp_path):
+def test_analytic_slopes_on_a_c_abi_without_them_are_refused():
     """The host sources reference pnol_alpha_pool_analytic weakly: linked against a C-ABI implementation without it (the unmodified
     stand-in, in a process where no libpnol_b200.so is loaded) they still build and load, and the analytic mode is refused with
     PNOL_ERR_NO_FUNCTOR instead of taking a forward difference."""
-    import shutil
     import subprocess
     import sys
-    if shutil.which("g++") is None:
+    so = host_standin.base_path()
+    if so is None:
         pytest.skip("no g++ on this box")
-    r = subprocess.run([sys.executable, "-c", _REFUSAL, UG.ROOT, str(tmp_path / "libstandin.so")], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-c", _REFUSAL, so], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     st, msg = r.stdout.strip().split(" ", 1)
     assert int(st) == capi.ERR_NO_FUNCTOR and "analytic line-search slopes (Runtime::setAnalyticSlope)" in msg, r.stdout

@@ -1,6 +1,6 @@
 /* Four objectives for the batched simplex tests (tests/test_gpu_simplex_batch.py), written to the functor concept of
  * include/pnol/functors.hpp, each steering simplexSort into one of its quirks. my_simplex_objectives.cu registers them with the library
- * (compiled out of tree, as my_objectives.cu is) and the CPU stand-in (tests/host_logic_simplex_batch.cpp) includes this header for
+ * (compiled out of tree, as my_objectives.cu is) and the CPU stand-in (tests/host_logic_standin.cpp) includes this header for
  * its oracle, so the host and device definitions are the same source. */
 #ifndef MY_SIMPLEX_OBJECTIVES_HPP_
 #define MY_SIMPLEX_OBJECTIVES_HPP_

@@ -2,18 +2,12 @@
 scalar objectives with analytic gradients register their launch tables and gradient launchers at load time. Also: the host side of
 the analytic gradient (the same __host__ __device__ partial() the kernels compile) and of the shared host/device math."""
 import ctypes as C
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 import user_functor_lib
 import user_jacobian_lib
 
-ROOT = user_functor_lib.ROOT
-SRC = user_functor_lib.SRC
-LIBDIR = user_functor_lib.LIBDIR
 MYG_F_TRID, MYG_F_STYBLINSKI = 1201, 1202
 
 _lib = None
@@ -22,18 +16,8 @@ _lib = None
 def build_and_load():
     """compile once per process; returns the ctypes handle of the user's library"""
     global _lib
-    if _lib is not None:
-        return _lib
-    from parallelnonlinearoptimizationlibrary_b200 import capi, hostapi
-    capi.load_library()
-    hostapi.lib()
-    d = tempfile.mkdtemp(prefix="pnol_user_gradient_")
-    out = os.path.join(d, "libmy_gradients.so")
-    cmd = [user_functor_lib.nvcc(), "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-fmad=false", "-Xcompiler",
-           "-fPIC,-ffp-contract=off", "-I" + os.path.join(ROOT, "include"), "-I" + SRC, "-shared", "-o", out,
-           os.path.join(SRC, "my_gradients.cu"), "-L" + LIBDIR, "-lpnol_b200", "-lpnol_b200_host", "-Xlinker", "-rpath", "-Xlinker", LIBDIR]
-    subprocess.run(cmd, check=True, cwd=d, capture_output=True, text=True)
-    _lib = C.CDLL(out, mode=C.RTLD_GLOBAL)
+    if _lib is None:
+        _lib = user_functor_lib.build_user_library("my_gradients.cu")
     return _lib
 
 

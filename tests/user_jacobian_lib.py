@@ -2,17 +2,11 @@
 residual models with analytic Jacobians register their launch tables at load time. Also: the host side of the analytic Jacobian
 (the same __host__ __device__ definitions the kernels compile) and a ctypes mirror of pnol_functor_params."""
 import ctypes as C
-import os
-import subprocess
-import tempfile
 
 import numpy as np
 
 import user_functor_lib
 
-ROOT = user_functor_lib.ROOT
-SRC = user_functor_lib.SRC
-LIBDIR = user_functor_lib.LIBDIR
 MYJ_F_LORENTZ, MYJ_F_GAUSS, MYJ_F_GAUSS_V1, MYJ_F_GAUSS_NOJAC = 2101, 2102, 2103, 2104
 
 _lib = None
@@ -26,18 +20,8 @@ class FunctorParams(C.Structure):
 def build_and_load():
     """compile once per process; returns the ctypes handle of the user's library"""
     global _lib
-    if _lib is not None:
-        return _lib
-    from parallelnonlinearoptimizationlibrary_b200 import capi, hostapi
-    capi.load_library()
-    hostapi.lib()
-    d = tempfile.mkdtemp(prefix="pnol_user_jacobian_")
-    out = os.path.join(d, "libmy_jacobians.so")
-    cmd = [user_functor_lib.nvcc(), "-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-fmad=false", "-Xcompiler",
-           "-fPIC,-ffp-contract=off", "-I" + os.path.join(ROOT, "include"), "-I" + SRC, "-shared", "-o", out,
-           os.path.join(SRC, "my_jacobians.cu"), "-L" + LIBDIR, "-lpnol_b200", "-lpnol_b200_host", "-Xlinker", "-rpath", "-Xlinker", LIBDIR]
-    subprocess.run(cmd, check=True, cwd=d, capture_output=True, text=True)
-    _lib = C.CDLL(out, mode=C.RTLD_GLOBAL)
+    if _lib is None:
+        _lib = user_functor_lib.build_user_library("my_jacobians.cu")
     return _lib
 
 
