@@ -6,6 +6,9 @@
 * refined_solution / backward_error: a Cholesky solution refined with residuals in long double (64-bit significand on x86-64),
   and the normwise backward error eta = ||b - A x||_inf / (||A||_inf ||x||_inf + ||b||_inf).
 * spd_family: the matrix families of the solve sweep.
+* GradedMatvec / GradedGemm / IntegerHinv: exact inputs and results of p = -D g, C = A B and updateHessianInv; the launchers'
+  path predicates restated (matvec_path, hinv_rank2_path, gemm_path, syrk_path); componentwise gamma_d bars against long-double
+  references (matvec_bar, gemm_bar, hinv_bar) with each kernel's summation depth.
 """
 import numpy as np
 import scipy.linalg
@@ -195,3 +198,260 @@ def solve_sizes():
         s.update(q + r for r in (-1, 0, 1, 2, 3))
     s.update((416, 417, 511, 512, 513, 703, 704))
     return sorted(v for v in s if 1 <= v <= 704)
+
+
+# ---- the dense BFGS pieces and the DMMA GEMM: exact constructions --------------------------------------------------------------
+#
+# Every value below is an integer times a power of two, and every product and every partial sum of the kernels' arithmetic is an
+# integer multiple of one power of two whose magnitude stays below 2^53 times it. Each is then representable, so the result is
+# the exact one in any summation order, fused or not: the kernels must return it bit for bit.
+
+def _exponents(n, lo, hi, rng):
+    """n exponents in [lo, hi], each value about equally often, permuted: every 4-wide lane group and 128-column group mixes them"""
+    return rng.permutation(np.arange(n) % (hi - lo + 1) + lo).astype(np.int32)
+
+
+def _zero_some(K, rng, rows=3, cols=2):
+    m, n = K.shape
+    if m > 2:
+        K[rng.choice(m, size=min(rows, m - 1), replace=False)] = 0
+    if n > 2:
+        K[:, rng.choice(n, size=min(cols, n - 1), replace=False)] = 0
+
+
+class GradedMatvec:
+    """p = -D g with D_ik = K_ik 2^(-r_i - t_k), g_k = G_k 2^(t_k): every product of row i is an integer times 2^(-r_i) and
+    n max|K| max|G| < 2^53, so p_i = -(K G)_i 2^(-r_i) exactly."""
+
+    def __init__(self, n, rng):
+        b = integer_bits(n)
+        self.K = rng.integers(-2 ** b, 2 ** b, size=(n, n), endpoint=True, dtype=np.int64)
+        self.G = rng.integers(-2 ** b, 2 ** b, size=n, endpoint=True, dtype=np.int64)
+        _zero_some(self.K, rng)
+        self.r, self.t = _exponents(n, 0, 30, rng), _exponents(n, -20, 20, rng)
+        self.D = np.ldexp(self.K.astype(np.float64), -self.r[:, None] - self.t[None, :])
+        self.g = np.ldexp(self.G.astype(np.float64), self.t)
+        self.peak = int(np.abs(self.K).max(initial=0)) * int(np.abs(self.G).max(initial=0)) * n   # bound of any partial sum / 2^-r_i
+        self.want = np.ldexp(-(self.K @ self.G).astype(np.float64), -self.r)
+
+
+class GradedGemm:
+    """C = A B with A_ik = K_ik 2^(-r_i), B_kj = L_kj 2^(-c_j), K_dim max|K| max|L| < 2^53: C_ij = (K L)_ij 2^(-r_i - c_j) exactly,
+    and numpy's float64 product of the integer matrices is exact too (test_exact_reference.py proves it against int64)."""
+
+    def __init__(self, M, N, K, rng):
+        b = integer_bits(K)
+        self.Ka = rng.integers(-2 ** b, 2 ** b, size=(M, K), endpoint=True, dtype=np.int64)
+        self.Lb = rng.integers(-2 ** b, 2 ** b, size=(K, N), endpoint=True, dtype=np.int64)
+        _zero_some(self.Ka, rng, rows=2, cols=1)
+        _zero_some(self.Lb, rng, rows=1, cols=2)
+        self.r, self.c = _exponents(M, 0, 40, rng), _exponents(N, 0, 40, rng)
+        self.A = np.ldexp(self.Ka.astype(np.float64), -self.r[:, None])
+        self.B = np.ldexp(self.Lb.astype(np.float64), -self.c[None, :])
+        self.peak = int(np.abs(self.Ka).max(initial=0)) * int(np.abs(self.Lb).max(initial=0)) * K
+
+    def int_product_f64(self):
+        """K L through float64 BLAS (exact by the bound)"""
+        return self.Ka.astype(np.float64) @ self.Lb.astype(np.float64)
+
+    def want(self, KL=None):
+        KL = self.int_product_f64() if KL is None else KL
+        return np.ldexp(np.ldexp(KL, -self.r[:, None]), -self.c[None, :])
+
+
+class IntegerHinv:
+    """updateHessianInv on an integer, nonsymmetric D and integer g, s with g_0 = 1 and s_0 chosen so that g.s = sign 2^k, i.e.
+    rho = sign 2^-k exactly. With u = D g, v = D^T g, gamma = g^T D g (int64):
+        4^k D_new = 4^k D - sign 2^k (s v^T + u s^T) + (gamma + sign 2^k) s s^T.
+    `peak` bounds (as an integer multiple of the finest power of two involved) every product and partial sum of the rank-2 form
+    (u, v, g.s, g.u, rho, cc, the per-entry sum) and of the literal form (M1 D, then (M1 D) M2, then + rho s s^T) in any order;
+    below 2^53 both forms are exact and equal `want` bit for bit."""
+
+    def __init__(self, n, k, sign, rng, dbits=None, vbits=None, symmetric=False):
+        self.n, self.k, self.sign = n, k, sign
+        # |D| <= 16, |g|, |s| <= 8; from n = 2048 on |D| <= 8, |g|, |s| <= 4: s_0 absorbs g.s (about sqrt(n) 2^(2 vbits)), and the
+        # literal form's bound grows like s_0^2 |g|^T|D||g|
+        dbits = (4 if n < 2048 else 3) if dbits is None else dbits
+        vbits = (3 if n < 2048 else 2) if vbits is None else vbits
+        D = rng.integers(-2 ** dbits, 2 ** dbits, size=(n, n), endpoint=True, dtype=np.int64)
+        if symmetric:
+            D = D + D.T
+        g = rng.integers(-2 ** vbits, 2 ** vbits, size=n, endpoint=True, dtype=np.int64)
+        s = rng.integers(-2 ** vbits, 2 ** vbits, size=n, endpoint=True, dtype=np.int64)
+        g[0] = 1
+        s[0] += sign * 2 ** k - int(g @ s)
+        assert int(g @ s) == sign * 2 ** k
+        self.Di, self.gi, self.si = D, g, s
+        self.D, self.g, self.s = D.astype(np.float64), g.astype(np.float64), s.astype(np.float64)
+        self.u, self.v = D @ g, D.T @ g
+        self.gamma = int(g @ self.u)
+        self.scaled = self.scaled_update(self.u, self.v)
+        self.peak = self._peak()
+        self.want = np.ldexp(self.scaled.astype(np.float64), -2 * k)
+
+    def scaled_update(self, u, v):
+        """4^k D_new in int64 from the given u (row sums) and v (column sums)"""
+        k, sg, s = self.k, self.sign, self.si
+        return 4 ** k * self.Di - sg * 2 ** k * (np.outer(s, v) + np.outer(u, s)) + (self.gamma + sg * 2 ** k) * np.outer(s, s)
+
+    def swapped(self):
+        """the same update with u and v exchanged (a kernel that reads a row partial where it wants a column partial)"""
+        return np.ldexp(self.scaled_update(self.v, self.u).astype(np.float64), -2 * self.k)
+
+    def _peak(self):
+        k = self.k
+        aD, ag, as_ = np.abs(self.Di), np.abs(self.gi), np.abs(self.si)
+        au, av = aD @ ag, aD.T @ ag                          # bounds of every partial sum of u, v
+        Gam = int(ag @ au)                                   # ... of g.u
+        cc = abs(self.gamma + self.sign * 2 ** k)            # 4^k |cc|
+        ms = int(as_.max())
+        # rank-2 entry: 4^k |D_ij| + 2^k |s_i| |v|_j + 2^k |u|_i |s_j| + 4^k |cc| |s_i| |s_j|, in units of 4^-k
+        r2 = 4 ** k * aD + 2 ** k * (np.outer(as_, av) + np.outer(au, as_)) + cc * np.outer(as_, as_)
+        # literal: 2^k (M1 D) partial sums <= X = 2^k |D| + |s| (|D|^T |g|)^T; 4^k ((M1 D) M2) <= 2^k X + (X |g|) |s|^T; + 2^k s s^T
+        X = 2 ** k * aD + np.outer(as_, av)
+        lit = 2 ** k * X + np.outer(X @ ag, as_) + 2 ** k * np.outer(as_, as_)
+        return max(int(au.max()), int(av.max()), Gam, int(ag @ as_), cc * ms, int(r2.max()), int(lit.max()),
+                   2 ** k + int(np.outer(as_, ag).max()))
+
+
+# ---- which kernel each launcher picks (restated from csrc/dense.cu and csrc/dmma.cu) -----------------------------------------
+# A device pointer is `offset` bytes past a 256-byte-aligned allocation, so its alignment is that of the offset.
+
+def _al(off, b):
+    return off % b == 0
+
+
+def matvec_path(n, off_D=0, off_g=0):
+    """launch_matvec_neg"""
+    return "v4" if n % 4 == 0 and _al(off_D, 32) and _al(off_g, 32) else "scalar"
+
+
+def hinv_rank2_path(n, off_D=0, off_g=0, off_s=0):
+    """launch_hinv_rank2: the three-launch v4 plan, or the five-launch plan with the double2 or the scalar pass 2"""
+    if n % 4 == 0 and _al(off_D, 32) and _al(off_g, 32) and _al(off_s, 32):
+        return "v4"
+    return "double2" if n % 2 == 0 and _al(off_D, 16) else "scalar"
+
+
+HINV_LAUNCHES = {"v4": 3, "double2": 5, "scalar": 5, "literal": 5}   # the literal form: dot2, M1/M2, two GEMMs, + rho s s^T
+
+
+def gemm_path(M, N, K, off_A=0, off_B=0, off_C=0):
+    """launch_dgemm_nn: gemm_nn_kernel<true> (16-byte pieces) or <false>"""
+    return "vec16" if N % 2 == 0 and K % 2 == 0 and _al(off_A, 16) and _al(off_B, 16) and _al(off_C, 16) else "scalar"
+
+
+def syrk_path(n, with_f, off_J=0, off_F=0):
+    """launch_syrk for m >= 1: the TMA kernels ("tma", "pair"), or the LDGSTS ring syrk_kernel<true> ("ldgsts16") / <false>"""
+    vec16 = n % 2 == 0 and _al(off_J, 16)
+    tma = vec16 and n % 16 == 0 and (not with_f or _al(off_F, 16))
+    if tma:
+        return "pair" if (n + 127) // 128 == 2 and not with_f else "tma"
+    return "ldgsts16" if vec16 else "ldgsts8"
+
+
+# ---- componentwise bars on real-valued data ------------------------------------------------------------------------------------
+
+UL = 2.0 ** -64                      # unit roundoff of the x86-64 long double (64-bit significand)
+
+
+def gamma(d, u=U):
+    """gamma_d = d u / (1 - d u): a sum whose terms each pass through at most d roundings is off by at most gamma_d sum |terms|"""
+    return d * u / (1 - d * u)
+
+
+def ld(a):
+    return np.asarray(a, dtype=np.longdouble)
+
+
+def matvec_depth(n, path):
+    """roundings a product of p = -D g passes through. v4: a chain of ceil(n / 128) FMA per lane and component, two adds for the
+    four components, five butterfly adds; scalar: ceil(n / 32) FMA per lane and five butterfly adds (-1 x: exact)"""
+    return -(-n // 128) + 7 if path == "v4" else -(-n // 32) + 5
+
+
+def gemm_depth(K):
+    """roundings a product of C = A B passes through in gemm_nn_kernel: one m8n8k4 DMMA per 4 k, each at most a rounded product
+    and four rounded adds into the accumulator for its own terms, four adds for the accumulator it carries"""
+    return 4 * (-(-K // 4)) + 1
+
+
+def hinv_v4_blocks(n, sm_count):
+    """(row blocks, rows per block R, column blocks) of hinv_pass1_v4_kernel, restated from launch_hinv_rank2"""
+    ncb = -(-n // 256)
+    wave = 2 * sm_count
+    nrb = (n + 111) // 112
+    waves = (nrb * ncb + wave // 2) // wave
+    if waves >= 1:
+        nrb = waves * wave // ncb
+    nrb = max(nrb, 1)
+    R = (-(-n // nrb) + 3) & ~3
+    return -(-n // R), R, ncb
+
+
+def hinv_depths(n, path, sm_count):
+    """(d_u, d_v, d_dot): roundings a term of u = D g, of v = D^T g and of the dot products g.s, g.u passes through"""
+    if path == "v4":
+        nrb, R, ncb = hinv_v4_blocks(n, sm_count)
+        d_u = 2 + 2 + 5 + -(-ncb // 8) + 8              # 2 FMA per chain, 2 adds, 5 butterfly adds, finish: chain + 8 group adds
+        d_v = 4 * -(-R // 32) + 8 + -(-nrb // 8) + 8     # FMA over the warp's rows, 8 warp adds, finish
+        d_dot = -(-n // 256) + 8                         # 256-thread chains and an 8-level tree
+    else:
+        nrb, ncb = -(-n // 32), -(-n // 512)
+        d_u = min(16, -(-n // 32)) + 5 + ncb             # chain over the 512-column block, butterfly, finish over column blocks
+        d_v = 4 + 8 + nrb                                # 4 rows per warp, 8 warp adds, finish over row blocks
+        d_dot = -(-n // 1024) + 10                       # dot2_kernel: 1024-thread chains and a 10-level tree
+    return d_u, d_v, d_dot
+
+
+def hinv_reference_ld(D, g, s):
+    """the rank-2 update in long double: (D_new, magnitude terms T = |D| + |rho||s|(|D|^T|g|)^T + |rho|(|D||g|)|s|^T
+    + (rho^2 |g|^T|D||g| + |rho|) |s||s|^T, condition of g.s = |g|^T|s| / |g.s|)"""
+    Dl, gl, sl = ld(D), ld(g), ld(s)
+    u, v = Dl @ gl, Dl.T @ gl
+    gs = gl @ sl
+    rho = 1 / gs
+    cc = rho * rho * (gl @ u) + rho
+    want = Dl - rho * np.outer(sl, v) - rho * np.outer(u, sl) + cc * np.outer(sl, sl)
+    aD, ag, as_ = np.abs(Dl), np.abs(gl), np.abs(sl)
+    au, av = aD @ ag, aD.T @ ag
+    T = aD + abs(rho) * (np.outer(as_, av) + np.outer(au, as_)) + (rho * rho * (ag @ au) + abs(rho)) * np.outer(as_, as_)
+    return want, T, (ag @ as_) / abs(gs)
+
+
+def hinv_bar(n, T, kappa_gs, d_u, d_v, d_dot):
+    """|D_hat - D_ld| <= (gamma_d + 2 eps_rho) T + (the same for the long-double reference), d = max(d_u, d_v) + d_dot + 8.
+    Derivation (first order in u): the computed v_j is off by gamma_{d_v} (|D|^T|g|)_j, u_i by gamma_{d_u} (|D||g|)_i, g.u by
+    (gamma_{d_u} + gamma_{d_dot}) |g|^T|D||g|; rho = RN(1 / g.s_hat) by eps_rho = (u + eta) / (1 - eta), eta = gamma_{d_dot} kappa_gs
+    relative. rho s_i v_j then carries eps_rho + 2 u + gamma_{d_v}, rho u_i s_j eps_rho + 2 u + gamma_{d_u}, cc s_i s_j (cc = rho^2 g.u
+    + rho: one product rounding, rho^2 doubles eps_rho, one add, two products with s) 2 eps_rho + 5 u + gamma_{d_u} + gamma_{d_dot},
+    and the sum D + (three terms) adds at most three roundings to each term. gamma_a + gamma_b <= gamma_{a+b} gathers all of it
+    under one gamma_d."""
+    def part(d_u, d_v, d_dot, u):
+        eta = gamma(d_dot, u) * kappa_gs
+        eps_rho = (u + eta) / (1 - eta)
+        return (gamma(max(d_u, d_v) + d_dot + 8, u) + 2 * eps_rho) * T
+    return part(d_u, d_v, d_dot, U) + part(n + 1, n + 1, n + 1, UL)
+
+
+def matvec_bar(D, g, d):
+    """(p in long double, bar): |p_hat - p| <= gamma_d (|D||g|)_i for the kernel's depth d, plus gamma_{n+1} in long double for
+    the reference's own error"""
+    n = g.size
+    return -(ld(D) @ ld(g)), (gamma(d) + gamma(n + 1, UL)) * (np.abs(ld(D)) @ np.abs(ld(g)))
+
+
+def gemm_bar(A, B, d):
+    """(C in long double, bar): gamma_d (|A||B|)_ij plus the long-double reference's gamma_{K+1}"""
+    K = A.shape[1]
+    return ld(A) @ ld(B), (gamma(d) + gamma(K + 1, UL)) * (np.abs(ld(A)) @ np.abs(ld(B)))
+
+
+def within(got, ref, bar):
+    """componentwise |got - ref| <= bar (in long double); NaN fails"""
+    return bool(np.all(np.abs(ld(got) - ref) <= bar))
+
+
+def graded_scaling(n):
+    """10^linspace(-6, 6): the spread of an LM-like inverse Hessian's diagonal"""
+    return 10.0 ** np.linspace(-6, 6, n)
