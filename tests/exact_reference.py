@@ -9,6 +9,9 @@
 * GradedMatvec / GradedGemm / IntegerHinv: exact inputs and results of p = -D g, C = A B and updateHessianInv; the launchers'
   path predicates restated (matvec_path, hinv_rank2_path, gemm_path, syrk_path); componentwise gamma_d bars against long-double
   references (matvec_bar, gemm_bar, hinv_bar) with each kernel's summation depth.
+* eval_batch_path / jacobian_tile_rows / max_n / recip_usable / dividend_in_range: the choices of the generic functor launchers
+  (include/pnol/device/functor_kernels.cuh) and of the FD quotient restated; order_witnesses: rows whose sequential sum no other
+  summation order reproduces.
 """
 import numpy as np
 import scipy.linalg
@@ -348,6 +351,89 @@ def syrk_path(n, with_f, off_J=0, off_F=0):
     if tma:
         return "pair" if (n + 127) // 128 == 2 and not with_f else "tma"
     return "ldgsts16" if vec16 else "ldgsts8"
+
+
+# ---- which kernel the functor launchers pick (restated from include/pnol/device/functor_kernels.cuh) ----------------------------
+# smem_optin is the device's opt-in shared memory per block (pnol_launch_env::smem_optin; 232 448 bytes on a B200).
+
+SMEM_OPTIN_B200 = 232_448
+EVAL_BATCH_PATHS = ("rowwise16", "rowwise", "warp32_full", "warp32_ragged", "warp_general", "tile16", "tile_scalar", "direct")
+
+
+def eval_batch_path(n, ld, off, B, smem_optin, separable=True):
+    """eval_batch (:302-325) and SeparableLaunch<F, true>::run (:269-298) for B >= 1: the set of branches the launch runs when
+    every row is evaluated. The warp-tile kernel (:136-184) runs "warp32_full" for whole 32-row batches at n == 32 (:152),
+    "warp32_ragged" for a last partial batch at n == 32 (:168), "warp_general" otherwise (:170); the tile kernel (:84-121) stages with
+    16-byte loads when ld == n, n is even and the rows are 16-byte aligned (:96), else element by element"""
+    if separable:
+        pitch = n | 1
+        smem = 4 * 32 * pitch * 8
+        rowwise_ok = n % 4 == 0 and ld % 4 == 0 and _al(off, 32)
+        if rowwise_ok:
+            return {"rowwise16" if n % 16 == 0 else "rowwise"}
+        if not (smem > smem_optin // 2 or B < 64 or n < 24):
+            if n != 32:
+                return {"warp_general"}
+            return ({"warp32_full"} if B >= 32 else set()) | ({"warp32_ragged"} if B % 32 else set())
+    if 128 * (n | 1) * 8 <= smem_optin:
+        return {"tile16" if ld == n and n % 2 == 0 and _al(off, 16) else "tile_scalar"}
+    return {"direct"}
+
+
+def jacobian_tile_rows(n, smem_optin):
+    """jacobian (:818-841): rows per tile, 128, 64 or 32, or None when the kernel runs untiled"""
+    xbytes, row_bytes = 8 * n, 8 * (n | 1)
+    threads = 128
+    while threads > 32 and xbytes + threads * row_bytes > smem_optin:
+        threads //= 2
+    return threads if xbytes + threads * row_bytes <= smem_optin else None
+
+
+def max_n(launcher, smem_optin):
+    """the largest n each launcher accepts (its PNOL_DEV_REQUIRE on the dynamic shared memory); n + 1 is refused"""
+    w = smem_optin // 8
+    return {
+        "fd_points": w,                                  # :363  8 n
+        "gradient": w,                                   # :407  8 n
+        "residual": w,                                   # :698  8 n
+        "fd_hessian": w,                                 # :467  8 n
+        "hessian": w - 32 * 33,                          # :539  8 (32 * 33 + n)
+        "alpha_pool": (smem_optin - 16) // 17,           # :601  17 n + 16
+        "alpha_slope": w // 2,                           # :668  8 (nfull + n), n = nfull
+        "fd_jacobian": (w - 128 * 33) // 3,              # :766  8 (3 n + 128 * 33)
+    }[launcher]
+
+
+def recip_usable(d):
+    """make_recip (include/pnol/device/exact_div.cuh:20-30) gives r = RN(1/d) != 0: |d| within 2^+-200, significand not all ones"""
+    b = int(np.array([d], dtype=np.float64).view(np.uint64)[0])
+    e = (b >> 52) & 0x7FF
+    return 1023 - 200 < e < 1023 + 200 and (b & (2 ** 52 - 1)) != 2 ** 52 - 1
+
+
+def dividend_in_range(x):
+    """div_exact (exact_div.cuh:52-65) takes its FMA sequence for a dividend within 2^+-700, or zero; `/` otherwise"""
+    b = int(np.array([x], dtype=np.float64).view(np.uint64)[0])
+    e = (b >> 52) & 0x7FF
+    return 1023 - 700 < e < 1023 + 700 or x == 0.0
+
+
+def order_witnesses(n):
+    """three rows whose sequential sum from 0 (Power with power 1: the terms are the entries) no other order reproduces, n >= 3:
+    [1, e, e, ...] sums to 1, [e, ..., e, 1] to 1 + (n - 1) e rounded once, [1, e, -1, e, ...] to (n - 3) e (e = 2^-53). An order
+    that adds two small entries before it meets the 1, or lets the 1 absorb a different set of them (pairwise, reversed, strided,
+    four at a time), changes at least one of the three sums (test_functor_kernels_cpu.py)"""
+    w = np.full((3, n), U)
+    w[0, 0] = w[1, n - 1] = w[2, 0] = 1.0
+    w[2, 2] = -1.0
+    return w
+
+
+def seq_sum(v):
+    s = 0.0
+    for t in v:
+        s = s + float(t)
+    return s
 
 
 # ---- componentwise bars on real-valued data ------------------------------------------------------------------------------------
